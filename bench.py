@@ -2,7 +2,7 @@
 """bench.py - EM link-updates/s of the MMSBM hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--shape kuzmin|uniform]
-                    [--skip cfg4,cfg3,fp32,k3,e2e,cpu,dist_check]
+                    [--skip cfg4,cfg3,fp32,k3,e2e,cpu,dist_check] [--dump-outputs DIR]
 
 A "step" is one EM iteration (Model.make_iteration, TIP.py:984-1043) over one rank's link shard.
 Headline workload at every N (weak scaling): BASELINE config 2 per GPU - Kuzmin-2018 trigenic shape, 6,000 genes,
@@ -17,6 +17,12 @@ host-buffer C-ABI call (H2D of rows/theta/p and D2H of theta/p inside the timed 
 dominant kernel (the slot-segmented pass kernel) by SURVEY section 8d's accounting and names what binds it;
 `cpu_baseline` is the reference's own Model.make_iteration (oracle/_ref, kind "reference") - or the oracle's
 literal-loop port when the reference script did not travel (kind "port") - on this box's host cores.
+
+`--dump-outputs DIR` writes what the last timed step of the headline computed - theta [P,K] and pr [K,K,K,2], the
+parameters Model.make_iteration leaves its caller - as DIR/theta.npy and DIR/pr.npy (float64).  The inputs are
+seeded, so two builds run with the same arguments can be compared output for output - to rounding, not bit for bit:
+the E-step flushes its statistics with fp64 atomic adds, whose order varies from run to run.  Apart from DIR,
+bench.py writes nothing into the source tree.
 """
 from __future__ import annotations
 
@@ -34,6 +40,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the tree may be read-only; leave no __pycache__ behind in it
 
 P_GENES, K_GROUPS = 6000, 10
 L_PER_GPU = 800_000
@@ -332,6 +339,11 @@ def run_ours(args):
     total_ms = tdist.max_over_ranks(sum(ms), device=dev, group=group)
     ms_per_step = total_ms / steps
     value = L_total / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # taken here, before the informational replays below move the parameters on
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "theta.npy"), eng.theta.reshape(P, K).cpu().numpy())
+        np.save(os.path.join(args.dump_outputs, "pr.npy"), eng.p.reshape(K, K, K, 2).cpu().numpy())
 
     # back-to-back replays, rows resident in L2 (how a real training run behaves) - informational
     torch.cuda.synchronize(dev)
@@ -813,8 +825,12 @@ def main():
                     help="N>1: how link-shard statistics are summed over NVLink peer memory: peer = statistics pushed into the "
                          "peers' inboxes, one handshake, local sum + M-step in one kernel; peer_rs = reduce-scatter + M-step + "
                          "all-gather in one kernel; peer_gather = every rank reads every buffer (round 1); nccl = NCCL allreduce")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write theta and pr after the last timed step of the headline as DIR/theta.npy, DIR/pr.npy (float64)")
     args = ap.parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes what the GPU path computed; it does not apply to --impl reference")
         return run_reference(args)
     return run_ours(args)
 

@@ -1,5 +1,5 @@
-"""bench.py contract checks that need no GPU: the reference arm runs on host cores only, and the committed round-1
-line carries every key the driver reads."""
+"""bench.py contract checks: the reference arm runs on host cores only, the committed bench lines carry every key of
+the result line, and (on a GPU) --dump-outputs writes what the last timed step computed."""
 import json
 import os
 import subprocess
@@ -49,3 +49,41 @@ def test_committed_bench_line_has_the_contract_keys(name):
         assert key in rec["e2e"], key
     assert rec["e2e"]["h2d_bytes_per_step"] > 0 and rec["e2e"]["value"] < rec["value"]
     assert rec["gpu_launches"] >= rec["steps"]
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_parameters_after_the_last_timed_step(tmp_path):
+    """--dump-outputs writes theta and pr as the headline leaves them after its warm-up and exactly --steps timed
+    iterations: the same as that many eager iterations of the engine on bench.py's seeded inputs."""
+    import numpy as np
+    import torch
+    from trigenicinteractionpredictor_b200 import synth
+    from trigenicinteractionpredictor_b200.engine import EMEngine
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", "3",
+                          "--skip", "cfg4,cfg3,fp32,k3,e2e,cpu", "--dump-outputs", str(tmp_path / "dump")],
+                         capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    lines = [l for l in out.stdout.splitlines() if l.startswith("{")]
+    assert len(lines) == 1
+    rec = json.loads(lines[0])
+    assert rec["steps"] == 2 and rec["warmup"] == 3
+    assert sorted(os.listdir(tmp_path / "dump")) == ["pr.npy", "theta.npy"]
+    theta, pr = np.load(tmp_path / "dump" / "theta.npy"), np.load(tmp_path / "dump" / "pr.npy")
+    assert theta.dtype == np.float64 and pr.dtype == np.float64
+    # bench.py's headline inputs: P=6000, K=10, 800,000 Kuzmin-shaped links of seed 100, parameters of default_rng(0)
+    P, K, dev = 6000, 10, torch.device("cuda", 0)
+    g1, g2, g3, lab = synth.kuzmin_links_soa(P, 800_000, seed=100, device=dev)
+    g1[:P] = torch.arange(P, dtype=torch.int32, device=dev)
+    rng = np.random.default_rng(0)
+    theta0 = rng.dirichlet(np.ones(K), size=P)
+    pr0 = rng.random((K, K, K, 2))
+    pr0 /= pr0.sum(axis=3, keepdims=True)
+    eng = EMEngine(P, K, device=dev)
+    eng.set_train_links(g1, g2, g3, 1 - lab, lab)
+    eng.set_params(theta0, pr0)
+    for _ in range(3 + 2):
+        eng.em_iteration()
+    th, p = eng.get_params()
+    assert theta.shape == th.shape and pr.shape == p.shape
+    np.testing.assert_allclose(theta, th, rtol=1e-11, atol=0)
+    np.testing.assert_allclose(pr, p, rtol=1e-11, atol=0)

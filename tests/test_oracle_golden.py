@@ -6,6 +6,7 @@ import random
 import numpy as np
 import pytest
 
+from oracle import fetch_ref
 from oracle import mmsbm_oracle as orc
 from tests.conftest import GOLDEN, read_lines
 
@@ -206,25 +207,18 @@ def test_training_loop_semantics():
     np.testing.assert_allclose(trace, man["checks"], rtol=1e-11)
 
 
-REF_SRC = "/root/reference/src"
-
-
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF_SRC, "TrigenicInteractionPredictor.py")),
-                    reason="the reference only exists in the build container")
+@pytest.mark.skipif(not os.path.exists(fetch_ref.DST),
+                    reason="needs the original TrigenicInteractionPredictor.py in oracle/_ref/ (python oracle/fetch_ref.py)")
 @pytest.mark.parametrize("seed", range(4))
 def test_oracle_against_the_live_reference_on_random_files(tmp_path, monkeypatch, seed):
-    """Build container only: the unmodified reference, imported from /root/reference, digests random files (unsorted
+    """The unmodified reference, loaded from its sha256-checked copy in oracle/_ref/, digests random files (unsorted
     names, duplicates, conflicts, test-only genes, ids of different digit counts), folds them and runs two EM
     iterations; the oracle must agree - dictionaries and fold files exactly, theta / p / log-likelihood to 1e-12."""
     import contextlib
     import io
     import random
-    import sys
-    sys.path.insert(0, REF_SRC)
-    try:
-        import TrigenicInteractionPredictor as ref
-    finally:
-        sys.path.remove(REF_SRC)
+    ref = fetch_ref.load_reference_module()
+    assert ref is not None, "oracle/_ref/ holds a file whose sha256 is not the pinned reference's"
     rng = np.random.default_rng(500 + seed)
     P = int(rng.integers(10, 60))
     names = ["G%d" % v for v in rng.permutation(3000)[:P]]
