@@ -178,6 +178,25 @@ int tip_sort_scores_workspace_bytes(int64_t T, size_t *bytes);
 int tip_sort_scores(const double *d_scores, int64_t T, void *d_ws, size_t ws_bytes, int32_t *d_order, double *d_sorted,
                     void *stream);
 
+/* ---- prediction: the N highest-scoring unseen triplets of a candidate gene list, exhaustively ----
+ * Candidates are all triplets of distinct genes of d_cand[n_cand] (gene ids, distinct, in decimal-string order: position =
+ * rank).  A triplet's slots are its ranks in ascending order, which is the reference's key slot order (TIP.py:353); its
+ * score is do_prediction (TIP.py:530-547, rating 1, no eps) averaged over the S parameter sets
+ * d_theta[S][P][K], d_p[S][K][K][K][2].  d_known[n_known]: sorted, distinct packed rank triples
+ * (ra << 42) | (rb << 21) | rc, ra < rb < rc, of triplets never to return (the known links among the candidates).
+ * Out: the first min(N, C(n_cand, 3) - n_known) triplets in the order (score descending, (ra, rb, rc) ascending), exact
+ * under any ties: d_out_ids[N][3] gene ids in slot order, d_out_scores[N], *h_n_out rows.
+ * Every score is recomputed in each pass on the fp64 tensor path (C(n, 3) * 2 S K flop per pass, no per-triplet storage);
+ * only scores above a threshold leave registers, and the host narrows the threshold between passes.  Synchronises the
+ * stream (the host decides how many passes to run); not capturable in a CUDA graph.  Limits: n_cand <= 2^21, S * K <= 384,
+ * N < 2^28.  Precondition: finite, non-negative parameters.  d_ws: tip_top_triplets_workspace_bytes() bytes. */
+int tip_top_triplets_workspace_bytes(int n_cand, int K, int S, int64_t n_known, int64_t N, size_t *bytes);
+int tip_top_triplets(int P, int K, int S, const double *d_theta, const double *d_p, const int32_t *d_cand, int n_cand,
+                     const uint64_t *d_known, int64_t n_known, int64_t N, void *d_ws, size_t ws_bytes, int32_t *d_out_ids,
+                     double *d_out_scores, int64_t *h_n_out, void *stream);
+/* scoring passes (full sweeps) the last tip_top_triplets of this thread ran (measurement) */
+int tip_top_triplets_last_passes(void);
+
 /* ---- testResultsReducer.py:160-184: mean / median / standard deviation of every test triplet across samples ----
  * d_scores[S][T]: score of triplet t in sample j at [j * T + t]; d_n[t] (or NULL = S) = how many leading samples of
  * triplet t are valid.  mean = sequential sum in sample order / n; median = the reference's rule (ascending sort;

@@ -556,6 +556,126 @@ class Model:
         return [precision, recall, fallout, auc]
 
     # ------------------------------------------------------------------------------------------
+    # kept parameters and prediction of unseen triplets (additions: the reference's loader, get_data, opens its file
+    # with "w+" and never reads one)
+    # ------------------------------------------------------------------------------------------
+    def _genes_in_id_order(self):
+        return [self.id_gene[i] for i in range(self.P)]
+
+    def save_parameters(self, path):
+        """Write theta, pr, K and the gene names in id order to an .npz file at exactly `path`."""
+        theta = np.asarray(self.theta, dtype=np.float64)
+        pr = np.asarray(self.pr, dtype=np.float64)
+        with open(path, "wb") as fh:
+            np.savez(fh, theta=theta, pr=pr, K=np.int64(self.K), genes=np.array(self._genes_in_id_order(), dtype=str))
+
+    def check_parameters_file(self, path):
+        """(theta [P][K], pr [K][K][K][2]) of an .npz written by save_parameters, checked against this model's digestion:
+        the same genes in the same id order, the model's K (when it has one), finite non-negative values.  Raises
+        ValueError with the reason otherwise.  Host only."""
+        try:
+            with np.load(path, allow_pickle=False) as z:
+                theta, pr, K, genes = z["theta"], z["pr"], int(z["K"]), [str(g) for g in z["genes"]]
+        except (OSError, KeyError, ValueError) as exc:
+            raise ValueError("%s is not a parameter file of save_parameters (%s)" % (path, exc)) from exc
+        return self._check_parameters(theta, pr, K, genes, str(path))
+
+    def _check_parameters(self, theta, pr, K, genes, what):
+        theta = np.asarray(theta, dtype=np.float64)
+        pr = np.asarray(pr, dtype=np.float64)
+        if genes is not None and genes != self._genes_in_id_order():
+            raise ValueError("%s: its gene list (%d genes) differs from the model's digestion (%d genes)"
+                             % (what, len(genes), self.P))
+        if self.K and K != self.K:
+            raise ValueError("%s: K = %d, the model has K = %d" % (what, K, self.K))
+        if theta.shape != (self.P, K) or pr.shape != (K, K, K, self.R):
+            raise ValueError("%s: theta %s / pr %s do not have the shapes (%d, %d) / (%d, %d, %d, %d)"
+                             % (what, theta.shape, pr.shape, self.P, K, K, K, K, self.R))
+        if not (np.isfinite(theta).all() and np.isfinite(pr).all()):
+            raise ValueError("%s: theta or pr holds a non-finite value" % what)
+        if (theta < 0).any() or (pr < 0).any():
+            raise ValueError("%s: theta or pr holds a negative value" % what)
+        return theta, pr
+
+    def load_parameters(self, path):
+        """Make the parameters of an .npz written by save_parameters the model's current theta / pr (see
+        check_parameters_file for what is refused)."""
+        with np.load(path, allow_pickle=False) as z:
+            K = int(z["K"]) if "K" in z.files else 0
+        theta, pr = self.check_parameters_file(path)
+        self.K = K
+        self._theta_host, self._pr_host = theta, pr
+        self._params_on, self._host_valid, self._exposed = "host", True, False
+
+    def predict_top_triplets(self, n, genes=None, exclude_known=True, params=None):
+        """The `n` most likely interacting triplets of distinct genes among `genes` (names; default all P genes), by
+        do_prediction (TIP.py:530-547) of the current theta / pr, or by the mean over the parameter sets in `params`
+        (.npz paths of save_parameters or (theta, pr) pairs).  With exclude_known the keys of links and test_links are
+        left out.  Exhaustive over C(n_genes, 3) triplets on the device.  Returns [[score, "a_b_c", "nameA_nameB_nameC"],
+        ...], best first; equal scores in ascending order of the triplets' positions in the decimal-string order of the
+        candidate ids.  The id key is the report's "ID of genes" column; names are sorted as in the fold files (TIP.py:486)."""
+        if self.P < 1 or len(self.id_gene) != self.P:
+            raise ValueError("predict_top_triplets needs a model digested from train / test files")
+        if params is None:
+            if self.K < 1:
+                raise ValueError("predict_top_triplets: initialize_parameters() or load_parameters() must run first")
+            sets = [self._check_parameters(self.theta, self.pr, self.K, None, "the model's parameters")]
+        else:
+            sets = []
+            for item in params:
+                if isinstance(item, (str, bytes, os.PathLike)):
+                    sets.append(self.check_parameters_file(item))
+                else:
+                    th, pr = item
+                    sets.append(self._check_parameters(th, pr, np.asarray(th).shape[-1], None, "a (theta, pr) pair"))
+            if not sets:
+                raise ValueError("predict_top_triplets: params is empty")
+            Ks = {th.shape[1] for th, _ in sets}
+            if len(Ks) != 1:
+                raise ValueError("predict_top_triplets: the parameter sets have different K (%s)" % sorted(Ks))
+        K = sets[0][0].shape[1]
+        if genes is None:
+            ids = list(range(self.P))
+        else:
+            missing = [g for g in genes if g not in self.gene_id]
+            if missing:
+                raise ValueError("unknown gene names: %s" % ", ".join(missing))
+            ids = sorted({self.gene_id[g] for g in genes})
+        cand = np.array(sorted(ids, key=str), dtype=np.int32)
+        known = np.empty(0, dtype=np.uint64)
+        if exclude_known:
+            known = self._known_packed(cand)
+        from .engine import EMEngine
+        eng = self._engine if (self._engine is not None and self._engine_key == (self.P, K)) else None
+        if eng is None:
+            eng = EMEngine(self.P, K, device=self._device, flags=self._flags)
+        out_ids, scores = eng.top_triplets(np.stack([th for th, _ in sets]), np.stack([pr for _, pr in sets]), cand, known, int(n))
+        rows = []
+        for (a, b, c), s in zip(out_ids.tolist(), scores.tolist()):
+            names = sorted((self.id_gene[a], self.id_gene[b], self.id_gene[c]))
+            rows.append([s, "%d_%d_%d" % (a, b, c), "_".join(names)])
+        return rows
+
+    def _known_packed(self, cand):
+        """Sorted packed rank triples (ra << 42 | rb << 21 | rc) of the keys of links and test_links whose three genes
+        are all candidates."""
+        rank = np.full(self.P, -1, dtype=np.int64)
+        rank[cand] = np.arange(cand.shape[0], dtype=np.int64)
+        parts = []
+        for table in (self.links, self.test_links):
+            if len(table) == 0:
+                continue
+            g = [np.asarray(x.cpu().numpy() if _is_torch(x) else x, dtype=np.int64) for x in self._soa(table)[:3]]
+            r = np.stack([rank[g[0]], rank[g[1]], rank[g[2]]], axis=1)
+            r = r[(r >= 0).all(axis=1)]
+            r.sort(axis=1)
+            r = r[(r[:, 0] < r[:, 1]) & (r[:, 1] < r[:, 2])]
+            parts.append((r[:, 0] << 42) | (r[:, 1] << 21) | r[:, 2])
+        if not parts:
+            return np.empty(0, dtype=np.uint64)
+        return np.unique(np.concatenate(parts)).astype(np.uint64)
+
+    # ------------------------------------------------------------------------------------------
     # report (TIP.py:793-904)
     # ------------------------------------------------------------------------------------------
     def to_string(self):
@@ -609,11 +729,14 @@ class Model:
 # gene list block so that the sample files feed testResultsReducer directly),
 # --mode auto|slots|fp64|segmented|fp32 (E-step formulation: slot-segmented 4K^2 per link without per-link atomics - the
 # default for K >= 4 -, K^3 per link, gene-segmented 2K^2 per link - all the same results to rounding -, or
-# fp32-compute / fp64-accumulate within 1e-5).
+# fp32-compute / fp64-accumulate within 1e-5), --save-params (write Sample_{s}_K{k}.npz, the trained theta / pr, next to each
+# report written; `python -m trigenicinteractionpredictor_b200.predict` ranks unseen triplets with them).
 # ----------------------------------------------------------------------------------------------
-def train_sample(model, k, iterations, fcheck, bcheck, outfile=None, verbose=True, log=print, reducible=False):
+def train_sample(model, k, iterations, fcheck, bcheck, outfile=None, verbose=True, log=print, reducible=False,
+                 params_file=None):
     """One random restart (TIP.py:1260-1279).  Returns (converged, iterations_done, checks).  reducible: append the
-    LIST OF REGISTERED GENES block (TIP.py:863-867, commented out in the reference) that testResultsReducer parses."""
+    LIST OF REGISTERED GENES block (TIP.py:863-867, commented out in the reference) that testResultsReducer parses.
+    params_file: where the report is written, also write the trained parameters there (Model.save_parameters)."""
     model.initialize_parameters(k)
     if verbose:
         log("Parameters have been initialized")
@@ -645,6 +768,8 @@ def train_sample(model, k, iterations, fcheck, bcheck, outfile=None, verbose=Tru
                         from .testResultsReducer import gene_list_block
                         with codecs.open(outfile, encoding='utf-8', mode="a") as fh:
                             fh.write(gene_list_block(model))
+                    if params_file is not None:
+                        model.save_parameters(params_file)
                 return True, it, checks
             like0 = like
     return False, it, checks
@@ -655,11 +780,12 @@ def main(argv=None):
     iterations, num_samples, sample_ini, fcheck, bcheck = 10000, 100, 0, 25, 100
     train = test = None
     outpath, argk = "", 1
-    seed, device, dist_mode, mode_flags, reducible = None, None, "none", None, False
+    seed, device, dist_mode, mode_flags, reducible, save_params = None, None, "none", None, False, False
     try:
         opts, _ = getopt.getopt(argv, "hi:n:s:f:b:o:t:e:k:",
                                 ["help", "num_iterations=", "num_samples=", "sample_ini=", "fcheck=", "bcheck=",
-                                 "out=", "train=", "test=", "k=", "seed=", "device=", "dist=", "mode=", "reducible"])
+                                 "out=", "train=", "test=", "k=", "seed=", "device=", "dist=", "mode=", "reducible",
+                                 "save-params"])
         for opt, arg in opts:
             if opt in ("-h", "--help"):
                 print(__doc__)
@@ -719,6 +845,8 @@ def main(argv=None):
                 dist_mode = arg
             elif opt == "--reducible":
                 reducible = True
+            elif opt == "--save-params":
+                save_params = True
             elif opt == "--mode":
                 if arg not in ("auto", "slots", "fp64", "segmented", "fp32"):
                     raise ValueError
@@ -766,7 +894,8 @@ def main(argv=None):
         if seed is not None:
             random.seed(seed + sample)
         write = outfile if (dist_mode != "links" or rk == 0) else None
-        train_sample(model, argk, iterations, fcheck, bcheck, outfile=write, reducible=reducible)
+        params = outpath + 'Sample_' + str(sample) + '_K' + str(argk) + '.npz' if (save_params and write) else None
+        train_sample(model, argk, iterations, fcheck, bcheck, outfile=write, reducible=reducible, params_file=params)
     return 0
 
 

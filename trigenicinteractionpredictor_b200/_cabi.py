@@ -52,6 +52,10 @@ SIGNATURES = {
     "tip_metrics": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_size_t, c_void_p, c_void_p]),
     "tip_sort_scores_workspace_bytes": (c_int, [c_int64, _psz]),
     "tip_sort_scores": (c_int, [c_void_p, c_int64, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p]),
+    "tip_top_triplets_workspace_bytes": (c_int, [c_int, c_int, c_int, c_int64, c_int64, _psz]),
+    "tip_top_triplets": (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int64, c_int64, c_void_p,
+                                 c_size_t, c_void_p, c_void_p, _pi64, c_void_p]),
+    "tip_top_triplets_last_passes": (c_int, []),
     "tip_reduce_samples": (c_int, [c_int, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "tip_em_iterations_host": (c_int, [c_int, c_int, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_int,
                                        c_uint]),

@@ -22,7 +22,7 @@ OBJ_DIR = os.path.join(HERE, "csrc", "_obj")
 LIB_PATH = os.path.join(HERE, "libtip.so")
 
 SOURCES = ["tip_api.cu", "tip_em.cu", "tip_generic.cu", "tip_mstep.cu", "tip_rows.cu", "tip_metrics.cu", "tip_peer.cu",
-           "tip_reduce.cu", "tip_seg3.cu", "tip_pairs.cu"]
+           "tip_reduce.cu", "tip_seg3.cu", "tip_pairs.cu", "tip_predict.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xptxas", "-v",

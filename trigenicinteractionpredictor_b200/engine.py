@@ -7,6 +7,7 @@ CUDA kernels behind the C ABI (include/tip.h).  There is no CPU path.
     eng.set_params(theta, p)                           # numpy fp64, reference layouts
     eng.em_iterations(n)                               # n x make_iteration (TIP.py:984-1043)
     eng.loglik("train")                                # compute_likelihood (TIP.py:952-974)
+    eng.top_triplets(thetas, ps, cand, known, n)       # exhaustive top-n of unseen triplets (tip_top_triplets)
 """
 from __future__ import annotations
 
@@ -473,6 +474,35 @@ class EMEngine:
                     "tip_sort_scores")
         self.launches += 2
         return order.cpu().numpy(), out.cpu().numpy()
+
+    @_on_device
+    def top_triplets(self, theta_stack, p_stack, cand, known, n: int):
+        """tip_top_triplets: the `n` best triplets of the candidate genes under the mean of S models.
+        theta_stack [S][P][K], p_stack [S][K][K][K][2] (numpy fp64); cand: gene ids in decimal-string order; known: sorted
+        packed rank triples to leave out.  Returns (ids [m][3] int32 in slot order, scores [m] float64), best first."""
+        th = np.ascontiguousarray(theta_stack, dtype=np.float64)
+        pp = np.ascontiguousarray(p_stack, dtype=np.float64)
+        S = int(th.shape[0])
+        assert th.shape == (S, self.P, self.K) and pp.shape == (S, self.K, self.K, self.K, 2)
+        cand = np.ascontiguousarray(cand, dtype=np.int32)
+        known = np.ascontiguousarray(known, dtype=np.uint64)
+        n_cand, n_known, n = int(cand.shape[0]), int(known.shape[0]), int(n)
+        nb = ctypes.c_size_t(0)
+        _cabi.check(self.lib.tip_top_triplets_workspace_bytes(n_cand, self.K, S, n_known, n, ctypes.byref(nb)),
+                    "tip_top_triplets_workspace_bytes")
+        d_th = torch.from_numpy(th.reshape(-1)).to(self.device)
+        d_p = torch.from_numpy(pp.reshape(-1)).to(self.device)
+        d_cand = torch.from_numpy(cand).to(self.device)
+        d_known = torch.from_numpy(known.view(np.int64)).to(self.device) if n_known else None
+        ws = torch.empty(max(nb.value, 1), dtype=torch.uint8, device=self.device)
+        out_ids = torch.empty((max(n, 1), 3), dtype=torch.int32, device=self.device)
+        out_sc = torch.empty(max(n, 1), dtype=torch.float64, device=self.device)
+        m = ctypes.c_int64(0)
+        _cabi.check(self.lib.tip_top_triplets(self.P, self.K, S, _ptr(d_th), _ptr(d_p), _ptr(d_cand), n_cand, _ptr(d_known),
+                                              n_known, n, _ptr(ws), nb.value, _ptr(out_ids), _ptr(out_sc), ctypes.byref(m),
+                                              self._stream()), "tip_top_triplets")
+        m = int(m.value)
+        return out_ids[:m].cpu().numpy(), out_sc[:m].cpu().numpy()
 
     @_on_device
     def metric_counts(self, scores: torch.Tensor, positives_number: int) -> dict:
