@@ -1,6 +1,8 @@
 """The C-ABI library builds, loads and exports every symbol include/tip.h declares (no compute calls)."""
 import ctypes
+import glob
 import os
+import re
 
 import pytest
 
@@ -75,3 +77,23 @@ def test_sass_is_sm100a_with_fp64_fma_and_cp_async():
     # round 2: the slot-segmented passes run their K^2 work on the fp64 tensor path and are chained by programmatic
     # dependent launches (griddepcontrol.wait = ACQBULK, launch_dependents = PREEXIT); the counting sort ranks with MATCH
     assert "DMMA.8x8x4" in out and "ACQBULK" in out and "PREEXIT" in out and "MATCH.ANY" in out
+    # the hot E-step templates are instantiated only for the configurations their launchers select
+    assert len(re.findall(r"Function : \S*em_fused_kernel", out)) == 74
+    assert len(re.findall(r"Function : \S*seg3_pass_kernel", out)) == 128
+
+
+def test_environment_reads_are_only_the_kept_hooks():
+    """The library and the package read no environment switch beyond the stream-entry hooks: TIP_HOST_NO_STREAM and
+    TIP_HOST_SEG3_AFTER_STREAM pick a variant of tip_em_iterations_host, TIP_STREAM_TIMEOUT_US and
+    TIP_STREAM_INJECT_FAULT exercise its give-up and checksum-repair paths."""
+    pkg = os.path.dirname(os.path.abspath(build.__file__))
+    names = set()
+    for path in glob.glob(os.path.join(pkg, "csrc", "*.cu")) + glob.glob(os.path.join(pkg, "csrc", "*.cuh")):
+        for args in re.findall(r"getenv\(([^)]*)\)", open(path).read()):
+            names.update(re.findall(r'"([^"]*)"', args))
+    py_read = re.compile(r"""os\.(?:environ\.get|getenv)\(\s*["'](TIP_\w+)["']|os\.environ\[\s*["'](TIP_\w+)["']\s*\](?!\s*=[^=])"""
+                         r"""|["'](TIP_\w+)["']\s+(?:not\s+)?in\s+os\.environ""")
+    for path in glob.glob(os.path.join(pkg, "**", "*.py"), recursive=True):
+        for groups in py_read.findall(open(path).read()):
+            names.update(g for g in groups if g)
+    assert names == {"TIP_HOST_NO_STREAM", "TIP_HOST_SEG3_AFTER_STREAM", "TIP_STREAM_TIMEOUT_US", "TIP_STREAM_INJECT_FAULT"}

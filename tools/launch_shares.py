@@ -17,14 +17,14 @@ for r in rows:
     tot[name] += ns
     cnt[name] += 1
 print("per-launch times under ncu are cold-cache and serialised: compare shares, not absolutes\n")
-# the headline iteration (round 2): prep, pass A, pass B + C (Kuzmin: the gather-through-L1 instances "..., 2, 1>"), finish, M-step;
+# the headline iteration (round 2): prep, pass A, pass B + C (Kuzmin: the gather-through-L1 instances "..., 1>"), finish, M-step;
 # round-1 lists (em_fused / em_finalize / stage_p) still match their own names
 seg3 = any("seg3_pass_kernel" in k for k in tot)
 if seg3:
-    l1 = any("seg3_pass_kernel" in k and k.rstrip().endswith("2, 1>") for k in tot)
+    l1 = any("seg3_pass_kernel" in k and k.rstrip().endswith(", 1>") for k in tot)
     step = {k: tot[k] / cnt[k] for k in tot
             if "seg3_prep" in k or "seg3_finish" in k or "normalise" in k
-            or ("seg3_pass_kernel" in k and k.rstrip().endswith("2, 1>" if l1 else "2, 0>"))}
+            or ("seg3_pass_kernel" in k and k.rstrip().endswith(", 1>" if l1 else ", 0>"))}
 else:
     step = {k: tot[k] / cnt[k] for k in tot
             if "tip::" in k and (("em_fused" in k and "double, 0, 0>" in k) or "em_finalize" in k or "stage_p_kernel<double>" in k

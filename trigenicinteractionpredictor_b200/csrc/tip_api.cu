@@ -426,14 +426,7 @@ extern "C" int tip_em_iterations_host(int P, int K, const void *h_rows, int64_t 
         g.h_err[0] = 0;
         TIP_CHECK_CUDA(cudaMemsetAsync(g.chk, 0, 32, g.st));
         if (compact && n_iter <= 1 && (rc = launch_rows_expand(g.rows8, g.rows, n_rows, g.st))) return rc;
-        if (getenv("TIP_HOST_STREAM_DEBUG")) fprintf(stderr, "stream dbg: checksum mismatch, iterations repeated from resident rows\n");
         if ((rc = run_resident(0))) return rc;
-    }
-    if (streamed && getenv("TIP_HOST_STREAM_DEBUG")) {
-        unsigned long long d[5];
-        memcpy(d, reinterpret_cast<unsigned long long *>(g.h_err) + 8, sizeof(d));
-        fprintf(stderr, "stream dbg: first rows +%.1f us, last rows +%.1f us, end +%.1f us, spins %llu\n", (d[1] - d[0]) * 1e-3,
-                (d[2] - d[0]) * 1e-3, (d[3] - d[0]) * 1e-3, d[4]);
     }
     if (streamed && g.h_err[0] != 0) {
         TIP_CHECK_CUDA(cudaStreamSynchronize(g.copy));

@@ -47,7 +47,7 @@ constexpr int kMaxTunedK = 32;      // K = 17..32: gene-segmented formulation on
 __constant__ double c_pem[kPBankDoubles];
 __device__ double g_pstage[kPBankDoubles];
 
-template <int K, int NBUF>
+template <int K>
 struct EmCfg {
     static constexpr int KP = K + (K & 1);                   // sub-row length (even)
     static constexpr int S3 = 3 * KP;
@@ -62,9 +62,9 @@ struct EmCfg {
     static constexpr int CSLOTS = kPrivateS ? 3 : 2;
     static constexpr int CA = kPrivateS ? KP : 0;            // offset of cb inside a row
     static constexpr int RC = CSLOTS * KP + (((CSLOTS * KP) % 4 == 2) ? 0 : 2);
-    // shared memory of one warp-CTA: NBUF theta stages + contribution buffer (doubles), then ids (NBUF x 32 int4)
-    static constexpr int WARP_DBL = NBUF * 32 * RS + 32 * RC;
-    static constexpr size_t SMEM = (size_t)WARP_DBL * 8 + NBUF * 32 * 16;
+    // shared memory of one warp-CTA: theta stage + contribution buffer (doubles), then ids (32 int4)
+    static constexpr int WARP_DBL = 32 * RS + 32 * RC;
+    static constexpr size_t SMEM = (size_t)WARP_DBL * 8 + 32 * 16;
 };
 
 // p[abc][r] (reference layout) -> [r][ab][c padded] staging copy (fp64, or fp32 for the fp32-compute mode),
@@ -199,7 +199,6 @@ struct StreamArrive {
     unsigned *err;
     int compact;
     unsigned long long timeout_ns;
-    unsigned long long *dbg;  // optional (TIP_HOST_STREAM_DEBUG): CTA 0 records {start, first rows, last rows, end, spins}
 };
 constexpr unsigned long long kRowSentinel = ~0ull;
 
@@ -218,21 +217,19 @@ constexpr int em_max_regs(int minb)
     return r > 255 ? 255 : r;
 }
 
-template <int K, int NBUF, int MINB, bool LL, typename T, bool SEG, bool STREAM = false>
+template <int K, int MINB, bool LL, typename T, bool SEG, bool STREAM = false>
 __global__ void __launch_bounds__(32) __maxnreg__(em_max_regs(MINB))
     em_fused_kernel(int P, const int4 *__restrict__ rows, int n_tiles, int n_tiles_r0, const double *__restrict__ theta,
                     int p_off0, int p_off1, double *__restrict__ stats, double *__restrict__ Mg,
-                    const double *__restrict__ Zg, int tune, StreamArrive sa)
+                    const double *__restrict__ Zg, StreamArrive sa)
 {
-    const int red_scatter = tune & 1;  // bit 0: per-lane REDs instead of bulk reductions (TIP_EM_SCATTER=red);
-                                       // bit 1: stage Z_g of single-gene tiles in shared memory (off: TIP_SEG_ZSMEM=0)
-    using C = EmCfg<K, NBUF>;
+    using C = EmCfg<K>;
     constexpr int KP = C::KP, RS = C::RS, K3 = C::K3, CB = C::CB, RC = C::RC, CA = C::CA;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x;
-    double *stage0 = reinterpret_cast<double *>(smem_raw);    // [NBUF][32][RS]
-    double *cbuf = stage0 + NBUF * 32 * RS;                   // [32][RC]
-    int4 *ids_sm = reinterpret_cast<int4 *>(cbuf + 32 * RC);  // [NBUF][32]
+    double *stage = reinterpret_cast<double *>(smem_raw);    // [32][RS]
+    double *cbuf = stage + 32 * RS;                          // [32][RC]
+    int4 *ids = reinterpret_cast<int4 *>(cbuf + 32 * RC);    // [32]
 
     // Tile bookkeeping (t, W, the rating of a tile, the p index) must stay on the uniform datapath.
     // ptxas gives every value ONE home: a single per-lane use of %ctaid.x / %nctaid.x (the row pointers
@@ -254,10 +251,7 @@ __global__ void __launch_bounds__(32) __maxnreg__(em_max_regs(MINB))
     // STREAM: per-lane tile index of the next fetch
     unsigned tile_v = bx_v;
     bool stream_dead = false;
-    unsigned long long dbg_spins = 0, consumed = 0;
-    if constexpr (STREAM) {
-        if (sa.dbg != nullptr && bx_v == 0 && lane == 0) sa.dbg[0] = global_timer_ns();
-    }
+    unsigned long long consumed = 0;
     auto next_rows = [&]() -> int4 {
         int4 v;
         if constexpr (STREAM) {
@@ -281,12 +275,6 @@ __global__ void __launch_bounds__(32) __maxnreg__(em_max_regs(MINB))
                 }
             }
             stream_dead = __any_sync(0xffffffffu, stream_dead);
-            if (sa.dbg != nullptr && bx_v == 0 && lane == 0) {
-                dbg_spins += spins;
-                if (tile_v == 0) sa.dbg[1] = global_timer_ns();
-                sa.dbg[2] = global_timer_ns();
-                sa.dbg[4] = dbg_spins;
-            }
             if (!stream_dead) consumed += q0 + q1;
             if (stream_dead) {
                 v = make_int4(0, 0, 0, 0);
@@ -342,42 +330,17 @@ __global__ void __launch_bounds__(32) __maxnreg__(em_max_regs(MINB))
         }
     };
 
-    // ---- software pipeline prologue (NBUF == 2: rows of the next tile are gathered one tile ahead) ----
+    // the rows of the next tile are loaded while the current tile is gathered
     int4 ids_next = make_int4(0, 0, 0, 0);
-    if (NBUF == 2 && w0 < n_tiles) {
-        ids_sm[lane] = next_rows();
-        __syncwarp();
-        gather_tile<K, RS, KP>(theta, ids_sm, stage0, lane);
-        cp_async_commit();
-        if (w0 + W < n_tiles) ids_next = next_rows();
-    } else if (NBUF == 1 && w0 < n_tiles) {
-        ids_next = next_rows();
-    }
+    if (w0 < n_tiles) ids_next = next_rows();
 
-    int buf = 0;
     for (int t = w0; t < n_tiles; t += W) {
-        double *stage = stage0 + buf * 32 * RS;
-        const int4 *ids = ids_sm + buf * 32;
-        if (NBUF == 2) {
-            const bool has_next = (t + W) < n_tiles;
-            if (has_next) {
-                ids_sm[(buf ^ 1) * 32 + lane] = ids_next;
-                __syncwarp();
-                gather_tile<K, RS, KP>(theta, ids_sm + (buf ^ 1) * 32, stage0 + (buf ^ 1) * 32 * RS, lane);
-                cp_async_commit();
-                if (t + 2 * W < n_tiles) ids_next = next_rows();
-                cp_async_wait<1>();
-            } else {
-                cp_async_wait<0>();
-            }
-        } else {
-            ids_sm[lane] = ids_next;
-            __syncwarp();
-            gather_tile<K, RS, KP>(theta, ids_sm, stage0, lane);
-            cp_async_commit();
-            if (t + W < n_tiles) ids_next = next_rows();
-            cp_async_wait<0>();
-        }
+        ids[lane] = ids_next;
+        __syncwarp();
+        gather_tile<K, RS, KP>(theta, ids, stage, lane);
+        cp_async_commit();
+        if (t + W < n_tiles) ids_next = next_rows();
+        cp_async_wait<0>();
         __syncwarp();
 
         const int4 me = ids[lane];
@@ -429,7 +392,7 @@ __global__ void __launch_bounds__(32) __maxnreg__(em_max_regs(MINB))
                 // kernel, profiles/r1_em_fused_k10_gene_segmented_before_zstage_summary.txt).  Mixed tiles read Z through L1 as before.
                 const double *Zrow = Zg + ((int64_t)r_v * P + me.x) * (K * K);
                 const int g0 = __shfl_sync(0xffffffffu, me.x, 0);
-                const bool one_gene = (tune & 2) && __all_sync(0xffffffffu, me.x == g0 && cnt != 0.0);
+                const bool one_gene = __all_sync(0xffffffffu, me.x == g0 && cnt != 0.0);
                 if (one_gene) {
 #pragma unroll
                     for (int e = lane; e < K * K; e += 32) {
@@ -595,8 +558,9 @@ __global__ void __launch_bounds__(32) __maxnreg__(em_max_regs(MINB))
             // (Tried: all 64 bulk reductions of a tile issued by lane 0 in an unrolled loop over the links, instead of
             // two per lane - ptxas wraps the uniform-datapath UBLKRED of each lane in an elect-one-lane loop, 16 % of
             // the kernel in the round-1 capture.  The single-lane loop still gets a one-trip elect loop per
-            // instruction and serialises the address set-up: 0.274 vs 0.258 ms at 800 k links - not kept.)
-            if (K % 2 == 0 && !red_scatter) {
+            // instruction and serialises the address set-up: 0.274 vs 0.258 ms at 800 k links - not kept.
+            // Per-lane REDs for even K as well measured equal to the bulk path within noise at K = 10.)
+            if constexpr (K % 2 == 0) {
                 // one bulk add-reduction per (link, slot): the 8K-byte row goes to the TMA unit
                 fence_async_smem();
                 if (cnt != 0.0) {
@@ -666,7 +630,6 @@ __global__ void __launch_bounds__(32) __maxnreg__(em_max_regs(MINB))
             flush_M(a_prev);
         }
         __syncwarp();
-        if (NBUF == 2) buf ^= 1;
     }
     if constexpr (C::kPrivateS) flush_S(cur_r);
     if constexpr (LL) {
@@ -674,7 +637,6 @@ __global__ void __launch_bounds__(32) __maxnreg__(em_max_regs(MINB))
         if (lane == 0 && ll != 0.0) red_add_f64(stats + stats_off_ll(P, K), ll);
     }
     if constexpr (STREAM) {
-        if (sa.dbg != nullptr && bx_v == 0 && lane == 0) sa.dbg[3] = global_timer_ns();
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) consumed += __shfl_xor_sync(0xffffffffu, consumed, o);
         if (lane == 0) atomicAdd(sa.chk, consumed);
@@ -933,55 +895,19 @@ static int launch_finalize_generic(int P, int K, const double *theta, const doub
 
 static int g_slot_counter = 0;
 
-// TIP_EM_VARIANT (environment, read once): 0 = the per-K default chosen in launch_em_fused, 1 / 2 / 3 / 4 = 16 / 14 /
-// 13 / 12 resident warp-CTAs per SM, for tuning runs.  (A double-buffered gather was measured slower: its shared
-// memory halves the resident warps; the NBUF template parameter keeps that variant buildable.)
-static int em_variant()
-{
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("TIP_EM_VARIANT");
-        v = e ? atoi(e) : 0;
-        if (v < 0 || v > 5) v = 0;
-    }
-    return v;
-}
-
-// TIP_EM_SCATTER=red (environment, read once): slot-b/c contributions with per-lane red.global.add.f64 instead of
-// the bulk add-reductions, for A/B timing (measured equal within noise at K=10; both give the same statistics)
-static int em_seg_zsmem()
-{
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("TIP_SEG_ZSMEM");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v;
-}
-
-static int em_red_scatter()
-{
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("TIP_EM_SCATTER");
-        v = (e && e[0] == 'r') ? 1 : 0;
-    }
-    return v;
-}
-
-template <int K, int NBUF, int MINB, bool LL, typename T = double, bool SEG = false, bool STREAM = false>
+template <int K, int MINB, bool LL, typename T = double, bool SEG = false, bool STREAM = false>
 static int launch_variant(int P, const int4 *rows, int64_t n_rows, int64_t n_rows_r0, const double *theta, int p_off0,
                           int p_off1, double *stats, double *Mg, cudaStream_t st, StreamArrive sa = StreamArrive{})
 {
-    using C = EmCfg<K, NBUF>;
+    using C = EmCfg<K>;
     static int blocks_per_sm = 0;
     if (blocks_per_sm == 0) {
-        TIP_CHECK_CUDA(cudaFuncSetAttribute(em_fused_kernel<K, NBUF, MINB, LL, T, SEG, STREAM>,
+        TIP_CHECK_CUDA(cudaFuncSetAttribute(em_fused_kernel<K, MINB, LL, T, SEG, STREAM>,
                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-        TIP_CHECK_CUDA(cudaFuncSetAttribute(em_fused_kernel<K, NBUF, MINB, LL, T, SEG, STREAM>,
+        TIP_CHECK_CUDA(cudaFuncSetAttribute(em_fused_kernel<K, MINB, LL, T, SEG, STREAM>,
                                             cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         int nb = 0;
-        TIP_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, em_fused_kernel<K, NBUF, MINB, LL, T, SEG, STREAM>, 32,
+        TIP_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, em_fused_kernel<K, MINB, LL, T, SEG, STREAM>, 32,
                                                                      C::SMEM));
         TIP_REQUIRE(nb >= 1, "em_fused_kernel<%d> does not fit on an SM (smem %zu)", K, C::SMEM);
         blocks_per_sm = nb;
@@ -991,9 +917,9 @@ static int launch_variant(int P, const int4 *rows, int64_t n_rows, int64_t n_row
     int64_t cap = (int64_t)sm_count() * blocks_per_sm;
     int grid = (int)(n_tiles < cap ? n_tiles : cap);
     if (grid < 1) grid = 1;
-    em_fused_kernel<K, NBUF, MINB, LL, T, SEG, STREAM><<<grid, 32, C::SMEM, st>>>(
+    em_fused_kernel<K, MINB, LL, T, SEG, STREAM><<<grid, 32, C::SMEM, st>>>(
         P, rows, (int)n_tiles, (int)(n_rows_r0 / 32), theta, p_off0, p_off1, stats, Mg,
-        SEG ? Mg + 2 * (size_t)P * K * K : nullptr, em_red_scatter() | (em_seg_zsmem() << 1), sa);
+        SEG ? Mg + 2 * (size_t)P * K * K : nullptr, sa);
     TIP_CHECK_CUDA(cudaGetLastError());
     return 0;
 }
@@ -1035,14 +961,14 @@ static int upload_p_slot(int K, const double *p, bool f32, cudaStream_t st, int 
 constexpr int kPhaseBegin = 1, kPhaseRun = 2, kPhaseEnd = 4;
 static int g_phase_off0 = 0, g_phase_off1 = 0;
 
-template <int K, int NBUF, int MINB, bool LL, typename T>
+template <int K, int MINB, bool LL, typename T>
 static int run_rows(int P, const int4 *rows, int64_t n_rows, int64_t n_rows_r0, const double *theta, const double *p,
                     double *stats, double *ws, cudaStream_t st)
 {
     constexpr int KP = K + (K & 1), TBL = K * K * KP;
     if constexpr (2 * TBL <= kPBankDoubles) {
-        return launch_variant<K, NBUF, MINB, LL, T>(P, rows, n_rows, n_rows_r0, theta, g_phase_off0, g_phase_off1, stats,
-                                                    ws, st);
+        return launch_variant<K, MINB, LL, T>(P, rows, n_rows, n_rows_r0, theta, g_phase_off0, g_phase_off1, stats, ws,
+                                              st);
     } else {
         // one rating fits the bank at a time: upload p_r, run that rating block, in stream order
         for (int r = 0; r < 2; ++r) {
@@ -1050,7 +976,7 @@ static int run_rows(int P, const int4 *rows, int64_t n_rows, int64_t n_rows_r0, 
             if (hi <= lo) continue;
             int rc = upload_p_const(K, p, r, 1, 0, sizeof(T) == 4, st);
             if (rc != 0) return rc;
-            rc = launch_variant<K, NBUF, MINB, LL, T>(P, rows + lo, hi - lo, r == 0 ? hi - lo : 0, theta, 0, 0, stats, ws, st);
+            rc = launch_variant<K, MINB, LL, T>(P, rows + lo, hi - lo, r == 0 ? hi - lo : 0, theta, 0, 0, stats, ws, st);
             if (rc != 0) return rc;
         }
         return 0;
@@ -1093,33 +1019,20 @@ static int launch_em_fused(int P, const int4 *rows, int64_t n_rows, int64_t n_ro
         rc = 0;
     } else if (seg) {
         if constexpr (K > 4)
-            rc = launch_variant<K, 1, 16, false, double, true>(P, rows, n_rows, n_rows_r0, theta, 0, 0, stats, ws, st);
+            rc = launch_variant<K, 16, false, double, true>(P, rows, n_rows, n_rows_r0, theta, 0, 0, stats, ws, st);
     } else if constexpr (K > 10) {
         // K >= 14 prefers 10 resident warps with ~198 registers and no spills (1e7 links: K=16 8.16 vs 8.96 ms,
-        // K=14 6.10 vs 6.27 ms); K = 11..13 stay at 12.  TIP_EM_VARIANT = 2 / 4 / 5 forces 14 / 12 / 10.
-        int v = em_variant();
-        if (v == 0) v = (K >= 14) ? 5 : 4;
-        switch (v) {
-            case 2: rc = run_rows<K, 1, 14, false, double>(P, rows, n_rows, n_rows_r0, theta, p, stats, ws, st); break;
-            case 5: rc = run_rows<K, 1, 10, false, double>(P, rows, n_rows, n_rows_r0, theta, p, stats, ws, st); break;
-            default: rc = run_rows<K, 1, 12, false, double>(P, rows, n_rows, n_rows_r0, theta, p, stats, ws, st); break;
-        }
+        // K=14 6.10 vs 6.27 ms); K = 11..13 stay at 12.
+        rc = run_rows<K, (K >= 14) ? 10 : 12, false, double>(P, rows, n_rows, n_rows_r0, theta, p, stats, ws, st);
     } else if (f32) {
-        rc = run_rows<K, 1, 16, false, float>(P, rows, n_rows, n_rows_r0, theta, p, stats, ws, st);
+        rc = run_rows<K, 16, false, float>(P, rows, n_rows, n_rows_r0, theta, p, stats, ws, st);
     } else if (with_ll) {
-        rc = run_rows<K, 1, 12, true, double>(P, rows, n_rows, n_rows_r0, theta, p, stats, ws, st);
+        rc = run_rows<K, 12, true, double>(P, rows, n_rows, n_rows_r0, theta, p, stats, ws, st);
     } else {
         // resident warp-CTAs per SM (register budget 65536 / (32 MINB)): measured at 1e7 links, K = 10 gains 6-7 % and
         // K = 8 2.6 % from 16 (128 registers, ~90 bytes of spills) over 12 (158 registers); K = 9 loses 1 %, K <= 6
-        // does not care.  TIP_EM_VARIANT = 1 / 2 / 3 / 4 forces 16 / 14 / 13 / 12 for tuning runs.
-        int v = em_variant();
-        if (v == 0) v = (K == 10 || K == 8) ? 1 : 4;
-        switch (v) {
-            case 1: rc = run_rows<K, 1, 16, false, double>(P, rows, n_rows, n_rows_r0, theta, p, stats, ws, st); break;
-            case 2: rc = run_rows<K, 1, 14, false, double>(P, rows, n_rows, n_rows_r0, theta, p, stats, ws, st); break;
-            case 3: rc = run_rows<K, 1, 13, false, double>(P, rows, n_rows, n_rows_r0, theta, p, stats, ws, st); break;
-            default: rc = run_rows<K, 1, 12, false, double>(P, rows, n_rows, n_rows_r0, theta, p, stats, ws, st); break;
-        }
+        // does not care.
+        rc = run_rows<K, (K == 10 || K == 8) ? 16 : 12, false, double>(P, rows, n_rows, n_rows_r0, theta, p, stats, ws, st);
     }
     if (rc != 0) return rc;
     if (!(phases & kPhaseEnd)) return 0;
@@ -1154,7 +1067,7 @@ static int launch_em_seg_large(int P, const int4 *rows, int64_t n_rows, int64_t 
         TIP_CHECK_CUDA(cudaMemsetAsync(ws, 0, sizeof(double) * 2 * (size_t)P * K * K, st));
     }
     if ((phases & kPhaseRun) && n_rows > 0) {
-        const int rc = launch_variant<K, 1, 8, false, double, true>(P, rows, n_rows, n_rows_r0, theta, 0, 0, stats, ws, st);
+        const int rc = launch_variant<K, 8, false, double, true>(P, rows, n_rows, n_rows_r0, theta, 0, 0, stats, ws, st);
         if (rc != 0) return rc;
     }
     if (phases & kPhaseEnd) return launch_finalize_generic(P, K, theta, p, ws, stats, st);
@@ -1172,7 +1085,7 @@ __global__ void __launch_bounds__(32, 16)
     loglik_fused_kernel(const int4 *__restrict__ rows, int n_tiles, int n_tiles_r0, const double *__restrict__ theta,
                         int p_slot, double *__restrict__ partials, unsigned *__restrict__ counter, double *__restrict__ out)
 {
-    using C = EmCfg<K, 1>;
+    using C = EmCfg<K>;
     constexpr int KP = C::KP, RS = C::RS;
     __shared__ __align__(16) double stage[32 * RS];
     __shared__ __align__(16) int4 ids_sm[32];
@@ -1383,7 +1296,7 @@ static int launch_streamed_k(int P, const void *rows, int64_t n_rows, int64_t n_
                              double *ws, StreamArrive sa, cudaStream_t st)
 {
     constexpr int MINB = (K == 10 || K == 8) ? 16 : 12;  // as in launch_em_fused
-    return launch_variant<K, 1, MINB, false, double, false, true>(P, reinterpret_cast<const int4 *>(rows), n_rows, n_rows_r0, theta,
+    return launch_variant<K, MINB, false, double, false, true>(P, reinterpret_cast<const int4 *>(rows), n_rows, n_rows_r0, theta,
                                                                   g_phase_off0, g_phase_off1, stats, ws, st, sa);
 }
 
@@ -1393,7 +1306,6 @@ int launch_em_streamed(int P, int K, const void *rows, int64_t n_rows, int64_t n
     StreamArrive sa;
     sa.chk = chk;
     TIP_CHECK_CUDA(cudaMemsetAsync(chk, 0, 4 * sizeof(unsigned long long), st));
-    sa.dbg = getenv("TIP_HOST_STREAM_DEBUG") ? reinterpret_cast<unsigned long long *>(err) + 8 : nullptr;
     sa.err = err;
     sa.compact = compact ? 1 : 0;
     // 5 s: a host that stopped feeding the copy stream must not hang the GPU (TIP_STREAM_TIMEOUT_US overrides it, so

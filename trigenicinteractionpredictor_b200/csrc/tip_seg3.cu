@@ -38,8 +38,6 @@
 // B + C checks the s it gathered and re-reads (ld.relaxed.gpu) the ones still NaN.  Every pass-A tile has been drawn by
 // a resident warp before the first pass-B tile can be (A's grid is one resident wave), so the wait is bounded; a wait of
 // more than ~2 s poisons the statistics with NaN instead of hanging.
-#include <stdlib.h>
-
 #include <cub/device/device_radix_sort.cuh>
 
 #include "tip_common.cuh"
@@ -106,7 +104,6 @@ struct S3Args {
     unsigned *counter;       // schedule position counter of this launch, zero on entry
     const int *sched;        // chunks of this launch: (first tile << 3) | tiles, by descending cost; 0 = end of the list
     int n_sched;             // entries in sched (real chunks first, zeros behind them)
-    int tune;                // bit 0: gather through L1 (cp.async.ca) instead of L2 only (.cg); bit 4: (launcher) no overlap
 };
 
 __device__ __forceinline__ void cp_async_16_ca(void *smem_dst, const void *gmem_src)
@@ -169,12 +166,12 @@ __device__ __forceinline__ void s3_gather(const double *__restrict__ theta, cons
     }
 }
 
-// NST stage buffers: the gathers of the next NST - 1 tiles are in flight while a tile is computed
-template <int K, bool FIRST, int NST, bool CA>
+// Two stage buffers: the gather of the next tile is in flight while a tile is computed
+template <int K, bool FIRST, bool CA>
 __global__ void __launch_bounds__(32, K <= 16 ? (FIRST ? 16 : 18) : 1) seg3_pass_kernel(const S3Args a)
 {
     using C = S3<K>;
-    constexpr int KK = C::KK, NB = C::NB, NKG = C::NKG, RS = C::RS, D = NST - 1;
+    constexpr int KK = C::KK, NB = C::NB, NKG = C::NKG, RS = C::RS;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x, li = lane & 3, ri = lane >> 2;
     if constexpr (FIRST) {
@@ -253,26 +250,23 @@ __global__ void __launch_bounds__(32, K <= 16 ? (FIRST ? 16 : 18) : 1) seg3_pass
         double *st = stage_of(buf);
         ids[lane] = me;
         __syncwarp();
-        if (!(a.tune & 2)) s3_gather<K, CA>(a.theta, ids, st, lane);   // (tune bit 1: timing experiment, wrong results)
-        if constexpr (!FIRST) if (!(a.tune & 8)) cp_async_8_zfill(st + 32 * RS + lane, a.sbuf + (me.w >= 0 ? me.w : 0), me.w >= 0 ? 8 : 0);
+        s3_gather<K, CA>(a.theta, ids, st, lane);
+        if constexpr (!FIRST) cp_async_8_zfill(st + 32 * RS + lane, a.sbuf + (me.w >= 0 ? me.w : 0), me.w >= 0 ? 8 : 0);
     };
 
-    // tq[0]: tile computed this iteration; tq[1 .. D-1]: gathers in flight; tq[D .. D+RQ-1]: rows held in registers
+    // tq[0]: tile computed this iteration (gathered into buffer cb); tq[1 .. RQ]: rows held in registers
     // (the rows come from HBM: RQ tiles of lookahead hide that latency)
     constexpr int RQ = 2;
-    int tq[D + RQ];
+    int tq[1 + RQ];
     int4 meq[RQ];
-#pragma unroll
-    for (int j = 0; j < D; ++j) {
-        tq[j] = next_tile();
-        if (tq[j] >= 0) issue_gather(j, a.rows[(int64_t)tq[j] * 32 + lane]);
-        cp_async_commit();
-    }
+    tq[0] = next_tile();
+    if (tq[0] >= 0) issue_gather(0, a.rows[(int64_t)tq[0] * 32 + lane]);
+    cp_async_commit();
 #pragma unroll
     for (int j = 0; j < RQ; ++j) {
-        tq[D + j] = next_tile();
+        tq[1 + j] = next_tile();
         meq[j] = make_int4(0, 0, 0, 0);
-        if (tq[D + j] >= 0) meq[j] = a.rows[(int64_t)tq[D + j] * 32 + lane];
+        if (tq[1 + j] >= 0) meq[j] = a.rows[(int64_t)tq[1 + j] * 32 + lane];
     }
 
     int cb = 0;    // buffer of tq[0]
@@ -291,18 +285,14 @@ __global__ void __launch_bounds__(32, K <= 16 ? (FIRST ? 16 : 18) : 1) seg3_pass
     };
 
     while (tq[0] >= 0) {
-        // ---- A: gather of the tile D ahead; B: rows of the tile D + 1 ahead ----
-        {
-            int gb = cb + D;
-            if (gb >= NST) gb -= NST;
-            if (tq[D] >= 0) issue_gather(gb, meq[0]);
-            cp_async_commit();
-        }
+        // ---- A: gather of the next tile into the other buffer; B: rows of the tile after it ----
+        if (tq[1] >= 0) issue_gather(cb ^ 1, meq[0]);
+        cp_async_commit();
         const int tn = next_tile();
 #pragma unroll
         for (int j = 0; j + 1 < RQ; ++j) meq[j] = meq[j + 1];
         if (tn >= 0) meq[RQ - 1] = a.rows[(int64_t)tn * 32 + lane];
-        cp_async_wait<D>();
+        cp_async_wait<1>();
         __syncwarp();
 
         const int t = tq[0];
@@ -409,12 +399,10 @@ __global__ void __launch_bounds__(32, K <= 16 ? (FIRST ? 16 : 18) : 1) seg3_pass
                 part += __shfl_xor_sync(0xffffffffu, part, 2);
                 if (li == rb) dsel = TIP_EPS + part;
             }
-            if constexpr (C::HOIST_Z && NST > 1) {
+            if constexpr (C::HOIST_Z) {
                 // Z fragments of the next tile's first run, requested now so that they land during the M phase below
                 if (tq[1] >= 0) {
-                    int nb_ = cb + 1;
-                    if (nb_ >= NST) nb_ -= NST;
-                    const int mnext = mbase_of(tq[1]) + ids_of(nb_)[0].x;
+                    const int mnext = mbase_of(tq[1]) + ids_of(cb ^ 1)[0].x;
                     if (mnext != zcur && mnext != znext) {
                         load_z(zn, mnext);
                         znext = mnext;
@@ -434,9 +422,7 @@ __global__ void __launch_bounds__(32, K <= 16 ? (FIRST ? 16 : 18) : 1) seg3_pass
         }
 
         // ---- M += (s th_x)^T . th_y over the runs of equal gene in this tile ----
-        if (a.tune & 4) {
-            // (tune bit 2: timing experiment, wrong results)
-        } else if (bm == 0u) {
+        if (bm == 0u) {
             // the whole tile continues the current run: eight unconditional k-steps
 #pragma unroll 4
             for (int ks = 0; ks < 8; ++ks) {
@@ -496,9 +482,9 @@ __global__ void __launch_bounds__(32, K <= 16 ? (FIRST ? 16 : 18) : 1) seg3_pass
         }
         __syncwarp();
 #pragma unroll
-        for (int j = 0; j + 1 < D + RQ; ++j) tq[j] = tq[j + 1];
-        tq[D + RQ - 1] = tn;
-        if (++cb == NST) cb = 0;
+        for (int j = 0; j < RQ; ++j) tq[j] = tq[j + 1];
+        tq[RQ] = tn;
+        cb ^= 1;
     }
 }
 
@@ -755,39 +741,6 @@ static S3Layout s3_layout(int P, int K, int64_t n_rows)
 
 size_t em_seg3_workspace_bytes(int P, int K, int64_t n_rows) { return s3_layout(P, K, n_rows).total * sizeof(double); }
 
-static int s3_tune()
-{
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("TIP_SEG3_TUNE");
-        v = e ? atoi(e) : 0;
-    }
-    return v;
-}
-
-// TIP_SEG3_SKIP (bit mask, timing experiments only - results are wrong): 4 pass A, 8 pass B+C, 16 finish
-static int s3_skip()
-{
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("TIP_SEG3_SKIP");
-        v = e ? atoi(e) : 0;
-    }
-    return v;
-}
-
-// stage buffers per warp: TIP_SEG3_STAGES_A / TIP_SEG3_STAGES_BC = 1 | 2 (1: no gather prefetch inside a warp, most warps per SM)
-static int s3_stages(bool first)
-{
-    static int v[2] = {-1, -1};
-    if (v[first] < 0) {
-        const char *e = getenv(first ? "TIP_SEG3_STAGES_A" : "TIP_SEG3_STAGES_BC");
-        v[first] = e ? atoi(e) : 2;
-        if (v[first] != 1 && v[first] != 2) v[first] = 2;
-    }
-    return v[first];
-}
-
 // Per-kernel timing of one E-step (tip_seg3_timing): CUDA events recorded on the launching stream between the five
 // stages.  Off by default (event records cannot be captured in a CUDA graph); bench.py switches it on around the
 // un-graphed steps it uses for the roofline of the dominant kernel.
@@ -802,29 +755,18 @@ static int s3_mark(int i, cudaStream_t st)
     return 0;
 }
 
-// TIP_SEG3_NO_OVERLAP=1: launch pass B + C without the programmatic-dependent-launch attribute (A/B comparison)
-static bool s3_no_overlap()
-{
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("TIP_SEG3_NO_OVERLAP");
-        v = (e && atoi(e) != 0) ? 1 : 0;
-    }
-    return v != 0;
-}
-
-template <int K, bool FIRST, int NST, bool CA>
-static int s3_launch_pass_n(const S3Args &a, cudaStream_t st, int *grid_only)
+template <int K, bool FIRST, bool CA>
+static int s3_launch_pass_ca(const S3Args &a, bool plain, cudaStream_t st, int *grid_only)
 {
     using C = S3<K>;
-    constexpr size_t smem = C::BUF_BYTES * NST;
+    constexpr size_t smem = C::BUF_BYTES * 2;
     static int blocks_per_sm = 0;
     if (blocks_per_sm == 0) {
-        TIP_CHECK_CUDA(cudaFuncSetAttribute(seg3_pass_kernel<K, FIRST, NST, CA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        TIP_CHECK_CUDA(cudaFuncSetAttribute(seg3_pass_kernel<K, FIRST, NST, CA>, cudaFuncAttributePreferredSharedMemoryCarveout,
+        TIP_CHECK_CUDA(cudaFuncSetAttribute(seg3_pass_kernel<K, FIRST, CA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        TIP_CHECK_CUDA(cudaFuncSetAttribute(seg3_pass_kernel<K, FIRST, CA>, cudaFuncAttributePreferredSharedMemoryCarveout,
                                             cudaSharedmemCarveoutMaxShared));
         int nb = 0;
-        TIP_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, seg3_pass_kernel<K, FIRST, NST, CA>, 32, smem));
+        TIP_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, seg3_pass_kernel<K, FIRST, CA>, 32, smem));
         TIP_REQUIRE(nb >= 1, "seg3_pass_kernel<%d> does not fit on an SM (smem %zu)", K, smem);
         blocks_per_sm = nb;
     }
@@ -835,7 +777,7 @@ static int s3_launch_pass_n(const S3Args &a, cudaStream_t st, int *grid_only)
         *grid_only = grid;
         return 0;
     }
-    if (!g_s3_timing && !s3_no_overlap() && !(a.tune & 16)) {
+    if (!g_s3_timing && !plain) {
         // pass B + C may start while pass A drains (see the header comment); it never waits for the grid dependency,
         // only for the s values it needs.  Pass A is launched the same way behind the prep kernel and DOES wait
         // (griddepcontrol.wait at its top): what it gains is its launch latency and CTA ramp
@@ -849,22 +791,22 @@ static int s3_launch_pass_n(const S3Args &a, cudaStream_t st, int *grid_only)
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        TIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, seg3_pass_kernel<K, FIRST, NST, CA>, a));
+        TIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, seg3_pass_kernel<K, FIRST, CA>, a));
         return 0;
     }
-    seg3_pass_kernel<K, FIRST, NST, CA><<<grid, 32, smem, st>>>(a);
+    seg3_pass_kernel<K, FIRST, CA><<<grid, 32, smem, st>>>(a);
     TIP_CHECK_CUDA(cudaGetLastError());
     return 0;
 }
 
-// grid_only != nullptr: only report the grid the launch would use (the prep kernel presets the schedule counters with it)
+// gather_l1: gather through L1 (cp.async.ca) instead of L2 only (.cg).  plain: launch without the programmatic dependency
+// on the previous kernel.  grid_only != nullptr: only report the grid the launch would use (the prep kernel presets the
+// schedule counters with it)
 template <int K, bool FIRST>
-static int s3_launch_pass(const S3Args &a, cudaStream_t st, int *grid_only = nullptr)
+static int s3_launch_pass(const S3Args &a, bool gather_l1, bool plain, cudaStream_t st, int *grid_only = nullptr)
 {
-    const bool ca = (a.tune & 1) != 0;
-    if (s3_stages(FIRST) == 1)
-        return ca ? s3_launch_pass_n<K, FIRST, 1, true>(a, st, grid_only) : s3_launch_pass_n<K, FIRST, 1, false>(a, st, grid_only);
-    return ca ? s3_launch_pass_n<K, FIRST, 2, true>(a, st, grid_only) : s3_launch_pass_n<K, FIRST, 2, false>(a, st, grid_only);
+    return gather_l1 ? s3_launch_pass_ca<K, FIRST, true>(a, plain, st, grid_only)
+                     : s3_launch_pass_ca<K, FIRST, false>(a, plain, st, grid_only);
 }
 
 static S3Push g_s3_push = {};
@@ -881,7 +823,6 @@ static int launch_em_seg3_k(int P, const int4 *rows, int64_t n_rows, int64_t n_r
     const S3Layout l = s3_layout(P, K, n_rows);
     const int KK = K * K;
     TIP_REQUIRE(n_rows / 32 < (1ll << 27), "tip_em_step: too many tiles in one shard for the slot-segmented kernels");
-    const int skip = s3_skip();
     S3Args a;
     a.P = P;
     a.rows = rows;
@@ -891,7 +832,6 @@ static int launch_em_seg3_k(int P, const int4 *rows, int64_t n_rows, int64_t n_r
     a.Zg = ws + l.off_Z;
     a.sbuf = ws + l.off_s;
     a.Mg = ws + l.off_M;
-    a.tune = s3_tune() | (gather_l1 ? 1 : 0);
     a.n_tiles = a.tiles_per_order;
     a.slot0 = 0;
     a.counter = reinterpret_cast<unsigned *>(ws + l.off_cnt);
@@ -906,9 +846,9 @@ static int launch_em_seg3_k(int P, const int4 *rows, int64_t n_rows, int64_t n_r
     bc.sched = sched + a.tiles_per_order;
     bc.n_sched = 2 * a.tiles_per_order;
     int grid_a = 0, grid_bc = 0;
-    int rc = s3_launch_pass<K, true>(a, st, &grid_a);
+    int rc = s3_launch_pass<K, true>(a, gather_l1, false, st, &grid_a);
     if (rc) return rc;
-    rc = s3_launch_pass<K, false>(bc, st, &grid_bc);
+    rc = s3_launch_pass<K, false>(bc, gather_l1, false, st, &grid_bc);
     if (rc) return rc;
     // M starts every E-step from zero, sbuf from NaN ("not published"), the schedule counters behind the statically
     // assigned positions: all written by the prep kernel (no memset launches)
@@ -928,18 +868,16 @@ static int launch_em_seg3_k(int P, const int4 *rows, int64_t n_rows, int64_t n_r
         TIP_CHECK_CUDA(cudaGetLastError());
     }
     if (s3_mark(2, st)) return -2;
-    rc = (skip & 4) ? 0 : s3_launch_pass<K, true>(a, st);
+    rc = s3_launch_pass<K, true>(a, gather_l1, false, st);
     if (rc) return rc;
     if (s3_mark(3, st)) return -2;
-    if (bc_wait) {
-        // (host-buffer entry) orders b and c are still being produced on another stream
-        TIP_CHECK_CUDA(cudaStreamWaitEvent(st, bc_wait, 0));
-        bc.tune |= 16;   // a plain launch behind the wait (no programmatic dependency on pass A)
-    }
-    rc = (skip & 8) ? 0 : s3_launch_pass<K, false>(bc, st);
+    // (host-buffer entry) orders b and c are still being produced on another stream: a plain launch behind the wait
+    // (no programmatic dependency on pass A)
+    if (bc_wait) TIP_CHECK_CUDA(cudaStreamWaitEvent(st, bc_wait, 0));
+    rc = s3_launch_pass<K, false>(bc, gather_l1, bc_wait != nullptr, st);
     if (rc) return rc;
     if (s3_mark(4, st)) return -2;
-    if (!(skip & 16)) {
+    {
         constexpr int NBC = (K * K + 7) / 8;
         const int n_kind2 = 2 * NBC * ((P + kFin3GeneChunk - 1) / kFin3GeneChunk);
         const int wpc = kFin3Threads / 32;

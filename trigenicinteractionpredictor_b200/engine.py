@@ -13,7 +13,6 @@ from __future__ import annotations
 
 import ctypes
 import functools
-import os
 
 import numpy as np
 import torch
@@ -358,8 +357,7 @@ class EMEngine:
         if self.peer is not None:
             if self.peer.mode == "rs":
                 par = 0                                   # no double buffering: see tip_peer_mstep
-            fused = (self.peer.mode == "push" and bool(self.flags & _cabi.TIP_EM_SLOT_SEGMENTED) and self.train.n_rows > 0
-                     and os.environ.get("TIP_PEER_FUSED", "1") != "0")
+            fused = self.peer.mode == "push" and bool(self.flags & _cabi.TIP_EM_SLOT_SEGMENTED) and self.train.n_rows > 0
             if fused:
                 # the finish kernel of this E-step stores Ntheta into the peers' inboxes as it produces it
                 pe = self.peer
