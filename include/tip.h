@@ -197,6 +197,26 @@ int tip_top_triplets(int P, int K, int S, const double *d_theta, const double *d
 /* scoring passes (full sweeps) the last tip_top_triplets of this thread ran (measurement) */
 int tip_top_triplets_last_passes(void);
 
+/* ---- prediction per gene: for every query gene, the N highest-scoring unseen triplets that contain it ----
+ * Rank space, score and known keys as tip_top_triplets: d_cand[n_cand] in decimal-string order (rank = position),
+ * d_known sorted packed rank triples.  d_query_ranks[n_query]: distinct ranks into d_cand (a query is itself a candidate;
+ * its partners are the other candidates).  For the query of rank r every pair x < y of other ranks is scored, in one of
+ * three regions by the query's slot: x < y < r (slot c), x < r < y (slot b), r < x < y (slot a).
+ * Out, per query q: the first min(N, C(n_cand - 1, 2) - its known keys) triplets in the order (score descending, (ra, rb, rc)
+ * ascending), exact under any ties: d_out_ids[n_query][N][3] gene ids in slot order, d_out_scores[n_query][N],
+ * h_n_out[n_query] rows (rows past h_n_out[q] are not written).  Each query has its own threshold, narrowed between sweeps
+ * as in tip_top_triplets; sweeps after the first score only the queries not yet resolved.  Out-of-range or duplicate query
+ * ranks are refused before any device work.  Synchronises the stream; not capturable in a CUDA graph.  Limits:
+ * n_cand <= 2^21, S * K <= 384, n_query <= n_cand, n_query * N <= 2^24.  Workspace O(n_cand S K + n_query (S K^2 + N)).
+ * Precondition: finite, non-negative parameters.  d_ws: tip_top_triplets_per_gene_workspace_bytes() bytes. */
+int tip_top_triplets_per_gene_workspace_bytes(int n_cand, int n_query, int K, int S, int64_t n_known, int64_t N, size_t *bytes);
+int tip_top_triplets_per_gene(int P, int K, int S, const double *d_theta, const double *d_p, const int32_t *d_cand, int n_cand,
+                              const int32_t *d_query_ranks, int n_query, const uint64_t *d_known, int64_t n_known, int64_t N,
+                              void *d_ws, size_t ws_bytes, int32_t *d_out_ids, double *d_out_scores, int64_t *h_n_out,
+                              void *stream);
+/* sweeps the last tip_top_triplets_per_gene of this thread ran (measurement) */
+int tip_top_triplets_per_gene_last_passes(void);
+
 /* ---- testResultsReducer.py:160-184: mean / median / standard deviation of every test triplet across samples ----
  * d_scores[S][T]: score of triplet t in sample j at [j * T + t]; d_n[t] (or NULL = S) = how many leading samples of
  * triplet t are valid.  mean = sequential sum in sample order / n; median = the reference's rule (ascending sort;

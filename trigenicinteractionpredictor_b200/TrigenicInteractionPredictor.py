@@ -18,6 +18,7 @@ CLI (same flags as TIP.py:1166-1167):
 from __future__ import annotations
 
 import codecs
+import collections
 import getopt
 import math
 import os
@@ -607,18 +608,14 @@ class Model:
         self._theta_host, self._pr_host = theta, pr
         self._params_on, self._host_valid, self._exposed = "host", True, False
 
-    def predict_top_triplets(self, n, genes=None, exclude_known=True, params=None):
-        """The `n` most likely interacting triplets of distinct genes among `genes` (names; default all P genes), by
-        do_prediction (TIP.py:530-547) of the current theta / pr, or by the mean over the parameter sets in `params`
-        (.npz paths of save_parameters or (theta, pr) pairs).  With exclude_known the keys of links and test_links are
-        left out.  Exhaustive over C(n_genes, 3) triplets on the device.  Returns [[score, "a_b_c", "nameA_nameB_nameC"],
-        ...], best first; equal scores in ascending order of the triplets' positions in the decimal-string order of the
-        candidate ids.  The id key is the report's "ID of genes" column; names are sorted as in the fold files (TIP.py:486)."""
+    def _prediction_sets(self, params, who):
+        """The checked (theta, pr) sets a prediction averages over: the current theta / pr, or `params` (.npz paths of
+        save_parameters or (theta, pr) pairs).  Raises ValueError (messages prefixed with `who`)."""
         if self.P < 1 or len(self.id_gene) != self.P:
-            raise ValueError("predict_top_triplets needs a model digested from train / test files")
+            raise ValueError(who + " needs a model digested from train / test files")
         if params is None:
             if self.K < 1:
-                raise ValueError("predict_top_triplets: initialize_parameters() or load_parameters() must run first")
+                raise ValueError(who + ": initialize_parameters() or load_parameters() must run first")
             sets = [self._check_parameters(self.theta, self.pr, self.K, None, "the model's parameters")]
         else:
             sets = []
@@ -629,10 +626,26 @@ class Model:
                     th, pr = item
                     sets.append(self._check_parameters(th, pr, np.asarray(th).shape[-1], None, "a (theta, pr) pair"))
             if not sets:
-                raise ValueError("predict_top_triplets: params is empty")
+                raise ValueError(who + ": params is empty")
             Ks = {th.shape[1] for th, _ in sets}
             if len(Ks) != 1:
-                raise ValueError("predict_top_triplets: the parameter sets have different K (%s)" % sorted(Ks))
+                raise ValueError(who + ": the parameter sets have different K (%s)" % sorted(Ks))
+        return sets
+
+    def _prediction_engine(self, K):
+        from .engine import EMEngine
+        if self._engine is not None and self._engine_key == (self.P, K):
+            return self._engine
+        return EMEngine(self.P, K, device=self._device, flags=self._flags)
+
+    def predict_top_triplets(self, n, genes=None, exclude_known=True, params=None):
+        """The `n` most likely interacting triplets of distinct genes among `genes` (names; default all P genes), by
+        do_prediction (TIP.py:530-547) of the current theta / pr, or by the mean over the parameter sets in `params`
+        (.npz paths of save_parameters or (theta, pr) pairs).  With exclude_known the keys of links and test_links are
+        left out.  Exhaustive over C(n_genes, 3) triplets on the device.  Returns [[score, "a_b_c", "nameA_nameB_nameC"],
+        ...], best first; equal scores in ascending order of the triplets' positions in the decimal-string order of the
+        candidate ids.  The id key is the report's "ID of genes" column; names are sorted as in the fold files (TIP.py:486)."""
+        sets = self._prediction_sets(params, "predict_top_triplets")
         K = sets[0][0].shape[1]
         if genes is None:
             ids = list(range(self.P))
@@ -645,16 +658,51 @@ class Model:
         known = np.empty(0, dtype=np.uint64)
         if exclude_known:
             known = self._known_packed(cand)
-        from .engine import EMEngine
-        eng = self._engine if (self._engine is not None and self._engine_key == (self.P, K)) else None
-        if eng is None:
-            eng = EMEngine(self.P, K, device=self._device, flags=self._flags)
+        eng = self._prediction_engine(K)
         out_ids, scores = eng.top_triplets(np.stack([th for th, _ in sets]), np.stack([pr for _, pr in sets]), cand, known, int(n))
         rows = []
         for (a, b, c), s in zip(out_ids.tolist(), scores.tolist()):
             names = sorted((self.id_gene[a], self.id_gene[b], self.id_gene[c]))
             rows.append([s, "%d_%d_%d" % (a, b, c), "_".join(names)])
         return rows
+
+    def predict_top_triplets_per_gene(self, queries, n, genes=None, exclude_known=True, params=None):
+        """For every gene of `queries` (names, distinct): the `n` most likely interacting triplets that contain it, its two
+        partners distinct genes of `genes` + `queries` (names; default all P genes; the queries are always candidates),
+        scored as in predict_top_triplets.  With exclude_known the keys of links and test_links are left out.  Exhaustive
+        over the C(n_candidates - 1, 2) pairs of every query on the device.  Returns {query name: [[score, "a_b_c",
+        "nameA_nameB_nameC"], ...]} in the order of `queries`, each list best first with ties in the order of
+        predict_top_triplets; a list is shorter than n when the query has fewer unseen triplets."""
+        sets = self._prediction_sets(params, "predict_top_triplets_per_gene")
+        K = sets[0][0].shape[1]
+        queries = list(queries)
+        if not queries:
+            raise ValueError("predict_top_triplets_per_gene: queries is empty")
+        names = queries + (list(genes) if genes is not None else [])
+        missing = [g for g in names if g not in self.gene_id]
+        if missing:
+            raise ValueError("unknown gene names: %s" % ", ".join(dict.fromkeys(missing)))
+        twice = [g for g, c in collections.Counter(queries).items() if c > 1]
+        if twice:
+            raise ValueError("predict_top_triplets_per_gene: duplicate query genes: %s" % ", ".join(twice))
+        if int(n) < 0:
+            raise ValueError("predict_top_triplets_per_gene: n must be >= 0 (got %d)" % int(n))
+        ids = set(range(self.P)) if genes is None else {self.gene_id[g] for g in names}
+        cand = np.array(sorted(ids, key=str), dtype=np.int32)
+        rank = {g: r for r, g in enumerate(cand.tolist())}
+        qr = np.array([rank[self.gene_id[q]] for q in queries], dtype=np.int32)
+        known = self._known_packed(cand) if exclude_known else np.empty(0, dtype=np.uint64)
+        eng = self._prediction_engine(K)
+        out_ids, scores, counts = eng.top_triplets_per_gene(np.stack([th for th, _ in sets]), np.stack([pr for _, pr in sets]),
+                                                            cand, qr, known, int(n))
+        res = {}
+        for qi, q in enumerate(queries):
+            rows = []
+            for (a, b, c), s in zip(out_ids[qi, :counts[qi]].tolist(), scores[qi, :counts[qi]].tolist()):
+                names3 = sorted((self.id_gene[a], self.id_gene[b], self.id_gene[c]))
+                rows.append([s, "%d_%d_%d" % (a, b, c), "_".join(names3)])
+            res[q] = rows
+        return res
 
     def _known_packed(self, cand):
         """Sorted packed rank triples (ra << 42 | rb << 21 | rc) of the keys of links and test_links whose three genes

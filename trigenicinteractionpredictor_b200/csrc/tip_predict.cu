@@ -15,10 +15,17 @@
 // continues on the packed rank triple, so the result is exact whatever the scores are.  The buffer is then sorted by
 // (score descending, packed ranks ascending) and the first N rows are written out.  Known triplets are dropped in the
 // epilogue (binary search in the sorted known keys), so they never count towards N.
+//
+// Per query gene (tip_top_triplets_per_gene): the pairs of a query of rank r split into three regions by r's slot, each a
+// product th_x^T M th_y with a K x K matrix of the query (tip_query_pass_kernel, which shares the Q tile, the DMMA block
+// loop and the epilogue with tip_predict_pass_kernel).  Each query has its own threshold, survivor count, histogram and
+// buffer; its first threshold is the best score of a per-query sample, and sweeps after the first score only the queries
+// whose threshold has not settled.  A segmented sort orders every query's buffer.
 #include <algorithm>
 #include <vector>
 
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_segmented_sort.cuh>
 
 #include "tip_common.cuh"
 
@@ -53,6 +60,23 @@ __host__ __device__ inline long long items_before(long long j)
     return kPredRows * q * (q + 1) / 2 + r * (q + 1);
 }
 
+// threshold state of one selection (one per call of tip_top_triplets, one per query of tip_top_triplets_per_gene)
+struct Sel {
+    int mode;                       // 0: keep bits >= lo; 1: keep bits > v, or bits == v and packed <= rhi
+    int shift;
+    unsigned long long lo, hi;      // mode 0: histogram range of score bits (bin 0 = highest)
+    unsigned long long v, rlo, rhi; // mode 1: tied score bits and the histogram range of packed ranks (bin 0 = lowest)
+};
+
+// where the scores of a work item sit: row ra and column rc are a triplet when ra < row_end, rc < col_end and (tri) rc > ra;
+// its packed rank triple is (ra << sh_r) | (rc << sh_c) | fixed
+struct TileMap {
+    int row_end, col_end;
+    bool tri;
+    int sh_r, sh_c;
+    unsigned long long fixed;
+};
+
 struct PassArgs {
     int n, S, K, SK, SKP;
     const double *tcat;             // [n_pad][SKP] theta of every model, rank order, zero padded
@@ -60,10 +84,7 @@ struct PassArgs {
     const unsigned long long *known;  // sorted packed rank triples
     long long n_known;
     long long n_items;
-    int mode;                       // 0: keep bits >= lo; 1: keep bits > v, or bits == v and packed <= rhi
-    unsigned long long lo, hi;      // mode 0: histogram range of score bits (bin 0 = highest)
-    unsigned long long v, rlo, rhi; // mode 1: tied score bits and the histogram range of packed ranks (bin 0 = lowest)
-    int shift;
+    Sel sel;
     unsigned long long *counter;    // [0] entries kept, [1] work-item cursor
     unsigned long long *hist;       // [kPredBins + 1]
     unsigned long long *out_bits, *out_packed;
@@ -81,6 +102,16 @@ __device__ __noinline__ bool is_known(const unsigned long long *known, long long
     return lo < n && __ldg(known + lo) == key;
 }
 
+// tcat[r][s K + k] = theta_s of candidate r, zero padded to n_pad rows and SKP columns
+__device__ __forceinline__ double tcat_entry(long long t, int S, int P, int K, int n, int SKP, const double *theta,
+                                             const int32_t *cand)
+{
+    const int r = (int)(t / SKP), col = (int)(t % SKP);
+    if (r >= n || col >= S * K) return 0.0;
+    const int s = col / K, k = col % K;
+    return theta[((long long)s * P + cand[r]) * K + k];
+}
+
 __global__ void tip_predict_prep_kernel(int S, int P, int K, int n, int n_pad, int SKP, const double *__restrict__ theta,
                                         const double *__restrict__ p, const int32_t *__restrict__ cand, double *__restrict__ tcat,
                                         double *__restrict__ W)
@@ -88,13 +119,7 @@ __global__ void tip_predict_prep_kernel(int S, int P, int K, int n, int n_pad, i
     const long long n_t = (long long)n_pad * SKP, KK = (long long)K * K, n_w = (long long)S * n * KK;
     for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < n_t + n_w; t += (long long)gridDim.x * blockDim.x) {
         if (t < n_t) {
-            const int r = (int)(t / SKP), col = (int)(t % SKP);
-            double v = 0.0;
-            if (r < n && col < S * K) {
-                const int s = col / K, k = col % K;
-                v = theta[((long long)s * P + cand[r]) * K + k];
-            }
-            tcat[t] = v;
+            tcat[t] = tcat_entry(t, S, P, K, n, SKP, theta, cand);
         } else {
             const long long u = t - n_t;
             const int s = (int)(u / ((long long)n * KK));
@@ -146,6 +171,107 @@ __global__ void tip_predict_sample_kernel(int n, int S, int K, int SKP, const do
     out[t] = (unsigned long long)__double_as_longlong(acc);
 }
 
+// ---- pieces of a scoring pass, shared by tip_predict_pass_kernel and tip_query_pass_kernel ----
+
+// Q tile: Q[i][s K + z] = sum_x th_{a0+i}[s K + x] M[s][x][z] (M of set s at M + s * m_stride); pad rows / columns are zero
+__device__ __forceinline__ void form_q_tile(double *Q, int qs, const double *tcat, int SKP, int SK, int K, int a0, int rows,
+                                            const double *M, long long m_stride)
+{
+    for (int e = threadIdx.x; e < kPredRows * SKP; e += kPredThreads) {
+        const int i = e / SKP, col = e % SKP;
+        double acc = 0.0;
+        if (i < rows && col < SK) {
+            const int s = col / K, z = col % K;
+            const double *th = tcat + (long long)(a0 + i) * SKP + s * K;
+            const double *Wb = M + s * m_stride + z;
+            for (int x = 0; x < K; ++x) acc = fma(__ldg(th + x), __ldg(Wb + x * K), acc);
+        }
+        Q[i * qs + col] = acc;
+    }
+}
+
+// a warp's 32 x 32 block of scores: acc[mi][ni][e] = row gq + 8 mi of Qw times column 8 ni + 2 tq + e of Bw
+__device__ __forceinline__ void dmma_block(double (&acc)[4][4][2], const double *Qw, int qs, const double *Bw, int SKP)
+{
+#pragma unroll
+    for (int mi = 0; mi < 4; ++mi)
+#pragma unroll
+        for (int ni = 0; ni < 4; ++ni) acc[mi][ni][0] = acc[mi][ni][1] = 0.0;
+#pragma unroll 2
+    for (int kk = 0; kk < SKP; kk += 4) {
+        double af[4], bf[4];
+#pragma unroll
+        for (int mi = 0; mi < 4; ++mi) af[mi] = Qw[mi * 8 * qs + kk];
+#pragma unroll
+        for (int ni = 0; ni < 4; ++ni) bf[ni] = __ldg(Bw + (long long)ni * 8 * SKP + kk);
+#pragma unroll
+        for (int mi = 0; mi < 4; ++mi)
+#pragma unroll
+            for (int ni = 0; ni < 4; ++ni) dmma884(acc[mi][ni][0], acc[mi][ni][1], af[mi], bf[ni]);
+    }
+}
+
+// epilogue of a block (ra0 = the lane's first row, rc0 = its first column): the threshold test runs in registers; only
+// survivors go further: known keys are dropped, the rest are histogrammed in sh_hist and appended to out_* (counted past cap)
+__device__ __forceinline__ void select_block(const double (&acc)[4][4][2], const Sel sel, const TileMap tm, int lane, int ra0,
+                                             int rc0, const unsigned long long *known, long long n_known, unsigned *sh_hist,
+                                             unsigned long long *counter, unsigned long long *out_bits,
+                                             unsigned long long *out_packed, long long cap)
+{
+    unsigned keep = 0;
+#pragma unroll
+    for (int mi = 0; mi < 4; ++mi)
+#pragma unroll
+        for (int ni = 0; ni < 4; ++ni)
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+                const unsigned long long bits = (unsigned long long)__double_as_longlong(acc[mi][ni][e]);
+                const bool pass = sel.mode == 0 ? bits >= sel.lo : bits >= sel.v;
+                keep |= (pass ? 1u : 0u) << ((mi * 4 + ni) * 2 + e);
+            }
+    if (!__any_sync(0xffffffffu, keep != 0)) return;
+#pragma unroll
+    for (int f = 0; f < 32; ++f) {
+        const int mi = f >> 3, ni = (f >> 1) & 3, e = f & 1;
+        const int ra = ra0 + mi * 8, rc = rc0 + ni * 8 + e;
+        const unsigned long long bits = (unsigned long long)__double_as_longlong(acc[mi][ni][e]);
+        const unsigned long long packed = ((unsigned long long)ra << tm.sh_r) | ((unsigned long long)rc << tm.sh_c) | tm.fixed;
+        bool q = ((keep >> f) & 1u) && ra < tm.row_end && rc < tm.col_end && (!tm.tri || rc > ra);
+        if (q && sel.mode == 1) q = bits > sel.v || packed <= sel.rhi;
+        if (q && n_known > 0) q = !is_known(known, n_known, packed);
+        int bin = kPredBins;
+        if (q) {
+            if (sel.mode == 0) {
+                if (bits <= sel.hi) bin = (int)((sel.hi - bits) >> sel.shift);
+            } else if (bits == sel.v && packed >= sel.rlo) {
+                bin = (int)((packed - sel.rlo) >> sel.shift);
+            }
+            atomicAdd(sh_hist + bin, 1u);
+        }
+        const unsigned m = __ballot_sync(0xffffffffu, q);
+        if (m == 0) continue;
+        unsigned long long base = 0;
+        if (lane == __ffs(m) - 1) base = atomicAdd(counter, (unsigned long long)__popc(m));
+        base = __shfl_sync(0xffffffffu, base, __ffs(m) - 1);
+        if (q) {
+            const unsigned long long idx = base + __popc(m & ((1u << lane) - 1u));
+            if ((long long)idx < cap) {
+                out_bits[idx] = bits;
+                out_packed[idx] = packed;
+            }
+        }
+    }
+}
+
+// add the CTA's shared bins to hist and clear them (all threads, between barriers)
+__device__ __forceinline__ void flush_hist(unsigned *sh_hist, unsigned long long *hist)
+{
+    for (int i = threadIdx.x; i <= kPredBins; i += kPredThreads) {
+        if (sh_hist[i]) atomicAdd(hist + i, (unsigned long long)sh_hist[i]);
+        sh_hist[i] = 0;
+    }
+}
+
 __global__ void __launch_bounds__(kPredThreads) tip_predict_pass_kernel(PassArgs A)
 {
     extern __shared__ __align__(16) unsigned char smem[];
@@ -177,103 +303,246 @@ __global__ void __launch_bounds__(kPredThreads) tip_predict_pass_kernel(PassArgs
         const int rows = min(kPredRows, j - a0);
         const int n_c = n - 1 - j;
 
-        // Q tile: Q[i][s K + z] = sum_x th_{a0+i}[s K + x] W[s][j][x][z]; pad columns are zero
-        for (int e = tid; e < kPredRows * SKP; e += kPredThreads) {
-            const int i = e / SKP, col = e % SKP;
-            double acc = 0.0;
-            if (i < rows && col < A.SK) {
-                const int s = col / K, z = col % K;
-                const double *th = A.tcat + (long long)(a0 + i) * SKP + s * K;
-                const double *Wb = A.W + ((long long)s * n + j) * K * K + z;
-                for (int x = 0; x < K; ++x) acc = fma(__ldg(th + x), __ldg(Wb + x * K), acc);
-            }
-            Q[i * qs + col] = acc;
-        }
+        form_q_tile(Q, qs, A.tcat, SKP, A.SK, K, a0, rows, A.W + (long long)j * K * K, (long long)n * K * K);
         __syncthreads();
 
-        const bool warp_rows = wr * 32 < rows;
-        if (warp_rows) {
+        const TileMap tm{j, n, false, 2 * kRankBits, 0, (unsigned long long)j << kRankBits};
+        if (wr * 32 < rows) {
             const double *Qw = Q + (wr * 32 + gq) * qs + tq;
             for (int c0 = j + 1 + wc * 32; c0 < n; c0 += 64) {
                 double acc[4][4][2];
-#pragma unroll
-                for (int mi = 0; mi < 4; ++mi)
-#pragma unroll
-                    for (int ni = 0; ni < 4; ++ni) acc[mi][ni][0] = acc[mi][ni][1] = 0.0;
-                const double *Bw = A.tcat + (long long)(c0 + gq) * SKP + tq;
-#pragma unroll 2
-                for (int kk = 0; kk < SKP; kk += 4) {
-                    double af[4], bf[4];
-#pragma unroll
-                    for (int mi = 0; mi < 4; ++mi) af[mi] = Qw[mi * 8 * qs + kk];
-#pragma unroll
-                    for (int ni = 0; ni < 4; ++ni) bf[ni] = __ldg(Bw + (long long)ni * 8 * SKP + kk);
-#pragma unroll
-                    for (int mi = 0; mi < 4; ++mi)
-#pragma unroll
-                        for (int ni = 0; ni < 4; ++ni) dmma884(acc[mi][ni][0], acc[mi][ni][1], af[mi], bf[ni]);
-                }
-                // epilogue: the threshold test runs in registers; only survivors go further
-                unsigned keep = 0;
-#pragma unroll
-                for (int mi = 0; mi < 4; ++mi)
-#pragma unroll
-                    for (int ni = 0; ni < 4; ++ni)
-#pragma unroll
-                        for (int e = 0; e < 2; ++e) {
-                            const unsigned long long bits = (unsigned long long)__double_as_longlong(acc[mi][ni][e]);
-                            const bool pass = A.mode == 0 ? bits >= A.lo : bits >= A.v;
-                            keep |= (pass ? 1u : 0u) << ((mi * 4 + ni) * 2 + e);
-                        }
-                if (!__any_sync(0xffffffffu, keep != 0)) continue;
-#pragma unroll
-                for (int f = 0; f < 32; ++f) {
-                    const int mi = f >> 3, ni = (f >> 1) & 3, e = f & 1;
-                    const int ra = a0 + wr * 32 + mi * 8 + gq, rc = c0 + ni * 8 + 2 * tq + e;
-                    const unsigned long long bits = (unsigned long long)__double_as_longlong(acc[mi][ni][e]);
-                    const unsigned long long packed = ((unsigned long long)ra << (2 * kRankBits)) |
-                                                      ((unsigned long long)j << kRankBits) | (unsigned long long)rc;
-                    bool q = ((keep >> f) & 1u) && ra < j && rc < n;
-                    if (q && A.mode == 1) q = bits > A.v || packed <= A.rhi;
-                    if (q && A.n_known > 0) q = !is_known(A.known, A.n_known, packed);
-                    int bin = kPredBins;
-                    if (q) {
-                        if (A.mode == 0) {
-                            if (bits <= A.hi) bin = (int)((A.hi - bits) >> A.shift);
-                        } else if (bits == A.v && packed >= A.rlo) {
-                            bin = (int)((packed - A.rlo) >> A.shift);
-                        }
-                        atomicAdd(sh_hist + bin, 1u);
-                    }
-                    const unsigned m = __ballot_sync(0xffffffffu, q);
-                    if (m == 0) continue;
-                    unsigned long long base = 0;
-                    if (lane == __ffs(m) - 1) base = atomicAdd(A.counter, (unsigned long long)__popc(m));
-                    base = __shfl_sync(0xffffffffu, base, __ffs(m) - 1);
-                    if (q) {
-                        const unsigned long long idx = base + __popc(m & ((1u << lane) - 1u));
-                        if ((long long)idx < A.cap) {
-                            A.out_bits[idx] = bits;
-                            A.out_packed[idx] = packed;
-                        }
-                    }
-                }
+                dmma_block(acc, Qw, qs, A.tcat + (long long)(c0 + gq) * SKP + tq, SKP);
+                select_block(acc, A.sel, tm, lane, a0 + wr * 32 + gq, c0 + 2 * tq, A.known, A.n_known, sh_hist, A.counter,
+                             A.out_bits, A.out_packed, A.cap);
             }
         }
         // shared bins are 32-bit: flush before they could overflow
         since_flush += (double)rows * n_c;
         if (since_flush > 2.0e9) {
             __syncthreads();
-            for (int i = tid; i <= kPredBins; i += kPredThreads) {
-                if (sh_hist[i]) atomicAdd(A.hist + i, (unsigned long long)sh_hist[i]);
-                sh_hist[i] = 0;
-            }
+            flush_hist(sh_hist, A.hist);
             since_flush = 0.0;
         }
     }
-    for (int i = tid; i <= kPredBins; i += kPredThreads)
-        if (sh_hist[i]) atomicAdd(A.hist + i, (unsigned long long)sh_hist[i]);
+    flush_hist(sh_hist, A.hist);
 }
+
+// ---- per query (tip_top_triplets_per_gene) ----
+// The pairs x < y of a query of rank r (both != r) fall into three regions by the query's slot; g = 0: x < y < r (slot c),
+// g = 1: x < r < y (slot b), g = 2: r < x < y (slot a).  In each the score is th_x^T M_g th_y with, per set,
+//     M_0[u][v] = sum_w th_q[w] p[u][v][w][1],   M_1[u][w] = sum_v th_q[v] p[u][v][w][1] (= W),   M_2[v][w] = sum_u th_q[u] p[u][v][w][1]
+// Regions 0 and 2 are triangles (y > x); region 1 is the rectangle tip_predict_pass_kernel sweeps for middle rank r.
+
+// tcat as tip_predict_prep_kernel writes it, and Mq[query][g][s][K][K]
+__global__ void tip_query_prep_kernel(int S, int P, int K, int n, int n_pad, int SKP, int n_query, const double *__restrict__ theta,
+                                      const double *__restrict__ p, const int32_t *__restrict__ cand,
+                                      const int32_t *__restrict__ qrank, double *__restrict__ tcat, double *__restrict__ Mq)
+{
+    const long long n_t = (long long)n_pad * SKP, KK = (long long)K * K, n_m = (long long)n_query * 3 * S * KK;
+    for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < n_t + n_m; t += (long long)gridDim.x * blockDim.x) {
+        if (t < n_t) {
+            tcat[t] = tcat_entry(t, S, P, K, n, SKP, theta, cand);
+        } else {
+            const long long u = t - n_t;
+            const int qi = (int)(u / (3 * S * KK)), g = (int)(u / (S * KK) % 3), s = (int)(u / KK % S);
+            const int x = (int)(u % KK) / K, z = (int)(u % KK) % K;
+            const double *th = theta + ((long long)s * P + cand[qrank[qi]]) * K;
+            const double *ps = p + (long long)s * 2 * K * K * K;
+            // index of p[.][.][.][1] with the query's group y in slot (2 - g) and (x, z) in the other two, in order
+            const long long step = g == 0 ? 1 : g == 1 ? K : KK;
+            const long long base = g == 0 ? ((long long)x * K + z) * K : g == 1 ? (long long)x * KK + z : (long long)x * K + z;
+            double acc = 0.0;
+            for (int y = 0; y < K; ++y) acc = fma(th[y], ps[(base + y * step) * 2 + 1], acc);
+            Mq[u] = acc;
+        }
+    }
+}
+
+// T[s] = bits of the largest row sum of theta_s over the candidates (T zeroed by the caller)
+__global__ void tip_query_rowsum_kernel(int n, int S, int K, int SKP, const double *__restrict__ tcat, unsigned long long *T)
+{
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n) return;
+    for (int s = 0; s < S; ++s) {
+        double sum = 0.0;
+        for (int k = 0; k < K; ++k) sum += tcat[(long long)r * SKP + s * K + k];
+        atomicMax(T + s, (unsigned long long)__double_as_longlong(sum));
+    }
+}
+
+// bound[q] >= every sum over the sets of a query's scores (non-negative parameters): th_x^T M th_y <= max(M) |th_x|_1 |th_y|_1
+__global__ void tip_query_bound_kernel(int n_query, int S, int K, const double *__restrict__ Mq, const unsigned long long *T,
+                                       double *__restrict__ bound)
+{
+    const int qi = blockIdx.x * blockDim.x + threadIdx.x;
+    if (qi >= n_query) return;
+    const long long KK = (long long)K * K;
+    double best = 0.0;
+    for (int g = 0; g < 3; ++g) {
+        double b = 0.0;
+        for (int s = 0; s < S; ++s) {
+            const double *m = Mq + (((long long)qi * 3 + g) * S + s) * KK;
+            double mx = 0.0;
+            for (long long e = 0; e < KK; ++e) mx = fmax(mx, m[e]);
+            const double t = __longlong_as_double((long long)T[s]);
+            b += mx * t * t;
+        }
+        best = fmax(best, b);
+    }
+    bound[qi] = best;
+}
+
+// best[q] = bits of the largest of n_samp scores (summed over the sets) of deterministic random pairs of query q; with
+// about pairs / n_samp scores above it, it places the query's first threshold (best zeroed by the caller)
+__global__ void tip_query_sample_kernel(int n, int S, int K, int SKP, int n_query, int n_samp, const int32_t *__restrict__ qrank,
+                                        const double *__restrict__ tcat, const double *__restrict__ Mq,
+                                        unsigned long long *__restrict__ best)
+{
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= (long long)n_query * n_samp) return;
+    const int qi = (int)(t / n_samp), r = qrank[qi];
+    unsigned long long h = splitmix64((unsigned long long)t * 3 + 0x7654321ull);
+    int x, y;
+    do {
+        h = splitmix64(h);
+        x = (int)(h % (unsigned long long)n);
+        h = splitmix64(h);
+        y = (int)(h % (unsigned long long)n);
+    } while (x == y || x == r || y == r);
+    if (x > y) { const int z = x; x = y; y = z; }
+    const int g = y < r ? 0 : x < r ? 1 : 2;
+    const long long KK = (long long)K * K;
+    double acc = 0.0;
+    for (int s = 0; s < S; ++s) {
+        const double *m = Mq + (((long long)qi * 3 + g) * S + s) * KK;
+        for (int u = 0; u < K; ++u) {
+            double q = 0.0;
+            for (int v = 0; v < K; ++v) q = fma(m[u * K + v], tcat[(long long)y * SKP + s * K + v], q);
+            acc = fma(tcat[(long long)x * SKP + s * K + u], q, acc);
+        }
+    }
+    atomicMax(best + qi, (unsigned long long)__double_as_longlong(acc));
+}
+
+// tiles of the three regions of the query of rank r: tc (g = 0, rows 0 .. r-2), tb (g = 1, rows 0 .. r-1, only when
+// r <= n-2), ta (g = 2, rows r+1 .. n-2)
+__host__ __device__ inline void query_tiles(int n, int r, int &tc, int &tb, int &ta)
+{
+    tc = (max(r - 1, 0) + kPredRows - 1) / kPredRows;
+    tb = r <= n - 2 ? (r + kPredRows - 1) / kPredRows : 0;
+    ta = (max(n - 2 - r, 0) + kPredRows - 1) / kPredRows;
+}
+
+struct QueryPassArgs {
+    int n, S, K, SK, SKP;
+    const double *tcat;               // [n_pad][SKP]
+    const double *Mq;                 // [n_query][3][S][K][K]
+    const int32_t *qrank;             // [n_query]
+    const int32_t *active;            // [n_active] queries this pass sweeps, ascending
+    const long long *item_start;      // [n_active + 1] first work item of each
+    long long n_items;
+    const Sel *sel;                   // [n_query]
+    const unsigned long long *known;  // sorted packed rank triples
+    long long n_known;
+    int n_active;
+    unsigned long long *counter;      // [n_query] entries kept
+    unsigned long long *cursor;       // work-item cursor
+    unsigned long long *hist;         // [n_active][kPredBins + 1]
+    unsigned long long *out_bits, *out_packed;   // [n_query][cap]
+    long long cap;
+};
+
+// work items are (query, region, 64-row tile), query-major, so a CTA flushes its shared histogram when the query changes
+__global__ void __launch_bounds__(kPredThreads, 4) tip_query_pass_kernel(QueryPassArgs A)
+{
+    extern __shared__ __align__(16) unsigned char smem[];
+    const int qs = q_stride(A.SKP);
+    double *Q = reinterpret_cast<double *>(smem);                                   // [64][qs]
+    unsigned *sh_hist = reinterpret_cast<unsigned *>(Q + (size_t)kPredRows * qs);  // [kPredBins + 1]
+    __shared__ long long sh_item;
+    __shared__ Sel sh_sel;       // the item's threshold and geometry: CTA-uniform, read from shared memory in the epilogue
+    __shared__ TileMap sh_tm;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int wr = warp & 1, wc = warp >> 1;
+    const int gq = lane >> 2, tq = lane & 3;
+    for (int i = tid; i <= kPredBins; i += kPredThreads) sh_hist[i] = 0;
+    double since_flush = 0.0;   // as in tip_predict_pass_kernel
+    int cur = -1;               // active slot whose entries sh_hist holds (CTA-uniform)
+    const int n = A.n, SKP = A.SKP, K = A.K;
+    const long long KK = (long long)K * K;
+
+    for (;;) {
+        __syncthreads();   // Q, sh_item and sh_hist of the previous item are no longer used
+        if (tid == 0) sh_item = (long long)atomicAdd(A.cursor, 1ull);
+        __syncthreads();
+        const long long item = sh_item;
+        if (item >= A.n_items) break;
+        int al = 0, ah = A.n_active - 1;
+        while (al < ah) {
+            const int mid = (al + ah + 1) >> 1;
+            if (A.item_start[mid] <= item) al = mid; else ah = mid - 1;
+        }
+        if (al != cur || since_flush > 2.0e9) {
+            if (cur >= 0) flush_hist(sh_hist, A.hist + (long long)cur * (kPredBins + 1));
+            cur = al;
+            since_flush = 0.0;
+        }
+        const int qi = A.active[al], r = A.qrank[qi];
+        int tc, tb, ta;
+        query_tiles(n, r, tc, tb, ta);
+        int t = (int)(item - A.item_start[al]);
+        int g, a0, col0;
+        TileMap tm;
+        if (t < tc) {
+            g = 0; a0 = t * kPredRows; col0 = a0 + 1;
+            tm = TileMap{r - 1, r, true, 2 * kRankBits, kRankBits, (unsigned long long)r};
+        } else if ((t -= tc) < tb) {
+            g = 1; a0 = t * kPredRows; col0 = r + 1;
+            tm = TileMap{r, n, false, 2 * kRankBits, 0, (unsigned long long)r << kRankBits};
+        } else {
+            t -= tb;
+            g = 2; a0 = r + 1 + t * kPredRows; col0 = a0 + 1;
+            tm = TileMap{n - 1, n, true, kRankBits, 0, (unsigned long long)r << (2 * kRankBits)};
+        }
+        const int rows = min(kPredRows, tm.row_end - a0);
+        if (tid == 0) {
+            sh_sel = A.sel[qi];
+            sh_tm = tm;
+        }
+
+        form_q_tile(Q, qs, A.tcat, SKP, A.SK, K, a0, rows, A.Mq + ((long long)qi * 3 + g) * A.S * KK, KK);
+        __syncthreads();
+
+        if (wr * 32 < rows) {
+            const double *Qw = Q + (wr * 32 + gq) * qs + tq;
+            for (int c0 = col0 + wc * 32; c0 < tm.col_end; c0 += 64) {
+                double acc[4][4][2];
+                dmma_block(acc, Qw, qs, A.tcat + (long long)(c0 + gq) * SKP + tq, SKP);
+                select_block(acc, sh_sel, sh_tm, lane, a0 + wr * 32 + gq, c0 + 2 * tq, A.known, A.n_known, sh_hist, A.counter + qi,
+                             A.out_bits + (long long)qi * A.cap, A.out_packed + (long long)qi * A.cap, A.cap);
+            }
+        }
+        since_flush += (double)rows * (tm.col_end - col0);
+    }
+    if (cur >= 0) flush_hist(sh_hist, A.hist + (long long)cur * (kPredBins + 1));
+}
+
+__global__ void tip_query_finish_kernel(int n_query, int N, long long cap, int S, const long long *__restrict__ m_rows,
+                                        const unsigned long long *__restrict__ bits, const unsigned long long *__restrict__ packed,
+                                        const int32_t *__restrict__ cand, int32_t *__restrict__ out_ids, double *__restrict__ out_scores)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (long long)n_query * N) return;
+    const long long qi = i / N, t = i % N;
+    if (t >= m_rows[qi]) return;
+    const long long src = qi * cap + t;
+    const unsigned long long pk = packed[src], mask = (1ull << kRankBits) - 1;
+    out_ids[3 * i + 0] = cand[(pk >> (2 * kRankBits)) & mask];
+    out_ids[3 * i + 1] = cand[(pk >> kRankBits) & mask];
+    out_ids[3 * i + 2] = cand[pk & mask];
+    out_scores[i] = __longlong_as_double((long long)bits[src]) / (double)S;
+}
+
 
 __global__ void tip_predict_finish_kernel(long long m, int S, const unsigned long long *__restrict__ bits,
                                           const unsigned long long *__restrict__ packed, const int32_t *__restrict__ cand,
@@ -342,6 +611,55 @@ int shift_for(unsigned long long span)
     int s = 0;
     while (s < 64 && (span >> s) >= (unsigned long long)kPredBins) ++s;
     return s;
+}
+
+// One narrowing step after a pass that kept more than cap entries, at least M of them needed: walk the pass's histogram in
+// result order to the bin where the count reaches M and set the next pass's threshold from it.  Under ties (a bin one score
+// wide that still holds too many) the selection continues on the packed ranks.  false: the histogram does not reach M.
+bool narrow(Sel &sel, long long M, long long cap, const unsigned long long *hist, unsigned long long max_packed)
+{
+    long long cum = (long long)hist[kPredBins];
+    if (sel.mode == 0 && cum >= M) {
+        // everything needed lies above the histogram's range
+        sel.lo = sel.hi + 1;
+        sel.hi = kInfBits;
+        sel.shift = shift_for(sel.hi - sel.lo);
+        return true;
+    }
+    int b = 0;
+    for (; b < kPredBins; ++b) {
+        cum += (long long)hist[b];
+        if (cum >= M) break;
+    }
+    if (b == kPredBins) return false;
+    if (sel.mode == 0) {
+        const unsigned long long top = sel.hi - ((unsigned long long)b << sel.shift);
+        const unsigned long long width = (sel.shift >= 64) ? ~0ull : (1ull << sel.shift);
+        const unsigned long long bottom = (top - sel.lo + 1 <= width) ? sel.lo : top - width + 1;
+        if (cum <= cap) {
+            sel.lo = bottom;
+        } else if (bottom == top) {
+            // every remaining candidate has the same score: continue on the packed ranks
+            sel.mode = 1;
+            sel.v = top;
+            sel.rlo = 0;
+            sel.rhi = max_packed;
+        } else {
+            sel.lo = bottom;
+            sel.hi = top;
+        }
+    } else {
+        const unsigned long long lo_b = sel.rlo + ((unsigned long long)b << sel.shift);
+        const unsigned long long hi_b = std::min(sel.rhi, lo_b + ((sel.shift >= 64) ? ~0ull : (1ull << sel.shift) - 1));
+        if (cum <= cap) {
+            sel.rhi = hi_b;
+        } else {
+            sel.rlo = lo_b;
+            sel.rhi = hi_b;
+        }
+    }
+    sel.shift = sel.mode == 0 ? shift_for(sel.hi - sel.lo) : shift_for(sel.rhi - sel.rlo);
+    return true;
 }
 
 }  // namespace
@@ -433,9 +751,9 @@ extern "C" int tip_top_triplets(int P, int K, int S, const double *d_theta, cons
     };
 
     // first threshold: everything when it fits the buffer, else a quantile of a deterministic sample
-    A.mode = 0;
-    A.hi = kInfBits;
-    A.lo = 0;
+    A.sel.mode = 0;
+    A.sel.hi = kInfBits;
+    A.sel.lo = 0;
     long long samp_idx = -1;
     unsigned long long *samp_sorted = samp2;
     auto sample_at = [&](long long idx, unsigned long long *v) -> int {
@@ -451,13 +769,13 @@ extern "C" int tip_top_triplets(int P, int K, int S, const double *d_theta, cons
         // expected survivors ~2 M: well inside the buffer (4 N + 2^18)
         samp_idx = (long long)((double)(2 * M) / (double)total * kPredSample);
         if (samp_idx < kPredSample) {
-            int rc = sample_at(samp_idx, &A.lo);
+            int rc = sample_at(samp_idx, &A.sel.lo);
             if (rc) return rc;
-            rc = sample_at(0, &A.hi);
+            rc = sample_at(0, &A.sel.hi);
             if (rc) return rc;
         }
     }
-    A.shift = shift_for(A.hi - A.lo);
+    A.sel.shift = shift_for(A.sel.hi - A.sel.lo);
 
     const unsigned long long max_packed = ((unsigned long long)(n - 1) << (2 * kRankBits)) | ((unsigned long long)(n - 1) << kRankBits) |
                                           (unsigned long long)(n - 1);
@@ -469,60 +787,21 @@ extern "C" int tip_top_triplets(int P, int K, int S, const double *d_theta, cons
         const long long C = (long long)h_cnt[0];
         if (C >= M && C <= L.cap) { kept = C; break; }
         if (C < M) {
-            if (A.mode == 0 && A.lo == 0) { M = C; kept = C; break; }   // every candidate is in the buffer
+            if (A.sel.mode == 0 && A.sel.lo == 0) { M = C; kept = C; break; }   // every candidate is in the buffer
             // the sample placed the threshold too high: lower it to a sample value below it, or to zero
-            unsigned long long v = A.lo;
-            while (v >= A.lo) {
+            unsigned long long v = A.sel.lo;
+            while (v >= A.sel.lo) {
                 samp_idx = samp_idx < 0 ? 0 : samp_idx * 4 + 16;
                 if (samp_idx >= kPredSample) { v = 0; break; }
                 if ((rc = sample_at(samp_idx, &v))) return rc;
             }
-            A.lo = v;
-            A.shift = shift_for(A.hi - A.lo);
+            A.sel.lo = v;
+            A.sel.shift = shift_for(A.sel.hi - A.sel.lo);
             continue;
         }
-        // too many for the buffer: walk the histogram in result order to the bin where the count reaches M
-        long long cum = (long long)h_hist[kPredBins];
-        if (A.mode == 0 && cum >= M) {
-            // everything needed lies above the histogram's range
-            A.lo = A.hi + 1;
-            A.hi = kInfBits;
-            A.shift = shift_for(A.hi - A.lo);
-            continue;
-        }
-        int b = 0;
-        for (; b < kPredBins; ++b) {
-            cum += (long long)h_hist[b];
-            if (cum >= M) break;
-        }
-        TIP_REQUIRE(b < kPredBins, "tip_top_triplets: histogram does not reach N (internal error)");
-        if (A.mode == 0) {
-            const unsigned long long top = A.hi - ((unsigned long long)b << A.shift);
-            const unsigned long long width = (A.shift >= 64) ? ~0ull : (1ull << A.shift);
-            const unsigned long long bottom = (top - A.lo + 1 <= width) ? A.lo : top - width + 1;
-            if (cum <= L.cap) {
-                A.lo = bottom;
-            } else if (bottom == top) {
-                // every remaining candidate has the same score: continue on the packed ranks
-                A.mode = 1;
-                A.v = top;
-                A.rlo = 0;
-                A.rhi = max_packed;
-            } else {
-                A.lo = bottom;
-                A.hi = top;
-            }
-        } else {
-            const unsigned long long lo_b = A.rlo + ((unsigned long long)b << A.shift);
-            const unsigned long long hi_b = std::min(A.rhi, lo_b + ((A.shift >= 64) ? ~0ull : (1ull << A.shift) - 1));
-            if (cum <= L.cap) {
-                A.rhi = hi_b;
-            } else {
-                A.rlo = lo_b;
-                A.rhi = hi_b;
-            }
-        }
-        A.shift = A.mode == 0 ? shift_for(A.hi - A.lo) : shift_for(A.rhi - A.rlo);
+        // too many for the buffer
+        TIP_REQUIRE(narrow(A.sel, M, L.cap, h_hist.data(), max_packed),
+                    "tip_top_triplets: histogram does not reach N (internal error)");
     }
     TIP_REQUIRE(kept >= 0, "tip_top_triplets: the threshold did not converge (internal error)");
     if (M <= 0) return 0;
@@ -539,3 +818,267 @@ extern "C" int tip_top_triplets(int P, int K, int S, const double *d_theta, cons
 }
 
 extern "C" int tip_top_triplets_last_passes(void) { return g_last_passes; }
+
+// ---- tip_top_triplets_per_gene ----
+namespace tip {
+namespace {
+
+constexpr long long kQueryMaxRows = 1ll << 24;   // n_query * N
+
+long long n_pairs(long long m) { return m < 2 ? 0 : m * (m - 1) / 2; }
+
+// buffer of a query: room for 4 N survivors plus slack, never more than its pairs
+long long query_capacity(int n, long long N) { return std::max(1ll, std::min(n_pairs(n - 1), 4 * N + 256)); }
+
+struct QueryLayout {
+    size_t o_tcat, o_M, o_T, o_bound, o_best, o_sel, o_active, o_start, o_cnt, o_mrows, o_beg, o_end, o_hist, o_bits, o_pk, o_bits2,
+        o_pk2, o_cub, cub_bytes, total;
+    int n_pad, SKP;
+    long long cap;
+};
+
+QueryLayout query_layout(int n, int n_query, int K, int S, long long N)
+{
+    QueryLayout L{};
+    L.n_pad = (n + 63) / 64 * 64 + 64;
+    L.SKP = (S * K + 3) / 4 * 4;
+    L.cap = query_capacity(n, N);
+    const long long items = (long long)n_query * L.cap;
+    size_t cb1 = 0, cb2 = 0;
+    cub::DeviceSegmentedSort::StableSortPairs(nullptr, cb1, (const unsigned long long *)nullptr, (unsigned long long *)nullptr,
+                                              (const unsigned long long *)nullptr, (unsigned long long *)nullptr, (int)items,
+                                              n_query, (const int *)nullptr, (const int *)nullptr, (cudaStream_t)0);
+    cub::DeviceSegmentedSort::StableSortPairsDescending(nullptr, cb2, (const unsigned long long *)nullptr,
+                                                        (unsigned long long *)nullptr, (const unsigned long long *)nullptr,
+                                                        (unsigned long long *)nullptr, (int)items, n_query, (const int *)nullptr,
+                                                        (const int *)nullptr, (cudaStream_t)0);
+    L.cub_bytes = std::max(cb1, cb2);
+    const size_t nq = (size_t)n_query;
+    size_t off = 0;
+    L.o_tcat = off;   off += a256((size_t)L.n_pad * L.SKP * 8);
+    L.o_M = off;      off += a256(nq * 3 * S * K * K * 8);
+    L.o_T = off;      off += a256((size_t)S * 8);
+    L.o_bound = off;  off += a256(nq * 8);
+    L.o_best = off;   off += a256(nq * 8);
+    L.o_sel = off;    off += a256(nq * sizeof(Sel));
+    L.o_active = off; off += a256(nq * 4);
+    L.o_start = off;  off += a256((nq + 1) * 8);
+    L.o_cnt = off;    off += a256((nq + 1) * 8);
+    L.o_mrows = off;  off += a256(nq * 8);
+    L.o_beg = off;    off += a256(nq * 4);
+    L.o_end = off;    off += a256(nq * 4);
+    L.o_hist = off;   off += a256(nq * (kPredBins + 1) * 8);
+    L.o_bits = off;   off += a256((size_t)items * 8);
+    L.o_pk = off;     off += a256((size_t)items * 8);
+    L.o_bits2 = off;  off += a256((size_t)items * 8);
+    L.o_pk2 = off;    off += a256((size_t)items * 8);
+    L.o_cub = off;    off += a256(L.cub_bytes);
+    L.total = off + 256;
+    return L;
+}
+
+}  // namespace
+}  // namespace tip
+
+static thread_local int g_last_query_passes = 0;
+
+static bool per_gene_args_ok(int n_cand, int n_query, int K, int S, int64_t n_known, int64_t N)
+{
+    return predict_args_ok(n_cand, K, S, n_known, N) && n_query >= 0 && n_query <= n_cand &&
+           (long long)n_query * N <= kQueryMaxRows;
+}
+
+extern "C" int tip_top_triplets_per_gene_workspace_bytes(int n_cand, int n_query, int K, int S, int64_t n_known, int64_t N,
+                                                         size_t *bytes)
+{
+    TIP_REQUIRE(bytes != nullptr && per_gene_args_ok(n_cand, n_query, K, S, n_known, N),
+                "tip_top_triplets_per_gene_workspace_bytes: bad arguments (n_cand <= 2^21, 0 <= n_query <= n_cand, "
+                "1 <= K <= %d, S >= 1, S*K <= %d, N >= 0, n_query*N <= 2^24)", TIP_MAX_K, kPredMaxSK);
+    *bytes = query_layout(n_cand, n_query, K, S, N).total;
+    return 0;
+}
+
+extern "C" int tip_top_triplets_per_gene(int P, int K, int S, const double *d_theta, const double *d_p, const int32_t *d_cand,
+                                         int n_cand, const int32_t *d_query_ranks, int n_query, const uint64_t *d_known,
+                                         int64_t n_known, int64_t N, void *d_ws, size_t ws_bytes, int32_t *d_out_ids,
+                                         double *d_out_scores, int64_t *h_n_out, void *stream)
+{
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    TIP_REQUIRE(P > 0 && n_cand <= P && per_gene_args_ok(n_cand, n_query, K, S, n_known, N) && (h_n_out || n_query == 0),
+                "tip_top_triplets_per_gene: bad arguments (P > 0, n_cand <= min(P, 2^21), 0 <= n_query <= n_cand, "
+                "1 <= K <= %d, S >= 1, S*K <= %d, n_known >= 0, N >= 0, n_query*N <= 2^24)", TIP_MAX_K, kPredMaxSK);
+    TIP_REQUIRE(d_theta && d_p && (d_cand || n_cand == 0) && (d_query_ranks || n_query == 0) && (d_known || n_known == 0) &&
+                    (N == 0 || n_query == 0 || (d_out_ids && d_out_scores)),
+                "tip_top_triplets_per_gene: null pointer");
+    g_last_query_passes = 0;
+    if (n_query == 0) return 0;
+    const int n = n_cand, nq = n_query;
+    // the query ranks are checked on the host before any device work
+    std::vector<int32_t> qr(nq);
+    TIP_CHECK_CUDA(cudaMemcpyAsync(qr.data(), d_query_ranks, (size_t)nq * 4, cudaMemcpyDeviceToHost, st));
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    {
+        std::vector<char> seen(n, 0);
+        for (int i = 0; i < nq; ++i) {
+            TIP_REQUIRE(qr[i] >= 0 && qr[i] < n, "tip_top_triplets_per_gene: query rank %d of query %d is not in [0, %d)", qr[i],
+                        i, n);
+            TIP_REQUIRE(!seen[qr[i]], "tip_top_triplets_per_gene: query rank %d appears twice", qr[i]);
+            seen[qr[i]] = 1;
+        }
+    }
+    for (int i = 0; i < nq; ++i) h_n_out[i] = 0;
+    const long long pairs = n_pairs(n - 1);
+    if (N == 0 || pairs == 0) return 0;
+    const QueryLayout L = query_layout(n, nq, K, S, N);
+    // sample size per query: about 4 N of its pairs score above the sample's best, at most 4096 samples
+    const int n_samp = (int)std::max(1ll, std::min(4096ll, pairs / (4 * std::min<long long>(N, pairs))));
+    TIP_REQUIRE(d_ws != nullptr && ws_bytes >= L.total, "tip_top_triplets_per_gene: workspace too small (%zu < %zu)", ws_bytes,
+                L.total);
+    char *base = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(d_ws) + 255) / 256 * 256);
+    double *tcat = reinterpret_cast<double *>(base + L.o_tcat), *Mq = reinterpret_cast<double *>(base + L.o_M);
+    auto *T = reinterpret_cast<unsigned long long *>(base + L.o_T);
+    double *bound = reinterpret_cast<double *>(base + L.o_bound);
+    auto *best = reinterpret_cast<unsigned long long *>(base + L.o_best);
+    Sel *d_sel = reinterpret_cast<Sel *>(base + L.o_sel);
+    auto *d_active = reinterpret_cast<int32_t *>(base + L.o_active);
+    auto *d_start = reinterpret_cast<long long *>(base + L.o_start);
+    auto *cnt = reinterpret_cast<unsigned long long *>(base + L.o_cnt);
+    auto *d_mrows = reinterpret_cast<long long *>(base + L.o_mrows);
+    auto *d_beg = reinterpret_cast<int *>(base + L.o_beg), *d_end = reinterpret_cast<int *>(base + L.o_end);
+    auto *hist = reinterpret_cast<unsigned long long *>(base + L.o_hist);
+    auto *bits = reinterpret_cast<unsigned long long *>(base + L.o_bits), *pk = reinterpret_cast<unsigned long long *>(base + L.o_pk);
+    auto *bits2 = reinterpret_cast<unsigned long long *>(base + L.o_bits2), *pk2 = reinterpret_cast<unsigned long long *>(base + L.o_pk2);
+    void *cub_tmp = base + L.o_cub;
+
+    {
+        const long long work = (long long)L.n_pad * L.SKP + (long long)nq * 3 * S * K * K;
+        const long long want = (work + 255) / 256;
+        tip_query_prep_kernel<<<(int)std::min<long long>(want, (long long)sm_count() * 16), 256, 0, st>>>(
+            S, P, K, n, L.n_pad, L.SKP, nq, d_theta, d_p, d_cand, d_query_ranks, tcat, Mq);
+        TIP_CHECK_CUDA(cudaGetLastError());
+        TIP_CHECK_CUDA(cudaMemsetAsync(T, 0, (size_t)S * 8, st));
+        tip_query_rowsum_kernel<<<(n + 255) / 256, 256, 0, st>>>(n, S, K, L.SKP, tcat, T);
+        TIP_CHECK_CUDA(cudaGetLastError());
+        tip_query_bound_kernel<<<(nq + 127) / 128, 128, 0, st>>>(nq, S, K, Mq, T, bound);
+        TIP_CHECK_CUDA(cudaGetLastError());
+        TIP_CHECK_CUDA(cudaMemsetAsync(best, 0, (size_t)nq * 8, st));
+        if (pairs > L.cap) {
+            const long long work = (long long)nq * n_samp;
+            tip_query_sample_kernel<<<(int)((work + 255) / 256), 256, 0, st>>>(n, S, K, L.SKP, nq, n_samp, d_query_ranks, tcat,
+                                                                                 Mq, best);
+            TIP_CHECK_CUDA(cudaGetLastError());
+        }
+    }
+    std::vector<double> h_bound(nq);
+    std::vector<unsigned long long> h_best(nq);
+    TIP_CHECK_CUDA(cudaMemcpyAsync(h_bound.data(), bound, (size_t)nq * 8, cudaMemcpyDeviceToHost, st));
+    TIP_CHECK_CUDA(cudaMemcpyAsync(h_best.data(), best, (size_t)nq * 8, cudaMemcpyDeviceToHost, st));
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+
+    const size_t smem = (size_t)kPredRows * q_stride(L.SKP) * 8 + (size_t)(kPredBins + 1) * 4;
+    static int smem_set = 0;
+    if ((int)smem > smem_set && smem > 48 * 1024) {
+        TIP_CHECK_CUDA(cudaFuncSetAttribute(tip_query_pass_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        smem_set = (int)smem;
+    }
+    int per_sm = 0;
+    TIP_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tip_query_pass_kernel, kPredThreads, smem));
+    TIP_REQUIRE(per_sm > 0, "tip_top_triplets_per_gene: S*K = %d does not fit one block's shared memory", S * K);
+
+    // first threshold of each query: everything when its pairs fit its buffer; else the best score of its sample, with the
+    // histogram spanning up to an upper bound of its scores.  Neither has to be right: entries above the bound are counted
+    // ahead of the range, and a threshold that keeps fewer than N moves down in a later pass; they set how many passes it
+    // takes, not the result
+    std::vector<Sel> sel(nq);
+    std::vector<long long> M(nq), kept(nq, -1);
+    for (int i = 0; i < nq; ++i) {
+        Sel &q = sel[i];
+        q = Sel{};
+        q.hi = kInfBits;
+        M[i] = std::min<long long>(N, pairs);
+        if (pairs > L.cap) {
+            const double hb = h_bound[i] * (1.0 + 1e-9);
+            q.hi = std::min<unsigned long long>((unsigned long long)__builtin_bit_cast(long long, hb), kInfBits);
+            q.lo = std::min(h_best[i], q.hi);
+        }
+        q.shift = shift_for(q.hi - q.lo);
+    }
+    const unsigned long long max_packed = ((unsigned long long)(n - 1) << (2 * kRankBits)) | ((unsigned long long)(n - 1) << kRankBits) |
+                                          (unsigned long long)(n - 1);
+    QueryPassArgs A{};
+    A.n = n; A.S = S; A.K = K; A.SK = S * K; A.SKP = L.SKP;
+    A.tcat = tcat; A.Mq = Mq; A.qrank = d_query_ranks; A.active = d_active; A.item_start = d_start; A.sel = d_sel;
+    A.known = reinterpret_cast<const unsigned long long *>(d_known); A.n_known = n_known;
+    A.counter = cnt; A.cursor = cnt + nq; A.hist = hist; A.out_bits = bits; A.out_packed = pk; A.cap = L.cap;
+    std::vector<int32_t> active;
+    std::vector<long long> start;
+    std::vector<unsigned long long> h_cnt(nq), h_hist;
+    for (int pass = 0;; ++pass) {
+        active.clear();
+        start.assign(1, 0);
+        for (int i = 0; i < nq; ++i) {
+            if (kept[i] >= 0) continue;
+            int tc, tb, ta;
+            query_tiles(n, qr[i], tc, tb, ta);
+            active.push_back(i);
+            start.push_back(start.back() + tc + tb + ta);
+        }
+        if (active.empty()) break;
+        TIP_REQUIRE(pass < 200, "tip_top_triplets_per_gene: the threshold did not converge (internal error)");
+        const int na = (int)active.size();
+        A.n_active = na;
+        A.n_items = start.back();
+        TIP_CHECK_CUDA(cudaMemcpyAsync(d_sel, sel.data(), (size_t)nq * sizeof(Sel), cudaMemcpyHostToDevice, st));
+        TIP_CHECK_CUDA(cudaMemcpyAsync(d_active, active.data(), (size_t)na * 4, cudaMemcpyHostToDevice, st));
+        TIP_CHECK_CUDA(cudaMemcpyAsync(d_start, start.data(), (size_t)(na + 1) * 8, cudaMemcpyHostToDevice, st));
+        TIP_CHECK_CUDA(cudaMemsetAsync(cnt, 0, (size_t)(nq + 1) * 8, st));
+        TIP_CHECK_CUDA(cudaMemsetAsync(hist, 0, (size_t)na * (kPredBins + 1) * 8, st));
+        const long long grid_l = std::min<long long>((long long)sm_count() * per_sm, A.n_items);
+        tip_query_pass_kernel<<<(int)grid_l, kPredThreads, smem, st>>>(A);
+        TIP_CHECK_CUDA(cudaGetLastError());
+        h_hist.resize((size_t)na * (kPredBins + 1));
+        TIP_CHECK_CUDA(cudaMemcpyAsync(h_cnt.data(), cnt, (size_t)nq * 8, cudaMemcpyDeviceToHost, st));
+        TIP_CHECK_CUDA(cudaMemcpyAsync(h_hist.data(), hist, h_hist.size() * 8, cudaMemcpyDeviceToHost, st));
+        TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+        ++g_last_query_passes;
+        for (int a = 0; a < na; ++a) {
+            const int i = active[a];
+            Sel &q = sel[i];
+            const long long C = (long long)h_cnt[i];
+            if (C >= M[i] && C <= L.cap) { kept[i] = C; continue; }
+            if (C < M[i]) {
+                if (q.mode == 0 && q.lo == 0) { M[i] = C; kept[i] = C; continue; }   // every candidate is in the buffer
+                // the threshold was too high: move it 16 binades down (to zero below the normal range)
+                q.lo = q.lo > (16ull << 52) ? q.lo - (16ull << 52) : 0;
+                q.shift = shift_for(q.hi - q.lo);
+                continue;
+            }
+            TIP_REQUIRE(narrow(q, M[i], L.cap, h_hist.data() + (size_t)a * (kPredBins + 1), max_packed),
+                        "tip_top_triplets_per_gene: histogram does not reach N (internal error)");
+        }
+    }
+    // order: per query, packed ranks ascending, then (stable) score descending
+    std::vector<int> beg(nq), end(nq);
+    for (int i = 0; i < nq; ++i) {
+        beg[i] = (int)((long long)i * L.cap);
+        end[i] = beg[i] + (int)kept[i];
+    }
+    TIP_CHECK_CUDA(cudaMemcpyAsync(d_beg, beg.data(), (size_t)nq * 4, cudaMemcpyHostToDevice, st));
+    TIP_CHECK_CUDA(cudaMemcpyAsync(d_end, end.data(), (size_t)nq * 4, cudaMemcpyHostToDevice, st));
+    TIP_CHECK_CUDA(cudaMemcpyAsync(d_mrows, M.data(), (size_t)nq * 8, cudaMemcpyHostToDevice, st));
+    const int items = (int)((long long)nq * L.cap);
+    size_t cb = L.cub_bytes;
+    TIP_CHECK_CUDA(cub::DeviceSegmentedSort::StableSortPairs(cub_tmp, cb, pk, pk2, bits, bits2, items, nq, d_beg, d_end, st));
+    cb = L.cub_bytes;
+    TIP_CHECK_CUDA(
+        cub::DeviceSegmentedSort::StableSortPairsDescending(cub_tmp, cb, bits2, bits, pk2, pk, items, nq, d_beg, d_end, st));
+    const long long rows = (long long)nq * N;
+    tip_query_finish_kernel<<<(int)((rows + 255) / 256), 256, 0, st>>>(nq, (int)N, L.cap, S, d_mrows, bits, pk, d_cand,
+                                                                         d_out_ids, d_out_scores);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    for (int i = 0; i < nq; ++i) h_n_out[i] = M[i];
+    return 0;
+}
+
+extern "C" int tip_top_triplets_per_gene_last_passes(void) { return g_last_query_passes; }

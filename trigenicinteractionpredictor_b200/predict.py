@@ -1,8 +1,8 @@
 """Rank the triplets a trained model has not seen: exhaustive top-N over all triplets of a gene set, on the device.
 
     python -m trigenicinteractionpredictor_b200.predict -t train0.dat -e test0.dat \\
-        -p results/Sample_0_K10.npz [-p results/Sample_1_K10.npz ...] [-n 100] [-g genes.txt] [--include-known] \\
-        [-o predictions.tsv] [--device cuda:0]
+        -p results/Sample_0_K10.npz [-p results/Sample_1_K10.npz ...] [-n 100] [-g genes.txt] [-q queries.txt] \\
+        [--include-known] [-o predictions.tsv] [--device cuda:0]
 
 The train / test files rebuild the model's digestion (gene ids in order of first appearance, TIP.py:321-423); every
 parameter file (the .npz that training with --save-params writes) must belong to it.  With several files the score of a
@@ -10,7 +10,11 @@ triplet is the mean of the models' scores.  Triplets that are keys of the train 
 --include-known.  -g: one gene name per line, the candidates (default: all genes).
 
 Output: a header line "Predicted Interaction<TAB>ID of genes<TAB>Genes", then one line per triplet, best first: the score,
-the id key as in the report's "ID of genes" column, and the gene names sorted by name (the fold-file format)."""
+the id key as in the report's "ID of genes" column, and the gene names sorted by name (the fold-file format).
+
+-q: one query gene name per line.  Then -n counts per query: for every query, in file order, the -n best triplets that
+contain it, the two partners taken from the -g genes plus the queries (default: all genes).  The header is
+"Query gene<TAB>Predicted Interaction<TAB>ID of genes<TAB>Genes" and every line starts with its query's name."""
 from __future__ import annotations
 
 import contextlib
@@ -19,6 +23,7 @@ import os
 import sys
 
 HEADER = "Predicted Interaction\tID of genes\tGenes\n"
+QUERY_HEADER = "Query gene\t" + HEADER
 
 
 def _fail(msg: str) -> int:
@@ -28,12 +33,12 @@ def _fail(msg: str) -> int:
 
 def main(argv=None) -> int:
     argv = sys.argv[1:] if argv is None else argv
-    train = test = out = device = genes_file = None
+    train = test = out = device = genes_file = queries_file = None
     params: list[str] = []
     top, include_known = 100, False
     try:
-        opts, rest = getopt.getopt(argv, "ht:e:p:n:g:o:", ["help", "train=", "test=", "params=", "top=", "genes=",
-                                                           "include-known", "out=", "device="])
+        opts, rest = getopt.getopt(argv, "ht:e:p:n:g:q:o:", ["help", "train=", "test=", "params=", "top=", "genes=",
+                                                             "queries=", "include-known", "out=", "device="])
     except getopt.GetoptError as exc:
         return _fail("argument error: %s" % exc)
     if rest:
@@ -57,6 +62,8 @@ def main(argv=None) -> int:
                 return _fail("--top must be positive (got %d)" % top)
         elif opt in ("-g", "--genes"):
             genes_file = arg
+        elif opt in ("-q", "--queries"):
+            queries_file = arg
         elif opt == "--include-known":
             include_known = True
         elif opt in ("-o", "--out"):
@@ -65,7 +72,7 @@ def main(argv=None) -> int:
             device = arg
     if train is None or test is None or not params:
         return _fail("-t/--train, -e/--test and at least one -p/--params are required")
-    for path in [train, test, *params] + ([genes_file] if genes_file else []):
+    for path in [train, test, *params] + [f for f in (genes_file, queries_file) if f]:
         if not os.path.isfile(path):
             return _fail("the file %s does not exist" % path)
     if out is not None and os.path.dirname(os.path.abspath(out)) and not os.path.isdir(os.path.dirname(os.path.abspath(out))):
@@ -82,6 +89,22 @@ def main(argv=None) -> int:
         unknown = [g for g in genes if g not in model.gene_id]
         if unknown:
             return _fail("genes not in the train / test files: %s" % ", ".join(unknown))
+    queries = None
+    if queries_file:
+        with open(queries_file, encoding="utf-8") as fh:
+            queries = [line.strip() for line in fh if line.strip()]
+        if not queries:
+            return _fail("the query file %s names no gene" % queries_file)
+        unknown = [g for g in queries if g not in model.gene_id]
+        if unknown:
+            return _fail("query genes not in the train / test files: %s" % ", ".join(unknown))
+        seen, twice = set(), []
+        for g in queries:
+            if g in seen and g not in twice:
+                twice.append(g)
+            seen.add(g)
+        if twice:
+            return _fail("query genes listed twice: %s" % ", ".join(twice))
     sets = []
     for path in params:
         try:
@@ -91,8 +114,13 @@ def main(argv=None) -> int:
     if len({th.shape[1] for th, _ in sets}) != 1:
         return _fail("the parameter files have different K")
 
-    rows = model.predict_top_triplets(top, genes=genes, exclude_known=not include_known, params=sets)
-    text = HEADER + "".join(str(s) + "\t" + key + "\t" + names + "\n" for s, key, names in rows)
+    if queries is None:
+        rows = model.predict_top_triplets(top, genes=genes, exclude_known=not include_known, params=sets)
+        text = HEADER + "".join(str(s) + "\t" + key + "\t" + names + "\n" for s, key, names in rows)
+    else:
+        per = model.predict_top_triplets_per_gene(queries, top, genes=genes, exclude_known=not include_known, params=sets)
+        text = QUERY_HEADER + "".join(q + "\t" + str(s) + "\t" + key + "\t" + names + "\n"
+                                      for q in queries for s, key, names in per[q])
     if out is None:
         sys.stdout.write(text)
     else:
