@@ -217,6 +217,27 @@ int tip_top_triplets_per_gene(int P, int K, int S, const double *d_theta, const 
 /* sweeps the last tip_top_triplets_per_gene of this thread ran (measurement) */
 int tip_top_triplets_per_gene_last_passes(void);
 
+/* ---- prediction per query pair: for every pair of genes, the N highest-scoring unseen triplets that contain both ----
+ * Rank space, score and known keys as tip_top_triplets: d_cand[n_cand] in decimal-string order (rank = position),
+ * d_known sorted packed rank triples (a repeated key counts once).  d_pair_ranks[n_pairs][2]: two distinct ranks into
+ * d_cand, in either order; duplicate pairs are answered independently.  For the pair ra < rb every other candidate rc is a partner, and its slot follows from
+ * rc: rc < ra gives (c, a, b), ra < rc < rb gives (a, c, b), rc > rb gives (a, b, c).
+ * Out, per pair q in the caller's order: the first min(N, n_cand - 2 - its known keys) triplets in the order (score
+ * descending, rc ascending, which is packed ranks ascending), exact under any ties: d_out_ids[n_pairs][N][3] gene ids in
+ * slot order, d_out_scores[n_pairs][N], h_n_out[n_pairs] rows (rows past h_n_out[q] are not written).  The pairs are sorted
+ * by (ra, rb) on the device and swept in tiles of 64; each tile selects its rows in shared memory: one sweep counts the
+ * scores, the next keeps those at or above each row's boundary, and a row whose buffer overflowed is swept again.  A rank out
+ * of range or a pair of one rank is refused before any device work.  Synchronises the stream; not capturable in a CUDA
+ * graph.  Limits: n_cand <= 2^21, S * K <= 384, n_pairs * N <= 2^24.  Workspace O(n_cand S K + n_pairs (S K + N)).
+ * Precondition: finite, non-negative parameters.  d_ws: tip_top_triplets_per_pair_workspace_bytes() bytes. */
+int tip_top_triplets_per_pair_workspace_bytes(int n_cand, int64_t n_pairs, int K, int S, int64_t n_known, int64_t N, size_t *bytes);
+int tip_top_triplets_per_pair(int P, int K, int S, const double *d_theta, const double *d_p, const int32_t *d_cand, int n_cand,
+                              const int32_t *d_pair_ranks, int64_t n_pairs, const uint64_t *d_known, int64_t n_known, int64_t N,
+                              void *d_ws, size_t ws_bytes, int32_t *d_out_ids, double *d_out_scores, int64_t *h_n_out,
+                              void *stream);
+/* sweeps the last tip_top_triplets_per_pair of this thread ran (measurement) */
+int tip_top_triplets_per_pair_last_passes(void);
+
 /* ---- testResultsReducer.py:160-184: mean / median / standard deviation of every test triplet across samples ----
  * d_scores[S][T]: score of triplet t in sample j at [j * T + t]; d_n[t] (or NULL = S) = how many leading samples of
  * triplet t are valid.  mean = sequential sum in sample order / n; median = the reference's rule (ascending sort;

@@ -704,6 +704,49 @@ class Model:
             res[q] = rows
         return res
 
+    def predict_top_triplets_per_pair(self, pairs, n, genes=None, exclude_known=True, params=None):
+        """For every query pair (nameA, nameB) of `pairs` (two distinct genes; no pair twice, in either order): the `n` most
+        likely interacting triplets that contain both, the third gene a distinct gene of `genes` + the pairs' genes (names;
+        default all P genes), scored as in predict_top_triplets.  With exclude_known the keys of links and test_links are
+        left out.  Exhaustive over every partner of every pair on the device.  Returns {(nameA, nameB): [[score, "a_b_c",
+        "nameA_nameB_nameC"], ...]} in the order of `pairs`, each list best first with ties in the order of
+        predict_top_triplets; a list is shorter than n when the pair has fewer unseen triplets."""
+        sets = self._prediction_sets(params, "predict_top_triplets_per_pair")
+        K = sets[0][0].shape[1]
+        pairs = [tuple(p) for p in pairs]
+        if not pairs:
+            raise ValueError("predict_top_triplets_per_pair: pairs is empty")
+        if any(len(p) != 2 for p in pairs):
+            raise ValueError("predict_top_triplets_per_pair: a pair is not two gene names")
+        names = [g for p in pairs for g in p] + (list(genes) if genes is not None else [])
+        missing = [g for g in names if g not in self.gene_id]
+        if missing:
+            raise ValueError("unknown gene names: %s" % ", ".join(dict.fromkeys(missing)))
+        single = [p for p in pairs if p[0] == p[1]]
+        if single:
+            raise ValueError("predict_top_triplets_per_pair: a pair of one gene: %s" % "+".join(single[0]))
+        twice = [p for p, c in collections.Counter(frozenset(p) for p in pairs).items() if c > 1]
+        if twice:
+            raise ValueError("predict_top_triplets_per_pair: duplicate pairs: %s" % ", ".join("+".join(sorted(p)) for p in twice))
+        if int(n) < 0:
+            raise ValueError("predict_top_triplets_per_pair: n must be >= 0 (got %d)" % int(n))
+        ids = set(range(self.P)) if genes is None else {self.gene_id[g] for g in names}
+        cand = np.array(sorted(ids, key=str), dtype=np.int32)
+        rank = {g: r for r, g in enumerate(cand.tolist())}
+        pr = np.array([[rank[self.gene_id[a]], rank[self.gene_id[b]]] for a, b in pairs], dtype=np.int32)
+        known = self._known_packed(cand) if exclude_known else np.empty(0, dtype=np.uint64)
+        eng = self._prediction_engine(K)
+        out_ids, scores, counts = eng.top_triplets_per_pair(np.stack([th for th, _ in sets]), np.stack([pr_ for _, pr_ in sets]),
+                                                            cand, pr, known, int(n))
+        res = {}
+        for qi, p in enumerate(pairs):
+            rows = []
+            for (a, b, c), s in zip(out_ids[qi, :counts[qi]].tolist(), scores[qi, :counts[qi]].tolist()):
+                names3 = sorted((self.id_gene[a], self.id_gene[b], self.id_gene[c]))
+                rows.append([s, "%d_%d_%d" % (a, b, c), "_".join(names3)])
+            res[p] = rows
+        return res
+
     def _known_packed(self, cand):
         """Sorted packed rank triples (ra << 42 | rb << 21 | rc) of the keys of links and test_links whose three genes
         are all candidates."""

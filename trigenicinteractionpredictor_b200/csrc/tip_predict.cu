@@ -26,6 +26,7 @@
 
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_segmented_sort.cuh>
+#include <cub/device/device_select.cuh>
 
 #include "tip_common.cuh"
 
@@ -1082,3 +1083,675 @@ extern "C" int tip_top_triplets_per_gene(int P, int K, int S, const double *d_th
 }
 
 extern "C" int tip_top_triplets_per_gene_last_passes(void) { return g_last_query_passes; }
+
+// ---- tip_top_triplets_per_pair ----
+// A query pair of ranks ra < rb and a partner of rank rc: the triplet's slots follow from rc (rc < ra: (c, a, b); ra < rc < rb:
+// (a, c, b); rc > rb: (a, b, c)), and its score is th_c . V_g with, per set (M_0, M_1 of gene b as tip_query_prep_kernel forms
+// them, so K^2 per pair and vector entry)
+//     V_0[x] = sum_y M_0[x][y] th_a[y],   V_1[y] = sum_x th_a[x] M_0[x][y],   V_2[z] = sum_x th_a[x] M_1[x][z]
+// The pairs are sorted by (ra, rb) on the device; a work item is a tile of 64 of them, swept over the columns in three phases,
+// one per region, each loading that region's V rows as the A tile of dmma_block; the epilogue masks each row to its region.
+// A CTA owns its rows for the whole sweep, so selection is CTA-local: each row's histogram lives in shared memory, and at the
+// end of the tile the CTA sets the row's next threshold from it.  First sweep: count every score in a range just below the
+// row's upper bound (known triplets included: the row's count of known triplets is added to what it needs).  Second: keep
+// the unknown scores at or above the boundary bin, appended to the row's slice of a buffer.  A row whose slice overflows
+// narrows as narrow() does, continuing on rc under ties, and is swept again.
+namespace tip {
+namespace {
+
+constexpr long long kPairMaxRows = 1ll << 24;           // n_pairs * N
+constexpr unsigned long long kPairSpan = 4ull << 52;    // first histogram range: 4 binades below the row's bound
+
+// selection state of one pair
+struct PairSel {
+    int state;                      // 0: count bits in [lo, hi] (histogram only); 1: keep bits >= lo; 2: keep bits > v, or
+                                    // bits == v and rc <= rhi; 3: resolved
+    int shift;
+    int rlo, rhi;                   // state 2: histogram range of rc (bin 0 = lowest)
+    unsigned long long lo, hi, v;   // states 0, 1: histogram range of score bits (bin 0 = highest); state 2: tied score bits
+};
+
+__host__ __device__ inline int pair_shift(unsigned long long span, int nb)
+{
+    int s = 0;
+    while (s < 64 && (span >> s) >= (unsigned long long)nb) ++s;
+    return s;
+}
+
+// sort keys (ra << 21) | rb with ra < rb, and the caller's index
+__global__ void tip_pair_keys_kernel(long long n_pairs, const int32_t *__restrict__ pr, unsigned long long *__restrict__ key,
+                                     int32_t *__restrict__ idx)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_pairs) return;
+    const int a = min(pr[2 * i], pr[2 * i + 1]), b = max(pr[2 * i], pr[2 * i + 1]);
+    key[i] = ((unsigned long long)a << kRankBits) | (unsigned long long)b;
+    idx[i] = (int32_t)i;
+}
+
+// per sorted pair: its ranks; active[i] = i lists every tile for the first sweep (there are fewer tiles than pairs)
+__global__ void tip_pair_split_kernel(long long n_pairs, const unsigned long long *__restrict__ key, int32_t *__restrict__ ra,
+                                      int32_t *__restrict__ rb, int32_t *__restrict__ active)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_pairs) return;
+    ra[i] = (int32_t)(key[i] >> kRankBits);
+    rb[i] = (int32_t)(key[i] & ((1ull << kRankBits) - 1));
+    active[i] = (int32_t)i;
+}
+
+// per sorted pair: its count of distinct known triplets (a known triple adds one to every pair it contains)
+__global__ void tip_pair_known_kernel(long long n_known, const unsigned long long *__restrict__ known, long long n_pairs,
+                                      const unsigned long long *__restrict__ key, unsigned long long *__restrict__ krow)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_known || (i > 0 && known[i] == known[i - 1])) return;   // a repeated key counts once
+    const unsigned long long k = known[i], m = (1ull << kRankBits) - 1;
+    const unsigned long long r0 = (k >> (2 * kRankBits)) & m, r1 = (k >> kRankBits) & m, r2 = k & m;
+    const unsigned long long want[3] = {(r0 << kRankBits) | r1, (r0 << kRankBits) | r2, (r1 << kRankBits) | r2};
+    for (int w = 0; w < 3; ++w) {
+        long long lo = 0, hi = n_pairs;
+        while (lo < hi) {
+            const long long mid = (lo + hi) >> 1;
+            if (key[mid] < want[w]) lo = mid + 1; else hi = mid;
+        }
+        for (; lo < n_pairs && key[lo] == want[w]; ++lo) atomicAdd(krow + lo, 1ull);
+    }
+}
+
+// V[pair][g][s K + x] for the pairs whose gene b is one of the chunk's genes [c0, c1) (Mq of the chunk, local index)
+__global__ void tip_pair_vec_kernel(long long n_pairs, int S, int K, int SKP, int c0, int c1, const int32_t *__restrict__ bidx,
+                                    const int32_t *__restrict__ ra, const int32_t *__restrict__ rb, const double *__restrict__ tcat,
+                                    const double *__restrict__ Mq, double *__restrict__ V)
+{
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n_pairs * 3 * SKP) return;
+    const long long p = t / (3 * SKP);
+    const int g = (int)(t / SKP % 3), col = (int)(t % SKP);
+    const int u = bidx[rb[p]];
+    if (u < c0 || u >= c1) return;
+    double acc = 0.0;
+    if (col < S * K) {
+        const int s = col / K, x = col % K;
+        const long long KK = (long long)K * K;
+        const double *th = tcat + (long long)ra[p] * SKP + s * K;
+        const double *M = Mq + (((long long)(u - c0) * 3 + (g == 2 ? 1 : 0)) * S + s) * KK;
+        if (g == 0) {
+            for (int y = 0; y < K; ++y) acc = fma(M[x * K + y], th[y], acc);
+        } else {
+            for (int y = 0; y < K; ++y) acc = fma(th[y], M[y * K + x], acc);
+        }
+    }
+    V[t] = acc;
+}
+
+// first state of every pair: rows to select (M) and to count (M + known triplets), and the first histogram range, up to
+// an upper bound of the row's scores: th_c . V_s <= max(V_s) |th_c|_1 <= max(V_s) T[s] (non-negative parameters)
+__global__ void tip_pair_init_kernel(long long n_pairs, int n, int S, int K, int SKP, long long N, long long cap, int nb,
+                                     const double *__restrict__ V, const unsigned long long *__restrict__ T,
+                                     const unsigned long long *__restrict__ krow, PairSel *__restrict__ sel,
+                                     long long *__restrict__ need0, long long *__restrict__ m_rows, long long *__restrict__ kept)
+{
+    const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n_pairs) return;
+    const long long k = (long long)krow[p];
+    const long long M = max(0ll, min(N, (long long)(n - 2) - k));
+    m_rows[p] = M;
+    need0[p] = M + k;
+    kept[p] = 0;
+    PairSel q{};
+    q.hi = kInfBits;
+    if (M == 0) {
+        q.state = 3;
+    } else if (n - 2 <= cap) {
+        q.state = 1;   // every partner fits the row's slice
+    } else {
+        double best = 0.0;
+        for (int g = 0; g < 3; ++g) {
+            double b = 0.0;
+            for (int s = 0; s < S; ++s) {
+                double mx = 0.0;
+                for (int x = 0; x < K; ++x) mx = fmax(mx, V[(p * 3 + g) * SKP + s * K + x]);
+                b += mx * __longlong_as_double((long long)T[s]);
+            }
+            best = fmax(best, b);
+        }
+        q.hi = min((unsigned long long)__double_as_longlong(best * (1.0 + 1e-9)), kInfBits);
+        q.lo = q.hi >= kPairSpan ? q.hi - kPairSpan + 1 : 0;
+    }
+    q.shift = pair_shift(q.hi - q.lo, nb);
+    sel[p] = q;
+}
+
+// is_known for the pair kernel: a second call site of is_known changes the code generated for it inside the two scoring
+// kernels above, so the pair kernel has its own copy
+__device__ __noinline__ bool pair_is_known(const unsigned long long *known, long long n, unsigned long long key)
+{
+    long long lo = 0, hi = n;
+    while (lo < hi) {
+        const long long mid = (lo + hi) >> 1;
+        if (__ldg(known + mid) < key) lo = mid + 1; else hi = mid;
+    }
+    return lo < n && __ldg(known + lo) == key;
+}
+
+struct PairPassArgs {
+    int n, SKP, nb;
+    const double *tcat;               // [n_pad][SKP]
+    const double *V;                  // [n_pairs][3][SKP], sorted pair order
+    const int32_t *ra, *rb;           // [n_pairs] sorted
+    const int32_t *active;            // [n_active] tiles this sweep scores (tile t = sorted pairs 64 t .. 64 t + 63), ascending
+    int n_active, n_pairs;
+    const unsigned long long *known;  // sorted packed rank triples
+    long long n_known;
+    PairSel *sel;                     // [n_pairs]
+    const long long *need0;           // [n_pairs] rows state 0 must reach (M + known triplets of the pair)
+    long long *m_rows, *kept;         // [n_pairs]
+    char *again;                      // [n_active] 1: a row of the tile is swept again
+    unsigned long long *ctl;          // [0] tile cursor, [1] rows not resolved, [2] internal errors
+    unsigned long long *out_bits, *out_rc;   // [n_pairs][cap]
+    long long cap;
+};
+
+// epilogue of a block for phase g (i0 = the lane's first row in the tile, rc0 = its first column)
+__device__ __forceinline__ void pair_select_block(const double (&acc)[4][4][2], int g, int i0, int rc0, const PairPassArgs &A,
+                                                  const PairSel *sh_sel, const int *sh_ra, const int *sh_rb, const int *sh_p,
+                                                  unsigned *sh_cnt, unsigned *sh_hist)
+{
+    const int nb = A.nb;
+#pragma unroll
+    for (int mi = 0; mi < 4; ++mi) {
+        const int i = i0 + mi * 8;
+        const PairSel q = sh_sel[i];
+        if (q.state == 3) continue;
+        const int ra = sh_ra[i], rb = sh_rb[i];
+        const int lo_c = g == 0 ? 0 : g == 1 ? ra + 1 : rb + 1, hi_c = g == 0 ? ra : g == 1 ? rb : A.n;
+        unsigned *h = sh_hist + i * (nb + 1);
+#pragma unroll
+        for (int ni = 0; ni < 4; ++ni)
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+                const int rc = rc0 + ni * 8 + e;
+                if (rc < lo_c || rc >= hi_c) continue;
+                const unsigned long long bits = (unsigned long long)__double_as_longlong(acc[mi][ni][e]);
+                if (q.state == 0) {
+                    if (bits >= q.lo) atomicAdd(h + (bits > q.hi ? nb : (int)((q.hi - bits) >> q.shift)), 1u);
+                    continue;
+                }
+                if (!(q.state == 1 ? bits >= q.lo : (bits > q.v || (bits == q.v && rc <= q.rhi)))) continue;
+                if (A.n_known > 0) {
+                    const unsigned long long a = ra, b = rb, c = rc;
+                    const unsigned long long packed = g == 0 ? (c << 42) | (a << 21) | b
+                                                    : g == 1 ? (a << 42) | (c << 21) | b : (a << 42) | (b << 21) | c;
+                    if (pair_is_known(A.known, A.n_known, packed)) continue;
+                }
+                int bin = nb;
+                if (q.state == 1) {
+                    if (bits <= q.hi) bin = (int)((q.hi - bits) >> q.shift);
+                } else if (bits == q.v && rc >= q.rlo) {
+                    bin = (rc - q.rlo) >> q.shift;
+                }
+                atomicAdd(h + bin, 1u);
+                const unsigned idx = atomicAdd(sh_cnt + i, 1u);
+                if ((long long)idx < A.cap) {
+                    const long long o = (long long)sh_p[i] * A.cap + idx;
+                    A.out_bits[o] = bits;
+                    A.out_rc[o] = (unsigned long long)rc;
+                }
+            }
+    }
+}
+
+// next state of a row after a sweep counted C kept entries into its histogram h: 1 resolved, 0 swept again, -1 error.
+// States 1 and 2 follow narrow(); state 0 places the boundary where the count reaches need0, or, when the range does not
+// reach it, counts everything below the range in the next sweep.
+__device__ int narrow_pair(PairSel &q, long long C, long long need0, long long &M, long long cap, const unsigned *h, int nb, int n)
+{
+    const unsigned long long width = q.shift >= 64 ? ~0ull : (1ull << q.shift);
+    if (q.state == 1 || q.state == 2) {
+        if (C >= M && C <= cap) return 1;
+        if (C < M) {
+            if (q.state == 2) return -1;
+            if (q.lo == 0) { M = C; return 1; }   // every unknown partner is in the slice
+            q.state = 0;                          // count again, everything below this range
+            q.hi = q.lo - 1;
+            q.lo = 0;
+            q.shift = pair_shift(q.hi - q.lo, nb);
+            return 0;
+        }
+    }
+    if (q.state == 0) {
+        long long cum = h[nb];
+        int b = 0;
+        if (cum < need0)
+            for (; b < nb; ++b)
+                if ((cum += h[b]) >= need0) break;
+        if (cum < need0 || b == nb) {
+            if (q.lo == 0) return -1;
+            q.hi = q.lo - 1;   // the range missed: the next one reaches down to zero
+            q.lo = 0;
+        } else if (h[nb] >= need0) {
+            q.state = 1;
+            q.lo = q.hi + 1;
+            q.hi = kInfBits;
+        } else {
+            const unsigned long long top = q.hi - ((unsigned long long)b << q.shift);
+            q.state = 1;
+            q.lo = (top - q.lo + 1 <= width) ? q.lo : top - width + 1;
+        }
+        q.shift = pair_shift(q.hi - q.lo, nb);
+        return 0;
+    }
+    // too many for the slice: the histogram holds exactly the kept entries
+    long long cum = h[nb];
+    if (q.state == 1 && cum >= M) {
+        q.lo = q.hi + 1;
+        q.hi = kInfBits;
+        q.shift = pair_shift(q.hi - q.lo, nb);
+        return 0;
+    }
+    int b = 0;
+    for (; b < nb; ++b)
+        if ((cum += h[b]) >= M) break;
+    if (b == nb) return -1;
+    if (q.state == 1) {
+        const unsigned long long top = q.hi - ((unsigned long long)b << q.shift);
+        const unsigned long long bottom = (top - q.lo + 1 <= width) ? q.lo : top - width + 1;
+        if (cum <= cap) {
+            q.lo = bottom;
+        } else if (bottom == top) {
+            q.state = 2;   // one score value holds too many: continue on rc
+            q.v = top;
+            q.rlo = 0;
+            q.rhi = n - 1;
+        } else {
+            q.lo = bottom;
+            q.hi = top;
+        }
+    } else {
+        const long long lo_b = q.rlo + ((long long)b << q.shift);
+        const int hi_b = (int)min((long long)q.rhi, lo_b + (long long)width - 1);
+        if (cum > cap) q.rlo = (int)lo_b;
+        q.rhi = hi_b;
+    }
+    q.shift = q.state == 1 ? pair_shift(q.hi - q.lo, nb) : pair_shift((unsigned long long)(q.rhi - q.rlo), nb);
+    return 0;
+}
+
+// work items are the active tiles of 64 sorted pairs; every tile sweeps the columns of each region of its rows.  A tile
+// holds the same rows in every sweep (resolved rows are skipped in the epilogue), so every score is computed at the same
+// place in the same DMMA fragment, with the same contraction order, in every sweep
+__global__ void __launch_bounds__(kPredThreads) tip_pair_pass_kernel(PairPassArgs A)
+{
+    extern __shared__ __align__(16) unsigned char smem[];
+    const int qs = q_stride(A.SKP), nb = A.nb;
+    double *At = reinterpret_cast<double *>(smem);                                        // [64][qs]
+    PairSel *sh_sel = reinterpret_cast<PairSel *>(At + (size_t)kPredRows * qs);          // [64]
+    int *sh_ra = reinterpret_cast<int *>(sh_sel + kPredRows), *sh_rb = sh_ra + kPredRows, *sh_p = sh_rb + kPredRows;
+    unsigned *sh_cnt = reinterpret_cast<unsigned *>(sh_p + kPredRows);                   // [64]
+    unsigned *sh_hist = sh_cnt + kPredRows;                                                // [64][nb + 1]
+    __shared__ long long sh_item;
+    __shared__ int sh_range[4];   // min ra, max ra, min rb, max rb of the tile
+    __shared__ int sh_again;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int wr = warp & 1, wc = warp >> 1;
+    const int gq = lane >> 2, tq = lane & 3;
+    const int n = A.n, SKP = A.SKP;
+
+    for (;;) {
+        __syncthreads();   // the previous tile is no longer read
+        if (tid == 0) sh_item = (long long)atomicAdd(A.ctl, 1ull);
+        __syncthreads();
+        const long long item = sh_item;
+        if (item >= A.n_active) break;
+        const int t0 = A.active[item] * kPredRows, rows = min(kPredRows, A.n_pairs - t0);
+        if (tid == 0) sh_again = 0;
+        if (tid < kPredRows) {
+            const int p = t0 + (tid < rows ? tid : 0);
+            sh_p[tid] = p;
+            sh_ra[tid] = A.ra[p];
+            sh_rb[tid] = A.rb[p];
+            PairSel q = A.sel[p];
+            if (tid >= rows) q.state = 3;
+            sh_sel[tid] = q;
+            sh_cnt[tid] = 0;
+        }
+        for (int i = tid; i < kPredRows * (nb + 1); i += kPredThreads) sh_hist[i] = 0;
+        __syncthreads();
+        if (tid == 0) {
+            int r0 = n, r1 = 0, r2 = n, r3 = 0;
+            for (int i = 0; i < rows; ++i) {
+                r0 = min(r0, sh_ra[i]); r1 = max(r1, sh_ra[i]);
+                r2 = min(r2, sh_rb[i]); r3 = max(r3, sh_rb[i]);
+            }
+            sh_range[0] = r0; sh_range[1] = r1; sh_range[2] = r2; sh_range[3] = r3;
+        }
+        __syncthreads();
+
+        for (int g = 0; g < 3; ++g) {
+            const int col0 = g == 0 ? 0 : g == 1 ? sh_range[0] + 1 : sh_range[2] + 1;
+            const int col_end = g == 0 ? sh_range[1] : g == 1 ? sh_range[3] : n;
+            if (col0 >= col_end) continue;
+            __syncthreads();   // the previous phase's A tile is no longer read
+            for (int e = tid; e < kPredRows * SKP; e += kPredThreads) {
+                const int i = e / SKP, col = e % SKP;
+                At[i * qs + col] = i < rows ? __ldg(A.V + ((long long)sh_p[i] * 3 + g) * SKP + col) : 0.0;
+            }
+            __syncthreads();
+            if (wr * 32 < rows) {
+                const double *Aw = At + (wr * 32 + gq) * qs + tq;
+                for (int c0 = col0 + wc * 32; c0 < col_end; c0 += 64) {
+                    double acc[4][4][2];
+                    dmma_block(acc, Aw, qs, A.tcat + (long long)(c0 + gq) * SKP + tq, SKP);
+                    pair_select_block(acc, g, wr * 32 + gq, c0 + 2 * tq, A, sh_sel, sh_ra, sh_rb, sh_p, sh_cnt, sh_hist);
+                }
+            }
+        }
+        __syncthreads();
+        if (tid < rows) {
+            const int p = sh_p[tid];
+            PairSel q = sh_sel[tid];
+            long long M = A.m_rows[p];
+            const long long C = sh_cnt[tid];
+            int r = 1;
+            if (q.state != 3) r = narrow_pair(q, C, A.need0[p], M, A.cap, sh_hist + tid * (nb + 1), nb, n);
+            if (r < 0) {
+                atomicAdd(A.ctl + 2, 1ull);
+                r = 1;
+            }
+            if (r == 1 && q.state != 3) {
+                q.state = 3;
+                A.kept[p] = C;
+                A.m_rows[p] = M;
+            }
+            A.sel[p] = q;
+            if (r == 0) {
+                sh_again = 1;
+                atomicAdd(A.ctl + 1, 1ull);
+            }
+        }
+        __syncthreads();
+        if (tid == 0) A.again[item] = (char)sh_again;
+    }
+}
+
+__global__ void tip_pair_segments_kernel(long long n_pairs, long long cap, const long long *__restrict__ kept, int *__restrict__ beg,
+                                         int *__restrict__ end)
+{
+    const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n_pairs) return;
+    beg[p] = (int)(p * cap);
+    end[p] = (int)(p * cap + kept[p]);
+}
+
+// row t of sorted pair p goes to the caller's pair perm[p]; ids in slot order (ranks ascending)
+__global__ void tip_pair_finish_kernel(long long n_pairs, long long N, long long cap, int S, const int32_t *__restrict__ perm,
+                                       const int32_t *__restrict__ ra, const int32_t *__restrict__ rb,
+                                       const long long *__restrict__ m_rows, const unsigned long long *__restrict__ bits,
+                                       const unsigned long long *__restrict__ rc, const int32_t *__restrict__ cand,
+                                       int32_t *__restrict__ out_ids, double *__restrict__ out_scores, int64_t *__restrict__ counts)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_pairs * N) return;
+    const long long p = i / N, t = i % N, o = (long long)perm[p] * N + t;
+    if (t == 0) counts[perm[p]] = m_rows[p];
+    if (t >= m_rows[p]) return;
+    const long long src = p * cap + t;
+    const int a = ra[p], b = rb[p], c = (int)rc[src];
+    const int x = min(c, a), z = max(c, b), y = a + b + c - x - z;
+    out_ids[3 * o + 0] = cand[x];
+    out_ids[3 * o + 1] = cand[y];
+    out_ids[3 * o + 2] = cand[z];
+    out_scores[o] = __longlong_as_double((long long)bits[src]) / (double)S;
+}
+
+// room for 4 N survivors plus slack in a row's slice, never more than its partners
+long long pair_capacity(int n, long long N) { return std::max(1ll, std::min((long long)n - 2, 4 * N + 64)); }
+
+struct PairLayout {
+    size_t o_tcat, o_M, o_T, o_key, o_key2, o_idx, o_perm, o_ra, o_rb, o_bidx, o_ub, o_krow, o_V, o_sel, o_need, o_mrows, o_kept,
+        o_again, o_act, o_act2, o_nsel, o_ctl, o_beg, o_end, o_counts, o_bits, o_rc, o_bits2, o_rc2, o_cub, cub_bytes, total;
+    int n_pad, SKP, chunk;
+    long long cap;
+};
+
+PairLayout pair_layout(int n, long long n_pairs, int K, int S, long long N)
+{
+    PairLayout L{};
+    L.n_pad = (n + 63) / 64 * 64 + 64;
+    L.SKP = (S * K + 3) / 4 * 4;
+    L.cap = pair_capacity(n, N);
+    // genes b whose K x K matrices are formed at a time: about n S K doubles
+    L.chunk = (int)std::max(1ll, std::min((long long)n, (long long)L.n_pad * L.SKP / (3ll * S * K * K)));
+    const long long items = n_pairs * L.cap;
+    const int np = (int)n_pairs;
+    size_t cb[5] = {0, 0, 0, 0, 0};
+    cub::DeviceRadixSort::SortPairs(nullptr, cb[0], (const unsigned long long *)nullptr, (unsigned long long *)nullptr,
+                                    (const int32_t *)nullptr, (int32_t *)nullptr, np, 0, 2 * kRankBits, (cudaStream_t)0);
+    cub::DeviceSelect::Flagged(nullptr, cb[1], (const int32_t *)nullptr, (const char *)nullptr, (int32_t *)nullptr, (int *)nullptr,
+                               np, (cudaStream_t)0);
+    cub::DeviceSegmentedSort::StableSortPairs(nullptr, cb[2], (const unsigned long long *)nullptr, (unsigned long long *)nullptr,
+                                              (const unsigned long long *)nullptr, (unsigned long long *)nullptr, (int)items, np,
+                                              (const int *)nullptr, (const int *)nullptr, (cudaStream_t)0);
+    cub::DeviceSegmentedSort::StableSortPairsDescending(nullptr, cb[3], (const unsigned long long *)nullptr,
+                                                        (unsigned long long *)nullptr, (const unsigned long long *)nullptr,
+                                                        (unsigned long long *)nullptr, (int)items, np, (const int *)nullptr,
+                                                        (const int *)nullptr, (cudaStream_t)0);
+    L.cub_bytes = *std::max_element(cb, cb + 5);
+    const size_t q = (size_t)n_pairs;
+    size_t off = 0;
+    L.o_tcat = off;   off += a256((size_t)L.n_pad * L.SKP * 8);
+    L.o_M = off;      off += a256((size_t)L.chunk * 3 * S * K * K * 8);
+    L.o_T = off;      off += a256((size_t)S * 8);
+    L.o_key = off;    off += a256(q * 8);
+    L.o_key2 = off;   off += a256(q * 8);
+    L.o_idx = off;    off += a256(q * 4);
+    L.o_perm = off;   off += a256(q * 4);
+    L.o_ra = off;     off += a256(q * 4);
+    L.o_rb = off;     off += a256(q * 4);
+    L.o_bidx = off;   off += a256((size_t)n * 4);
+    L.o_ub = off;     off += a256((size_t)n * 4);
+    L.o_krow = off;   off += a256(q * 8);
+    L.o_V = off;      off += a256(q * 3 * L.SKP * 8);
+    L.o_sel = off;    off += a256(q * sizeof(PairSel));
+    L.o_need = off;   off += a256(q * 8);
+    L.o_mrows = off;  off += a256(q * 8);
+    L.o_kept = off;   off += a256(q * 8);
+    L.o_again = off;  off += a256(q);
+    L.o_act = off;    off += a256(q * 4);
+    L.o_act2 = off;   off += a256(q * 4);
+    L.o_nsel = off;   off += 256;
+    L.o_ctl = off;    off += 256;
+    L.o_beg = off;    off += a256(q * 4);
+    L.o_end = off;    off += a256(q * 4);
+    L.o_counts = off; off += a256(q * 8);
+    L.o_bits = off;   off += a256((size_t)items * 8);
+    L.o_rc = off;     off += a256((size_t)items * 8);
+    L.o_bits2 = off;  off += a256((size_t)items * 8);
+    L.o_rc2 = off;    off += a256((size_t)items * 8);
+    L.o_cub = off;    off += a256(L.cub_bytes);
+    L.total = off + 256;
+    return L;
+}
+
+// bins per row of the shared histograms: the most of 256, 128, 64 that fit beside the A tile
+size_t pair_smem(int SKP, int nb)
+{
+    return (size_t)kPredRows * q_stride(SKP) * 8 + (size_t)kPredRows * (sizeof(PairSel) + 16) + (size_t)kPredRows * (nb + 1) * 4;
+}
+
+}  // namespace
+}  // namespace tip
+
+static thread_local int g_last_pair_passes = 0;
+
+static bool per_pair_args_ok(int n_cand, int64_t n_pairs, int K, int S, int64_t n_known, int64_t N)
+{
+    return predict_args_ok(n_cand, K, S, n_known, N) && n_pairs >= 0 && n_pairs <= kPairMaxRows &&
+           (N == 0 || n_pairs <= kPairMaxRows / N);
+}
+
+extern "C" int tip_top_triplets_per_pair_workspace_bytes(int n_cand, int64_t n_pairs, int K, int S, int64_t n_known, int64_t N,
+                                                         size_t *bytes)
+{
+    TIP_REQUIRE(bytes != nullptr && per_pair_args_ok(n_cand, n_pairs, K, S, n_known, N),
+                "tip_top_triplets_per_pair_workspace_bytes: bad arguments (n_cand <= 2^21, n_pairs >= 0, 1 <= K <= %d, S >= 1, "
+                "S*K <= %d, N >= 0, n_pairs*N <= 2^24)", TIP_MAX_K, kPredMaxSK);
+    *bytes = pair_layout(n_cand, n_pairs, K, S, N).total;
+    return 0;
+}
+
+extern "C" int tip_top_triplets_per_pair(int P, int K, int S, const double *d_theta, const double *d_p, const int32_t *d_cand,
+                                         int n_cand, const int32_t *d_pair_ranks, int64_t n_pairs, const uint64_t *d_known,
+                                         int64_t n_known, int64_t N, void *d_ws, size_t ws_bytes, int32_t *d_out_ids,
+                                         double *d_out_scores, int64_t *h_n_out, void *stream)
+{
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    TIP_REQUIRE(P > 0 && n_cand <= P && per_pair_args_ok(n_cand, n_pairs, K, S, n_known, N) && (h_n_out || n_pairs == 0),
+                "tip_top_triplets_per_pair: bad arguments (P > 0, n_cand <= min(P, 2^21), n_pairs >= 0, 1 <= K <= %d, S >= 1, "
+                "S*K <= %d, n_known >= 0, N >= 0, n_pairs*N <= 2^24)", TIP_MAX_K, kPredMaxSK);
+    TIP_REQUIRE(d_theta && d_p && (d_cand || n_cand == 0) && (d_pair_ranks || n_pairs == 0) && (d_known || n_known == 0) &&
+                    (N == 0 || n_pairs == 0 || (d_out_ids && d_out_scores)),
+                "tip_top_triplets_per_pair: null pointer");
+    g_last_pair_passes = 0;
+    if (n_pairs == 0) return 0;
+    const int n = n_cand;
+    const long long Q = n_pairs;
+    // the pair ranks are checked on the host before any device work
+    std::vector<int32_t> pr((size_t)Q * 2);
+    TIP_CHECK_CUDA(cudaMemcpyAsync(pr.data(), d_pair_ranks, (size_t)Q * 8, cudaMemcpyDeviceToHost, st));
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    std::vector<int32_t> bidx(std::max(n, 1), -1), ub;
+    for (long long i = 0; i < Q; ++i) {
+        for (int e = 0; e < 2; ++e)
+            TIP_REQUIRE(pr[2 * i + e] >= 0 && pr[2 * i + e] < n, "tip_top_triplets_per_pair: rank %d of pair %lld is not in [0, %d)",
+                        pr[2 * i + e], i, n);
+        TIP_REQUIRE(pr[2 * i] != pr[2 * i + 1], "tip_top_triplets_per_pair: pair %lld has the same rank twice (%d)", i, pr[2 * i]);
+        bidx[std::max(pr[2 * i], pr[2 * i + 1])] = 0;
+    }
+    for (long long i = 0; i < Q; ++i) h_n_out[i] = 0;
+    if (N == 0 || n < 3) return 0;
+    for (int r = 0; r < n; ++r)
+        if (bidx[r] == 0) {
+            bidx[r] = (int32_t)ub.size();
+            ub.push_back(r);
+        }
+    const PairLayout L = pair_layout(n, Q, K, S, N);
+    TIP_REQUIRE(d_ws != nullptr && ws_bytes >= L.total, "tip_top_triplets_per_pair: workspace too small (%zu < %zu)", ws_bytes,
+                L.total);
+    char *base = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(d_ws) + 255) / 256 * 256);
+    double *tcat = reinterpret_cast<double *>(base + L.o_tcat), *Mq = reinterpret_cast<double *>(base + L.o_M);
+    auto *T = reinterpret_cast<unsigned long long *>(base + L.o_T);
+    auto *key = reinterpret_cast<unsigned long long *>(base + L.o_key), *key2 = reinterpret_cast<unsigned long long *>(base + L.o_key2);
+    auto *idx = reinterpret_cast<int32_t *>(base + L.o_idx), *perm = reinterpret_cast<int32_t *>(base + L.o_perm);
+    auto *ra = reinterpret_cast<int32_t *>(base + L.o_ra), *rb = reinterpret_cast<int32_t *>(base + L.o_rb);
+    auto *d_bidx = reinterpret_cast<int32_t *>(base + L.o_bidx), *d_ub = reinterpret_cast<int32_t *>(base + L.o_ub);
+    auto *krow = reinterpret_cast<unsigned long long *>(base + L.o_krow);
+    double *V = reinterpret_cast<double *>(base + L.o_V);
+    PairSel *sel = reinterpret_cast<PairSel *>(base + L.o_sel);
+    auto *need0 = reinterpret_cast<long long *>(base + L.o_need), *m_rows = reinterpret_cast<long long *>(base + L.o_mrows);
+    auto *kept = reinterpret_cast<long long *>(base + L.o_kept);
+    char *again = base + L.o_again;
+    auto *act = reinterpret_cast<int32_t *>(base + L.o_act), *act2 = reinterpret_cast<int32_t *>(base + L.o_act2);
+    auto *nsel = reinterpret_cast<int *>(base + L.o_nsel);
+    auto *ctl = reinterpret_cast<unsigned long long *>(base + L.o_ctl);
+    auto *d_beg = reinterpret_cast<int *>(base + L.o_beg), *d_end = reinterpret_cast<int *>(base + L.o_end);
+    auto *counts = reinterpret_cast<int64_t *>(base + L.o_counts);
+    auto *bits = reinterpret_cast<unsigned long long *>(base + L.o_bits), *rcs = reinterpret_cast<unsigned long long *>(base + L.o_rc);
+    auto *bits2 = reinterpret_cast<unsigned long long *>(base + L.o_bits2), *rcs2 = reinterpret_cast<unsigned long long *>(base + L.o_rc2);
+    void *cub_tmp = base + L.o_cub;
+    const int g1 = (int)((Q + 255) / 256);
+
+    // pairs sorted by (ra, rb), with the permutation back to the caller's order
+    tip_pair_keys_kernel<<<g1, 256, 0, st>>>(Q, d_pair_ranks, key, idx);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    size_t cb = L.cub_bytes;
+    TIP_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(cub_tmp, cb, key, key2, idx, perm, (int)Q, 0, 2 * kRankBits, st));
+    tip_pair_split_kernel<<<g1, 256, 0, st>>>(Q, key2, ra, rb, act);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    TIP_CHECK_CUDA(cudaMemsetAsync(krow, 0, (size_t)Q * 8, st));
+    if (n_known > 0) {
+        tip_pair_known_kernel<<<(int)((n_known + 255) / 256), 256, 0, st>>>(n_known, reinterpret_cast<const unsigned long long *>(d_known),
+                                                                              Q, key2, krow);
+        TIP_CHECK_CUDA(cudaGetLastError());
+    }
+    // V of every pair, from the matrices of its gene b, a chunk of genes at a time
+    TIP_CHECK_CUDA(cudaMemcpyAsync(d_bidx, bidx.data(), (size_t)n * 4, cudaMemcpyHostToDevice, st));
+    TIP_CHECK_CUDA(cudaMemcpyAsync(d_ub, ub.data(), ub.size() * 4, cudaMemcpyHostToDevice, st));
+    const int n_ub = (int)ub.size();
+    for (int c0 = 0; c0 < n_ub; c0 += L.chunk) {
+        const int c1 = std::min(n_ub, c0 + L.chunk);
+        const long long work = (long long)L.n_pad * L.SKP + (long long)(c1 - c0) * 3 * S * K * K;
+        tip_query_prep_kernel<<<(int)std::min<long long>((work + 255) / 256, (long long)sm_count() * 16), 256, 0, st>>>(
+            S, P, K, n, L.n_pad, L.SKP, c1 - c0, d_theta, d_p, d_cand, d_ub + c0, tcat, Mq);
+        TIP_CHECK_CUDA(cudaGetLastError());
+        tip_pair_vec_kernel<<<(int)((Q * 3 * L.SKP + 255) / 256), 256, 0, st>>>(Q, S, K, L.SKP, c0, c1, d_bidx, ra, rb, tcat, Mq, V);
+        TIP_CHECK_CUDA(cudaGetLastError());
+    }
+    TIP_CHECK_CUDA(cudaMemsetAsync(T, 0, (size_t)S * 8, st));
+    tip_query_rowsum_kernel<<<(n + 255) / 256, 256, 0, st>>>(n, S, K, L.SKP, tcat, T);
+    TIP_CHECK_CUDA(cudaGetLastError());
+
+    int dev = 0, optin = 0;
+    TIP_CHECK_CUDA(cudaGetDevice(&dev));
+    TIP_CHECK_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    int nb = 256;
+    while (nb > 64 && pair_smem(L.SKP, nb) + 1024 > (size_t)optin) nb /= 2;
+    const size_t smem = pair_smem(L.SKP, nb);
+    static int smem_set = 0;
+    if ((int)smem > smem_set && smem > 48 * 1024) {
+        TIP_CHECK_CUDA(cudaFuncSetAttribute(tip_pair_pass_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        smem_set = (int)smem;
+    }
+    int per_sm = 0;
+    TIP_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tip_pair_pass_kernel, kPredThreads, smem));
+    TIP_REQUIRE(per_sm > 0, "tip_top_triplets_per_pair: S*K = %d does not fit one block's shared memory", S * K);
+
+    tip_pair_init_kernel<<<g1, 256, 0, st>>>(Q, n, S, K, L.SKP, N, L.cap, nb, V, T, krow, sel, need0, m_rows, kept);
+    TIP_CHECK_CUDA(cudaGetLastError());
+
+    PairPassArgs A{};
+    A.n = n; A.SKP = L.SKP; A.nb = nb;
+    A.tcat = tcat; A.V = V; A.ra = ra; A.rb = rb; A.active = act; A.n_active = (int)((Q + kPredRows - 1) / kPredRows);
+    A.n_pairs = (int)Q;
+    A.known = reinterpret_cast<const unsigned long long *>(d_known); A.n_known = n_known;
+    A.sel = sel; A.need0 = need0; A.m_rows = m_rows; A.kept = kept; A.again = again; A.ctl = ctl;
+    A.out_bits = bits; A.out_rc = rcs; A.cap = L.cap;
+    unsigned long long h_ctl[3];
+    for (int pass = 0;; ++pass) {
+        TIP_REQUIRE(pass < 200, "tip_top_triplets_per_pair: the threshold did not converge (internal error)");
+        TIP_CHECK_CUDA(cudaMemsetAsync(ctl, 0, 24, st));
+        tip_pair_pass_kernel<<<(int)std::min<long long>((long long)sm_count() * per_sm, A.n_active), kPredThreads, smem, st>>>(A);
+        TIP_CHECK_CUDA(cudaGetLastError());
+        ++g_last_pair_passes;
+        // the tiles that hold a row not yet resolved, in order
+        int32_t *next = A.active == act ? act2 : act;
+        cb = L.cub_bytes;
+        TIP_CHECK_CUDA(cub::DeviceSelect::Flagged(cub_tmp, cb, A.active, again, next, nsel, A.n_active, st));
+        int h_nsel = 0;
+        TIP_CHECK_CUDA(cudaMemcpyAsync(h_ctl, ctl, 24, cudaMemcpyDeviceToHost, st));
+        TIP_CHECK_CUDA(cudaMemcpyAsync(&h_nsel, nsel, 4, cudaMemcpyDeviceToHost, st));
+        TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+        TIP_REQUIRE(h_ctl[2] == 0, "tip_top_triplets_per_pair: the histogram does not reach N (internal error)");
+        if (h_nsel == 0) break;
+        A.active = next;
+        A.n_active = h_nsel;
+    }
+    // order: per pair, rc ascending, then (stable) score descending
+    tip_pair_segments_kernel<<<g1, 256, 0, st>>>(Q, L.cap, kept, d_beg, d_end);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    const int items = (int)(Q * L.cap);
+    cb = L.cub_bytes;
+    TIP_CHECK_CUDA(cub::DeviceSegmentedSort::StableSortPairs(cub_tmp, cb, rcs, rcs2, bits, bits2, items, (int)Q, d_beg, d_end, st));
+    cb = L.cub_bytes;
+    TIP_CHECK_CUDA(
+        cub::DeviceSegmentedSort::StableSortPairsDescending(cub_tmp, cb, bits2, bits, rcs2, rcs, items, (int)Q, d_beg, d_end, st));
+    tip_pair_finish_kernel<<<(int)((Q * N + 255) / 256), 256, 0, st>>>(Q, N, L.cap, S, perm, ra, rb, m_rows, bits, rcs, d_cand,
+                                                                         d_out_ids, d_out_scores, counts);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    TIP_CHECK_CUDA(cudaMemcpyAsync(h_n_out, counts, (size_t)Q * 8, cudaMemcpyDeviceToHost, st));
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
+extern "C" int tip_top_triplets_per_pair_last_passes(void) { return g_last_pair_passes; }

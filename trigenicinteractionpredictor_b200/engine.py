@@ -9,6 +9,7 @@ CUDA kernels behind the C ABI (include/tip.h).  There is no CPU path.
     eng.loglik("train")                                # compute_likelihood (TIP.py:952-974)
     eng.top_triplets(thetas, ps, cand, known, n)       # exhaustive top-n of unseen triplets (tip_top_triplets)
     eng.top_triplets_per_gene(thetas, ps, cand, q, known, n)   # the same per query gene (tip_top_triplets_per_gene)
+    eng.top_triplets_per_pair(thetas, ps, cand, pr, known, n)  # the same per query pair (tip_top_triplets_per_pair)
 """
 from __future__ import annotations
 
@@ -537,6 +538,42 @@ class EMEngine:
         m = int(counts.max()) if n_query else 0
         ids = out_ids[:n_query * n].reshape(n_query, n, 3)[:, :m].cpu().numpy()
         sc = out_sc[:n_query * n].reshape(n_query, n)[:, :m].cpu().numpy()
+        return ids, sc, counts
+
+    @_on_device
+    def top_triplets_per_pair(self, theta_stack, p_stack, cand, pair_ranks, known, n: int):
+        """tip_top_triplets_per_pair: for every pair of ranks (into `cand`, [Q][2], either order), the `n` best triplets of
+        candidate genes that contain both, under the mean of S models; arguments otherwise as top_triplets.  Returns (ids
+        [Q][m][3] int32 in slot order, scores [Q][m] float64, counts [Q]), best first per pair, m = the largest count; a
+        pair's rows past its count are -1 / NaN."""
+        th = np.ascontiguousarray(theta_stack, dtype=np.float64)
+        pp = np.ascontiguousarray(p_stack, dtype=np.float64)
+        S = int(th.shape[0])
+        assert th.shape == (S, self.P, self.K) and pp.shape == (S, self.K, self.K, self.K, 2)
+        cand = np.ascontiguousarray(cand, dtype=np.int32)
+        pr = np.ascontiguousarray(np.asarray(pair_ranks, dtype=np.int32).reshape(-1, 2))
+        known = np.ascontiguousarray(known, dtype=np.uint64)
+        n_cand, n_pairs, n_known, n = int(cand.shape[0]), int(pr.shape[0]), int(known.shape[0]), int(n)
+        nb = ctypes.c_size_t(0)
+        _cabi.check(self.lib.tip_top_triplets_per_pair_workspace_bytes(n_cand, n_pairs, self.K, S, n_known, n, ctypes.byref(nb)),
+                    "tip_top_triplets_per_pair_workspace_bytes")
+        d_th = torch.from_numpy(th.reshape(-1)).to(self.device)
+        d_p = torch.from_numpy(pp.reshape(-1)).to(self.device)
+        d_cand = torch.from_numpy(cand).to(self.device)
+        d_pr = torch.from_numpy(pr.reshape(-1)).to(self.device)
+        d_known = torch.from_numpy(known.view(np.int64)).to(self.device) if n_known else None
+        ws = torch.empty(max(nb.value, 1), dtype=torch.uint8, device=self.device)
+        out_ids = torch.full((max(n_pairs * n, 1), 3), -1, dtype=torch.int32, device=self.device)
+        out_sc = torch.full((max(n_pairs * n, 1),), float("nan"), dtype=torch.float64, device=self.device)
+        counts = np.zeros(max(n_pairs, 1), dtype=np.int64)
+        _cabi.check(self.lib.tip_top_triplets_per_pair(
+            self.P, self.K, S, _ptr(d_th), _ptr(d_p), _ptr(d_cand), n_cand, _ptr(d_pr), n_pairs, _ptr(d_known), n_known, n,
+            _ptr(ws), nb.value, _ptr(out_ids), _ptr(out_sc), counts.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)),
+            self._stream()), "tip_top_triplets_per_pair")
+        counts = counts[:n_pairs]
+        m = int(counts.max()) if n_pairs else 0
+        ids = out_ids[:n_pairs * n].reshape(n_pairs, n, 3)[:, :m].cpu().numpy()
+        sc = out_sc[:n_pairs * n].reshape(n_pairs, n)[:, :m].cpu().numpy()
         return ids, sc, counts
 
     @_on_device

@@ -1,8 +1,8 @@
 """Rank the triplets a trained model has not seen: exhaustive top-N over all triplets of a gene set, on the device.
 
     python -m trigenicinteractionpredictor_b200.predict -t train0.dat -e test0.dat \\
-        -p results/Sample_0_K10.npz [-p results/Sample_1_K10.npz ...] [-n 100] [-g genes.txt] [-q queries.txt] \\
-        [--include-known] [-o predictions.tsv] [--device cuda:0]
+        -p results/Sample_0_K10.npz [-p results/Sample_1_K10.npz ...] [-n 100] [-g genes.txt] \\
+        [-q queries.txt | -r pairs.txt] [--include-known] [-o predictions.tsv] [--device cuda:0]
 
 The train / test files rebuild the model's digestion (gene ids in order of first appearance, TIP.py:321-423); every
 parameter file (the .npz that training with --save-params writes) must belong to it.  With several files the score of a
@@ -14,7 +14,13 @@ the id key as in the report's "ID of genes" column, and the gene names sorted by
 
 -q: one query gene name per line.  Then -n counts per query: for every query, in file order, the -n best triplets that
 contain it, the two partners taken from the -g genes plus the queries (default: all genes).  The header is
-"Query gene<TAB>Predicted Interaction<TAB>ID of genes<TAB>Genes" and every line starts with its query's name."""
+"Query gene<TAB>Predicted Interaction<TAB>ID of genes<TAB>Genes" and every line starts with its query's name.
+
+-r: one query pair per line, written nameA+nameB (the raw screens' notation for a double-mutant query) or as two
+whitespace-separated names.  Then -n counts per pair: for every pair, in file order, the -n best triplets that contain
+both genes, the third taken from the -g genes plus the pairs' genes (default: all genes).  The header is
+"Query pair<TAB>Predicted Interaction<TAB>ID of genes<TAB>Genes" and every line starts with its pair, written nameA+nameB.
+-q and -r exclude each other."""
 from __future__ import annotations
 
 import contextlib
@@ -24,6 +30,7 @@ import sys
 
 HEADER = "Predicted Interaction\tID of genes\tGenes\n"
 QUERY_HEADER = "Query gene\t" + HEADER
+PAIR_HEADER = "Query pair\t" + HEADER
 
 
 def _fail(msg: str) -> int:
@@ -33,12 +40,12 @@ def _fail(msg: str) -> int:
 
 def main(argv=None) -> int:
     argv = sys.argv[1:] if argv is None else argv
-    train = test = out = device = genes_file = queries_file = None
+    train = test = out = device = genes_file = queries_file = pairs_file = None
     params: list[str] = []
     top, include_known = 100, False
     try:
-        opts, rest = getopt.getopt(argv, "ht:e:p:n:g:q:o:", ["help", "train=", "test=", "params=", "top=", "genes=",
-                                                             "queries=", "include-known", "out=", "device="])
+        opts, rest = getopt.getopt(argv, "ht:e:p:n:g:q:r:o:", ["help", "train=", "test=", "params=", "top=", "genes=",
+                                                               "queries=", "pairs=", "include-known", "out=", "device="])
     except getopt.GetoptError as exc:
         return _fail("argument error: %s" % exc)
     if rest:
@@ -64,6 +71,8 @@ def main(argv=None) -> int:
             genes_file = arg
         elif opt in ("-q", "--queries"):
             queries_file = arg
+        elif opt in ("-r", "--pairs"):
+            pairs_file = arg
         elif opt == "--include-known":
             include_known = True
         elif opt in ("-o", "--out"):
@@ -72,7 +81,9 @@ def main(argv=None) -> int:
             device = arg
     if train is None or test is None or not params:
         return _fail("-t/--train, -e/--test and at least one -p/--params are required")
-    for path in [train, test, *params] + [f for f in (genes_file, queries_file) if f]:
+    if queries_file and pairs_file:
+        return _fail("-q/--queries and -r/--pairs exclude each other")
+    for path in [train, test, *params] + [f for f in (genes_file, queries_file, pairs_file) if f]:
         if not os.path.isfile(path):
             return _fail("the file %s does not exist" % path)
     if out is not None and os.path.dirname(os.path.abspath(out)) and not os.path.isdir(os.path.dirname(os.path.abspath(out))):
@@ -105,6 +116,32 @@ def main(argv=None) -> int:
             seen.add(g)
         if twice:
             return _fail("query genes listed twice: %s" % ", ".join(twice))
+    pairs = None
+    if pairs_file:
+        pairs = []
+        with open(pairs_file, encoding="utf-8") as fh:
+            for no, line in enumerate(fh, 1):
+                if not line.strip():
+                    continue
+                pair = line.strip().split("+") if "+" in line else line.split()
+                if len(pair) != 2 or not all(g.strip() for g in pair) or any(len(g.split()) != 1 for g in pair):
+                    return _fail("line %d of %s is not a pair nameA+nameB or nameA nameB: %r" % (no, pairs_file, line.strip()))
+                pairs.append((pair[0].strip(), pair[1].strip()))
+        if not pairs:
+            return _fail("the pair file %s names no pair" % pairs_file)
+        unknown = list(dict.fromkeys(g for p in pairs for g in p if g not in model.gene_id))
+        if unknown:
+            return _fail("pair genes not in the train / test files: %s" % ", ".join(unknown))
+        single = [p for p in pairs if p[0] == p[1]]
+        if single:
+            return _fail("a pair of one gene: %s" % "+".join(single[0]))
+        seen, twice = set(), []
+        for p in pairs:
+            if frozenset(p) in seen and "+".join(p) not in twice:
+                twice.append("+".join(p))
+            seen.add(frozenset(p))
+        if twice:
+            return _fail("pairs listed twice: %s" % ", ".join(twice))
     sets = []
     for path in params:
         try:
@@ -114,7 +151,11 @@ def main(argv=None) -> int:
     if len({th.shape[1] for th, _ in sets}) != 1:
         return _fail("the parameter files have different K")
 
-    if queries is None:
+    if pairs is not None:
+        per = model.predict_top_triplets_per_pair(pairs, top, genes=genes, exclude_known=not include_known, params=sets)
+        text = PAIR_HEADER + "".join(p[0] + "+" + p[1] + "\t" + str(s) + "\t" + key + "\t" + names + "\n"
+                                     for p in pairs for s, key, names in per[p])
+    elif queries is None:
         rows = model.predict_top_triplets(top, genes=genes, exclude_known=not include_known, params=sets)
         text = HEADER + "".join(str(s) + "\t" + key + "\t" + names + "\n" for s, key, names in rows)
     else:
