@@ -165,7 +165,8 @@ int tip_score(int P, int K, const int32_t *d_g1, const int32_t *d_g2, const int3
  *                   tp, fp, fn, tn, bit pattern of cut_value}
  * positives_number = int(positives_fraction * T) computed by the caller (TIP.py:592); cut_value is
  * the positives_number-th largest score, or 0.0 when positives_number >= T (TIP.py:595-599).
- * The ratios are formed by the caller in Python so ZeroDivisionError behaves as in the reference. */
+ * The ratios are formed by the caller in Python so ZeroDivisionError behaves as in the reference.
+ * Needs 0 < T < 2^31 (the negatives before each rank are counted by an int32 scan); refused otherwise. */
 int tip_metrics_workspace_bytes(int64_t T, size_t *bytes);
 int tip_metrics(const double *d_scores, const int32_t *d_labels, int64_t T, int64_t positives_number,
                 void *d_ws, size_t ws_bytes, int64_t *d_out, void *stream);

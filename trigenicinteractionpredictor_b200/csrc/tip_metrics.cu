@@ -148,6 +148,9 @@ extern "C" int tip_metrics(const double *d_scores, const int32_t *d_labels, int6
 {
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     TIP_REQUIRE(T > 0, "tip_metrics: empty test set (the reference raises ZeroDivisionError; the caller handles it)");
+    // the exclusive scan of the int32 negative flags accumulates in int32 (CUB takes the input type), so neg_before
+    // would wrap past 2^31 - 1 negatives
+    TIP_REQUIRE(T < (1ll << 31), "tip_metrics: T = %lld; need T < 2^31", (long long)T);
     TIP_REQUIRE(positives_number >= 0, "tip_metrics: negative positives_number");
     const size_t need = metrics_layout(T, nullptr, nullptr);
     TIP_REQUIRE(d_ws != nullptr && ws_bytes >= need, "tip_metrics: workspace too small (%zu < %zu)", ws_bytes, need);
