@@ -239,6 +239,22 @@ int tip_top_triplets_per_pair(int P, int K, int S, const double *d_theta, const 
 /* sweeps the last tip_top_triplets_per_pair of this thread ran (measurement) */
 int tip_top_triplets_per_pair_last_passes(void);
 
+/* ---- histogram of the scores of all triplets of a candidate gene list (ranks of held-out triplets, DESIGN §4.8) ----
+ * Candidates and parameters as tip_top_triplets.  Every one of the C(n_cand, 3) triplets is scored by the sweep of
+ * tip_top_triplets (the bits of the ensemble SUM over the S sets) and counted, never stored, into d_hist_out[n_binades *
+ * 2^log2_bins + 2] (uint64, zeroed by the call).  With key(x) = bits(x) >> (52 - log2_bins) and key_top = ((top_exp + 1)
+ * << log2_bins) - 1, a score goes to bin 0 when key > key_top, to bin 1 + key_top - key when key_top - key < n_binades *
+ * 2^log2_bins, and to the last bin otherwise (everything below the range, exact zeros included).  Bin 0 holds the
+ * highest scores.  *h_top_exp returns the biased exponent of the range's top binade: that of an upper bound of the
+ * scores, sum_s max(p_s[..][1]) (largest row sum of theta_s)^3.  Bad arguments are refused before any device work.
+ * Synchronises the stream.  Limits: n_cand <= 2^21, S * K <= 384, 0 <= log2_bins <= 10, n_binades >= 1,
+ * n_binades * 2^log2_bins <= 2^14, and the Q tile plus the bins must fit one block's shared memory.  Precondition:
+ * finite, non-negative parameters.  d_ws: tip_score_histogram_workspace_bytes() bytes, O(n_cand S K + n_cand S K^2). */
+int tip_score_histogram_workspace_bytes(int n_cand, int K, int S, int log2_bins, int n_binades, size_t *bytes);
+int tip_score_histogram(int P, int K, int S, const double *d_theta, const double *d_p, const int32_t *d_cand, int n_cand,
+                        int log2_bins, int n_binades, int *h_top_exp, uint64_t *d_hist_out, void *d_ws, size_t ws_bytes,
+                        void *stream);
+
 /* ---- testResultsReducer.py:160-184: mean / median / standard deviation of every test triplet across samples ----
  * d_scores[S][T]: score of triplet t in sample j at [j * T + t]; d_n[t] (or NULL = S) = how many leading samples of
  * triplet t are valid.  mean = sequential sum in sample order / n; median = the reference's rule (ascending sort;

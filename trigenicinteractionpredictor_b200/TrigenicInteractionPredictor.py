@@ -766,6 +766,124 @@ class Model:
             return np.empty(0, dtype=np.uint64)
         return np.unique(np.concatenate(parts)).astype(np.uint64)
 
+    def _train_packed(self, cand):
+        """Sorted packed rank triples of the keys of links (not test_links) whose three genes are distinct candidates."""
+        if len(self.links) == 0:
+            return np.empty(0, dtype=np.uint64)
+        rank = np.full(self.P, -1, dtype=np.int64)
+        rank[cand] = np.arange(cand.shape[0], dtype=np.int64)
+        g = [np.asarray(x.cpu().numpy() if _is_torch(x) else x, dtype=np.int64) for x in self._soa(self.links)[:3]]
+        r = np.sort(np.stack([rank[g[0]], rank[g[1]], rank[g[2]]], axis=1), axis=1)
+        r = r[(r[:, 0] >= 0) & (r[:, 0] < r[:, 1]) & (r[:, 1] < r[:, 2])]
+        return np.unique((r[:, 0] << 42) | (r[:, 1] << 21) | r[:, 2]).astype(np.uint64)
+
+    def rank_held_out(self, n_exact=100000, genes=None, params=None, recall_at=(100, 1000, 10000, 100000)):
+        """Where the test triplets land among all unseen triplets (addition; DESIGN §4.8).
+
+        The universe U is every triplet of three distinct genes of `genes` (names; default all P genes) that is not a key
+        of links; test keys stay in U.  Triplets are ordered as in predict_top_triplets (score descending, then the
+        triplets' positions in the decimal-string order of the candidate ids), scored by the current theta / pr or by the
+        mean over the sets of `params`.  A test triplet's rank is 1 + the number of triplets of U before it.  The first
+        `n_exact` triplets of U are listed exactly, so a test triplet among them gets its exact rank; every other one
+        gets an interval [rank_lo, rank_hi] from a histogram of all scores, which always contains the exact rank
+        (rank_lo == rank_hi only when the rank is exact).  Test keys that are also keys of links, or that name a gene
+        outside `genes`, have no rank and are counted as excluded.  Labels follow calculate_metrics: 0 if n0 != 0 else 1.
+
+        Returns a dict:
+          rows: [[key "a_b_c", names, label, score, rank_lo, rank_hi], ...] for the ranked test triplets, in rank order;
+          universe, n_exact, positives, negatives, excluded_train, excluded_genes;
+          recall_at: {N: {"positives": (lo, hi), "negatives": (lo, hi)}}, the fraction ranked <= N (lo == hi when exact,
+            always when N <= n_exact);
+          median_rank: (lo, hi) of the positives' median rank;
+          auc: (lo, hi) of the mean over positives of (|U| - rank) / (|U| - 1).
+        Values that need a positive or |U| > 1 are None without them."""
+        who = "rank_held_out"
+        sets = self._prediction_sets(params, who)
+        K = sets[0][0].shape[1]
+        if len(self.test_links) == 0:
+            raise ValueError(who + ": the model has no test links")
+        if genes is not None:
+            missing = [g for g in genes if g not in self.gene_id]
+            if missing:
+                raise ValueError("unknown gene names: %s" % ", ".join(dict.fromkeys(missing)))
+        n_exact = int(n_exact)
+        if n_exact < 0 or n_exact >= 1 << 28:
+            raise ValueError(who + ": n_exact must be in [0, 2^28) (got %d)" % n_exact)
+        recall_at = [int(x) for x in recall_at]
+        ids = set(range(self.P)) if genes is None else {self.gene_id[g] for g in genes}
+        cand = np.array(sorted(ids, key=str), dtype=np.int32)
+        n = int(cand.shape[0])
+        rank = np.full(self.P, -1, dtype=np.int64)
+        rank[cand] = np.arange(n, dtype=np.int64)
+        train = self._train_packed(cand)
+        universe = (n * (n - 1) // 2 * (n - 2) // 3 if n >= 3 else 0) - int(train.shape[0])
+
+        t1, t2, t3, t_n0, _ = [np.asarray(x.cpu().numpy() if _is_torch(x) else x, dtype=np.int64) for x in self._soa(self.test_links)]
+        r = np.sort(np.stack([rank[t1], rank[t2], rank[t3]], axis=1), axis=1)
+        triplet = (r[:, 0] >= 0) & (r[:, 0] < r[:, 1]) & (r[:, 1] < r[:, 2])
+        packed = ((r[:, 0] << 42) | (r[:, 1] << 21) | r[:, 2]).astype(np.uint64)
+        at = np.minimum(np.searchsorted(train, packed), max(len(train) - 1, 0))
+        in_train = triplet & (train[at] == packed) if len(train) else np.zeros_like(triplet)
+        sel = np.flatnonzero(triplet & ~in_train)
+        packed, r = packed[sel], r[sel]
+        labels = np.where(t_n0[sel] != 0, 0, 1)
+
+        thetas = np.stack([th for th, _ in sets])
+        prs = np.stack([pr for _, pr in sets])
+        S = len(sets)
+        eng = self._prediction_engine(K)
+        # exact ranks at the top: the first n_exact triplets of U, and where the test triplets sit among them
+        m_exact = min(n_exact, universe)
+        pos = np.full(len(sel), -1, dtype=np.int64)
+        top_sc = np.empty(0)
+        if m_exact > 0:
+            top_ids, top_sc = eng.top_triplets(thetas, prs, cand, train, m_exact)
+            tr = np.sort(rank[top_ids.astype(np.int64)], axis=1)
+            pos = eng.find_keys(((tr[:, 0] << 42) | (tr[:, 1] << 21) | tr[:, 2]).astype(np.uint64), packed)
+        # every other test triplet: an interval from the histogram of all C(n, 3) scores minus the train keys
+        layout, hist = eng.score_histogram(thetas, prs, cand)
+        t_sum = eng.score_sum(thetas, prs, cand[r])
+        tk = np.stack([(train >> np.uint64(s)) & np.uint64((1 << 21) - 1) for s in (42, 21, 0)], axis=1).astype(np.int64)
+        k_first, k_last = layout.bins_widened(eng.score_sum(thetas, prs, cand[tk]))
+        t_first, t_last = layout.bins_widened(t_sum)
+        nb = layout.n_bins
+        above = np.concatenate([[0], np.cumsum(hist)])                       # above[b]: triplets in bins < b
+        k_surely = np.concatenate([[0], np.cumsum(np.bincount(k_last, minlength=nb))])    # train keys surely in bins < b
+        k_maybe = np.concatenate([[0], np.cumsum(np.bincount(k_first, minlength=nb))])    # ... possibly in bins < b
+        lo = 1 + above[t_first] - k_maybe[t_first]
+        hi = np.minimum(above[t_last + 1] - k_surely[t_last + 1], universe)
+        lo = np.maximum(lo, m_exact + 1)
+        score = t_sum / S
+        exact = pos >= 0
+        lo[exact] = hi[exact] = pos[exact] + 1
+        score[exact] = top_sc[pos[exact]]
+
+        order = np.lexsort((packed, hi, lo))
+        g = cand[r[order]].astype(np.int64)
+        names = np.array(self._genes_in_id_order())[g]
+        names.sort(axis=1)
+        rows = [list(x) for x in zip([f"{a}_{b}_{c}" for a, b, c in g.tolist()], ["_".join(t) for t in names.tolist()],
+                                     labels[order].tolist(), score[order].tolist(), lo[order].tolist(), hi[order].tolist())]
+        positive = labels == 1
+        n_pos, n_neg = int(positive.sum()), int((~positive).sum())
+
+        def frac(mask, N):
+            total = int(mask.sum())
+            if total == 0:
+                return None
+            return (int((hi[mask] <= N).sum()) / total, int((lo[mask] <= N).sum()) / total)
+
+        res = {"rows": rows, "universe": universe, "n_exact": m_exact, "positives": n_pos, "negatives": n_neg,
+               "excluded_train": int(in_train.sum()), "excluded_genes": int((~triplet).sum()),
+               "recall_at": {N: {"positives": frac(positive, N), "negatives": frac(~positive, N)} for N in recall_at},
+               "median_rank": None, "auc": None}
+        if n_pos:
+            res["median_rank"] = (float(np.median(lo[positive])), float(np.median(hi[positive])))
+            if universe > 1:
+                res["auc"] = (float(np.mean((universe - hi[positive]) / (universe - 1))),
+                              float(np.mean((universe - lo[positive]) / (universe - 1))))
+        return res
+
     # ------------------------------------------------------------------------------------------
     # report (TIP.py:793-904)
     # ------------------------------------------------------------------------------------------

@@ -21,7 +21,11 @@
 // loop and the epilogue with tip_predict_pass_kernel).  Each query has its own threshold, survivor count, histogram and
 // buffer; its first threshold is the best score of a per-query sample, and sweeps after the first score only the queries
 // whose threshold has not settled.  A segmented sort orders every query's buffer.
+//
+// Histogram of all scores (tip_score_histogram): the same sweep as tip_top_triplets, counting every score into a fixed
+// log-spaced histogram of its bits (tip_hist_pass_kernel); the ranks of held-out triplets among all triplets follow from it.
 #include <algorithm>
+#include <cmath>
 #include <vector>
 
 #include <cub/device/device_radix_sort.cuh>
@@ -1755,3 +1759,256 @@ extern "C" int tip_top_triplets_per_pair(int P, int K, int S, const double *d_th
 }
 
 extern "C" int tip_top_triplets_per_pair_last_passes(void) { return g_last_pair_passes; }
+
+// ---- tip_score_histogram ----
+// Every triplet of the candidates is scored by the same work items, Q tiles and DMMA block loop as tip_predict_pass_kernel,
+// and counted into a fixed log-spaced histogram of the bits of its ensemble sum; no score is stored.  With B = 2^log2_bins
+// bins per binade, key(x) = bits(x) >> (52 - log2_bins) (the biased exponent and the top log2_bins mantissa bits) and
+// key_top = ((top_exp + 1) << log2_bins) - 1, the bin of a score is
+//     0                   when key > key_top (above the range)
+//     1 + key_top - key   when key_top - key < n_binades B
+//     n_binades B + 1     otherwise (below the range, down to exact zeros)
+// so bin 0 holds the highest scores, every bin is an interval of score bits, and the host bins any double the same way.
+namespace tip {
+namespace {
+
+constexpr int kHistMaxLog2Bins = 10;
+constexpr long long kHistMaxRange = 1ll << 14;   // n_binades * B: shared bins beside the Q tile
+
+__host__ __device__ inline int hist_bin(unsigned long long bits, int shift, unsigned long long key_top, unsigned long long n_range)
+{
+    const unsigned long long key = bits >> shift;
+    if (key > key_top) return 0;
+    const unsigned long long d = key_top - key;
+    return d < n_range ? (int)d + 1 : (int)n_range + 1;
+}
+
+// bound[0] = sum_s max(p_s[.][.][.][1]) T_s^3 >= every ensemble sum of scores (non-negative parameters, T_s the largest
+// row sum of theta_s over the candidates); one block
+__global__ void tip_hist_bound_kernel(int S, int K, const double *__restrict__ p, const unsigned long long *__restrict__ T,
+                                      double *__restrict__ bound)
+{
+    __shared__ double sh_max[256];
+    const long long KKK = (long long)K * K * K;
+    double sum = 0.0;
+    for (int s = 0; s < S; ++s) {
+        double mx = 0.0;
+        for (long long e = threadIdx.x; e < KKK; e += blockDim.x) mx = fmax(mx, p[((long long)s * KKK + e) * 2 + 1]);
+        sh_max[threadIdx.x] = mx;
+        __syncthreads();
+        for (int w = blockDim.x / 2; w > 0; w >>= 1) {
+            if ((int)threadIdx.x < w) sh_max[threadIdx.x] = fmax(sh_max[threadIdx.x], sh_max[threadIdx.x + w]);
+            __syncthreads();
+        }
+        const double t = __longlong_as_double((long long)T[s]);
+        sum += sh_max[0] * t * t * t;
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) bound[0] = sum;
+}
+
+struct HistPassArgs {
+    int n, SK, SKP, K;
+    const double *tcat;             // [n_pad][SKP]
+    const double *W;                // [S][n][K][K]
+    long long n_items;
+    int shift;                      // 52 - log2_bins
+    unsigned long long key_top, n_range;
+    int n_bins;                     // n_range + 2
+    unsigned long long *cursor;     // work-item cursor
+    unsigned long long *hist;       // [n_bins]
+};
+
+// epilogue of a block: every valid score into its shared bin, one shared atomic per distinct bin of the warp
+__device__ __forceinline__ void hist_block(const double (&acc)[4][4][2], int lane, int ra0, int rc0, int row_end, int n,
+                                           const HistPassArgs &A, unsigned *sh_hist)
+{
+#pragma unroll
+    for (int f = 0; f < 32; ++f) {
+        const int mi = f >> 3, ni = (f >> 1) & 3, e = f & 1;
+        const int ra = ra0 + mi * 8, rc = rc0 + ni * 8 + e;
+        const int bin = (ra < row_end && rc < n)
+                            ? hist_bin((unsigned long long)__double_as_longlong(acc[mi][ni][e]), A.shift, A.key_top, A.n_range)
+                            : -1;
+        const unsigned peers = __match_any_sync(0xffffffffu, bin);
+        if (bin >= 0 && lane == __ffs(peers) - 1) atomicAdd(sh_hist + bin, (unsigned)__popc(peers));
+    }
+}
+
+__device__ __forceinline__ void hist_flush(unsigned *sh_hist, unsigned long long *hist, int n_bins)
+{
+    for (int i = threadIdx.x; i < n_bins; i += kPredThreads) {
+        if (sh_hist[i]) atomicAdd(hist + i, (unsigned long long)sh_hist[i]);
+        sh_hist[i] = 0;
+    }
+}
+
+// the sweep of tip_predict_pass_kernel (same items, Q tiles and DMMA blocks) with a counting epilogue
+__global__ void __launch_bounds__(kPredThreads) tip_hist_pass_kernel(HistPassArgs A)
+{
+    extern __shared__ __align__(16) unsigned char smem[];
+    const int qs = q_stride(A.SKP);
+    double *Q = reinterpret_cast<double *>(smem);                                   // [64][qs]
+    unsigned *sh_hist = reinterpret_cast<unsigned *>(Q + (size_t)kPredRows * qs);  // [n_bins]
+    __shared__ long long sh_item;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int wr = warp & 1, wc = warp >> 1;
+    const int gq = lane >> 2, tq = lane & 3;
+    for (int i = tid; i < A.n_bins; i += kPredThreads) sh_hist[i] = 0;
+    double since_flush = 0.0;   // as in tip_predict_pass_kernel
+    const int n = A.n, SKP = A.SKP, K = A.K;
+
+    for (;;) {
+        __syncthreads();
+        if (tid == 0) sh_item = (long long)atomicAdd(A.cursor, 1ull);
+        __syncthreads();
+        const long long item = sh_item;
+        if (item >= A.n_items) break;
+        int jl = 1, jh = n - 2;
+        while (jl < jh) {
+            const int mid = (jl + jh + 1) >> 1;
+            if (items_before(mid) <= item) jl = mid; else jh = mid - 1;
+        }
+        const int j = jl;
+        const int a0 = (int)(item - items_before(j)) * kPredRows;
+        const int rows = min(kPredRows, j - a0);
+        const int n_c = n - 1 - j;
+
+        form_q_tile(Q, qs, A.tcat, SKP, A.SK, K, a0, rows, A.W + (long long)j * K * K, (long long)n * K * K);
+        __syncthreads();
+
+        if (wr * 32 < rows) {
+            const double *Qw = Q + (wr * 32 + gq) * qs + tq;
+            for (int c0 = j + 1 + wc * 32; c0 < n; c0 += 64) {
+                double acc[4][4][2];
+                dmma_block(acc, Qw, qs, A.tcat + (long long)(c0 + gq) * SKP + tq, SKP);
+                hist_block(acc, lane, a0 + wr * 32 + gq, c0 + 2 * tq, j, n, A, sh_hist);
+            }
+        }
+        since_flush += (double)rows * n_c;
+        if (since_flush > 2.0e9) {
+            __syncthreads();
+            hist_flush(sh_hist, A.hist, A.n_bins);
+            since_flush = 0.0;
+        }
+    }
+    hist_flush(sh_hist, A.hist, A.n_bins);
+}
+
+struct HistLayout {
+    size_t o_tcat, o_W, o_T, o_bound, o_cursor, total;
+    int n_pad, SKP;
+};
+
+HistLayout hist_layout(int n, int K, int S)
+{
+    HistLayout L{};
+    L.n_pad = (n + 63) / 64 * 64 + 64;
+    L.SKP = (S * K + 3) / 4 * 4;
+    size_t off = 0;
+    L.o_tcat = off;   off += a256((size_t)L.n_pad * L.SKP * 8);
+    L.o_W = off;      off += a256((size_t)S * n * K * K * 8);
+    L.o_T = off;      off += a256((size_t)S * 8);
+    L.o_bound = off;  off += 256;
+    L.o_cursor = off; off += 256;
+    L.total = off + 256;
+    return L;
+}
+
+size_t hist_smem(int SKP, long long n_bins) { return (size_t)kPredRows * q_stride(SKP) * 8 + (size_t)n_bins * 4; }
+
+}  // namespace
+}  // namespace tip
+
+static bool hist_args_ok(int n_cand, int K, int S, int log2_bins, int n_binades)
+{
+    return predict_args_ok(n_cand, K, S, 0, 0) && log2_bins >= 0 && log2_bins <= kHistMaxLog2Bins && n_binades >= 1 &&
+           ((long long)n_binades << log2_bins) <= kHistMaxRange;
+}
+
+#define TIP_HIST_LIMITS "n_cand <= 2^21, 1 <= K <= %d, S >= 1, S*K <= %d, 0 <= log2_bins <= %d, n_binades >= 1, " \
+                        "n_binades * 2^log2_bins <= %lld"
+
+extern "C" int tip_score_histogram_workspace_bytes(int n_cand, int K, int S, int log2_bins, int n_binades, size_t *bytes)
+{
+    TIP_REQUIRE(bytes != nullptr && hist_args_ok(n_cand, K, S, log2_bins, n_binades),
+                "tip_score_histogram_workspace_bytes: bad arguments (" TIP_HIST_LIMITS ")", TIP_MAX_K, kPredMaxSK,
+                kHistMaxLog2Bins, kHistMaxRange);
+    *bytes = hist_layout(n_cand, K, S).total;
+    return 0;
+}
+
+extern "C" int tip_score_histogram(int P, int K, int S, const double *d_theta, const double *d_p, const int32_t *d_cand,
+                                   int n_cand, int log2_bins, int n_binades, int *h_top_exp, uint64_t *d_hist_out, void *d_ws,
+                                   size_t ws_bytes, void *stream)
+{
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    TIP_REQUIRE(P > 0 && n_cand <= P && hist_args_ok(n_cand, K, S, log2_bins, n_binades) && h_top_exp != nullptr,
+                "tip_score_histogram: bad arguments (P > 0, n_cand <= P, " TIP_HIST_LIMITS ")", TIP_MAX_K, kPredMaxSK,
+                kHistMaxLog2Bins, kHistMaxRange);
+    TIP_REQUIRE(d_theta && d_p && (d_cand || n_cand == 0) && d_hist_out, "tip_score_histogram: null pointer");
+    const int n = n_cand;
+    const HistLayout L = hist_layout(n, K, S);
+    TIP_REQUIRE(d_ws != nullptr && ws_bytes >= L.total, "tip_score_histogram: workspace too small (%zu < %zu)", ws_bytes, L.total);
+    const long long n_range = (long long)n_binades << log2_bins, n_bins = n_range + 2;
+    const size_t smem = hist_smem(L.SKP, n_bins);
+    int dev = 0, optin = 0;
+    TIP_CHECK_CUDA(cudaGetDevice(&dev));
+    TIP_CHECK_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    TIP_REQUIRE(smem + 64 <= (size_t)optin,
+                "tip_score_histogram: the Q tile of S*K = %d and %lld bins need %zu bytes of shared memory (the device has %d)",
+                S * K, n_bins, smem, optin);
+    static int smem_set = 0;
+    if ((int)smem > smem_set && smem > 48 * 1024) {
+        TIP_CHECK_CUDA(cudaFuncSetAttribute(tip_hist_pass_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        smem_set = (int)smem;
+    }
+    int per_sm = 0;
+    TIP_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tip_hist_pass_kernel, kPredThreads, smem));
+    TIP_REQUIRE(per_sm > 0, "tip_score_histogram: S*K = %d does not fit one block's shared memory", S * K);
+
+    char *base = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(d_ws) + 255) / 256 * 256);
+    double *tcat = reinterpret_cast<double *>(base + L.o_tcat), *W = reinterpret_cast<double *>(base + L.o_W);
+    auto *T = reinterpret_cast<unsigned long long *>(base + L.o_T);
+    double *bound = reinterpret_cast<double *>(base + L.o_bound);
+    auto *cursor = reinterpret_cast<unsigned long long *>(base + L.o_cursor);
+    TIP_CHECK_CUDA(cudaMemsetAsync(d_hist_out, 0, (size_t)n_bins * 8, st));
+    *h_top_exp = 0;
+    if (n < 3) {
+        TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+        return 0;
+    }
+    {
+        const long long work = (long long)L.n_pad * L.SKP + (long long)S * n * K * K;
+        tip_predict_prep_kernel<<<(int)std::min<long long>((work + 255) / 256, (long long)sm_count() * 16), 256, 0, st>>>(
+            S, P, K, n, L.n_pad, L.SKP, d_theta, d_p, d_cand, tcat, W);
+        TIP_CHECK_CUDA(cudaGetLastError());
+        TIP_CHECK_CUDA(cudaMemsetAsync(T, 0, (size_t)S * 8, st));
+        tip_query_rowsum_kernel<<<(n + 255) / 256, 256, 0, st>>>(n, S, K, L.SKP, tcat, T);
+        TIP_CHECK_CUDA(cudaGetLastError());
+        tip_hist_bound_kernel<<<1, 256, 0, st>>>(S, K, d_p, T, bound);
+        TIP_CHECK_CUDA(cudaGetLastError());
+    }
+    double h_bound = 0.0;
+    TIP_CHECK_CUDA(cudaMemcpyAsync(&h_bound, bound, 8, cudaMemcpyDeviceToHost, st));
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    // the range's top binade holds the bound (with a margin for its rounding); a score above it lands in bin 0
+    const double hb = h_bound * (1.0 + 1e-9);
+    const int top_exp = std::isfinite(hb) ? (int)((unsigned long long)__builtin_bit_cast(long long, hb) >> 52) & 0x7FF : 2046;
+    *h_top_exp = std::min(top_exp, 2046);
+
+    HistPassArgs A{};
+    A.n = n; A.SK = S * K; A.SKP = L.SKP; A.K = K;
+    A.tcat = tcat; A.W = W;
+    A.n_items = items_before(n - 1);
+    A.shift = 52 - log2_bins;
+    A.key_top = (((unsigned long long)*h_top_exp + 1) << log2_bins) - 1;
+    A.n_range = (unsigned long long)n_range;
+    A.n_bins = (int)n_bins;
+    A.cursor = cursor; A.hist = reinterpret_cast<unsigned long long *>(d_hist_out);
+    TIP_CHECK_CUDA(cudaMemsetAsync(cursor, 0, 8, st));
+    tip_hist_pass_kernel<<<(int)std::min<long long>((long long)sm_count() * per_sm, A.n_items), kPredThreads, smem, st>>>(A);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}

@@ -10,11 +10,13 @@ CUDA kernels behind the C ABI (include/tip.h).  There is no CPU path.
     eng.top_triplets(thetas, ps, cand, known, n)       # exhaustive top-n of unseen triplets (tip_top_triplets)
     eng.top_triplets_per_gene(thetas, ps, cand, q, known, n)   # the same per query gene (tip_top_triplets_per_gene)
     eng.top_triplets_per_pair(thetas, ps, cand, pr, known, n)  # the same per query pair (tip_top_triplets_per_pair)
+    eng.score_histogram(thetas, ps, cand)              # histogram of all C(n, 3) scores (tip_score_histogram)
 """
 from __future__ import annotations
 
 import ctypes
 import functools
+from typing import NamedTuple
 
 import numpy as np
 import torch
@@ -25,6 +27,35 @@ from . import dist as _dist
 # libtip.so keeps per-process caches that belong to ONE device (SM count, function attributes, the constant-bank
 # staging buffer, events, the host-entry scratch): one CUDA device per process, the first engine decides which.
 _PROCESS_DEVICE = None
+
+
+class BinLayout(NamedTuple):
+    """Bins of tip_score_histogram (DESIGN §4.8): 2^log2_bins bins per binade over n_binades binades, the top one of
+    biased exponent top_exp; bin 0 is above the range, the last bin below it."""
+    log2_bins: int
+    n_binades: int
+    top_exp: int
+
+    @property
+    def n_bins(self) -> int:
+        return (self.n_binades << self.log2_bins) + 2
+
+    def bins(self, values) -> np.ndarray:
+        """The bin of every double, by the integer formula the kernel uses: bit-exact on any value."""
+        bits = np.ascontiguousarray(values, dtype=np.float64).view(np.uint64)
+        key = bits >> np.uint64(52 - self.log2_bins)
+        key_top = np.uint64(((self.top_exp + 1) << self.log2_bins) - 1)
+        n_range = self.n_binades << self.log2_bins
+        d = (key_top - np.minimum(key, key_top)).astype(np.int64)
+        return np.where(key > key_top, 0, np.where(d < n_range, d + 1, n_range + 1)).astype(np.int64)
+
+    def bins_widened(self, values, rel: float = 2.0 ** -40):
+        """(first, last): the bins of values * (1 + rel) and values * (1 - rel), for non-negative values.  A score
+        computed in another summation order lies in one of the bins first..last; first < last only when the value is
+        within a relative `rel` of a bin edge."""
+        v = np.asarray(values, dtype=np.float64)
+        with np.errstate(over="ignore"):
+            return self.bins(v * (1.0 + rel)), self.bins(v * (1.0 - rel))
 
 
 def _ptr(t):
@@ -575,6 +606,65 @@ class EMEngine:
         ids = out_ids[:n_pairs * n].reshape(n_pairs, n, 3)[:, :m].cpu().numpy()
         sc = out_sc[:n_pairs * n].reshape(n_pairs, n)[:, :m].cpu().numpy()
         return ids, sc, counts
+
+    @_on_device
+    def score_histogram(self, theta_stack, p_stack, cand, log2_bins: int = 7, n_binades: int = 64):
+        """tip_score_histogram: every score (the bits of the sum over the S sets) of the C(n, 3) triplets of the candidate
+        genes, counted into log-spaced bins; arguments as top_triplets.  Returns (BinLayout, counts [n_bins] int64),
+        bin 0 the highest scores."""
+        th = np.ascontiguousarray(theta_stack, dtype=np.float64)
+        pp = np.ascontiguousarray(p_stack, dtype=np.float64)
+        S = int(th.shape[0])
+        assert th.shape == (S, self.P, self.K) and pp.shape == (S, self.K, self.K, self.K, 2)
+        cand = np.ascontiguousarray(cand, dtype=np.int32)
+        n_cand = int(cand.shape[0])
+        nb = ctypes.c_size_t(0)
+        _cabi.check(self.lib.tip_score_histogram_workspace_bytes(n_cand, self.K, S, int(log2_bins), int(n_binades),
+                                                                 ctypes.byref(nb)), "tip_score_histogram_workspace_bytes")
+        d_th = torch.from_numpy(th.reshape(-1)).to(self.device)
+        d_p = torch.from_numpy(pp.reshape(-1)).to(self.device)
+        d_cand = torch.from_numpy(cand).to(self.device)
+        ws = torch.empty(max(nb.value, 1), dtype=torch.uint8, device=self.device)
+        hist = torch.empty((int(n_binades) << int(log2_bins)) + 2, dtype=torch.int64, device=self.device)
+        top = ctypes.c_int(0)
+        _cabi.check(self.lib.tip_score_histogram(self.P, self.K, S, _ptr(d_th), _ptr(d_p), _ptr(d_cand), n_cand, int(log2_bins),
+                                                 int(n_binades), ctypes.byref(top), _ptr(hist), _ptr(ws), nb.value,
+                                                 self._stream()), "tip_score_histogram")
+        return BinLayout(int(log2_bins), int(n_binades), int(top.value)), hist.cpu().numpy()
+
+    @_on_device
+    def score_sum(self, theta_stack, p_stack, ids):
+        """Sum over the S parameter sets, in set order, of tip_score (do_prediction at rating 1) of the triplets `ids`
+        [T][3] (gene ids in slot order).  Returns float64 [T]."""
+        th = np.ascontiguousarray(theta_stack, dtype=np.float64)
+        pp = np.ascontiguousarray(p_stack, dtype=np.float64)
+        S = int(th.shape[0])
+        assert th.shape == (S, self.P, self.K) and pp.shape == (S, self.K, self.K, self.K, 2)
+        g = torch.from_numpy(np.ascontiguousarray(np.asarray(ids, dtype=np.int32).reshape(-1, 3).T)).to(self.device)
+        T = int(g.shape[1])
+        acc = torch.zeros(T, dtype=torch.float64, device=self.device)
+        if T == 0:
+            return acc.cpu().numpy()
+        out = torch.empty(T, dtype=torch.float64, device=self.device)
+        for s in range(S):
+            d_th = torch.from_numpy(th[s].reshape(-1)).to(self.device)
+            d_p = torch.from_numpy(pp[s].reshape(-1)).to(self.device)
+            _cabi.check(self.lib.tip_score(self.P, self.K, _ptr(g[0]), _ptr(g[1]), _ptr(g[2]), T, _ptr(d_th), _ptr(d_p),
+                                           _ptr(out), self._stream()), "tip_score")
+            acc += out
+        return acc.cpu().numpy()
+
+    @_on_device
+    def find_keys(self, keys, queries):
+        """Position in `keys` (distinct uint64) of every query key, or -1: a sort and a binary search per query on the
+        device."""
+        k = torch.from_numpy(np.ascontiguousarray(keys, dtype=np.uint64).view(np.int64)).to(self.device)
+        q = torch.from_numpy(np.ascontiguousarray(queries, dtype=np.uint64).view(np.int64)).to(self.device)
+        if k.numel() == 0 or q.numel() == 0:
+            return np.full(q.numel(), -1, dtype=np.int64)
+        sk, perm = torch.sort(k)      # packed rank triples are < 2^63: the signed order is the unsigned one
+        i = torch.searchsorted(sk, q).clamp_(max=k.numel() - 1)
+        return torch.where(sk[i] == q, perm[i], torch.full_like(i, -1)).cpu().numpy()
 
     @_on_device
     def metric_counts(self, scores: torch.Tensor, positives_number: int) -> dict:

@@ -2,7 +2,7 @@
 
     python -m trigenicinteractionpredictor_b200.predict -t train0.dat -e test0.dat \\
         -p results/Sample_0_K10.npz [-p results/Sample_1_K10.npz ...] [-n 100] [-g genes.txt] \\
-        [-q queries.txt | -r pairs.txt] [--include-known] [-o predictions.tsv] [--device cuda:0]
+        [-q queries.txt | -r pairs.txt | --held-out] [--include-known] [-o predictions.tsv] [--device cuda:0]
 
 The train / test files rebuild the model's digestion (gene ids in order of first appearance, TIP.py:321-423); every
 parameter file (the .npz that training with --save-params writes) must belong to it.  With several files the score of a
@@ -20,7 +20,15 @@ contain it, the two partners taken from the -g genes plus the queries (default: 
 whitespace-separated names.  Then -n counts per pair: for every pair, in file order, the -n best triplets that contain
 both genes, the third taken from the -g genes plus the pairs' genes (default: all genes).  The header is
 "Query pair<TAB>Predicted Interaction<TAB>ID of genes<TAB>Genes" and every line starts with its pair, written nameA+nameB.
--q and -r exclude each other."""
+-q and -r exclude each other.
+
+--held-out: where the test file's triplets land among all unseen triplets (Model.rank_held_out, DESIGN §4.8): the
+universe is every triplet of the -g genes (default: all genes) that is not a key of the train file, ranked by score, and
+-n is the number of its best triplets ranked exactly (default 100000).  Below them a rank is an interval lo-hi that holds
+the exact rank.  Output: summary lines "Name:<TAB>value" (universe size, counts, recall at N for the positives and the
+negatives, the positives' median rank and AUC against the universe, each as lo or lo-hi), then the header
+"Rank<TAB>Predicted Interaction<TAB>Real Interaction<TAB>ID of genes<TAB>Genes" and one line per ranked test triplet, best
+first.  --held-out excludes -q, -r and --include-known."""
 from __future__ import annotations
 
 import contextlib
@@ -31,6 +39,8 @@ import sys
 HEADER = "Predicted Interaction\tID of genes\tGenes\n"
 QUERY_HEADER = "Query gene\t" + HEADER
 PAIR_HEADER = "Query pair\t" + HEADER
+HELD_OUT_HEADER = "Rank\tPredicted Interaction\tReal Interaction\tID of genes\tGenes\n"
+RECALL_AT = (100, 1000, 10000, 100000)
 
 
 def _fail(msg: str) -> int:
@@ -42,10 +52,11 @@ def main(argv=None) -> int:
     argv = sys.argv[1:] if argv is None else argv
     train = test = out = device = genes_file = queries_file = pairs_file = None
     params: list[str] = []
-    top, include_known = 100, False
+    top, include_known, held_out = None, False, False
     try:
         opts, rest = getopt.getopt(argv, "ht:e:p:n:g:q:r:o:", ["help", "train=", "test=", "params=", "top=", "genes=",
-                                                               "queries=", "pairs=", "include-known", "out=", "device="])
+                                                               "queries=", "pairs=", "include-known", "held-out", "out=",
+                                                               "device="])
     except getopt.GetoptError as exc:
         return _fail("argument error: %s" % exc)
     if rest:
@@ -65,8 +76,6 @@ def main(argv=None) -> int:
                 top = int(arg)
             except ValueError:
                 return _fail("--top must be an integer (got %r)" % arg)
-            if top < 1:
-                return _fail("--top must be positive (got %d)" % top)
         elif opt in ("-g", "--genes"):
             genes_file = arg
         elif opt in ("-q", "--queries"):
@@ -75,10 +84,22 @@ def main(argv=None) -> int:
             pairs_file = arg
         elif opt == "--include-known":
             include_known = True
+        elif opt == "--held-out":
+            held_out = True
         elif opt in ("-o", "--out"):
             out = arg
         elif opt == "--device":
             device = arg
+    if held_out:
+        if queries_file or pairs_file or include_known:
+            return _fail("--held-out excludes -q/--queries, -r/--pairs and --include-known")
+        top = 100000 if top is None else top
+        if top < 0:
+            return _fail("--top must be >= 0 with --held-out (got %d)" % top)
+    else:
+        top = 100 if top is None else top
+        if top < 1:
+            return _fail("--top must be positive (got %d)" % top)
     if train is None or test is None or not params:
         return _fail("-t/--train, -e/--test and at least one -p/--params are required")
     if queries_file and pairs_file:
@@ -151,7 +172,13 @@ def main(argv=None) -> int:
     if len({th.shape[1] for th, _ in sets}) != 1:
         return _fail("the parameter files have different K")
 
-    if pairs is not None:
+    if held_out:
+        try:
+            res = model.rank_held_out(top, genes=genes, params=sets, recall_at=RECALL_AT)
+        except ValueError as exc:
+            return _fail(str(exc))
+        text = held_out_text(res)
+    elif pairs is not None:
         per = model.predict_top_triplets_per_pair(pairs, top, genes=genes, exclude_known=not include_known, params=sets)
         text = PAIR_HEADER + "".join(p[0] + "+" + p[1] + "\t" + str(s) + "\t" + key + "\t" + names + "\n"
                                      for p in pairs for s, key, names in per[p])
@@ -168,6 +195,28 @@ def main(argv=None) -> int:
         with open(out, "w", encoding="utf-8") as fh:
             fh.write(text)
     return 0
+
+
+def _interval(v) -> str:
+    if v is None:
+        return "n/a"
+    lo, hi = v
+    return str(lo) if lo == hi else "%s-%s" % (lo, hi)
+
+
+def held_out_text(res: dict) -> str:
+    """Summary lines and the table of ranked test triplets of Model.rank_held_out."""
+    lines = ["Universe size:\t%d" % res["universe"], "Exactly ranked:\t%d" % res["n_exact"],
+             "Ranked positives:\t%d" % res["positives"], "Ranked negatives:\t%d" % res["negatives"],
+             "Excluded train keys:\t%d" % res["excluded_train"], "Excluded outside the genes:\t%d" % res["excluded_genes"]]
+    for N, r in res["recall_at"].items():
+        lines.append("Recall at %d:\t%s" % (N, _interval(r["positives"])))
+        lines.append("Negatives at %d:\t%s" % (N, _interval(r["negatives"])))
+    lines.append("Median rank of positives:\t%s" % _interval(res["median_rank"]))
+    lines.append("Universe AUC:\t%s" % _interval(res["auc"]))
+    body = "".join("%s\t%s\t%d\t%s\t%s\n" % (_interval((lo, hi)), score, label, key, names)
+                   for key, names, label, score, lo, hi in res["rows"])
+    return "\n".join(lines) + "\n" + HELD_OUT_HEADER + body
 
 
 if __name__ == "__main__":
