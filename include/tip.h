@@ -255,6 +255,30 @@ int tip_score_histogram(int P, int K, int S, const double *d_theta, const double
                         int log2_bins, int n_binades, int *h_top_exp, uint64_t *d_hist_out, void *d_ws, size_t ws_bytes,
                         void *stream);
 
+/* ---- held-out ranks per query pair: each test partner's exact rank among its pair's unseen partners (DESIGN §4.9) ----
+ * Candidates, pairs, scores and order as tip_top_triplets_per_pair: d_cand[n_cand] in decimal-string order (rank =
+ * position), d_pair_ranks[n_pairs][2] two distinct ranks in either order (duplicate pairs are answered independently),
+ * score bits of the ensemble SUM over the S sets, partners of the pair ra < rb ordered by (score descending, rc ascending).
+ * d_known: sorted packed rank triples, the train keys (a repeated key counts once).  The universe of a pair is every
+ * partner rc whose triplet is not a known key.  Test entry j is (d_test_pair[j], an index into the caller's pairs;
+ * d_test_rc[j], the partner's rank).  Out: d_rank_out[n_test] = 1 + the partners of the universe ordered before the entry
+ * (0 when its triplet is a known key), exact under any ties; d_score_out[n_test] the mean score; d_universe_out[n_pairs]
+ * |U| = n_cand - 2 - the known keys that contain the pair.  Every score is computed as tip_top_triplets_per_pair computes
+ * it (same tiles of 64 sorted pairs, same fragment position), so a test partner that it returns at position k, with the
+ * same pairs and known keys, has rank k + 1.  One sweep records the bits of the test partners, a second counts every
+ * score of a pair ahead of its entries; a tile's entries are held in shared memory in rounds.  A rank out of range, a
+ * pair of one rank, a test pair index out of range and a test rank that is out of range or one of its pair's are refused
+ * before any device work.  Synchronises the stream.  Limits: n_cand <= 2^21, S * K <= 384, n_pairs <= 2^24, n_known <=
+ * 2^29, n_test < 2^31.  Workspace O(n_cand S K + n_pairs S K + n_test + n_known).  Precondition: finite, non-negative
+ * parameters.  d_ws: tip_rank_per_pair_workspace_bytes() bytes. */
+int tip_rank_per_pair_workspace_bytes(int n_cand, int64_t n_pairs, int K, int S, int64_t n_known, int64_t n_test,
+                                      size_t *bytes);
+int tip_rank_per_pair(int P, int K, int S, const double *d_theta, const double *d_p, const int32_t *d_cand, int n_cand,
+                      const int32_t *d_pair_ranks, int64_t n_pairs, const uint64_t *d_known, int64_t n_known,
+                      const int32_t *d_test_pair, const int32_t *d_test_rc, int64_t n_test,
+                      void *d_ws, size_t ws_bytes, int64_t *d_rank_out, double *d_score_out,
+                      int64_t *d_universe_out, void *stream);
+
 /* ---- testResultsReducer.py:160-184: mean / median / standard deviation of every test triplet across samples ----
  * d_scores[S][T]: score of triplet t in sample j at [j * T + t]; d_n[t] (or NULL = S) = how many leading samples of
  * triplet t are valid.  mean = sequential sum in sample order / n; median = the reference's rule (ascending sort;

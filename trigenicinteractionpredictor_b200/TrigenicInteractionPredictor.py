@@ -884,6 +884,138 @@ class Model:
                               float(np.mean((universe - lo[positive]) / (universe - 1))))
         return res
 
+    def rank_held_out_per_pair(self, pairs=None, genes=None, params=None, hits_at=(1, 5, 10, 20, 50, 100)):
+        """Where each held-out triplet lands among its query pair's unseen partners (addition; DESIGN §4.9).
+
+        A view is a pair {a, b} and a test triplet {a, b, c}.  With pairs=None every ranked test triplet gives three views,
+        one per pair of its genes; the candidates are `genes` (names; default all P genes).  With `pairs` (name pairs,
+        two distinct genes, no pair twice in either order) a view is a listed pair and a test triplet that contains both
+        of its genes; the candidates are `genes` + the pairs' genes.  A test triplet is ranked when its three genes are
+        distinct candidates and it is not a key of links; the others are counted as excluded.  The universe U_ab of a
+        pair is every candidate partner c whose triplet is not a key of links (test keys stay in it), ordered as in
+        predict_top_triplets_per_pair (score descending, then rank order of c), scored by the current theta / pr or by
+        the mean over the sets of `params`.  rank = 1 + the partners of U_ab before c, exact.  Labels follow
+        calculate_metrics: 0 if n0 != 0 else 1.
+
+        Returns a dict:
+          rows: [[pair "nameA+nameB", key "a_b_c", names, label, score, rank, universe], ...] in pair order (the order
+            of `pairs`, or sorted names), each pair's views in rank order;
+          pairs: [[pair, universe, positives, negatives, best positive rank, pair AUC], ...] in the same order (a listed
+            pair without a test triplet has zero counts);
+          views, positives, negatives, excluded_train, excluded_genes;
+          hits_at: {N: {"positives": fraction, "negatives": fraction}}, the share of views with rank <= N;
+          median_rank of the positive views; mrr, the mean over pairs with a positive of 1 / its best positive rank;
+          auc_micro / auc_macro: the mean of (|U| - rank) / (|U| - 1) over positive views / over pairs (each the mean of
+            its positives).
+        Values that need a positive, or |U| > 1, are None without them."""
+        who = "rank_held_out_per_pair"
+        sets = self._prediction_sets(params, who)
+        K = sets[0][0].shape[1]
+        if len(self.test_links) == 0:
+            raise ValueError(who + ": the model has no test links")
+        names = list(genes) if genes is not None else []
+        if pairs is not None:
+            pairs = [tuple(p) for p in pairs]
+            if not pairs:
+                raise ValueError(who + ": pairs is empty")
+            if any(len(p) != 2 for p in pairs):
+                raise ValueError(who + ": a pair is not two gene names")
+            names = [g for p in pairs for g in p] + names
+        missing = [g for g in names if g not in self.gene_id]
+        if missing:
+            raise ValueError("unknown gene names: %s" % ", ".join(dict.fromkeys(missing)))
+        if pairs is not None:
+            single = [p for p in pairs if p[0] == p[1]]
+            if single:
+                raise ValueError(who + ": a pair of one gene: %s" % "+".join(single[0]))
+            twice = [p for p, c in collections.Counter(frozenset(p) for p in pairs).items() if c > 1]
+            if twice:
+                raise ValueError(who + ": duplicate pairs: %s" % ", ".join("+".join(sorted(p)) for p in twice))
+        hits_at = [int(x) for x in hits_at]
+        ids = set(range(self.P)) if genes is None else {self.gene_id[g] for g in names}
+        cand = np.array(sorted(ids, key=str), dtype=np.int32)
+        n = int(cand.shape[0])
+        rank = np.full(self.P, -1, dtype=np.int64)
+        rank[cand] = np.arange(n, dtype=np.int64)
+        train = self._train_packed(cand)
+
+        t1, t2, t3, t_n0, _ = [np.asarray(x.cpu().numpy() if _is_torch(x) else x, dtype=np.int64) for x in self._soa(self.test_links)]
+        r = np.sort(np.stack([rank[t1], rank[t2], rank[t3]], axis=1), axis=1)
+        triplet = (r[:, 0] >= 0) & (r[:, 0] < r[:, 1]) & (r[:, 1] < r[:, 2])
+        packed = ((r[:, 0] << 42) | (r[:, 1] << 21) | r[:, 2]).astype(np.uint64)
+        at = np.minimum(np.searchsorted(train, packed), max(len(train) - 1, 0))
+        in_train = triplet & (train[at] == packed) if len(train) else np.zeros_like(triplet)
+        sel = np.flatnonzero(triplet & ~in_train)
+        r, labels = r[sel], np.where(t_n0[sel] != 0, 0, 1)
+
+        # views: (pair key ra << 21 | rb, partner rank, test triplet)
+        m = len(sel)
+        v_pk = np.concatenate([(r[:, 0] << 21) | r[:, 1], (r[:, 0] << 21) | r[:, 2], (r[:, 1] << 21) | r[:, 2]])
+        v_c = np.concatenate([r[:, 2], r[:, 1], r[:, 0]])
+        v_t = np.tile(np.arange(m, dtype=np.int64), 3)
+        gene_name = np.array(self._genes_in_id_order())
+        if pairs is None:
+            upk = np.unique(v_pk)
+            a_names = gene_name[cand[upk >> 21]]
+            b_names = gene_name[cand[upk & ((1 << 21) - 1)]]
+            first = a_names <= b_names
+            lo_n, hi_n = np.where(first, a_names, b_names), np.where(first, b_names, a_names)
+            order = np.lexsort((hi_n, lo_n))
+            upk = upk[order]
+            labels_p = ["%s+%s" % (x, y) for x, y in zip(lo_n[order].tolist(), hi_n[order].tolist())]
+            pr = np.stack([upk >> 21, upk & ((1 << 21) - 1)], axis=1)
+        else:
+            pr = np.array([sorted((rank[self.gene_id[a]], rank[self.gene_id[b]])) for a, b in pairs], dtype=np.int64).reshape(-1, 2)
+            upk = (pr[:, 0] << 21) | pr[:, 1]
+            labels_p = ["%s+%s" % p for p in pairs]
+        srt = np.argsort(upk, kind="stable")
+        pos = np.minimum(np.searchsorted(upk[srt], v_pk), max(len(upk) - 1, 0))
+        keep = upk[srt][pos] == v_pk if len(upk) else np.zeros(len(v_pk), dtype=bool)
+        v_pair = srt[pos[keep]]
+        v_c, v_t = v_c[keep], v_t[keep]
+
+        thetas = np.stack([th for th, _ in sets])
+        prs = np.stack([p_ for _, p_ in sets])
+        eng = self._prediction_engine(K)
+        v_rank, v_score, universe = eng.rank_per_pair(thetas, prs, cand, pr, train, v_pair, v_c)
+
+        order = np.lexsort((v_rank, v_pair))
+        v_pair, v_t, v_rank, v_score = v_pair[order], v_t[order], v_rank[order], v_score[order]
+        v_lab = labels[v_t]
+        g = cand[r[v_t]].astype(np.int64)
+        nm = gene_name[g]
+        nm.sort(axis=1)
+        v_u = universe[v_pair]
+        rows = [list(x) for x in zip([labels_p[i] for i in v_pair.tolist()], ["%d_%d_%d" % tuple(x) for x in g.tolist()],
+                                     ["_".join(t) for t in nm.tolist()], v_lab.tolist(), v_score.tolist(), v_rank.tolist(),
+                                     v_u.tolist())]
+        positive = v_lab == 1
+        Q = len(labels_p)
+        n_pos_p = np.bincount(v_pair[positive], minlength=Q)
+        n_neg_p = np.bincount(v_pair[~positive], minlength=Q)
+        best = np.full(Q, np.iinfo(np.int64).max)
+        np.minimum.at(best, v_pair[positive], v_rank[positive])
+        auc_ok = positive & (v_u > 1)
+        auc_v = (v_u[auc_ok] - v_rank[auc_ok]) / (v_u[auc_ok] - 1)
+        auc_n = np.bincount(v_pair[auc_ok], minlength=Q)
+        auc_s = np.bincount(v_pair[auc_ok], weights=auc_v, minlength=Q)
+        pair_rows = [[labels_p[q], int(universe[q]), int(n_pos_p[q]), int(n_neg_p[q]),
+                      int(best[q]) if n_pos_p[q] else None, float(auc_s[q] / auc_n[q]) if auc_n[q] else None] for q in range(Q)]
+
+        def frac(mask, N):
+            total = int(mask.sum())
+            return int((v_rank[mask] <= N).sum()) / total if total else None
+
+        has_pos = n_pos_p > 0
+        return {"rows": rows, "pairs": pair_rows, "views": len(rows), "positives": int(positive.sum()),
+                "negatives": int((~positive).sum()), "excluded_train": int(in_train.sum()),
+                "excluded_genes": int((~triplet).sum()),
+                "hits_at": {N: {"positives": frac(positive, N), "negatives": frac(~positive, N)} for N in hits_at},
+                "median_rank": float(np.median(v_rank[positive])) if positive.any() else None,
+                "mrr": float(np.mean(1.0 / best[has_pos])) if has_pos.any() else None,
+                "auc_micro": float(np.mean(auc_v)) if len(auc_v) else None,
+                "auc_macro": float(np.mean(auc_s[auc_n > 0] / auc_n[auc_n > 0])) if (auc_n > 0).any() else None}
+
     # ------------------------------------------------------------------------------------------
     # report (TIP.py:793-904)
     # ------------------------------------------------------------------------------------------

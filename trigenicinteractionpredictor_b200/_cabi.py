@@ -67,6 +67,9 @@ SIGNATURES = {
     "tip_score_histogram_workspace_bytes": (c_int, [c_int, c_int, c_int, c_int, c_int, _psz]),
     "tip_score_histogram": (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
                                     ctypes.POINTER(c_int), c_void_p, c_void_p, c_size_t, c_void_p]),
+    "tip_rank_per_pair_workspace_bytes": (c_int, [c_int, c_int64, c_int, c_int, c_int64, c_int64, _psz]),
+    "tip_rank_per_pair": (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int64, c_void_p, c_int64,
+                                  c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_void_p]),
     "tip_reduce_samples": (c_int, [c_int, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "tip_em_iterations_host": (c_int, [c_int, c_int, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_int,
                                        c_uint]),

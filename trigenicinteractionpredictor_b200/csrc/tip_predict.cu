@@ -24,6 +24,9 @@
 //
 // Histogram of all scores (tip_score_histogram): the same sweep as tip_top_triplets, counting every score into a fixed
 // log-spaced histogram of its bits (tip_hist_pass_kernel); the ranks of held-out triplets among all triplets follow from it.
+//
+// Ranks per query pair (tip_rank_per_pair): the tiles and column phases of tip_top_triplets_per_pair, swept once to record
+// the scores of the held-out partners and once to count, per pair, the scores ahead of each of them (tip_rank_pass_kernel).
 #include <algorithm>
 #include <cmath>
 #include <vector>
@@ -2008,6 +2011,606 @@ extern "C" int tip_score_histogram(int P, int K, int S, const double *d_theta, c
     A.cursor = cursor; A.hist = reinterpret_cast<unsigned long long *>(d_hist_out);
     TIP_CHECK_CUDA(cudaMemsetAsync(cursor, 0, 8, st));
     tip_hist_pass_kernel<<<(int)std::min<long long>((long long)sm_count() * per_sm, A.n_items), kPredThreads, smem, st>>>(A);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
+// ---- tip_rank_per_pair ----
+// The exact rank of every held-out partner among its query pair's unseen partners.  The sorted pairs, their V rows, the
+// tiles of 64 sorted pairs, the three column phases and dmma_block are those of tip_top_triplets_per_pair, so every score is
+// computed at the same fragment position, with the same contraction order, as there.  Test entries (pair, rc) are sorted by
+// (sorted pair, rc); the train partners of a pair (the distinct known keys that contain it) by (the first sorted position
+// of the pair, rc).
+// Capture sweep: each warp jumps to the column blocks that hold a test partner of one of its rows and records its bits.
+// Count sweep: a tile's entries sit in shared memory, per row in the order (bits descending, rc ascending), at most e_max of
+// them per round (a tile with more is swept once per round).  Every score of a row is tested in registers against the
+// row's weakest entry of the round; train partners, found by a cursor that walks the row's sorted train list along the
+// columns, are skipped; a score that passes is placed among the entries by binary search and counted at its slot (the
+// scores ahead of every entry of the round in a register per row).  rank = 1 + the slot counts up to the entry.
+namespace tip {
+namespace {
+
+constexpr int kRankMaxEntries = 2048;             // entries of a count round in shared memory, 16 bytes each
+constexpr int kRankMinEntries = 256;              // fewer beside the A tile: refused (bounds the rounds in the workspace)
+constexpr int kRankKeyBits = kRankBits + 24;      // (sorted pair << 21) | rc, n_pairs <= 2^24
+constexpr unsigned long long kRcMask = (1ull << kRankBits) - 1;
+
+struct RankPassArgs {
+    int n, SKP, n_pairs, mode;          // mode 0: capture the bits of the test entries; 1: count
+    const double *tcat;                 // [n_pad][SKP]
+    const double *V;                    // [n_pairs][3][SKP], sorted pair order
+    const int32_t *ra, *rb;             // [n_pairs] sorted
+    const int4 *items;                  // {tile, g0, g1, 0}: the count sweep ranks the entries [g0, g1) of the tile
+    int n_items;
+    const int32_t *te_off;              // [n_pairs + 1] test entries of sorted pair p: [te_off[p], te_off[p + 1])
+    const unsigned long long *te_key;   // [n_test] (p << 21) | rc, ascending
+    const int32_t *tr_beg, *tr_end;     // [n_pairs] train partners of sorted pair p in tr_key
+    const unsigned long long *tr_key;   // (first sorted position of the pair << 21) | rc, ascending
+    unsigned long long *te_bits;        // capture: [n_test] score bits, te_key order
+    const unsigned long long *ord_bits; // count: [n_test] score bits, per pair in the order (bits descending, rc ascending)
+    const int32_t *ord_pos;             // count: [n_test] the te_key position of each entry of that order
+    const int32_t *te_idx;              // [n_test] the caller's index of each te_key entry
+    int64_t *rank;                      // count: [n_test] caller's order
+    unsigned long long *ctl;            // [0] item cursor
+};
+
+__device__ __forceinline__ long long lower_bound_u64(const unsigned long long *a, long long n, unsigned long long key)
+{
+    long long lo = 0, hi = n;
+    while (lo < hi) {
+        const long long mid = (lo + hi) >> 1;
+        if (a[mid] < key) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+
+// per caller's pair: its sorted position
+__global__ void tip_rank_inverse_kernel(long long n_pairs, const int32_t *__restrict__ perm, int32_t *__restrict__ inv)
+{
+    const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p < n_pairs) inv[perm[p]] = (int32_t)p;
+}
+
+__global__ void tip_rank_test_keys_kernel(long long n_test, const int32_t *__restrict__ test_pair, const int32_t *__restrict__ test_rc,
+                                          const int32_t *__restrict__ inv, unsigned long long *__restrict__ key,
+                                          int32_t *__restrict__ idx)
+{
+    const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n_test) return;
+    key[j] = ((unsigned long long)inv[test_pair[j]] << kRankBits) | (unsigned long long)test_rc[j];
+    idx[j] = (int32_t)j;
+}
+
+// the train partners: per distinct known key (ascending ranks, all < n) and each of its three pairs that is listed, the
+// key's third rank, tagged with the pair's first sorted position
+__global__ void tip_rank_train_kernel(long long n_known, const unsigned long long *__restrict__ known, int n, long long n_pairs,
+                                      const unsigned long long *__restrict__ key, unsigned long long *__restrict__ tr_key,
+                                      unsigned long long *n_tr)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_known || (i > 0 && known[i] == known[i - 1])) return;   // a repeated key counts once
+    const unsigned long long k = known[i];
+    const unsigned long long r0 = (k >> (2 * kRankBits)) & kRcMask, r1 = (k >> kRankBits) & kRcMask, r2 = k & kRcMask;
+    if (!(r0 < r1 && r1 < r2 && r2 < (unsigned long long)n)) return;
+    const unsigned long long want[3] = {(r0 << kRankBits) | r1, (r0 << kRankBits) | r2, (r1 << kRankBits) | r2};
+    const unsigned long long third[3] = {r2, r1, r0};
+    for (int w = 0; w < 3; ++w) {
+        const long long pos = lower_bound_u64(key, n_pairs, want[w]);
+        if (pos < n_pairs && key[pos] == want[w])
+            tr_key[atomicAdd(n_tr, 1ull)] = ((unsigned long long)pos << kRankBits) | third[w];
+    }
+}
+
+// per sorted pair: its test entries, its train partners and |U| (in the caller's order)
+__global__ void tip_rank_rows_kernel(long long n_pairs, int n, const unsigned long long *__restrict__ key, const int32_t *__restrict__ perm,
+                                     long long n_test, const unsigned long long *__restrict__ te_key, long long n_tr,
+                                     const unsigned long long *__restrict__ tr_key, int32_t *__restrict__ te_off,
+                                     int32_t *__restrict__ rep, int32_t *__restrict__ tr_beg, int32_t *__restrict__ tr_end,
+                                     int64_t *__restrict__ universe)
+{
+    const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n_pairs) return;
+    const unsigned long long r = (unsigned long long)lower_bound_u64(key, n_pairs, key[p]);
+    te_off[p] = (int32_t)lower_bound_u64(te_key, n_test, (unsigned long long)p << kRankBits);
+    if (p == n_pairs - 1) te_off[n_pairs] = (int32_t)n_test;
+    const long long b = lower_bound_u64(tr_key, n_tr, r << kRankBits), e = lower_bound_u64(tr_key, n_tr, (r + 1) << kRankBits);
+    rep[p] = (int32_t)r;
+    tr_beg[p] = (int32_t)b;
+    tr_end[p] = (int32_t)e;
+    universe[perm[p]] = max(0ll, (long long)n - 2 - (e - b));
+}
+
+__global__ void tip_rank_iota_kernel(long long m, int32_t *__restrict__ out)
+{
+    const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j < m) out[j] = (int32_t)j;
+}
+
+// the lane's score at column offset off (from the lane's first column) of row mi of its block, if the lane holds it
+__device__ __forceinline__ bool lane_score(const double (&acc)[4][4][2], int mi, int off, double &v)
+{
+    bool hit = false;
+#pragma unroll
+    for (int ni = 0; ni < 4; ++ni)
+#pragma unroll
+        for (int e = 0; e < 2; ++e)
+            if (off == ni * 8 + e) {
+                v = acc[mi][ni][e];
+                hit = true;
+            }
+    return hit;
+}
+
+// work items are tiles of 64 sorted pairs (the tiles of tip_pair_pass_kernel, swept over the same column ranges)
+__global__ void __launch_bounds__(kPredThreads) tip_rank_pass_kernel(RankPassArgs A)
+{
+    extern __shared__ __align__(16) unsigned char smem[];
+    const int qs = q_stride(A.SKP);
+    double *At = reinterpret_cast<double *>(smem);                                                     // [64][qs]
+    const bool count = A.mode == 1;
+    unsigned long long *sh_eb = reinterpret_cast<unsigned long long *>(At + (size_t)kPredRows * qs);  // count: entry bits
+    int *sh_erc = nullptr;                                                                             // entry rc
+    unsigned *sh_cnt = nullptr;                                                                        // slot counts
+    __shared__ int sh_ra[kPredRows], sh_rb[kPredRows], sh_lb[kPredRows], sh_le[kPredRows], sh_elo[kPredRows], sh_ehi[kPredRows];
+    __shared__ long long sh_item;
+    __shared__ int sh_range[4];   // min ra, max ra, min rb, max rb of the tile
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int wr = warp & 1, wc = warp >> 1;
+    const int gq = lane >> 2, tq = lane & 3;
+    const int n = A.n, SKP = A.SKP;
+    const unsigned long long *list = count ? A.tr_key : A.te_key;   // the column lists the cursors walk
+
+    for (;;) {
+        __syncthreads();   // the previous tile is no longer read
+        if (tid == 0) sh_item = (long long)atomicAdd(A.ctl, 1ull);
+        __syncthreads();
+        const long long item = sh_item;
+        if (item >= A.n_items) break;
+        const int4 it = A.items[item];
+        const int t0 = it.x * kPredRows, rows = min(kPredRows, A.n_pairs - t0), n_e = it.z - it.y;
+        sh_erc = reinterpret_cast<int *>(sh_eb + n_e);
+        sh_cnt = reinterpret_cast<unsigned *>(sh_erc + n_e);
+        if (tid < kPredRows) {
+            const int p = t0 + (tid < rows ? tid : 0);
+            sh_ra[tid] = A.ra[p];
+            sh_rb[tid] = A.rb[p];
+            const int b = A.te_off[p], e = A.te_off[p + 1];
+            const bool in = tid < rows;
+            sh_lb[tid] = !in ? 0 : count ? A.tr_beg[p] : b;
+            sh_le[tid] = !in ? 0 : count ? A.tr_end[p] : e;
+            const int elo = max(b, it.y) - it.y, ehi = min(e, it.z) - it.y;
+            sh_elo[tid] = in && count ? elo : 0;
+            sh_ehi[tid] = in && count ? max(elo, ehi) : 0;
+        }
+        if (count)
+            for (int e = tid; e < n_e; e += kPredThreads) {
+                const int g = it.y + e;
+                sh_eb[e] = A.ord_bits[g];
+                sh_erc[e] = (int)(A.te_key[A.ord_pos[g]] & kRcMask);
+                sh_cnt[e] = 0;
+            }
+        __syncthreads();
+        if (tid == 0) {
+            int r0 = n, r1 = 0, r2 = n, r3 = 0;
+            for (int i = 0; i < rows; ++i) {
+                r0 = min(r0, sh_ra[i]); r1 = max(r1, sh_ra[i]);
+                r2 = min(r2, sh_rb[i]); r3 = max(r3, sh_rb[i]);
+            }
+            sh_range[0] = r0; sh_range[1] = r1; sh_range[2] = r2; sh_range[3] = r3;
+        }
+        __syncthreads();
+
+        for (int g = 0; g < 3; ++g) {
+            const int col0 = g == 0 ? 0 : g == 1 ? sh_range[0] + 1 : sh_range[2] + 1;
+            const int col_end = g == 0 ? sh_range[1] : g == 1 ? sh_range[3] : n;
+            if (col0 >= col_end) continue;
+            __syncthreads();   // the previous phase's A tile is no longer read
+            for (int e = tid; e < kPredRows * SKP; e += kPredThreads) {
+                const int i = e / SKP, col = e % SKP;
+                At[i * qs + col] = i < rows ? __ldg(A.V + ((long long)(t0 + i) * 3 + g) * SKP + col) : 0.0;
+            }
+            __syncthreads();
+            if (wr * 32 >= rows) continue;
+            const int ib = wr * 32 + gq;   // the lane's first row
+            int cur[4], lim[4];
+            unsigned ahead[4] = {0u, 0u, 0u, 0u};   // count: scores ahead of every entry of the round, per row
+            bool any = false;
+#pragma unroll
+            for (int mi = 0; mi < 4; ++mi) {
+                const int i = ib + mi * 8;
+                const bool act = !count || sh_elo[i] < sh_ehi[i];
+                cur[mi] = act ? sh_lb[i] : 0;
+                lim[mi] = act ? sh_le[i] : 0;
+                any |= count ? act : cur[mi] < lim[mi];
+            }
+            if (!__any_sync(0xffffffffu, any)) continue;
+            const double *Aw = At + ib * qs + tq;
+            const int cbase = col0 + wc * 32;
+            for (int c0 = cbase; c0 < col_end; c0 += 64) {
+                if (!count) {
+                    // the warp's next column, at or after c0, that holds a test partner of one of its rows in the row's region
+                    int nxt = INT_MAX;
+#pragma unroll
+                    for (int mi = 0; mi < 4; ++mi) {
+                        const int i = ib + mi * 8, ra = sh_ra[i], rb = sh_rb[i];
+                        const int lo_c = g == 0 ? 0 : g == 1 ? ra + 1 : rb + 1, hi_c = g == 0 ? ra : g == 1 ? rb : n;
+                        const int from = max(c0, lo_c);
+                        while (cur[mi] < lim[mi] && (int)(__ldg(list + cur[mi]) & kRcMask) < from) ++cur[mi];
+                        if (cur[mi] < lim[mi]) {
+                            const int r = (int)(__ldg(list + cur[mi]) & kRcMask);
+                            if (r < hi_c) nxt = min(nxt, r);
+                        }
+                    }
+                    nxt = __reduce_min_sync(0xffffffffu, nxt);
+                    if (nxt >= col_end) break;
+                    const int c1 = cbase + (nxt - cbase) / 64 * 64;
+                    c0 = c1;
+                    if (nxt - c1 >= 32) continue;   // in the other column half: look again from the next block
+                }
+                double acc[4][4][2];
+                dmma_block(acc, Aw, qs, A.tcat + (long long)(c0 + gq) * SKP + tq, SKP);
+                const int rc0 = c0 + 2 * tq;
+#pragma unroll
+                for (int mi = 0; mi < 4; ++mi) {
+                    const int i = ib + mi * 8, ra = sh_ra[i], rb = sh_rb[i];
+                    const int lo_c = g == 0 ? 0 : g == 1 ? ra + 1 : rb + 1, hi_c = g == 0 ? ra : g == 1 ? rb : n;
+                    if (!count) {
+                        // the row's test partners in this block (the cursor is at the first at or after max(c0, lo_c))
+                        while (cur[mi] < lim[mi]) {
+                            const int r = (int)(__ldg(list + cur[mi]) & kRcMask);
+                            if (r >= c0 + 32 || r >= hi_c) break;
+                            double v = 0.0;
+                            if (lane_score(acc, mi, r - rc0, v)) A.te_bits[cur[mi]] = (unsigned long long)__double_as_longlong(v);
+                            ++cur[mi];
+                        }
+                        continue;
+                    }
+                    const int elo = sh_elo[i], ehi = sh_ehi[i];
+                    if (elo == ehi) continue;
+                    // the row's train partners among the lane's columns of this block
+                    unsigned skip = 0;
+                    while (cur[mi] < lim[mi]) {
+                        const int r = (int)(__ldg(list + cur[mi]) & kRcMask);
+                        if (r >= c0 + 32) break;
+                        const int off = r - rc0;
+#pragma unroll
+                        for (int f = 0; f < 8; ++f)
+                            if (off == (f >> 1) * 8 + (f & 1)) skip |= 1u << f;
+                        ++cur[mi];
+                    }
+                    const unsigned long long wb = sh_eb[ehi - 1], fb = sh_eb[elo];
+                    const int wrc = sh_erc[ehi - 1], frc = sh_erc[elo];
+#pragma unroll
+                    for (int ni = 0; ni < 4; ++ni)
+#pragma unroll
+                        for (int e = 0; e < 2; ++e) {
+                            const int rc = rc0 + ni * 8 + e;
+                            if (rc < lo_c || rc >= hi_c || ((skip >> (ni * 2 + e)) & 1u)) continue;
+                            const unsigned long long bits = (unsigned long long)__double_as_longlong(acc[mi][ni][e]);
+                            if (!(bits > wb || (bits == wb && rc < wrc))) continue;   // not ahead of the weakest entry
+                            if (bits > fb || (bits == fb && rc < frc)) {
+                                ++ahead[mi];
+                                continue;
+                            }
+                            // the first entry in (elo, ehi) the score is ahead of
+                            int lo = elo + 1, hi = ehi - 1;
+                            while (lo < hi) {
+                                const int mid = (lo + hi) >> 1;
+                                const unsigned long long mb = sh_eb[mid];
+                                if (bits > mb || (bits == mb && rc < sh_erc[mid])) hi = mid; else lo = mid + 1;
+                            }
+                            atomicAdd(sh_cnt + lo, 1u);
+                        }
+                }
+            }
+            if (count) {
+#pragma unroll
+                for (int mi = 0; mi < 4; ++mi) {
+                    unsigned a = ahead[mi];
+                    a += __shfl_xor_sync(0xffffffffu, a, 1);
+                    a += __shfl_xor_sync(0xffffffffu, a, 2);
+                    const int i = ib + mi * 8;
+                    if (tq == 0 && a) atomicAdd(sh_cnt + sh_elo[i], a);
+                }
+            }
+        }
+        __syncthreads();
+        if (count && tid < rows) {
+            long long run = 0;
+            for (int s = sh_elo[tid]; s < sh_ehi[tid]; ++s) {
+                run += sh_cnt[s];
+                A.rank[A.te_idx[A.ord_pos[it.y + s]]] = (int64_t)(1 + run);
+            }
+        }
+    }
+}
+
+// per test entry (te_key order): the mean score, and rank 0 when its triplet is a train partner of its pair
+__global__ void tip_rank_finish_kernel(long long n_test, int S, const unsigned long long *__restrict__ te_key,
+                                       const int32_t *__restrict__ te_idx, const unsigned long long *__restrict__ bits,
+                                       const int32_t *__restrict__ rep, long long n_tr, const unsigned long long *__restrict__ tr_key,
+                                       int64_t *__restrict__ rank, double *__restrict__ score)
+{
+    const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n_test) return;
+    const unsigned long long k = te_key[j];
+    const unsigned long long want = ((unsigned long long)rep[k >> kRankBits] << kRankBits) | (k & kRcMask);
+    const long long at = lower_bound_u64(tr_key, n_tr, want);
+    const int o = te_idx[j];
+    score[o] = __longlong_as_double((long long)bits[j]) / (double)S;
+    if (at < n_tr && tr_key[at] == want) rank[o] = 0;
+}
+
+struct RankLayout {
+    size_t o_tcat, o_M, o_key, o_key2, o_idx, o_perm, o_inv, o_ra, o_rb, o_act, o_bidx, o_ub, o_V, o_tk, o_tk2, o_ti, o_ti2,
+        o_bits, o_obits, o_opos0, o_opos, o_toff, o_rep, o_trb, o_tre, o_trk, o_trk2, o_ntr, o_ctl, o_items, o_cub, cub_bytes,
+        total;
+    int n_pad, SKP, chunk;
+    long long max_items;
+};
+
+RankLayout rank_layout(int n, long long n_pairs, int K, int S, long long n_known, long long n_test)
+{
+    RankLayout L{};
+    L.n_pad = (n + 63) / 64 * 64 + 64;
+    L.SKP = (S * K + 3) / 4 * 4;
+    L.chunk = (int)std::max(1ll, std::min((long long)n, (long long)L.n_pad * L.SKP / (3ll * S * K * K)));
+    const long long tiles = (n_pairs + kPredRows - 1) / kPredRows;
+    L.max_items = 2 * tiles + n_test / kRankMinEntries + 1;   // the capture items, then the count rounds
+    const int np = (int)n_pairs, nt = (int)n_test, ntr = (int)(3 * n_known);
+    size_t cb[5] = {0, 0, 0, 0, 0};
+    cub::DeviceRadixSort::SortPairs(nullptr, cb[0], (const unsigned long long *)nullptr, (unsigned long long *)nullptr,
+                                    (const int32_t *)nullptr, (int32_t *)nullptr, np, 0, 2 * kRankBits, (cudaStream_t)0);
+    cub::DeviceRadixSort::SortPairs(nullptr, cb[1], (const unsigned long long *)nullptr, (unsigned long long *)nullptr,
+                                    (const int32_t *)nullptr, (int32_t *)nullptr, nt, 0, kRankKeyBits, (cudaStream_t)0);
+    cub::DeviceRadixSort::SortKeys(nullptr, cb[2], (const unsigned long long *)nullptr, (unsigned long long *)nullptr, ntr, 0,
+                                   kRankKeyBits, (cudaStream_t)0);
+    cub::DeviceSegmentedSort::StableSortPairsDescending(nullptr, cb[3], (const unsigned long long *)nullptr,
+                                                        (unsigned long long *)nullptr, (const int32_t *)nullptr, (int32_t *)nullptr,
+                                                        nt, np, (const int *)nullptr, (const int *)nullptr, (cudaStream_t)0);
+    L.cub_bytes = *std::max_element(cb, cb + 5);
+    const size_t q = (size_t)n_pairs, t = (size_t)n_test;
+    size_t off = 0;
+    L.o_tcat = off;   off += a256((size_t)L.n_pad * L.SKP * 8);
+    L.o_M = off;      off += a256((size_t)L.chunk * 3 * S * K * K * 8);
+    L.o_key = off;    off += a256(q * 8);
+    L.o_key2 = off;   off += a256(q * 8);
+    L.o_idx = off;    off += a256(q * 4);
+    L.o_perm = off;   off += a256(q * 4);
+    L.o_inv = off;    off += a256(q * 4);
+    L.o_ra = off;     off += a256(q * 4);
+    L.o_rb = off;     off += a256(q * 4);
+    L.o_act = off;    off += a256(q * 4);
+    L.o_bidx = off;   off += a256((size_t)n * 4);
+    L.o_ub = off;     off += a256((size_t)n * 4);
+    L.o_V = off;      off += a256(q * 3 * L.SKP * 8);
+    L.o_tk = off;     off += a256(t * 8);
+    L.o_tk2 = off;    off += a256(t * 8);
+    L.o_ti = off;     off += a256(t * 4);
+    L.o_ti2 = off;    off += a256(t * 4);
+    L.o_bits = off;   off += a256(t * 8);
+    L.o_obits = off;  off += a256(t * 8);
+    L.o_opos0 = off;  off += a256(t * 4);
+    L.o_opos = off;   off += a256(t * 4);
+    L.o_toff = off;   off += a256((q + 1) * 4);
+    L.o_rep = off;    off += a256(q * 4);
+    L.o_trb = off;    off += a256(q * 4);
+    L.o_tre = off;    off += a256(q * 4);
+    L.o_trk = off;    off += a256((size_t)n_known * 3 * 8);
+    L.o_trk2 = off;   off += a256((size_t)n_known * 3 * 8);
+    L.o_ntr = off;    off += 256;
+    L.o_ctl = off;    off += 256;
+    L.o_items = off;  off += a256((size_t)L.max_items * sizeof(int4));
+    L.o_cub = off;    off += a256(L.cub_bytes);
+    L.total = off + 256;
+    return L;
+}
+
+size_t rank_smem(int SKP, int e_max) { return (size_t)kPredRows * q_stride(SKP) * 8 + (size_t)e_max * 16; }
+
+}  // namespace
+}  // namespace tip
+
+static bool rank_args_ok(int n_cand, int64_t n_pairs, int K, int S, int64_t n_known, int64_t n_test)
+{
+    return predict_args_ok(n_cand, K, S, n_known, 0) && n_pairs >= 0 && n_pairs <= kPairMaxRows && n_known <= (1ll << 29) &&
+           n_test >= 0 && n_test < (1ll << 31);
+}
+
+#define TIP_RANK_LIMITS "n_cand <= 2^21, 1 <= K <= %d, S >= 1, S*K <= %d, 0 <= n_pairs <= 2^24, 0 <= n_known <= 2^29, " \
+                        "0 <= n_test < 2^31"
+
+extern "C" int tip_rank_per_pair_workspace_bytes(int n_cand, int64_t n_pairs, int K, int S, int64_t n_known, int64_t n_test,
+                                                 size_t *bytes)
+{
+    TIP_REQUIRE(bytes != nullptr && rank_args_ok(n_cand, n_pairs, K, S, n_known, n_test),
+                "tip_rank_per_pair_workspace_bytes: bad arguments (" TIP_RANK_LIMITS ")", TIP_MAX_K, kPredMaxSK);
+    *bytes = rank_layout(n_cand, n_pairs, K, S, n_known, n_test).total;
+    return 0;
+}
+
+extern "C" int tip_rank_per_pair(int P, int K, int S, const double *d_theta, const double *d_p, const int32_t *d_cand, int n_cand,
+                                 const int32_t *d_pair_ranks, int64_t n_pairs, const uint64_t *d_known, int64_t n_known,
+                                 const int32_t *d_test_pair, const int32_t *d_test_rc, int64_t n_test, void *d_ws, size_t ws_bytes,
+                                 int64_t *d_rank_out, double *d_score_out, int64_t *d_universe_out, void *stream)
+{
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    TIP_REQUIRE(P > 0 && n_cand <= P && rank_args_ok(n_cand, n_pairs, K, S, n_known, n_test),
+                "tip_rank_per_pair: bad arguments (P > 0, n_cand <= P, " TIP_RANK_LIMITS ")", TIP_MAX_K, kPredMaxSK);
+    TIP_REQUIRE(d_theta && d_p && (d_cand || n_cand == 0) && (d_known || n_known == 0) &&
+                    (n_pairs == 0 || (d_pair_ranks && d_universe_out)) &&
+                    (n_test == 0 || (d_test_pair && d_test_rc && d_rank_out && d_score_out)),
+                "tip_rank_per_pair: null pointer");
+    const int n = n_cand;
+    const long long Q = n_pairs, T = n_test;
+    // pair ranks and test entries are checked on the host before any device work
+    std::vector<int32_t> pr((size_t)Q * 2), tp((size_t)T), trc((size_t)T);
+    if (Q) TIP_CHECK_CUDA(cudaMemcpyAsync(pr.data(), d_pair_ranks, (size_t)Q * 8, cudaMemcpyDeviceToHost, st));
+    if (T) {
+        TIP_CHECK_CUDA(cudaMemcpyAsync(tp.data(), d_test_pair, (size_t)T * 4, cudaMemcpyDeviceToHost, st));
+        TIP_CHECK_CUDA(cudaMemcpyAsync(trc.data(), d_test_rc, (size_t)T * 4, cudaMemcpyDeviceToHost, st));
+    }
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    std::vector<int32_t> bidx(std::max(n, 1), -1), ub;
+    for (long long i = 0; i < Q; ++i) {
+        for (int e = 0; e < 2; ++e)
+            TIP_REQUIRE(pr[2 * i + e] >= 0 && pr[2 * i + e] < n, "tip_rank_per_pair: rank %d of pair %lld is not in [0, %d)",
+                        pr[2 * i + e], i, n);
+        TIP_REQUIRE(pr[2 * i] != pr[2 * i + 1], "tip_rank_per_pair: pair %lld has the same rank twice (%d)", i, pr[2 * i]);
+        bidx[std::max(pr[2 * i], pr[2 * i + 1])] = 0;
+    }
+    for (long long j = 0; j < T; ++j) {
+        TIP_REQUIRE(tp[j] >= 0 && tp[j] < Q, "tip_rank_per_pair: test entry %lld names pair %d, not in [0, %lld)", j, tp[j], Q);
+        const int32_t a = pr[2 * (size_t)tp[j]], b = pr[2 * (size_t)tp[j] + 1];
+        TIP_REQUIRE(trc[j] >= 0 && trc[j] < n && trc[j] != a && trc[j] != b,
+                    "tip_rank_per_pair: test entry %lld has partner rank %d, not a rank in [0, %d) other than its pair's (%d, %d)",
+                    j, trc[j], n, a, b);
+    }
+    if (Q == 0) return 0;
+    for (int r = 0; r < n; ++r)
+        if (bidx[r] == 0) {
+            bidx[r] = (int32_t)ub.size();
+            ub.push_back(r);
+        }
+    const RankLayout L = rank_layout(n, Q, K, S, n_known, T);
+    TIP_REQUIRE(d_ws != nullptr && ws_bytes >= L.total, "tip_rank_per_pair: workspace too small (%zu < %zu)", ws_bytes, L.total);
+    int dev = 0, optin = 0;
+    TIP_CHECK_CUDA(cudaGetDevice(&dev));
+    TIP_CHECK_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    cudaFuncAttributes fa{};
+    TIP_CHECK_CUDA(cudaFuncGetAttributes(&fa, tip_rank_pass_kernel));
+    const long long room = ((long long)optin - 1024 - (long long)fa.sharedSizeBytes - (long long)rank_smem(L.SKP, 0)) / 16;
+    const int e_max = (int)std::min<long long>(kRankMaxEntries, room);
+    TIP_REQUIRE(e_max >= kRankMinEntries, "tip_rank_per_pair: S*K = %d leaves room for %d entries beside the A tile (internal error)",
+                S * K, e_max);
+
+    char *base = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(d_ws) + 255) / 256 * 256);
+    double *tcat = reinterpret_cast<double *>(base + L.o_tcat), *Mq = reinterpret_cast<double *>(base + L.o_M);
+    auto *key = reinterpret_cast<unsigned long long *>(base + L.o_key), *key2 = reinterpret_cast<unsigned long long *>(base + L.o_key2);
+    auto *idx = reinterpret_cast<int32_t *>(base + L.o_idx), *perm = reinterpret_cast<int32_t *>(base + L.o_perm);
+    auto *inv = reinterpret_cast<int32_t *>(base + L.o_inv);
+    auto *ra = reinterpret_cast<int32_t *>(base + L.o_ra), *rb = reinterpret_cast<int32_t *>(base + L.o_rb);
+    auto *act = reinterpret_cast<int32_t *>(base + L.o_act);
+    auto *d_bidx = reinterpret_cast<int32_t *>(base + L.o_bidx), *d_ub = reinterpret_cast<int32_t *>(base + L.o_ub);
+    double *V = reinterpret_cast<double *>(base + L.o_V);
+    auto *tk = reinterpret_cast<unsigned long long *>(base + L.o_tk), *tk2 = reinterpret_cast<unsigned long long *>(base + L.o_tk2);
+    auto *ti = reinterpret_cast<int32_t *>(base + L.o_ti), *ti2 = reinterpret_cast<int32_t *>(base + L.o_ti2);
+    auto *bits = reinterpret_cast<unsigned long long *>(base + L.o_bits);
+    auto *obits = reinterpret_cast<unsigned long long *>(base + L.o_obits);
+    auto *opos0 = reinterpret_cast<int32_t *>(base + L.o_opos0), *opos = reinterpret_cast<int32_t *>(base + L.o_opos);
+    auto *toff = reinterpret_cast<int32_t *>(base + L.o_toff), *rep = reinterpret_cast<int32_t *>(base + L.o_rep);
+    auto *trb = reinterpret_cast<int32_t *>(base + L.o_trb), *tre = reinterpret_cast<int32_t *>(base + L.o_tre);
+    auto *trk = reinterpret_cast<unsigned long long *>(base + L.o_trk), *trk2 = reinterpret_cast<unsigned long long *>(base + L.o_trk2);
+    auto *ntr = reinterpret_cast<unsigned long long *>(base + L.o_ntr), *ctl = reinterpret_cast<unsigned long long *>(base + L.o_ctl);
+    auto *items = reinterpret_cast<int4 *>(base + L.o_items);
+    void *cub_tmp = base + L.o_cub;
+    const int g1 = (int)((Q + 255) / 256), gt = (int)((T + 255) / 256);
+    size_t cb = 0;
+
+    // pairs sorted by (ra, rb) as tip_top_triplets_per_pair sorts them, with the permutation back to the caller's order
+    tip_pair_keys_kernel<<<g1, 256, 0, st>>>(Q, d_pair_ranks, key, idx);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    cb = L.cub_bytes;
+    TIP_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(cub_tmp, cb, key, key2, idx, perm, (int)Q, 0, 2 * kRankBits, st));
+    tip_pair_split_kernel<<<g1, 256, 0, st>>>(Q, key2, ra, rb, act);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    tip_rank_inverse_kernel<<<g1, 256, 0, st>>>(Q, perm, inv);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    // test entries by (sorted pair, rc)
+    if (T) {
+        tip_rank_test_keys_kernel<<<gt, 256, 0, st>>>(T, d_test_pair, d_test_rc, inv, tk, ti);
+        TIP_CHECK_CUDA(cudaGetLastError());
+        cb = L.cub_bytes;
+        TIP_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(cub_tmp, cb, tk, tk2, ti, ti2, (int)T, 0, kRankKeyBits, st));
+    }
+    // train partners by (first sorted position of the pair, rc)
+    TIP_CHECK_CUDA(cudaMemsetAsync(ntr, 0, 8, st));
+    if (n_known > 0) {
+        tip_rank_train_kernel<<<(int)((n_known + 255) / 256), 256, 0, st>>>(
+            n_known, reinterpret_cast<const unsigned long long *>(d_known), n, Q, key2, trk, ntr);
+        TIP_CHECK_CUDA(cudaGetLastError());
+    }
+    unsigned long long h_ntr = 0;
+    TIP_CHECK_CUDA(cudaMemcpyAsync(&h_ntr, ntr, 8, cudaMemcpyDeviceToHost, st));
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    const long long NT = (long long)h_ntr;
+    if (NT) {
+        cb = L.cub_bytes;
+        TIP_CHECK_CUDA(cub::DeviceRadixSort::SortKeys(cub_tmp, cb, trk, trk2, (int)NT, 0, kRankKeyBits, st));
+    }
+    tip_rank_rows_kernel<<<g1, 256, 0, st>>>(Q, n, key2, perm, T, tk2, NT, trk2, toff, rep, trb, tre, d_universe_out);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    if (T == 0) {
+        TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+        return 0;
+    }
+
+    // V of every pair, from the matrices of its gene b, a chunk of genes at a time (as tip_top_triplets_per_pair)
+    TIP_CHECK_CUDA(cudaMemcpyAsync(d_bidx, bidx.data(), (size_t)n * 4, cudaMemcpyHostToDevice, st));
+    TIP_CHECK_CUDA(cudaMemcpyAsync(d_ub, ub.data(), ub.size() * 4, cudaMemcpyHostToDevice, st));
+    const int n_ub = (int)ub.size();
+    for (int c0 = 0; c0 < n_ub; c0 += L.chunk) {
+        const int c1 = std::min(n_ub, c0 + L.chunk);
+        const long long work = (long long)L.n_pad * L.SKP + (long long)(c1 - c0) * 3 * S * K * K;
+        tip_query_prep_kernel<<<(int)std::min<long long>((work + 255) / 256, (long long)sm_count() * 16), 256, 0, st>>>(
+            S, P, K, n, L.n_pad, L.SKP, c1 - c0, d_theta, d_p, d_cand, d_ub + c0, tcat, Mq);
+        TIP_CHECK_CUDA(cudaGetLastError());
+        tip_pair_vec_kernel<<<(int)((Q * 3 * L.SKP + 255) / 256), 256, 0, st>>>(Q, S, K, L.SKP, c0, c1, d_bidx, ra, rb, tcat, Mq, V);
+        TIP_CHECK_CUDA(cudaGetLastError());
+    }
+
+    // work items: the tiles that hold a test entry (capture), then each of them in rounds of at most e_max entries (count)
+    std::vector<int32_t> h_off((size_t)Q + 1);
+    TIP_CHECK_CUDA(cudaMemcpyAsync(h_off.data(), toff, ((size_t)Q + 1) * 4, cudaMemcpyDeviceToHost, st));
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    std::vector<int4> h_items;
+    const long long tiles = (Q + kPredRows - 1) / kPredRows;
+    for (long long t = 0; t < tiles; ++t) {
+        const int b = h_off[(size_t)(t * kPredRows)], e = h_off[(size_t)std::min(Q, (t + 1) * kPredRows)];
+        if (e > b) h_items.push_back(make_int4((int)t, b, e, 0));
+    }
+    const int n_capture = (int)h_items.size();
+    for (int k = 0; k < n_capture; ++k)
+        for (int b = h_items[k].y; b < h_items[k].z; b += e_max)
+            h_items.push_back(make_int4(h_items[k].x, b, std::min(h_items[k].z, b + e_max), 0));
+    const int n_count = (int)h_items.size() - n_capture;
+    TIP_REQUIRE((long long)h_items.size() <= L.max_items, "tip_rank_per_pair: %zu work items (internal error)", h_items.size());
+    TIP_CHECK_CUDA(cudaMemcpyAsync(items, h_items.data(), h_items.size() * sizeof(int4), cudaMemcpyHostToDevice, st));
+
+    const size_t smem0 = rank_smem(L.SKP, 0), smem1 = rank_smem(L.SKP, e_max);
+    static int smem_set = 0;
+    if ((int)smem1 > smem_set && smem1 > 48 * 1024) {
+        TIP_CHECK_CUDA(cudaFuncSetAttribute(tip_rank_pass_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
+        smem_set = (int)smem1;
+    }
+    int per_sm0 = 0, per_sm1 = 0;
+    TIP_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm0, tip_rank_pass_kernel, kPredThreads, smem0));
+    TIP_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm1, tip_rank_pass_kernel, kPredThreads, smem1));
+    TIP_REQUIRE(per_sm0 > 0 && per_sm1 > 0, "tip_rank_per_pair: S*K = %d does not fit one block's shared memory", S * K);
+
+    RankPassArgs A{};
+    A.n = n; A.SKP = L.SKP; A.n_pairs = (int)Q;
+    A.tcat = tcat; A.V = V; A.ra = ra; A.rb = rb;
+    A.te_off = toff; A.te_key = tk2; A.tr_beg = trb; A.tr_end = tre; A.tr_key = trk2;
+    A.te_bits = bits; A.ord_bits = obits; A.ord_pos = opos; A.te_idx = ti2; A.rank = d_rank_out; A.ctl = ctl;
+    // capture sweep
+    A.mode = 0; A.items = items; A.n_items = n_capture;
+    TIP_CHECK_CUDA(cudaMemsetAsync(ctl, 0, 8, st));
+    tip_rank_pass_kernel<<<(int)std::min<long long>((long long)sm_count() * per_sm0, n_capture), kPredThreads, smem0, st>>>(A);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    // per pair: entries in the order (bits descending, rc ascending): a stable sort of the (pair, rc) order
+    tip_rank_iota_kernel<<<gt, 256, 0, st>>>(T, opos0);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    cb = L.cub_bytes;
+    TIP_CHECK_CUDA(cub::DeviceSegmentedSort::StableSortPairsDescending(cub_tmp, cb, bits, obits, opos0, opos, (int)T, (int)Q, toff,
+                                                                      toff + 1, st));
+    // count sweep
+    A.mode = 1; A.items = items + n_capture; A.n_items = n_count;
+    TIP_CHECK_CUDA(cudaMemsetAsync(ctl, 0, 8, st));
+    tip_rank_pass_kernel<<<(int)std::min<long long>((long long)sm_count() * per_sm1, n_count), kPredThreads, smem1, st>>>(A);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    tip_rank_finish_kernel<<<gt, 256, 0, st>>>(T, S, tk2, ti2, bits, rep, NT, trk2, d_rank_out, d_score_out);
     TIP_CHECK_CUDA(cudaGetLastError());
     TIP_CHECK_CUDA(cudaStreamSynchronize(st));
     return 0;

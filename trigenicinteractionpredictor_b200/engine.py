@@ -11,6 +11,7 @@ CUDA kernels behind the C ABI (include/tip.h).  There is no CPU path.
     eng.top_triplets_per_gene(thetas, ps, cand, q, known, n)   # the same per query gene (tip_top_triplets_per_gene)
     eng.top_triplets_per_pair(thetas, ps, cand, pr, known, n)  # the same per query pair (tip_top_triplets_per_pair)
     eng.score_histogram(thetas, ps, cand)              # histogram of all C(n, 3) scores (tip_score_histogram)
+    eng.rank_per_pair(thetas, ps, cand, pr, known, tp, trc)   # held-out ranks per query pair (tip_rank_per_pair)
 """
 from __future__ import annotations
 
@@ -606,6 +607,43 @@ class EMEngine:
         ids = out_ids[:n_pairs * n].reshape(n_pairs, n, 3)[:, :m].cpu().numpy()
         sc = out_sc[:n_pairs * n].reshape(n_pairs, n)[:, :m].cpu().numpy()
         return ids, sc, counts
+
+    @_on_device
+    def rank_per_pair(self, theta_stack, p_stack, cand, pair_ranks, known, test_pair, test_rc):
+        """tip_rank_per_pair: the exact rank of every test entry (test_pair[j], an index into `pair_ranks`; test_rc[j], the
+        partner's rank) among its pair's partners whose triplet is not a key of `known`, in the order of
+        top_triplets_per_pair; arguments otherwise as there.  Returns (rank [T] int64, 0 when the entry is a known key;
+        score [T] float64, the mean over the S sets; universe [Q] int64, the partners that are not known keys)."""
+        th = np.ascontiguousarray(theta_stack, dtype=np.float64)
+        pp = np.ascontiguousarray(p_stack, dtype=np.float64)
+        S = int(th.shape[0])
+        assert th.shape == (S, self.P, self.K) and pp.shape == (S, self.K, self.K, self.K, 2)
+        cand = np.ascontiguousarray(cand, dtype=np.int32)
+        pr = np.ascontiguousarray(np.asarray(pair_ranks, dtype=np.int32).reshape(-1, 2))
+        known = np.ascontiguousarray(known, dtype=np.uint64)
+        tp = np.ascontiguousarray(test_pair, dtype=np.int32).reshape(-1)
+        trc = np.ascontiguousarray(test_rc, dtype=np.int32).reshape(-1)
+        assert tp.shape == trc.shape
+        n_cand, n_pairs, n_known, n_test = int(cand.shape[0]), int(pr.shape[0]), int(known.shape[0]), int(tp.shape[0])
+        nb = ctypes.c_size_t(0)
+        _cabi.check(self.lib.tip_rank_per_pair_workspace_bytes(n_cand, n_pairs, self.K, S, n_known, n_test, ctypes.byref(nb)),
+                    "tip_rank_per_pair_workspace_bytes")
+        d_th = torch.from_numpy(th.reshape(-1)).to(self.device)
+        d_p = torch.from_numpy(pp.reshape(-1)).to(self.device)
+        d_cand = torch.from_numpy(cand).to(self.device)
+        d_pr = torch.from_numpy(pr.reshape(-1)).to(self.device)
+        d_known = torch.from_numpy(known.view(np.int64)).to(self.device) if n_known else None
+        d_tp = torch.from_numpy(tp).to(self.device)
+        d_trc = torch.from_numpy(trc).to(self.device)
+        ws = torch.empty(max(nb.value, 1), dtype=torch.uint8, device=self.device)
+        rank = torch.zeros(max(n_test, 1), dtype=torch.int64, device=self.device)
+        score = torch.zeros(max(n_test, 1), dtype=torch.float64, device=self.device)
+        universe = torch.zeros(max(n_pairs, 1), dtype=torch.int64, device=self.device)
+        _cabi.check(self.lib.tip_rank_per_pair(
+            self.P, self.K, S, _ptr(d_th), _ptr(d_p), _ptr(d_cand), n_cand, _ptr(d_pr), n_pairs, _ptr(d_known), n_known,
+            _ptr(d_tp), _ptr(d_trc), n_test, _ptr(ws), nb.value, _ptr(rank), _ptr(score), _ptr(universe), self._stream()),
+            "tip_rank_per_pair")
+        return rank[:n_test].cpu().numpy(), score[:n_test].cpu().numpy(), universe[:n_pairs].cpu().numpy()
 
     @_on_device
     def score_histogram(self, theta_stack, p_stack, cand, log2_bins: int = 7, n_binades: int = 64):

@@ -2,7 +2,8 @@
 
     python -m trigenicinteractionpredictor_b200.predict -t train0.dat -e test0.dat \\
         -p results/Sample_0_K10.npz [-p results/Sample_1_K10.npz ...] [-n 100] [-g genes.txt] \\
-        [-q queries.txt | -r pairs.txt | --held-out] [--include-known] [-o predictions.tsv] [--device cuda:0]
+        [-q queries.txt | -r pairs.txt | --held-out | --held-out-pairs [-r pairs.txt]] [--include-known]
+        [-o predictions.tsv] [--device cuda:0]
 
 The train / test files rebuild the model's digestion (gene ids in order of first appearance, TIP.py:321-423); every
 parameter file (the .npz that training with --save-params writes) must belong to it.  With several files the score of a
@@ -28,7 +29,16 @@ universe is every triplet of the -g genes (default: all genes) that is not a key
 the exact rank.  Output: summary lines "Name:<TAB>value" (universe size, counts, recall at N for the positives and the
 negatives, the positives' median rank and AUC against the universe, each as lo or lo-hi), then the header
 "Rank<TAB>Predicted Interaction<TAB>Real Interaction<TAB>ID of genes<TAB>Genes" and one line per ranked test triplet, best
-first.  --held-out excludes -q, -r and --include-known."""
+first.  --held-out excludes -q, -r and --include-known.
+
+--held-out-pairs: where each test triplet lands among its query pair's unseen partners (Model.rank_held_out_per_pair,
+DESIGN §4.9).  Without -r every test triplet of the -g genes gives three views, one per pair of its genes; with -r a view
+is a listed pair and a test triplet that contains both of its genes, the third taken from the -g genes plus the pairs'
+genes.  A pair's universe is every partner whose triplet is not a key of the train file, and every rank is exact.
+Output: summary lines "Name:<TAB>value" (counts, hits at N for the positives and the negatives, the positives' median
+rank, MRR and AUC against the pair universes), then the header "Query pair<TAB>Rank<TAB>Pair universe<TAB>Predicted
+Interaction<TAB>Real Interaction<TAB>ID of genes<TAB>Genes" and one line per view, by pair (file order, or sorted names)
+and rank.  --held-out-pairs excludes -q, -n, --held-out and --include-known."""
 from __future__ import annotations
 
 import contextlib
@@ -40,7 +50,9 @@ HEADER = "Predicted Interaction\tID of genes\tGenes\n"
 QUERY_HEADER = "Query gene\t" + HEADER
 PAIR_HEADER = "Query pair\t" + HEADER
 HELD_OUT_HEADER = "Rank\tPredicted Interaction\tReal Interaction\tID of genes\tGenes\n"
+HELD_OUT_PAIRS_HEADER = "Query pair\tRank\tPair universe\tPredicted Interaction\tReal Interaction\tID of genes\tGenes\n"
 RECALL_AT = (100, 1000, 10000, 100000)
+HITS_AT = (1, 5, 10, 20, 50, 100)
 
 
 def _fail(msg: str) -> int:
@@ -52,11 +64,11 @@ def main(argv=None) -> int:
     argv = sys.argv[1:] if argv is None else argv
     train = test = out = device = genes_file = queries_file = pairs_file = None
     params: list[str] = []
-    top, include_known, held_out = None, False, False
+    top, include_known, held_out, held_out_pairs = None, False, False, False
     try:
         opts, rest = getopt.getopt(argv, "ht:e:p:n:g:q:r:o:", ["help", "train=", "test=", "params=", "top=", "genes=",
-                                                               "queries=", "pairs=", "include-known", "held-out", "out=",
-                                                               "device="])
+                                                               "queries=", "pairs=", "include-known", "held-out",
+                                                               "held-out-pairs", "out=", "device="])
     except getopt.GetoptError as exc:
         return _fail("argument error: %s" % exc)
     if rest:
@@ -86,11 +98,16 @@ def main(argv=None) -> int:
             include_known = True
         elif opt == "--held-out":
             held_out = True
+        elif opt == "--held-out-pairs":
+            held_out_pairs = True
         elif opt in ("-o", "--out"):
             out = arg
         elif opt == "--device":
             device = arg
-    if held_out:
+    if held_out_pairs:
+        if queries_file or held_out or include_known or top is not None:
+            return _fail("--held-out-pairs excludes -q/--queries, -n/--top, --held-out and --include-known")
+    elif held_out:
         if queries_file or pairs_file or include_known:
             return _fail("--held-out excludes -q/--queries, -r/--pairs and --include-known")
         top = 100000 if top is None else top
@@ -172,7 +189,13 @@ def main(argv=None) -> int:
     if len({th.shape[1] for th, _ in sets}) != 1:
         return _fail("the parameter files have different K")
 
-    if held_out:
+    if held_out_pairs:
+        try:
+            res = model.rank_held_out_per_pair(pairs, genes=genes, params=sets, hits_at=HITS_AT)
+        except ValueError as exc:
+            return _fail(str(exc))
+        text = held_out_pairs_text(res)
+    elif held_out:
         try:
             res = model.rank_held_out(top, genes=genes, params=sets, recall_at=RECALL_AT)
         except ValueError as exc:
@@ -217,6 +240,25 @@ def held_out_text(res: dict) -> str:
     body = "".join("%s\t%s\t%d\t%s\t%s\n" % (_interval((lo, hi)), score, label, key, names)
                    for key, names, label, score, lo, hi in res["rows"])
     return "\n".join(lines) + "\n" + HELD_OUT_HEADER + body
+
+
+def _value(v) -> str:
+    return "n/a" if v is None else str(v)
+
+
+def held_out_pairs_text(res: dict) -> str:
+    """Summary lines and the table of views of Model.rank_held_out_per_pair."""
+    lines = ["Query pairs:\t%d" % len(res["pairs"]), "Views:\t%d" % res["views"], "Positive views:\t%d" % res["positives"],
+             "Negative views:\t%d" % res["negatives"], "Excluded train keys:\t%d" % res["excluded_train"],
+             "Excluded outside the genes:\t%d" % res["excluded_genes"]]
+    for N, r in res["hits_at"].items():
+        lines.append("Hits at %d:\t%s" % (N, _value(r["positives"])))
+        lines.append("Negatives at %d:\t%s" % (N, _value(r["negatives"])))
+    lines += ["Median rank of positives:\t%s" % _value(res["median_rank"]), "MRR:\t%s" % _value(res["mrr"]),
+              "Pair AUC (micro):\t%s" % _value(res["auc_micro"]), "Pair AUC (macro):\t%s" % _value(res["auc_macro"])]
+    body = "".join("%s\t%d\t%d\t%s\t%d\t%s\t%s\n" % (pair, rank, universe, score, label, key, names)
+                   for pair, key, names, label, score, rank, universe in res["rows"])
+    return "\n".join(lines) + "\n" + HELD_OUT_PAIRS_HEADER + body
 
 
 if __name__ == "__main__":
