@@ -279,6 +279,30 @@ int tip_rank_per_pair(int P, int K, int S, const double *d_theta, const double *
                       void *d_ws, size_t ws_bytes, int64_t *d_rank_out, double *d_score_out,
                       int64_t *d_universe_out, void *stream);
 
+/* ---- held-out ranks per query gene: each test triplet's exact rank among its query's unseen triplets (DESIGN §4.10) ----
+ * Candidates, queries, scores and order as tip_top_triplets_per_gene: d_cand[n_cand] in decimal-string order (rank =
+ * position), d_query_ranks[n_query] distinct ranks into d_cand, score bits of the ensemble SUM over the S sets, the pairs
+ * of a query ordered by (score descending, packed ranks ascending).  d_known: sorted packed rank triples, the train keys (a
+ * repeated key counts once).  The universe of a query is every pair of other candidates whose triplet is not a known key.
+ * Test entry j is (d_test_query[j], an index into the caller's queries; d_test_u[j], d_test_v[j], the two other ranks in
+ * either order).  Out: d_rank_out[n_test] = 1 + the pairs of the universe ordered before the entry (0 when its triplet is
+ * a known key), exact under any ties; d_score_out[n_test] the mean score; d_universe_out[n_query] |U| = C(n_cand - 1, 2) -
+ * the known keys that contain the query.  Every score is computed as tip_top_triplets_per_gene computes it (same work
+ * item, Q tile and fragment position), so a triplet that it returns at position k for a query, with the known keys alone,
+ * has rank k + 1 and the same score bits.  One sweep records the bits of the test and train triplets of the queries, a
+ * second counts every score of a query ahead of its test entries, held in shared memory in rounds; the train triplets
+ * ahead of an entry are subtracted.  A query rank out of range or given twice, a test query index out of range and a test
+ * rank that is out of range, equal to its query's or to its other rank are refused before any device work.  Synchronises
+ * the stream.  Limits: n_cand <= 2^21, S * K <= 384, n_query <= n_cand, n_known <= 2^29, n_test < 2^31 (and the test
+ * entries plus the queries' train triplets < 2^31).  Workspace O(n_cand S K + n_query S K^2 + n_test + n_known).
+ * Precondition: finite, non-negative parameters.  d_ws: tip_rank_per_gene_workspace_bytes() bytes. */
+int tip_rank_per_gene_workspace_bytes(int n_cand, int n_query, int K, int S, int64_t n_known, int64_t n_test, size_t *bytes);
+int tip_rank_per_gene(int P, int K, int S, const double *d_theta, const double *d_p, const int32_t *d_cand, int n_cand,
+                      const int32_t *d_query_ranks, int n_query, const uint64_t *d_known, int64_t n_known,
+                      const int32_t *d_test_query, const int32_t *d_test_u, const int32_t *d_test_v, int64_t n_test,
+                      void *d_ws, size_t ws_bytes, int64_t *d_rank_out, double *d_score_out,
+                      int64_t *d_universe_out, void *stream);
+
 /* ---- testResultsReducer.py:160-184: mean / median / standard deviation of every test triplet across samples ----
  * d_scores[S][T]: score of triplet t in sample j at [j * T + t]; d_n[t] (or NULL = S) = how many leading samples of
  * triplet t are valid.  mean = sequential sum in sample order / n; median = the reference's rule (ascending sort;

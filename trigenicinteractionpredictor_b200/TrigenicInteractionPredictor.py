@@ -1016,6 +1016,127 @@ class Model:
                 "auc_micro": float(np.mean(auc_v)) if len(auc_v) else None,
                 "auc_macro": float(np.mean(auc_s[auc_n > 0] / auc_n[auc_n > 0])) if (auc_n > 0).any() else None}
 
+    def rank_held_out_per_gene(self, queries=None, genes=None, params=None, hits_at=(1, 10, 20, 100, 1000, 10000)):
+        """Where each held-out triplet lands among its query gene's unseen triplets (addition; DESIGN §4.10).
+
+        A view is a query gene q and a test triplet that contains it.  With queries=None every ranked test triplet gives
+        three views, one per gene; the candidates are `genes` (names; default all P genes).  With `queries` (names,
+        distinct) a view is a listed query and a test triplet that contains it; the candidates are `genes` + the queries.
+        A test triplet is ranked when its three genes are distinct candidates and it is not a key of links; the others are
+        counted as excluded.  The universe U_q of a query is every pair {x, y} of other candidates whose triplet {q, x, y}
+        is not a key of links (test keys stay in it), ordered as in predict_top_triplets_per_gene (score descending, then
+        the triplets' positions in the decimal-string order of the candidate ids), scored by the current theta / pr or by
+        the mean over the sets of `params`.  rank = 1 + the triplets of U_q before the view's triplet, exact.  Labels follow
+        calculate_metrics: 0 if n0 != 0 else 1.
+
+        Returns a dict:
+          rows: [[query gene, key "a_b_c", names, label, score, rank, universe], ...] in query order (the order of
+            `queries`, or sorted names), each query's views in rank order;
+          genes: [[gene, universe, positives, negatives, best positive rank, gene AUC], ...] in the same order (a listed
+            query without a test triplet has zero counts);
+          views, positives, negatives, excluded_train, excluded_genes;
+          hits_at: {N: {"positives": fraction, "negatives": fraction}}, the share of views with rank <= N;
+          median_rank of the positive views; mrr, the mean over genes with a positive of 1 / its best positive rank;
+          auc_micro / auc_macro: the mean of (|U| - rank) / (|U| - 1) over positive views / over genes (each the mean of
+            its positives).
+        Values that need a positive, or |U| > 1, are None without them."""
+        who = "rank_held_out_per_gene"
+        sets = self._prediction_sets(params, who)
+        K = sets[0][0].shape[1]
+        if len(self.test_links) == 0:
+            raise ValueError(who + ": the model has no test links")
+        names = list(genes) if genes is not None else []
+        if queries is not None:
+            queries = list(queries)
+            if not queries:
+                raise ValueError(who + ": queries is empty")
+            names = queries + names
+        missing = [g for g in names if g not in self.gene_id]
+        if missing:
+            raise ValueError("unknown gene names: %s" % ", ".join(dict.fromkeys(missing)))
+        if queries is not None:
+            twice = [g for g, c in collections.Counter(queries).items() if c > 1]
+            if twice:
+                raise ValueError(who + ": duplicate query genes: %s" % ", ".join(twice))
+        hits_at = [int(x) for x in hits_at]
+        ids = set(range(self.P)) if genes is None else {self.gene_id[g] for g in names}
+        cand = np.array(sorted(ids, key=str), dtype=np.int32)
+        n = int(cand.shape[0])
+        rank = np.full(self.P, -1, dtype=np.int64)
+        rank[cand] = np.arange(n, dtype=np.int64)
+        train = self._train_packed(cand)
+
+        t1, t2, t3, t_n0, _ = [np.asarray(x.cpu().numpy() if _is_torch(x) else x, dtype=np.int64) for x in self._soa(self.test_links)]
+        r = np.sort(np.stack([rank[t1], rank[t2], rank[t3]], axis=1), axis=1)
+        triplet = (r[:, 0] >= 0) & (r[:, 0] < r[:, 1]) & (r[:, 1] < r[:, 2])
+        packed = ((r[:, 0] << 42) | (r[:, 1] << 21) | r[:, 2]).astype(np.uint64)
+        at = np.minimum(np.searchsorted(train, packed), max(len(train) - 1, 0))
+        in_train = triplet & (train[at] == packed) if len(train) else np.zeros_like(triplet)
+        sel = np.flatnonzero(triplet & ~in_train)
+        r, labels = r[sel], np.where(t_n0[sel] != 0, 0, 1)
+
+        # views: (query rank, the other two ranks, test triplet)
+        m = len(sel)
+        v_qr = np.concatenate([r[:, 0], r[:, 1], r[:, 2]])
+        v_u = np.concatenate([r[:, 1], r[:, 0], r[:, 0]])
+        v_v = np.concatenate([r[:, 2], r[:, 2], r[:, 1]])
+        v_t = np.tile(np.arange(m, dtype=np.int64), 3)
+        gene_name = np.array(self._genes_in_id_order())
+        if queries is None:
+            uq = np.unique(v_qr)
+            q_names = gene_name[cand[uq]]
+            order = np.argsort(q_names, kind="stable")
+            uq, labels_q = uq[order], q_names[order].tolist()
+        else:
+            uq = np.array([rank[self.gene_id[g]] for g in queries], dtype=np.int64)
+            labels_q = queries
+        qidx = np.full(n, -1, dtype=np.int64)
+        qidx[uq] = np.arange(len(uq), dtype=np.int64)
+        keep = qidx[v_qr] >= 0
+        v_query, v_u, v_v, v_t = qidx[v_qr[keep]], v_u[keep], v_v[keep], v_t[keep]
+
+        thetas = np.stack([th for th, _ in sets])
+        prs = np.stack([p_ for _, p_ in sets])
+        eng = self._prediction_engine(K)
+        v_rank, v_score, universe = eng.rank_per_gene(thetas, prs, cand, uq, train, v_query, v_u, v_v)
+
+        order = np.lexsort((v_rank, v_query))
+        v_query, v_t, v_rank, v_score = v_query[order], v_t[order], v_rank[order], v_score[order]
+        v_lab = labels[v_t]
+        g = cand[r[v_t]].astype(np.int64)
+        nm = gene_name[g]
+        nm.sort(axis=1)
+        v_uni = universe[v_query]
+        rows = [list(x) for x in zip([labels_q[i] for i in v_query.tolist()], ["%d_%d_%d" % tuple(x) for x in g.tolist()],
+                                     ["_".join(t) for t in nm.tolist()], v_lab.tolist(), v_score.tolist(), v_rank.tolist(),
+                                     v_uni.tolist())]
+        positive = v_lab == 1
+        Q = len(labels_q)
+        n_pos_q = np.bincount(v_query[positive], minlength=Q)
+        n_neg_q = np.bincount(v_query[~positive], minlength=Q)
+        best = np.full(Q, np.iinfo(np.int64).max)
+        np.minimum.at(best, v_query[positive], v_rank[positive])
+        auc_ok = positive & (v_uni > 1)
+        auc_v = (v_uni[auc_ok] - v_rank[auc_ok]) / (v_uni[auc_ok] - 1)
+        auc_n = np.bincount(v_query[auc_ok], minlength=Q)
+        auc_s = np.bincount(v_query[auc_ok], weights=auc_v, minlength=Q)
+        gene_rows = [[labels_q[q], int(universe[q]), int(n_pos_q[q]), int(n_neg_q[q]),
+                      int(best[q]) if n_pos_q[q] else None, float(auc_s[q] / auc_n[q]) if auc_n[q] else None] for q in range(Q)]
+
+        def frac(mask, N):
+            total = int(mask.sum())
+            return int((v_rank[mask] <= N).sum()) / total if total else None
+
+        has_pos = n_pos_q > 0
+        return {"rows": rows, "genes": gene_rows, "views": len(rows), "positives": int(positive.sum()),
+                "negatives": int((~positive).sum()), "excluded_train": int(in_train.sum()),
+                "excluded_genes": int((~triplet).sum()),
+                "hits_at": {N: {"positives": frac(positive, N), "negatives": frac(~positive, N)} for N in hits_at},
+                "median_rank": float(np.median(v_rank[positive])) if positive.any() else None,
+                "mrr": float(np.mean(1.0 / best[has_pos])) if has_pos.any() else None,
+                "auc_micro": float(np.mean(auc_v)) if len(auc_v) else None,
+                "auc_macro": float(np.mean(auc_s[auc_n > 0] / auc_n[auc_n > 0])) if (auc_n > 0).any() else None}
+
     # ------------------------------------------------------------------------------------------
     # report (TIP.py:793-904)
     # ------------------------------------------------------------------------------------------

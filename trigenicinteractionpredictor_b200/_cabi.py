@@ -70,6 +70,10 @@ SIGNATURES = {
     "tip_rank_per_pair_workspace_bytes": (c_int, [c_int, c_int64, c_int, c_int, c_int64, c_int64, _psz]),
     "tip_rank_per_pair": (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int64, c_void_p, c_int64,
                                   c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "tip_rank_per_gene_workspace_bytes": (c_int, [c_int, c_int, c_int, c_int, c_int64, c_int64, _psz]),
+    "tip_rank_per_gene": (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int64,
+                                  c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p,
+                                  c_void_p]),
     "tip_reduce_samples": (c_int, [c_int, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "tip_em_iterations_host": (c_int, [c_int, c_int, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_int,
                                        c_uint]),

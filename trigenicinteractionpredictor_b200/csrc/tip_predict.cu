@@ -27,11 +27,16 @@
 //
 // Ranks per query pair (tip_rank_per_pair): the tiles and column phases of tip_top_triplets_per_pair, swept once to record
 // the scores of the held-out partners and once to count, per pair, the scores ahead of each of them (tip_rank_pass_kernel).
+//
+// Ranks per query gene (tip_rank_per_gene): the work items, Q tiles and column blocks of tip_top_triplets_per_gene, swept
+// once to record the scores of the held-out and train triplets of the queries and once to count, per query, the scores
+// ahead of each held-out one (tip_gene_rank_pass_kernel); the train triplets ahead are subtracted.
 #include <algorithm>
 #include <cmath>
 #include <vector>
 
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 #include <cub/device/device_segmented_sort.cuh>
 #include <cub/device/device_select.cuh>
 
@@ -2611,6 +2616,630 @@ extern "C" int tip_rank_per_pair(int P, int K, int S, const double *d_theta, con
     tip_rank_pass_kernel<<<(int)std::min<long long>((long long)sm_count() * per_sm1, n_count), kPredThreads, smem1, st>>>(A);
     TIP_CHECK_CUDA(cudaGetLastError());
     tip_rank_finish_kernel<<<gt, 256, 0, st>>>(T, S, tk2, ti2, bits, rep, NT, trk2, d_rank_out, d_score_out);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
+// ---- tip_rank_per_gene ----
+// The exact rank of every held-out triplet among its query gene's unseen triplets.  The work items (query, region, 64-row
+// tile) of query_tiles, the Q tiles that form_q_tile builds from the Mq of tip_query_prep_kernel, the column blocks from
+// col0 + wc 32 in steps of 64 and dmma_block are those of tip_query_pass_kernel, so every score is computed at the same
+// fragment position, with the same contraction order, as tip_top_triplets_per_gene computes it.  In a triplet {q, u, v}
+// with u < v the row is u and the column v.  Entries are keyed (query index << 42) | (u << 21) | v; for a fixed query this
+// order is the packed order of the triplets.  They are the test entries and the train entries: per distinct known key, each
+// of its genes that is a query.
+// Capture sweep: only the tiles that hold an entry; each warp jumps to the column blocks that hold an entry of one of its rows
+// and the lane that holds the score writes its bits.  A segmented stable sort then orders each query's entries by (bits
+// descending, key ascending), and a scan of the test flags gives every test entry its place among the query's test entries
+// and the number of train entries ahead of it.
+// Count sweep: items (query, round, region, tile), query-major; a round is at most e_max of the query's test entries, held in
+// shared memory.  Every score is tested in registers against the round's weakest entry, then its first; the scores between
+// them are placed by binary search and counted at their slot with a shared atomic.  Slot counts go to global memory, one
+// atomic per slot, when the CTA's (query, round) changes.  rank = 1 + the round's slot counts up to the entry - the train
+// entries ahead of it: train triplets are counted like any other score and subtracted, not skipped.
+namespace tip {
+namespace {
+
+constexpr int kGeneEntryBytes = 20;                      // a count round's entry in shared memory: bits, key, slot count
+constexpr unsigned long long kUvMask = (1ull << (2 * kRankBits)) - 1;
+
+struct GeneRankArgs {
+    int n, S, K, SK, SKP, mode;           // mode 0: capture the bits of the entries; 1: count
+    const double *tcat;                   // [n_pad][SKP]
+    const double *Mq;                     // [n_query][3][S][K][K]
+    const int32_t *qrank;                 // [n_query]
+    const long long *seg_start;           // capture: [n_query + 1] first item of each query; count: [n_seg + 1] of each round
+    const int4 *seg;                      // count: [n_seg] {query, first, end, 0}: the round's entries in the t_* arrays
+    int n_seg;
+    const long long *items;               // capture: [n_items] the item ids that hold an entry
+    long long n_items;
+    int e_max;                            // count: entries of a round in shared memory
+    const unsigned long long *key;        // capture: [n_entries] sorted entry keys
+    const int32_t *q_off;                 // capture: [n_query + 1] each query's entries in key
+    unsigned long long *bits;             // capture: [n_entries] score bits, key order
+    const unsigned long long *t_bits;     // count: test entries per query in the order (bits descending, key ascending)
+    const unsigned long long *t_uv;       // count: (u << 21) | v of each
+    unsigned long long *t_cnt;            // count: slot counts
+    unsigned long long *ctl;              // [0] item cursor
+};
+
+__device__ __forceinline__ unsigned long long lane_bits(double v) { return (unsigned long long)__double_as_longlong(v); }
+
+__global__ void __launch_bounds__(kPredThreads) tip_gene_rank_pass_kernel(GeneRankArgs A)
+{
+    extern __shared__ __align__(16) unsigned char smem[];
+    const int qs = q_stride(A.SKP);
+    double *Q = reinterpret_cast<double *>(smem);                                                  // [64][qs]
+    unsigned long long *sh_eb = reinterpret_cast<unsigned long long *>(Q + (size_t)kPredRows * qs);  // count: entry bits
+    unsigned long long *sh_ek = sh_eb + A.e_max;                                                   // entry (u << 21) | v
+    unsigned *sh_cnt = reinterpret_cast<unsigned *>(sh_ek + A.e_max);                              // slot counts
+    __shared__ long long sh_item;
+    __shared__ long long sh_lb[kPredRows], sh_le[kPredRows];   // capture: each row's entries in key
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int wr = warp & 1, wc = warp >> 1;
+    const int gq = lane >> 2, tq = lane & 3;
+    const int n = A.n, SKP = A.SKP, K = A.K;
+    const long long KK = (long long)K * K;
+    const bool count = A.mode == 1;
+    int cur_seg = -1, ne = 0;   // count: the round whose entries and slot counts shared memory holds (CTA-uniform)
+    double since_flush = 0.0;   // as in tip_predict_pass_kernel: the 32-bit slot counts are flushed before they could overflow
+
+    for (;;) {
+        __syncthreads();   // Q, the entries and sh_item of the previous item are no longer read
+        if (tid == 0) sh_item = (long long)atomicAdd(A.ctl, 1ull);
+        __syncthreads();
+        const long long it = sh_item;
+        if (it >= A.n_items) break;
+        const long long item = count ? it : A.items[it];
+        int sl = 0, sh = A.n_seg - 1;
+        while (sl < sh) {
+            const int mid = (sl + sh + 1) >> 1;
+            if (A.seg_start[mid] <= item) sl = mid; else sh = mid - 1;
+        }
+        const int qi = count ? A.seg[sl].x : sl, r = A.qrank[qi];
+        if (count && (sl != cur_seg || since_flush > 2.0e9)) {
+            // the same thread flushes, clears and reloads an index: no barrier between the loops
+            for (int e = tid; e < ne; e += kPredThreads) {
+                if (sh_cnt[e]) atomicAdd(A.t_cnt + A.seg[cur_seg].y + e, (unsigned long long)sh_cnt[e]);
+                sh_cnt[e] = 0;
+            }
+            if (sl != cur_seg) {
+                const int4 s = A.seg[sl];
+                ne = s.z - s.y;
+                for (int e = tid; e < ne; e += kPredThreads) {
+                    sh_eb[e] = A.t_bits[s.y + e];
+                    sh_ek[e] = A.t_uv[s.y + e];
+                    sh_cnt[e] = 0;
+                }
+                cur_seg = sl;
+            }
+            since_flush = 0.0;
+        }
+        int tc, tb, ta;
+        query_tiles(n, r, tc, tb, ta);
+        int t = (int)(item - A.seg_start[sl]);
+        int g, a0, col0, row_end;
+        bool tri;
+        if (t < tc) {
+            g = 0; a0 = t * kPredRows; col0 = a0 + 1; row_end = r - 1; tri = true;
+        } else if ((t -= tc) < tb) {
+            g = 1; a0 = t * kPredRows; col0 = r + 1; row_end = r; tri = false;
+        } else {
+            t -= tb;
+            g = 2; a0 = r + 1 + t * kPredRows; col0 = a0 + 1; row_end = n - 1; tri = true;
+        }
+        const int col_end = g == 0 ? r : n;
+        const int rows = min(kPredRows, row_end - a0);
+        if (!count && tid < kPredRows) {
+            long long b = 0, e = 0;
+            if (tid < rows) {
+                const long long qb = A.q_off[qi], qe = A.q_off[qi + 1];
+                const unsigned long long k0 = ((unsigned long long)qi << (2 * kRankBits)) | ((unsigned long long)(a0 + tid) << kRankBits);
+                b = qb + lower_bound_u64(A.key + qb, qe - qb, k0);
+                e = b + lower_bound_u64(A.key + b, qe - b, k0 + (1ull << kRankBits));
+            }
+            sh_lb[tid] = b;
+            sh_le[tid] = e;
+        }
+
+        form_q_tile(Q, qs, A.tcat, SKP, A.SK, K, a0, rows, A.Mq + ((long long)qi * 3 + g) * A.S * KK, KK);
+        __syncthreads();
+
+        if (wr * 32 < rows) {
+            const int ib = wr * 32 + gq;   // the lane's first row in the tile
+            const double *Qw = Q + ib * qs + tq;
+            const int cbase = col0 + wc * 32;
+            if (!count) {
+                long long cur[4], lim[4];
+                bool any = false;
+#pragma unroll
+                for (int mi = 0; mi < 4; ++mi) {
+                    cur[mi] = sh_lb[ib + mi * 8];
+                    lim[mi] = sh_le[ib + mi * 8];
+                    any |= cur[mi] < lim[mi];
+                }
+                const bool warp_any = __any_sync(0xffffffffu, any);
+                for (int c0 = cbase; warp_any && c0 < col_end; c0 += 64) {
+                    // the warp's next column, at or after c0, that holds an entry of one of its rows in this region
+                    int nxt = INT_MAX;
+#pragma unroll
+                    for (int mi = 0; mi < 4; ++mi) {
+                        const int ra = a0 + ib + mi * 8;
+                        const int from = max(c0, tri ? ra + 1 : col0);
+                        while (cur[mi] < lim[mi] && (int)(__ldg(A.key + cur[mi]) & kRcMask) < from) ++cur[mi];
+                        if (cur[mi] < lim[mi]) {
+                            const int v = (int)(__ldg(A.key + cur[mi]) & kRcMask);
+                            if (v < col_end) nxt = min(nxt, v);
+                        }
+                    }
+                    nxt = __reduce_min_sync(0xffffffffu, nxt);
+                    if (nxt >= col_end) break;
+                    c0 = cbase + (nxt - cbase) / 64 * 64;
+                    if (nxt - c0 >= 32) continue;   // in the other column half: look again from the next block
+                    double acc[4][4][2];
+                    dmma_block(acc, Qw, qs, A.tcat + (long long)(c0 + gq) * SKP + tq, SKP);
+                    const int rc0 = c0 + 2 * tq;
+#pragma unroll
+                    for (int mi = 0; mi < 4; ++mi)
+                        while (cur[mi] < lim[mi]) {
+                            const int v = (int)(__ldg(A.key + cur[mi]) & kRcMask);
+                            if (v >= c0 + 32 || v >= col_end) break;
+                            double s = 0.0;
+                            if (lane_score(acc, mi, v - rc0, s)) A.bits[cur[mi]] = lane_bits(s);
+                            ++cur[mi];
+                        }
+                }
+            } else {
+                const unsigned long long wb = sh_eb[ne - 1], wk = sh_ek[ne - 1], fb = sh_eb[0], fk = sh_ek[0];
+                const int ra0 = a0 + ib;
+                unsigned ahead = 0;   // scores ahead of every entry of the round
+                for (int c0 = cbase; c0 < col_end; c0 += 64) {
+                    double acc[4][4][2];
+                    dmma_block(acc, Qw, qs, A.tcat + (long long)(c0 + gq) * SKP + tq, SKP);
+                    const int rc0 = c0 + 2 * tq;
+#pragma unroll
+                    for (int mi = 0; mi < 4; ++mi)
+#pragma unroll
+                        for (int ni = 0; ni < 4; ++ni)
+#pragma unroll
+                            for (int e = 0; e < 2; ++e) {
+                                const int ra = ra0 + mi * 8, rc = rc0 + ni * 8 + e;
+                                if (ra >= row_end || rc >= col_end || (tri && rc <= ra)) continue;
+                                const unsigned long long b = lane_bits(acc[mi][ni][e]);
+                                const unsigned long long k = ((unsigned long long)ra << kRankBits) | (unsigned long long)rc;
+                                if (!(b > wb || (b == wb && k < wk))) continue;   // not ahead of the weakest entry
+                                if (b > fb || (b == fb && k < fk)) {
+                                    ++ahead;
+                                    continue;
+                                }
+                                // the first entry in (0, ne - 1] the score is ahead of
+                                int lo = 1, hi = ne - 1;
+                                while (lo < hi) {
+                                    const int mid = (lo + hi) >> 1;
+                                    const unsigned long long mb = sh_eb[mid];
+                                    if (b > mb || (b == mb && k < sh_ek[mid])) hi = mid; else lo = mid + 1;
+                                }
+                                atomicAdd(sh_cnt + lo, 1u);
+                            }
+                }
+                ahead = __reduce_add_sync(0xffffffffu, ahead);
+                if (lane == 0 && ahead) atomicAdd(sh_cnt, ahead);
+            }
+        }
+        since_flush += (double)rows * (col_end - col0);
+    }
+    if (count)
+        for (int e = tid; e < ne; e += kPredThreads)
+            if (sh_cnt[e]) atomicAdd(A.t_cnt + A.seg[cur_seg].y + e, (unsigned long long)sh_cnt[e]);
+}
+
+// entries: test entry j is ((query << 42) | (min(u, v) << 21) | max(u, v), j)
+__global__ void tip_gene_test_keys_kernel(long long n_test, const int32_t *__restrict__ tq, const int32_t *__restrict__ tu,
+                                          const int32_t *__restrict__ tv, unsigned long long *__restrict__ key,
+                                          int32_t *__restrict__ idx)
+{
+    const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n_test) return;
+    const unsigned long long u = (unsigned long long)min(tu[j], tv[j]), v = (unsigned long long)max(tu[j], tv[j]);
+    key[j] = ((unsigned long long)tq[j] << (2 * kRankBits)) | (u << kRankBits) | v;
+    idx[j] = (int32_t)j;
+}
+
+// the train entries: per distinct known key (ascending ranks, all < n) and each of its genes that is a query, the key's other
+// two ranks, appended after the n_test test entries with an index >= n_test
+__global__ void tip_gene_train_kernel(long long n_known, const unsigned long long *__restrict__ known, int n,
+                                      const int32_t *__restrict__ qidx, long long n_test, unsigned long long *__restrict__ key,
+                                      int32_t *__restrict__ idx, unsigned long long *n_tr)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_known || (i > 0 && known[i] == known[i - 1])) return;   // a repeated key counts once
+    const unsigned long long k = known[i];
+    const unsigned long long r0 = (k >> (2 * kRankBits)) & kRcMask, r1 = (k >> kRankBits) & kRcMask, r2 = k & kRcMask;
+    if (!(r0 < r1 && r1 < r2 && r2 < (unsigned long long)n)) return;
+    const unsigned long long self[3] = {r0, r1, r2};
+    const unsigned long long other[3] = {(r1 << kRankBits) | r2, (r0 << kRankBits) | r2, (r0 << kRankBits) | r1};
+    for (int w = 0; w < 3; ++w) {
+        const int q = qidx[self[w]];
+        if (q < 0) continue;
+        const long long at = n_test + (long long)atomicAdd(n_tr, 1ull);
+        key[at] = ((unsigned long long)q << (2 * kRankBits)) | other[w];
+        idx[at] = (int32_t)at;
+    }
+}
+
+// per query: its first entry in the sorted keys
+__global__ void tip_gene_offsets_kernel(int n_query, long long n_entries, const unsigned long long *__restrict__ key,
+                                        int32_t *__restrict__ off)
+{
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q > n_query) return;
+    off[q] = (int32_t)lower_bound_u64(key, n_entries, (unsigned long long)q << (2 * kRankBits));
+}
+
+// per sorted entry: the work item (query_tiles numbering from item_start[query]) that holds its score
+__global__ void tip_gene_items_kernel(long long n_entries, int n, const unsigned long long *__restrict__ key,
+                                      const int32_t *__restrict__ qrank, const long long *__restrict__ item_start,
+                                      unsigned long long *__restrict__ item)
+{
+    const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n_entries) return;
+    const unsigned long long k = key[p];
+    const int q = (int)(k >> (2 * kRankBits)), u = (int)((k >> kRankBits) & kRcMask), v = (int)(k & kRcMask), r = qrank[q];
+    int tc, tb, ta;
+    query_tiles(n, r, tc, tb, ta);
+    const int t = v < r ? u / kPredRows : u < r ? tc + u / kPredRows : tc + tb + (u - r - 1) / kPredRows;
+    item[p] = (unsigned long long)(item_start[q] + t);
+}
+
+// per entry in the query order (bits descending, key ascending): 1 when it is a test entry
+__global__ void tip_gene_flags_kernel(long long n_entries, const int32_t *__restrict__ ord_pos, const int32_t *__restrict__ idx,
+                                      long long n_test, int32_t *__restrict__ flag)
+{
+    const long long o = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (o < n_entries) flag[o] = idx[ord_pos[o]] < n_test ? 1 : 0;
+}
+
+// the test entries of each query in that order (tscan: exclusive scan of the flags), with the train entries ahead of each,
+// -1 when its triplet is a train entry itself (the last entry of its key's run is then a train entry)
+__global__ void tip_gene_compact_kernel(long long n_entries, long long n_test, const unsigned long long *__restrict__ key,
+                                        const int32_t *__restrict__ idx, const int32_t *__restrict__ q_off,
+                                        const unsigned long long *__restrict__ ord_bits, const int32_t *__restrict__ ord_pos,
+                                        const int32_t *__restrict__ tscan, unsigned long long *__restrict__ t_bits,
+                                        unsigned long long *__restrict__ t_uv, int32_t *__restrict__ t_idx,
+                                        int32_t *__restrict__ t_train)
+{
+    const long long o = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (o >= n_entries) return;
+    const long long p = ord_pos[o];
+    if (idx[p] >= n_test) return;
+    const unsigned long long k = key[p];
+    const int q = (int)(k >> (2 * kRankBits));
+    const long long qb = q_off[q], qe = q_off[q + 1];
+    const long long last = p + lower_bound_u64(key + p, qe - p, k + 1) - 1;
+    const int t = tscan[o];
+    t_bits[t] = ord_bits[o];
+    t_uv[t] = k & kUvMask;
+    t_idx[t] = idx[p];
+    t_train[t] = idx[last] >= n_test ? -1 : (int32_t)((o - qb) - (t - tscan[qb]));
+}
+
+// per query: its first test entry in the t_* arrays and |U| = C(n - 1, 2) - its train entries
+__global__ void tip_gene_universe_kernel(int n_query, long long n_entries, long long n_test, long long pairs,
+                                         const int32_t *__restrict__ q_off, const int32_t *__restrict__ tscan,
+                                         int32_t *__restrict__ t_off, int64_t *__restrict__ universe)
+{
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q > n_query) return;
+    auto tests_before = [&](long long o) -> long long { return n_test == 0 ? 0 : o < n_entries ? tscan[o] : n_test; };
+    t_off[q] = (int32_t)tests_before(q_off[q]);
+    if (q == n_query) return;
+    const long long train = (q_off[q + 1] - q_off[q]) - (tests_before(q_off[q + 1]) - tests_before(q_off[q]));
+    universe[q] = pairs - train;
+}
+
+// per round: rank = 1 + the round's slot counts up to the entry - the train entries ahead of it (0 for a train triplet)
+__global__ void tip_gene_finish_kernel(int n_seg, int S, const int4 *__restrict__ seg, const unsigned long long *__restrict__ t_cnt,
+                                       const unsigned long long *__restrict__ t_bits, const int32_t *__restrict__ t_idx,
+                                       const int32_t *__restrict__ t_train, int64_t *__restrict__ rank, double *__restrict__ score)
+{
+    const int s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= n_seg) return;
+    long long run = 0;
+    for (int k = seg[s].y; k < seg[s].z; ++k) {
+        run += (long long)t_cnt[k];
+        const int j = t_idx[k];
+        score[j] = __longlong_as_double((long long)t_bits[k]) / (double)S;
+        rank[j] = t_train[k] < 0 ? 0 : 1 + run - t_train[k];
+    }
+}
+
+struct GeneRankLayout {
+    size_t o_tcat, o_M, o_qidx, o_istart, o_qoff, o_toff, o_key, o_key2, o_idx, o_idx2, o_bits, o_obits, o_opos0, o_opos, o_flag,
+        o_scan, o_item, o_item2, o_uitem, o_tbits, o_tuv, o_tcnt, o_tidx, o_ttr, o_seg, o_sstart, o_cnt, o_cub, cub_bytes, total;
+    int n_pad, SKP;
+    long long max_seg;
+};
+
+GeneRankLayout gene_rank_layout(int n, int n_query, int K, int S, long long n_known, long long n_test)
+{
+    GeneRankLayout L{};
+    L.n_pad = (n + 63) / 64 * 64 + 64;
+    L.SKP = (S * K + 3) / 4 * 4;
+    L.max_seg = n_query + n_test / kRankMinEntries + 1;
+    const long long e_all = n_test + 3 * n_known;
+    const int ne = (int)std::min<long long>(e_all, INT_MAX), nq = std::max(n_query, 1);
+    size_t cb[5] = {0, 0, 0, 0, 0};
+    cub::DeviceRadixSort::SortPairs(nullptr, cb[0], (const unsigned long long *)nullptr, (unsigned long long *)nullptr,
+                                    (const int32_t *)nullptr, (int32_t *)nullptr, ne, 0, 64, (cudaStream_t)0);
+    cub::DeviceRadixSort::SortKeys(nullptr, cb[1], (const unsigned long long *)nullptr, (unsigned long long *)nullptr, ne, 0, 64,
+                                   (cudaStream_t)0);
+    cub::DeviceSelect::Unique(nullptr, cb[2], (const unsigned long long *)nullptr, (unsigned long long *)nullptr, (int *)nullptr, ne,
+                              (cudaStream_t)0);
+    cub::DeviceSegmentedSort::StableSortPairsDescending(nullptr, cb[3], (const unsigned long long *)nullptr,
+                                                        (unsigned long long *)nullptr, (const int32_t *)nullptr, (int32_t *)nullptr,
+                                                        ne, nq, (const int *)nullptr, (const int *)nullptr, (cudaStream_t)0);
+    cub::DeviceScan::ExclusiveSum(nullptr, cb[4], (const int32_t *)nullptr, (int32_t *)nullptr, ne, (cudaStream_t)0);
+    L.cub_bytes = *std::max_element(cb, cb + 5);
+    const size_t e = (size_t)e_all, t = (size_t)n_test, q = (size_t)n_query;
+    size_t off = 0;
+    L.o_tcat = off;   off += a256((size_t)L.n_pad * L.SKP * 8);
+    L.o_M = off;      off += a256(q * 3 * S * K * K * 8);
+    L.o_qidx = off;   off += a256((size_t)n * 4);
+    L.o_istart = off; off += a256((q + 1) * 8);
+    L.o_qoff = off;   off += a256((q + 1) * 4);
+    L.o_toff = off;   off += a256((q + 1) * 4);
+    L.o_key = off;    off += a256(e * 8);
+    L.o_key2 = off;   off += a256(e * 8);
+    L.o_idx = off;    off += a256(e * 4);
+    L.o_idx2 = off;   off += a256(e * 4);
+    L.o_bits = off;   off += a256(e * 8);
+    L.o_obits = off;  off += a256(e * 8);
+    L.o_opos0 = off;  off += a256(e * 4);
+    L.o_opos = off;   off += a256(e * 4);
+    L.o_flag = off;   off += a256(e * 4);
+    L.o_scan = off;   off += a256(e * 4);
+    L.o_item = off;   off += a256(e * 8);
+    L.o_item2 = off;  off += a256(e * 8);
+    L.o_uitem = off;  off += a256(e * 8);
+    L.o_tbits = off;  off += a256(t * 8);
+    L.o_tuv = off;    off += a256(t * 8);
+    L.o_tcnt = off;   off += a256(t * 8);
+    L.o_tidx = off;   off += a256(t * 4);
+    L.o_ttr = off;    off += a256(t * 4);
+    L.o_seg = off;    off += a256((size_t)L.max_seg * sizeof(int4));
+    L.o_sstart = off; off += a256(((size_t)L.max_seg + 1) * 8);
+    L.o_cnt = off;    off += 256;
+    L.o_cub = off;    off += a256(L.cub_bytes);
+    L.total = off + 256;
+    return L;
+}
+
+size_t gene_rank_smem(int SKP, int e_max) { return (size_t)kPredRows * q_stride(SKP) * 8 + (size_t)e_max * kGeneEntryBytes; }
+
+int bits_for(long long x)
+{
+    int b = 0;
+    while (b < 63 && (1ll << b) <= x) ++b;
+    return b;
+}
+
+}  // namespace
+}  // namespace tip
+
+static bool gene_rank_args_ok(int n_cand, int n_query, int K, int S, int64_t n_known, int64_t n_test)
+{
+    return predict_args_ok(n_cand, K, S, n_known, 0) && n_query >= 0 && n_query <= n_cand && n_known <= (1ll << 29) &&
+           n_test >= 0 && n_test < (1ll << 31);
+}
+
+#define TIP_GENE_RANK_LIMITS "n_cand <= 2^21, 1 <= K <= %d, S >= 1, S*K <= %d, 0 <= n_query <= n_cand, 0 <= n_known <= 2^29, " \
+                             "0 <= n_test < 2^31"
+
+extern "C" int tip_rank_per_gene_workspace_bytes(int n_cand, int n_query, int K, int S, int64_t n_known, int64_t n_test,
+                                                 size_t *bytes)
+{
+    TIP_REQUIRE(bytes != nullptr && gene_rank_args_ok(n_cand, n_query, K, S, n_known, n_test),
+                "tip_rank_per_gene_workspace_bytes: bad arguments (" TIP_GENE_RANK_LIMITS ")", TIP_MAX_K, kPredMaxSK);
+    *bytes = gene_rank_layout(n_cand, n_query, K, S, n_known, n_test).total;
+    return 0;
+}
+
+extern "C" int tip_rank_per_gene(int P, int K, int S, const double *d_theta, const double *d_p, const int32_t *d_cand, int n_cand,
+                                 const int32_t *d_query_ranks, int n_query, const uint64_t *d_known, int64_t n_known,
+                                 const int32_t *d_test_query, const int32_t *d_test_u, const int32_t *d_test_v, int64_t n_test,
+                                 void *d_ws, size_t ws_bytes, int64_t *d_rank_out, double *d_score_out, int64_t *d_universe_out,
+                                 void *stream)
+{
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    TIP_REQUIRE(P > 0 && n_cand <= P && gene_rank_args_ok(n_cand, n_query, K, S, n_known, n_test),
+                "tip_rank_per_gene: bad arguments (P > 0, n_cand <= P, " TIP_GENE_RANK_LIMITS ")", TIP_MAX_K, kPredMaxSK);
+    TIP_REQUIRE(d_theta && d_p && (d_cand || n_cand == 0) && (d_known || n_known == 0) &&
+                    (n_query == 0 || (d_query_ranks && d_universe_out)) &&
+                    (n_test == 0 || (d_test_query && d_test_u && d_test_v && d_rank_out && d_score_out)),
+                "tip_rank_per_gene: null pointer");
+    const int n = n_cand, nq = n_query;
+    const long long T = n_test;
+    // query ranks and test entries are checked on the host before any device work
+    std::vector<int32_t> qr(nq), tq((size_t)T), tu((size_t)T), tv((size_t)T);
+    if (nq) TIP_CHECK_CUDA(cudaMemcpyAsync(qr.data(), d_query_ranks, (size_t)nq * 4, cudaMemcpyDeviceToHost, st));
+    if (T) {
+        TIP_CHECK_CUDA(cudaMemcpyAsync(tq.data(), d_test_query, (size_t)T * 4, cudaMemcpyDeviceToHost, st));
+        TIP_CHECK_CUDA(cudaMemcpyAsync(tu.data(), d_test_u, (size_t)T * 4, cudaMemcpyDeviceToHost, st));
+        TIP_CHECK_CUDA(cudaMemcpyAsync(tv.data(), d_test_v, (size_t)T * 4, cudaMemcpyDeviceToHost, st));
+    }
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    std::vector<int32_t> qidx(std::max(n, 1), -1);
+    for (int i = 0; i < nq; ++i) {
+        TIP_REQUIRE(qr[i] >= 0 && qr[i] < n, "tip_rank_per_gene: query rank %d of query %d is not in [0, %d)", qr[i], i, n);
+        TIP_REQUIRE(qidx[qr[i]] < 0, "tip_rank_per_gene: query rank %d appears twice", qr[i]);
+        qidx[qr[i]] = i;
+    }
+    for (long long j = 0; j < T; ++j) {
+        TIP_REQUIRE(tq[j] >= 0 && tq[j] < nq, "tip_rank_per_gene: test entry %lld names query %d, not in [0, %d)", j, tq[j], nq);
+        const int32_t r = qr[tq[j]];
+        TIP_REQUIRE(tu[j] >= 0 && tu[j] < n && tv[j] >= 0 && tv[j] < n && tu[j] != r && tv[j] != r && tu[j] != tv[j],
+                    "tip_rank_per_gene: test entry %lld has ranks (%d, %d), not two distinct ranks in [0, %d) other than its "
+                    "query's (%d)", j, tu[j], tv[j], n, r);
+    }
+    if (nq == 0) return 0;
+    const GeneRankLayout L = gene_rank_layout(n, nq, K, S, n_known, T);
+    TIP_REQUIRE(d_ws != nullptr && ws_bytes >= L.total, "tip_rank_per_gene: workspace too small (%zu < %zu)", ws_bytes, L.total);
+    int dev = 0, optin = 0;
+    TIP_CHECK_CUDA(cudaGetDevice(&dev));
+    TIP_CHECK_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    cudaFuncAttributes fa{};
+    TIP_CHECK_CUDA(cudaFuncGetAttributes(&fa, tip_gene_rank_pass_kernel));
+    const long long room =
+        ((long long)optin - 1024 - (long long)fa.sharedSizeBytes - (long long)gene_rank_smem(L.SKP, 0)) / kGeneEntryBytes;
+    const int e_max = (int)std::min<long long>(kRankMaxEntries, room);
+    TIP_REQUIRE(e_max >= kRankMinEntries, "tip_rank_per_gene: S*K = %d leaves room for %d entries beside the Q tile (internal error)",
+                S * K, e_max);
+
+    char *base = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(d_ws) + 255) / 256 * 256);
+    double *tcat = reinterpret_cast<double *>(base + L.o_tcat), *Mq = reinterpret_cast<double *>(base + L.o_M);
+    auto *d_qidx = reinterpret_cast<int32_t *>(base + L.o_qidx);
+    auto *istart = reinterpret_cast<long long *>(base + L.o_istart);
+    auto *qoff = reinterpret_cast<int32_t *>(base + L.o_qoff), *toff = reinterpret_cast<int32_t *>(base + L.o_toff);
+    auto *key = reinterpret_cast<unsigned long long *>(base + L.o_key), *key2 = reinterpret_cast<unsigned long long *>(base + L.o_key2);
+    auto *idx = reinterpret_cast<int32_t *>(base + L.o_idx), *idx2 = reinterpret_cast<int32_t *>(base + L.o_idx2);
+    auto *bits = reinterpret_cast<unsigned long long *>(base + L.o_bits);
+    auto *obits = reinterpret_cast<unsigned long long *>(base + L.o_obits);
+    auto *opos0 = reinterpret_cast<int32_t *>(base + L.o_opos0), *opos = reinterpret_cast<int32_t *>(base + L.o_opos);
+    auto *flag = reinterpret_cast<int32_t *>(base + L.o_flag), *tscan = reinterpret_cast<int32_t *>(base + L.o_scan);
+    auto *item = reinterpret_cast<unsigned long long *>(base + L.o_item);
+    auto *item2 = reinterpret_cast<unsigned long long *>(base + L.o_item2);
+    auto *uitem = reinterpret_cast<unsigned long long *>(base + L.o_uitem);
+    auto *t_bits = reinterpret_cast<unsigned long long *>(base + L.o_tbits), *t_uv = reinterpret_cast<unsigned long long *>(base + L.o_tuv);
+    auto *t_cnt = reinterpret_cast<unsigned long long *>(base + L.o_tcnt);
+    auto *t_idx = reinterpret_cast<int32_t *>(base + L.o_tidx), *t_tr = reinterpret_cast<int32_t *>(base + L.o_ttr);
+    auto *seg = reinterpret_cast<int4 *>(base + L.o_seg);
+    auto *sstart = reinterpret_cast<long long *>(base + L.o_sstart);
+    auto *cnt = reinterpret_cast<unsigned long long *>(base + L.o_cnt);   // [0] train entries, [1] item cursor, [2] unique items
+    void *cub_tmp = base + L.o_cub;
+    size_t cb = 0;
+
+    // the work items of every query, numbered as tip_query_pass_kernel numbers them, query after query
+    std::vector<long long> h_istart((size_t)nq + 1, 0);
+    for (int i = 0; i < nq; ++i) {
+        int tc, tb, ta;
+        query_tiles(n, qr[i], tc, tb, ta);
+        h_istart[i + 1] = h_istart[i] + tc + tb + ta;
+    }
+    TIP_CHECK_CUDA(cudaMemcpyAsync(d_qidx, qidx.data(), (size_t)n * 4, cudaMemcpyHostToDevice, st));
+    TIP_CHECK_CUDA(cudaMemcpyAsync(istart, h_istart.data(), ((size_t)nq + 1) * 8, cudaMemcpyHostToDevice, st));
+    TIP_CHECK_CUDA(cudaMemsetAsync(cnt, 0, 3 * 8, st));
+    // entries: the test entries, then the train entries of the queries; sorted by (query, u, v)
+    if (T) {
+        tip_gene_test_keys_kernel<<<(int)((T + 255) / 256), 256, 0, st>>>(T, d_test_query, d_test_u, d_test_v, key, idx);
+        TIP_CHECK_CUDA(cudaGetLastError());
+    }
+    if (n_known > 0) {
+        tip_gene_train_kernel<<<(int)((n_known + 255) / 256), 256, 0, st>>>(
+            n_known, reinterpret_cast<const unsigned long long *>(d_known), n, d_qidx, T, key, idx, cnt);
+        TIP_CHECK_CUDA(cudaGetLastError());
+    }
+    unsigned long long h_ntr = 0;
+    TIP_CHECK_CUDA(cudaMemcpyAsync(&h_ntr, cnt, 8, cudaMemcpyDeviceToHost, st));
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    const long long E = T + (long long)h_ntr;
+    TIP_REQUIRE(E < (1ll << 31), "tip_rank_per_gene: %lld test and train entries, more than 2^31 - 1", E);
+    const int end_bit = 2 * kRankBits + bits_for(nq - 1);
+    if (E) {
+        cb = L.cub_bytes;
+        TIP_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(cub_tmp, cb, key, key2, idx, idx2, (int)E, 0, end_bit, st));
+    }
+    tip_gene_offsets_kernel<<<(nq + 256) / 256, 256, 0, st>>>(nq, E, key2, qoff);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    const long long pairs = n_pairs(n - 1);
+    if (T == 0) {
+        tip_gene_universe_kernel<<<(nq + 256) / 256, 256, 0, st>>>(nq, E, 0, pairs, qoff, tscan, toff, d_universe_out);
+        TIP_CHECK_CUDA(cudaGetLastError());
+        TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+        return 0;
+    }
+
+    // tcat and the query matrices as tip_top_triplets_per_gene forms them
+    {
+        const long long work = (long long)L.n_pad * L.SKP + (long long)nq * 3 * S * K * K;
+        tip_query_prep_kernel<<<(int)std::min<long long>((work + 255) / 256, (long long)sm_count() * 16), 256, 0, st>>>(
+            S, P, K, n, L.n_pad, L.SKP, nq, d_theta, d_p, d_cand, d_query_ranks, tcat, Mq);
+        TIP_CHECK_CUDA(cudaGetLastError());
+    }
+    // capture items: the distinct items that hold an entry
+    const int ge = (int)((E + 255) / 256);
+    tip_gene_items_kernel<<<ge, 256, 0, st>>>(E, n, key2, d_query_ranks, istart, item);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    cb = L.cub_bytes;
+    TIP_CHECK_CUDA(cub::DeviceRadixSort::SortKeys(cub_tmp, cb, item, item2, (int)E, 0, std::max(1, bits_for(h_istart[nq])), st));
+    cb = L.cub_bytes;
+    TIP_CHECK_CUDA(cub::DeviceSelect::Unique(cub_tmp, cb, item2, uitem, reinterpret_cast<int *>(cnt + 2), (int)E, st));
+    int n_capture = 0;
+    TIP_CHECK_CUDA(cudaMemcpyAsync(&n_capture, cnt + 2, 4, cudaMemcpyDeviceToHost, st));
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+
+    const size_t smem0 = gene_rank_smem(L.SKP, 0), smem1 = gene_rank_smem(L.SKP, e_max);
+    static int smem_set = 0;
+    if ((int)smem1 > smem_set && smem1 > 48 * 1024) {
+        TIP_CHECK_CUDA(cudaFuncSetAttribute(tip_gene_rank_pass_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
+        smem_set = (int)smem1;
+    }
+    int per_sm0 = 0, per_sm1 = 0;
+    TIP_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm0, tip_gene_rank_pass_kernel, kPredThreads, smem0));
+    TIP_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm1, tip_gene_rank_pass_kernel, kPredThreads, smem1));
+    TIP_REQUIRE(per_sm0 > 0 && per_sm1 > 0, "tip_rank_per_gene: S*K = %d does not fit one block's shared memory", S * K);
+
+    GeneRankArgs A{};
+    A.n = n; A.S = S; A.K = K; A.SK = S * K; A.SKP = L.SKP;
+    A.tcat = tcat; A.Mq = Mq; A.qrank = d_query_ranks; A.ctl = cnt + 1;
+    // capture sweep
+    A.mode = 0; A.seg_start = istart; A.n_seg = nq; A.items = reinterpret_cast<const long long *>(uitem); A.n_items = n_capture;
+    A.key = key2; A.q_off = qoff; A.bits = bits;
+    if (n_capture > 0) {
+        tip_gene_rank_pass_kernel<<<(int)std::min<long long>((long long)sm_count() * per_sm0, n_capture), kPredThreads, smem0, st>>>(A);
+        TIP_CHECK_CUDA(cudaGetLastError());
+    }
+    // per query: entries in the order (bits descending, key ascending), a stable sort of the key order; the test entries
+    // of that order with the train entries ahead of each
+    tip_rank_iota_kernel<<<ge, 256, 0, st>>>(E, opos0);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    cb = L.cub_bytes;
+    TIP_CHECK_CUDA(cub::DeviceSegmentedSort::StableSortPairsDescending(cub_tmp, cb, bits, obits, opos0, opos, (int)E, nq, qoff,
+                                                                      qoff + 1, st));
+    tip_gene_flags_kernel<<<ge, 256, 0, st>>>(E, opos, idx2, T, flag);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    cb = L.cub_bytes;
+    TIP_CHECK_CUDA(cub::DeviceScan::ExclusiveSum(cub_tmp, cb, flag, tscan, (int)E, st));
+    tip_gene_compact_kernel<<<ge, 256, 0, st>>>(E, T, key2, idx2, qoff, obits, opos, tscan, t_bits, t_uv, t_idx, t_tr);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    tip_gene_universe_kernel<<<(nq + 256) / 256, 256, 0, st>>>(nq, E, T, pairs, qoff, tscan, toff, d_universe_out);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    TIP_CHECK_CUDA(cudaMemsetAsync(t_cnt, 0, (size_t)T * 8, st));
+
+    // count items: every tile of every query with a test entry, once per round of at most e_max of its test entries
+    std::vector<int32_t> h_toff((size_t)nq + 1);
+    TIP_CHECK_CUDA(cudaMemcpyAsync(h_toff.data(), toff, ((size_t)nq + 1) * 4, cudaMemcpyDeviceToHost, st));
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    std::vector<int4> h_seg;
+    std::vector<long long> h_sstart(1, 0);
+    for (int i = 0; i < nq; ++i)
+        for (int b = h_toff[i]; b < h_toff[i + 1]; b += e_max) {
+            h_seg.push_back(make_int4(i, b, std::min(h_toff[i + 1], b + e_max), 0));
+            h_sstart.push_back(h_sstart.back() + (h_istart[i + 1] - h_istart[i]));
+        }
+    const int n_seg = (int)h_seg.size();
+    TIP_REQUIRE(n_seg <= L.max_seg, "tip_rank_per_gene: %d rounds (internal error)", n_seg);
+    TIP_CHECK_CUDA(cudaMemcpyAsync(seg, h_seg.data(), (size_t)n_seg * sizeof(int4), cudaMemcpyHostToDevice, st));
+    TIP_CHECK_CUDA(cudaMemcpyAsync(sstart, h_sstart.data(), ((size_t)n_seg + 1) * 8, cudaMemcpyHostToDevice, st));
+    // count sweep
+    A.mode = 1; A.seg_start = sstart; A.seg = seg; A.n_seg = n_seg; A.items = nullptr; A.n_items = h_sstart.back();
+    A.e_max = e_max; A.t_bits = t_bits; A.t_uv = t_uv; A.t_cnt = t_cnt;
+    TIP_CHECK_CUDA(cudaMemsetAsync(cnt + 1, 0, 8, st));
+    if (A.n_items > 0) {
+        tip_gene_rank_pass_kernel<<<(int)std::min<long long>((long long)sm_count() * per_sm1, A.n_items), kPredThreads, smem1, st>>>(A);
+        TIP_CHECK_CUDA(cudaGetLastError());
+    }
+    tip_gene_finish_kernel<<<(n_seg + 127) / 128, 128, 0, st>>>(n_seg, S, seg, t_cnt, t_bits, t_idx, t_tr, d_rank_out, d_score_out);
     TIP_CHECK_CUDA(cudaGetLastError());
     TIP_CHECK_CUDA(cudaStreamSynchronize(st));
     return 0;

@@ -12,6 +12,7 @@ CUDA kernels behind the C ABI (include/tip.h).  There is no CPU path.
     eng.top_triplets_per_pair(thetas, ps, cand, pr, known, n)  # the same per query pair (tip_top_triplets_per_pair)
     eng.score_histogram(thetas, ps, cand)              # histogram of all C(n, 3) scores (tip_score_histogram)
     eng.rank_per_pair(thetas, ps, cand, pr, known, tp, trc)   # held-out ranks per query pair (tip_rank_per_pair)
+    eng.rank_per_gene(thetas, ps, cand, q, known, tq, tu, tv)   # held-out ranks per query gene (tip_rank_per_gene)
 """
 from __future__ import annotations
 
@@ -644,6 +645,43 @@ class EMEngine:
             _ptr(d_tp), _ptr(d_trc), n_test, _ptr(ws), nb.value, _ptr(rank), _ptr(score), _ptr(universe), self._stream()),
             "tip_rank_per_pair")
         return rank[:n_test].cpu().numpy(), score[:n_test].cpu().numpy(), universe[:n_pairs].cpu().numpy()
+
+    @_on_device
+    def rank_per_gene(self, theta_stack, p_stack, cand, query_ranks, known, test_query, test_u, test_v):
+        """tip_rank_per_gene: the exact rank of every test entry (test_query[j], an index into `query_ranks`; test_u[j],
+        test_v[j], the other two ranks) among its query's pairs whose triplet is not a key of `known`, in the order of
+        top_triplets_per_gene; arguments otherwise as there.  Returns (rank [T] int64, 0 when the entry is a known key;
+        score [T] float64, the mean over the S sets; universe [Q] int64, the pairs that are not known keys)."""
+        th = np.ascontiguousarray(theta_stack, dtype=np.float64)
+        pp = np.ascontiguousarray(p_stack, dtype=np.float64)
+        S = int(th.shape[0])
+        assert th.shape == (S, self.P, self.K) and pp.shape == (S, self.K, self.K, self.K, 2)
+        cand = np.ascontiguousarray(cand, dtype=np.int32)
+        qr = np.ascontiguousarray(query_ranks, dtype=np.int32).reshape(-1)
+        known = np.ascontiguousarray(known, dtype=np.uint64)
+        tq = np.ascontiguousarray(test_query, dtype=np.int32).reshape(-1)
+        tu = np.ascontiguousarray(test_u, dtype=np.int32).reshape(-1)
+        tv = np.ascontiguousarray(test_v, dtype=np.int32).reshape(-1)
+        assert tq.shape == tu.shape == tv.shape
+        n_cand, n_query, n_known, n_test = int(cand.shape[0]), int(qr.shape[0]), int(known.shape[0]), int(tq.shape[0])
+        nb = ctypes.c_size_t(0)
+        _cabi.check(self.lib.tip_rank_per_gene_workspace_bytes(n_cand, n_query, self.K, S, n_known, n_test, ctypes.byref(nb)),
+                    "tip_rank_per_gene_workspace_bytes")
+        d_th = torch.from_numpy(th.reshape(-1)).to(self.device)
+        d_p = torch.from_numpy(pp.reshape(-1)).to(self.device)
+        d_cand = torch.from_numpy(cand).to(self.device)
+        d_qr = torch.from_numpy(qr).to(self.device)
+        d_known = torch.from_numpy(known.view(np.int64)).to(self.device) if n_known else None
+        d_tq, d_tu, d_tv = (torch.from_numpy(x).to(self.device) for x in (tq, tu, tv))
+        ws = torch.empty(max(nb.value, 1), dtype=torch.uint8, device=self.device)
+        rank = torch.zeros(max(n_test, 1), dtype=torch.int64, device=self.device)
+        score = torch.zeros(max(n_test, 1), dtype=torch.float64, device=self.device)
+        universe = torch.zeros(max(n_query, 1), dtype=torch.int64, device=self.device)
+        _cabi.check(self.lib.tip_rank_per_gene(
+            self.P, self.K, S, _ptr(d_th), _ptr(d_p), _ptr(d_cand), n_cand, _ptr(d_qr), n_query, _ptr(d_known), n_known,
+            _ptr(d_tq), _ptr(d_tu), _ptr(d_tv), n_test, _ptr(ws), nb.value, _ptr(rank), _ptr(score), _ptr(universe),
+            self._stream()), "tip_rank_per_gene")
+        return rank[:n_test].cpu().numpy(), score[:n_test].cpu().numpy(), universe[:n_query].cpu().numpy()
 
     @_on_device
     def score_histogram(self, theta_stack, p_stack, cand, log2_bins: int = 7, n_binades: int = 64):

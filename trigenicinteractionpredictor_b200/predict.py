@@ -2,8 +2,8 @@
 
     python -m trigenicinteractionpredictor_b200.predict -t train0.dat -e test0.dat \\
         -p results/Sample_0_K10.npz [-p results/Sample_1_K10.npz ...] [-n 100] [-g genes.txt] \\
-        [-q queries.txt | -r pairs.txt | --held-out | --held-out-pairs [-r pairs.txt]] [--include-known]
-        [-o predictions.tsv] [--device cuda:0]
+        [-q queries.txt | -r pairs.txt | --held-out | --held-out-pairs [-r pairs.txt] | --held-out-genes [-q queries.txt]]
+        [--include-known] [-o predictions.tsv] [--device cuda:0]
 
 The train / test files rebuild the model's digestion (gene ids in order of first appearance, TIP.py:321-423); every
 parameter file (the .npz that training with --save-params writes) must belong to it.  With several files the score of a
@@ -38,7 +38,16 @@ genes.  A pair's universe is every partner whose triplet is not a key of the tra
 Output: summary lines "Name:<TAB>value" (counts, hits at N for the positives and the negatives, the positives' median
 rank, MRR and AUC against the pair universes), then the header "Query pair<TAB>Rank<TAB>Pair universe<TAB>Predicted
 Interaction<TAB>Real Interaction<TAB>ID of genes<TAB>Genes" and one line per view, by pair (file order, or sorted names)
-and rank.  --held-out-pairs excludes -q, -n, --held-out and --include-known."""
+and rank.  --held-out-pairs excludes -q, -n, --held-out and --include-known.
+
+--held-out-genes: where each test triplet lands among its query gene's unseen triplets (Model.rank_held_out_per_gene,
+DESIGN §4.10).  Without -q every test triplet of the -g genes gives three views, one per gene; with -q a view is a listed
+query and a test triplet that contains it, the partners taken from the -g genes plus the queries.  A query's universe is
+every pair of other genes whose triplet is not a key of the train file, and every rank is exact.  Output: summary lines
+"Name:<TAB>value" (counts, hits at N for the positives and the negatives, the positives' median rank, MRR and AUC against
+the gene universes), then the header "Query gene<TAB>Rank<TAB>Gene universe<TAB>Predicted Interaction<TAB>Real
+Interaction<TAB>ID of genes<TAB>Genes" and one line per view, by query (file order, or sorted names) and rank.
+--held-out-genes excludes -r, -n, --held-out, --held-out-pairs and --include-known."""
 from __future__ import annotations
 
 import contextlib
@@ -51,8 +60,10 @@ QUERY_HEADER = "Query gene\t" + HEADER
 PAIR_HEADER = "Query pair\t" + HEADER
 HELD_OUT_HEADER = "Rank\tPredicted Interaction\tReal Interaction\tID of genes\tGenes\n"
 HELD_OUT_PAIRS_HEADER = "Query pair\tRank\tPair universe\tPredicted Interaction\tReal Interaction\tID of genes\tGenes\n"
+HELD_OUT_GENES_HEADER = "Query gene\tRank\tGene universe\tPredicted Interaction\tReal Interaction\tID of genes\tGenes\n"
 RECALL_AT = (100, 1000, 10000, 100000)
 HITS_AT = (1, 5, 10, 20, 50, 100)
+GENE_HITS_AT = (1, 10, 20, 100, 1000, 10000)
 
 
 def _fail(msg: str) -> int:
@@ -64,11 +75,11 @@ def main(argv=None) -> int:
     argv = sys.argv[1:] if argv is None else argv
     train = test = out = device = genes_file = queries_file = pairs_file = None
     params: list[str] = []
-    top, include_known, held_out, held_out_pairs = None, False, False, False
+    top, include_known, held_out, held_out_pairs, held_out_genes = None, False, False, False, False
     try:
         opts, rest = getopt.getopt(argv, "ht:e:p:n:g:q:r:o:", ["help", "train=", "test=", "params=", "top=", "genes=",
                                                                "queries=", "pairs=", "include-known", "held-out",
-                                                               "held-out-pairs", "out=", "device="])
+                                                               "held-out-pairs", "held-out-genes", "out=", "device="])
     except getopt.GetoptError as exc:
         return _fail("argument error: %s" % exc)
     if rest:
@@ -100,11 +111,16 @@ def main(argv=None) -> int:
             held_out = True
         elif opt == "--held-out-pairs":
             held_out_pairs = True
+        elif opt == "--held-out-genes":
+            held_out_genes = True
         elif opt in ("-o", "--out"):
             out = arg
         elif opt == "--device":
             device = arg
-    if held_out_pairs:
+    if held_out_genes:
+        if pairs_file or top is not None or held_out or held_out_pairs or include_known:
+            return _fail("--held-out-genes excludes -r/--pairs, -n/--top, --held-out, --held-out-pairs and --include-known")
+    elif held_out_pairs:
         if queries_file or held_out or include_known or top is not None:
             return _fail("--held-out-pairs excludes -q/--queries, -n/--top, --held-out and --include-known")
     elif held_out:
@@ -189,7 +205,13 @@ def main(argv=None) -> int:
     if len({th.shape[1] for th, _ in sets}) != 1:
         return _fail("the parameter files have different K")
 
-    if held_out_pairs:
+    if held_out_genes:
+        try:
+            res = model.rank_held_out_per_gene(queries, genes=genes, params=sets, hits_at=GENE_HITS_AT)
+        except ValueError as exc:
+            return _fail(str(exc))
+        text = held_out_genes_text(res)
+    elif held_out_pairs:
         try:
             res = model.rank_held_out_per_pair(pairs, genes=genes, params=sets, hits_at=HITS_AT)
         except ValueError as exc:
@@ -259,6 +281,21 @@ def held_out_pairs_text(res: dict) -> str:
     body = "".join("%s\t%d\t%d\t%s\t%d\t%s\t%s\n" % (pair, rank, universe, score, label, key, names)
                    for pair, key, names, label, score, rank, universe in res["rows"])
     return "\n".join(lines) + "\n" + HELD_OUT_PAIRS_HEADER + body
+
+
+def held_out_genes_text(res: dict) -> str:
+    """Summary lines and the table of views of Model.rank_held_out_per_gene."""
+    lines = ["Query genes:\t%d" % len(res["genes"]), "Views:\t%d" % res["views"], "Positive views:\t%d" % res["positives"],
+             "Negative views:\t%d" % res["negatives"], "Excluded train keys:\t%d" % res["excluded_train"],
+             "Excluded outside the genes:\t%d" % res["excluded_genes"]]
+    for N, r in res["hits_at"].items():
+        lines.append("Hits at %d:\t%s" % (N, _value(r["positives"])))
+        lines.append("Negatives at %d:\t%s" % (N, _value(r["negatives"])))
+    lines += ["Median rank of positives:\t%s" % _value(res["median_rank"]), "MRR:\t%s" % _value(res["mrr"]),
+              "Gene AUC (micro):\t%s" % _value(res["auc_micro"]), "Gene AUC (macro):\t%s" % _value(res["auc_macro"])]
+    body = "".join("%s\t%d\t%d\t%s\t%d\t%s\t%s\n" % (gene, rank, universe, score, label, key, names)
+                   for gene, key, names, label, score, rank, universe in res["rows"])
+    return "\n".join(lines) + "\n" + HELD_OUT_GENES_HEADER + body
 
 
 if __name__ == "__main__":
