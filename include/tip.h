@@ -303,6 +303,43 @@ int tip_rank_per_gene(int P, int K, int S, const double *d_theta, const double *
                       void *d_ws, size_t ws_bytes, int64_t *d_rank_out, double *d_score_out,
                       int64_t *d_universe_out, void *stream);
 
+/* ---- the digenic model: pair scores and the N best unseen gene pairs (DESIGN §4.11) ----
+ * The score of the id pair (a, b), a in the key's first slot, is sum_ij th_a[i] th_b[j] q[i][j][1] (rating 1, no eps);
+ * q is not symmetric, so slot order matters, and the slot order of a key is the decimal-string order of its ids.
+ *   tip_score_pairs   d_out[t] = score of (d_a[t], d_b[t]) under d_theta[P][K], d_q[K][K][2] (one parameter set).
+ * Top-N: candidates d_cand[n_cand] in decimal-string order (rank = position), so every pair of ranks ra < rb is in slot
+ * order; parameters d_theta[S][P][K], d_q[S][K][K][2]; pairs are ordered by the bits of the score SUM over the S sets,
+ * descending, then by the packed ranks (ra << 21) | rb ascending, exact under any ties; d_out_scores are the means.
+ * d_known[n_known]: sorted packed rank pairs never to return (a repeated key counts once).  Every score is computed
+ * once, on the fp64 tensor path, in chunks of at most TIP_PAIR_CHUNK pairs; the chunk size follows from this constant and
+ * is not an argument.  Synchronises the stream; not capturable in a CUDA graph.  Precondition: finite, non-negative
+ * parameters.
+ *   tip_top_pairs           the first min(N, unseen pairs) of all C(n_cand, 2) pairs: d_out_ids[N][2] gene ids in slot
+ *                           order, d_out_scores[N], *h_n_out rows.  Limits: n_cand <= 2^21, S * K <= 384, N < 2^28.
+ *                           Workspace O(n_cand S K + N + TIP_PAIR_CHUNK).
+ *   tip_top_pairs_per_gene  for every query rank r of d_query_ranks[n_query] (distinct ranks into d_cand), its pairs with
+ *                           every other candidate x, (x, r) for x < r and (r, x) for x > r, ordered by score descending,
+ *                           then x ascending: d_out_ids[n_query][N][2], d_out_scores[n_query][N], h_n_out[n_query] rows
+ *                           (rows past h_n_out[q] are not written).  Queries are answered in chunks of
+ *                           max(1, TIP_PAIR_CHUNK / (n_cand - 1)).  An out-of-range or repeated query rank is refused
+ *                           before any device work.  Limits: n_cand <= 2^21, S * K <= 384, n_query <= n_cand,
+ *                           n_query * N <= 2^24.  Workspace O(n_cand S K + TIP_PAIR_CHUNK).
+ *   *_last_chunks           chunks the last such call of this thread swept (measurement). */
+#define TIP_PAIR_CHUNK (1 << 21)
+int tip_score_pairs(int P, int K, const double *d_theta, const double *d_q, const int32_t *d_a, const int32_t *d_b, int64_t T,
+                    double *d_out, void *stream);
+int tip_top_pairs_workspace_bytes(int n_cand, int K, int S, int64_t N, size_t *bytes);
+int tip_top_pairs(int P, int K, int S, const double *d_theta, const double *d_q, const int32_t *d_cand, int n_cand,
+                  const uint64_t *d_known, int64_t n_known, int64_t N, void *d_ws, size_t ws_bytes, int32_t *d_out_ids,
+                  double *d_out_scores, int64_t *h_n_out, void *stream);
+int tip_top_pairs_last_chunks(void);
+int tip_top_pairs_per_gene_workspace_bytes(int n_cand, int n_query, int K, int S, int64_t N, size_t *bytes);
+int tip_top_pairs_per_gene(int P, int K, int S, const double *d_theta, const double *d_q, const int32_t *d_cand, int n_cand,
+                           const int32_t *d_query_ranks, int n_query, const uint64_t *d_known, int64_t n_known, int64_t N,
+                           void *d_ws, size_t ws_bytes, int32_t *d_out_ids, double *d_out_scores, int64_t *h_n_out,
+                           void *stream);
+int tip_top_pairs_per_gene_last_chunks(void);
+
 /* ---- testResultsReducer.py:160-184: mean / median / standard deviation of every test triplet across samples ----
  * d_scores[S][T]: score of triplet t in sample j at [j * T + t]; d_n[t] (or NULL = S) = how many leading samples of
  * triplet t are valid.  mean = sequential sum in sample order / n; median = the reference's rule (ascending sort;

@@ -74,7 +74,16 @@ SIGNATURES = {
     "tip_rank_per_gene": (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p, c_int64,
                                   c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p,
                                   c_void_p]),
-    "tip_reduce_samples": (c_int, [c_int, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "tip_score_pairs": (c_int, [c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
+    "tip_top_pairs_workspace_bytes": (c_int, [c_int, c_int, c_int, c_int64, _psz]),
+    "tip_top_pairs": (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int64, c_int64, c_void_p,
+                              c_size_t, c_void_p, c_void_p, _pi64, c_void_p]),
+    "tip_top_pairs_last_chunks": (c_int, []),
+    "tip_top_pairs_per_gene_workspace_bytes": (c_int, [c_int, c_int, c_int, c_int, c_int64, _psz]),
+    "tip_top_pairs_per_gene": (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p,
+                                       c_int64, c_int64, c_void_p, c_size_t, c_void_p, c_void_p, _pi64, c_void_p]),
+    "tip_top_pairs_per_gene_last_chunks": (c_int, []),
+    "tip_reduce_samples":(c_int, [c_int, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "tip_em_iterations_host": (c_int, [c_int, c_int, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_int,
                                        c_uint]),
     "tip_rows_compact_host": (c_int, [c_void_p, c_int64, c_void_p]),

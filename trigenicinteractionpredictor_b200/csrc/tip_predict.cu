@@ -31,6 +31,8 @@
 // Ranks per query gene (tip_rank_per_gene): the work items, Q tiles and column blocks of tip_top_triplets_per_gene, swept
 // once to record the scores of the held-out and train triplets of the queries and once to count, per query, the scores
 // ahead of each held-out one (tip_gene_rank_pass_kernel); the train triplets ahead are subtracted.
+//
+// The digenic model's gene pairs (tip_top_pairs, tip_top_pairs_per_gene, tip_score_pairs): see the last section.
 #include <algorithm>
 #include <cmath>
 #include <vector>
@@ -3244,3 +3246,526 @@ extern "C" int tip_rank_per_gene(int P, int K, int S, const double *d_theta, con
     TIP_CHECK_CUDA(cudaStreamSynchronize(st));
     return 0;
 }
+
+// ---- the digenic model: top-N gene pairs (tip_top_pairs, tip_top_pairs_per_gene) and test-set pair scores ----
+// A pair of ranks a < b (already in key slot order) scores
+//     score(a, b) = sum_ij th_a[i] qr[i][j][1] th_b[j] = V[a] . tcat[b],   V[x][s K + j] = sum_i th_x[s K + i] qr_s[i][j][1]
+// (tip_pair_prep_kernel), the ensemble sum being the same dot product, S K long.  The pair universe is C(n, 2), so every score
+// is computed once, in chunks of at most TIP_PAIR_CHUNK pairs, each scored into a bounded buffer and merged:
+//   global    items of 64 rows x 128 columns of the upper triangle (tip_top_pairs_pass_kernel); a chunk keeps the scores at or
+//             above the N-th best so far, appends them behind the running best N, and two stable radix sorts (packed ranks
+//             ascending, then bits descending) put the running best N first again;
+//   per gene  a chunk of queries x (n - 1) partners (tip_top_pairs_gene_kernel: the query's V row against the partners'
+//             theta for x > r, the partners' V rows against the query's theta for x < r), then a stable segmented sort
+//             by bits descending of the partners in ascending order, and the first N of every segment.
+namespace tip {
+namespace {
+
+constexpr int kTpRows = 64;                 // rows of a global item (2 warps x 32)
+constexpr int kTpCols = 128;                // columns of a global item (2 warps x 2 x 32)
+constexpr long long kTpItemPairs = (long long)kTpRows * kTpCols;
+constexpr long long kTpChunk = TIP_PAIR_CHUNK;
+constexpr int kTpMaxRows = 1 << 24;         // per gene: n_query * N
+
+// tcat[r] = theta rows of candidate r (tcat_entry), V[r] = its rows times qr[..][1]; Tq / Vq: the same rows of the queries,
+// in the order of qsorted (per gene only)
+__global__ void tip_pair_prep_kernel(int S, int P, int K, int n, int n_pad, int SKP, const double *__restrict__ theta,
+                                     const double *__restrict__ q, const int32_t *__restrict__ cand, int n_q, int nq_pad,
+                                     const int32_t *__restrict__ qsorted, double *__restrict__ tcat, double *__restrict__ V,
+                                     double *__restrict__ Tq, double *__restrict__ Vq)
+{
+    const long long n_t = (long long)n_pad * SKP, n_qt = (long long)nq_pad * SKP;
+    for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < 2 * n_t + 2 * n_qt;
+         t += (long long)gridDim.x * blockDim.x) {
+        const bool is_q = t >= 2 * n_t;
+        const long long u = is_q ? t - 2 * n_t : t, m = is_q ? n_qt : n_t;
+        const bool is_v = u >= m;
+        const long long e = is_v ? u - m : u;
+        long long row = e / SKP;
+        const int col = (int)(e % SKP);
+        if (is_q) row = row < n_q ? qsorted[row] : n;         // pad rows map to a zero row
+        double val = 0.0;
+        if (row < n && col < S * K) {
+            const int s = col / K, j = col % K;
+            const double *th = theta + ((long long)s * P + cand[row]) * K;
+            if (is_v) {
+                const double *qs = q + (long long)s * 2 * K * K;
+                for (int i = 0; i < K; ++i) val = fma(th[i], qs[((long long)i * K + j) * 2 + 1], val);
+            } else {
+                val = th[j];
+            }
+        }
+        double *out = is_q ? (is_v ? Vq : Tq) : (is_v ? V : tcat);
+        out[e] = val;
+    }
+}
+
+__device__ __forceinline__ bool pair_key_known(const unsigned long long *known, long long n, unsigned long long key)
+{
+    long long lo = 0, hi = n;
+    while (lo < hi) {
+        const long long mid = (lo + hi) >> 1;
+        if (__ldg(known + mid) < key) lo = mid + 1; else hi = mid;
+    }
+    return lo < n && __ldg(known + lo) == key;
+}
+
+struct TopPairArgs {
+    int n, SKP;
+    const double *V, *tcat;             // [n_pad][SKP]
+    const unsigned long long *known;    // sorted packed pairs (ra << 21) | rb
+    long long n_known;
+    const long long *tile_item;         // [n_tiles + 1] first item of every row tile
+    int n_tiles;
+    long long item0;                    // first item of the chunk
+    const unsigned long long *thr;      // [0]: bits of the N-th best so far (0: keep everything)
+    unsigned long long *counter;        // entries appended
+    unsigned long long *out_bits, *out_packed;
+};
+
+// an item is 64 rows a0.. of one row tile and 128 columns c0..; pairs b > a only
+__global__ void __launch_bounds__(kPredThreads) tip_top_pairs_pass_kernel(TopPairArgs A)
+{
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int wr = warp & 1, wc = warp >> 1;
+    const int gq = lane >> 2, tq = lane & 3;
+    const long long item = A.item0 + blockIdx.x;
+    int tl = 0, th = A.n_tiles - 1;
+    while (tl < th) {
+        const int mid = (tl + th + 1) >> 1;
+        if (A.tile_item[mid] <= item) tl = mid; else th = mid - 1;
+    }
+    const int a0 = tl * kTpRows + wr * 32;
+    const int cs = tl * kTpRows + (int)(item - A.tile_item[tl]) * kTpCols;
+    const int n = A.n, SKP = A.SKP;
+    const unsigned long long thr = *A.thr;
+    if (a0 >= n - 1) return;
+    for (int h = 0; h < 2; ++h) {
+        const int c0 = cs + h * 64 + wc * 32;
+        if (c0 >= n || c0 + 31 <= a0) continue;       // outside the candidates, or wholly on or below the diagonal
+        double acc[4][4][2];
+        dmma_block(acc, A.V + (long long)(a0 + gq) * SKP + tq, SKP, A.tcat + (long long)(c0 + gq) * SKP + tq, SKP);
+#pragma unroll
+        for (int f = 0; f < 32; ++f) {
+            const int mi = f >> 3, ni = (f >> 1) & 3, e = f & 1;
+            const int ra = a0 + gq + mi * 8, rb = c0 + 2 * tq + ni * 8 + e;
+            const unsigned long long bits = (unsigned long long)__double_as_longlong(acc[mi][ni][e]);
+            const unsigned long long packed = ((unsigned long long)ra << kRankBits) | (unsigned long long)rb;
+            bool keep = rb < n && rb > ra && bits >= thr;
+            if (keep && A.n_known > 0) keep = !pair_key_known(A.known, A.n_known, packed);
+            const unsigned m = __ballot_sync(0xffffffffu, keep);
+            if (m == 0) continue;
+            unsigned long long base = 0;
+            if (lane == __ffs(m) - 1) base = atomicAdd(A.counter, (unsigned long long)__popc(m));
+            base = __shfl_sync(0xffffffffu, base, __ffs(m) - 1);
+            if (keep) {
+                const unsigned long long idx = base + __popc(m & ((1u << lane) - 1u));
+                A.out_bits[idx] = bits;
+                A.out_packed[idx] = packed;
+            }
+        }
+    }
+}
+
+__global__ void tip_top_pairs_finish_kernel(long long m, int S, const unsigned long long *__restrict__ bits,
+                                            const unsigned long long *__restrict__ packed, const int32_t *__restrict__ cand,
+                                            int32_t *__restrict__ out_ids, double *__restrict__ out_scores)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= m) return;
+    const unsigned long long pk = packed[i], mask = (1ull << kRankBits) - 1;
+    out_ids[2 * i + 0] = cand[(pk >> kRankBits) & mask];
+    out_ids[2 * i + 1] = cand[pk & mask];
+    out_scores[i] = __longlong_as_double((long long)bits[i]) / (double)S;
+}
+
+struct GenePairArgs {
+    int n, SKP, n_q;
+    const double *V, *tcat;             // [n_pad][SKP]
+    const double *Vq, *Tq;              // [nq_pad][SKP] rows of the chunk's queries
+    const int32_t *qrank;               // [n_q] ranks of the chunk's queries, ascending
+    const unsigned long long *known;
+    long long n_known;
+    unsigned long long *key;            // [n_q][n - 1]: bits + 1 of partner x at x - (x > r); 0 for a known pair
+    int32_t *part;                      // [n_q][n - 1]: x
+};
+
+// a CTA: 64 queries (blockIdx.y) x 128 partners (blockIdx.x); per warp block, x > r takes Vq[q] . tcat[x] and x < r takes
+// Tq[q] . V[x], each product run only when the block holds such a partner
+__global__ void __launch_bounds__(kPredThreads, 4) tip_top_pairs_gene_kernel(GenePairArgs A)
+{
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int wr = warp & 1, wc = warp >> 1;
+    const int gq = lane >> 2, tq = lane & 3;
+    const int q0 = blockIdx.y * kTpRows + wr * 32;
+    const int n = A.n, SKP = A.SKP;
+    if (q0 >= A.n_q) return;
+    const int rmin = A.qrank[q0], rmax = A.qrank[min(q0 + 31, A.n_q - 1)];
+    int r[4];
+#pragma unroll
+    for (int mi = 0; mi < 4; ++mi) r[mi] = q0 + gq + mi * 8 < A.n_q ? A.qrank[q0 + gq + mi * 8] : -1;
+    const long long stride = n - 1;
+    for (int h = 0; h < 2; ++h) {
+        const int c0 = blockIdx.x * kTpCols + h * 64 + wc * 32;
+        if (c0 >= n) continue;
+        for (int side = 0; side < 2; ++side) {         // 0: partners x > r, 1: partners x < r
+            if (side == 0 ? c0 + 31 <= rmin : c0 >= rmax) continue;
+            double acc[4][4][2];
+            const double *Aq = side == 0 ? A.Vq : A.Tq, *Bx = side == 0 ? A.tcat : A.V;
+            dmma_block(acc, Aq + (long long)(q0 + gq) * SKP + tq, SKP, Bx + (long long)(c0 + gq) * SKP + tq, SKP);
+#pragma unroll
+            for (int f = 0; f < 32; ++f) {
+                const int mi = f >> 3, ni = (f >> 1) & 3, e = f & 1;
+                const int x = c0 + 2 * tq + ni * 8 + e, rq = r[mi];
+                if (rq < 0 || x >= n || (side == 0 ? x <= rq : x >= rq)) continue;
+                const unsigned long long packed = side == 0 ? ((unsigned long long)rq << kRankBits) | (unsigned long long)x
+                                                            : ((unsigned long long)x << kRankBits) | (unsigned long long)rq;
+                const bool known = A.n_known > 0 && pair_key_known(A.known, A.n_known, packed);
+                const long long pos = (long long)(q0 + gq + mi * 8) * stride + x - (side == 0 ? 1 : 0);
+                A.key[pos] = known ? 0ull : (unsigned long long)__double_as_longlong(acc[mi][ni][e]) + 1ull;
+                A.part[pos] = x;
+            }
+        }
+    }
+}
+
+// the first min(N, n - 1) entries of every sorted segment that are not known pairs; out row of query qi: oq[qi]
+__global__ void tip_top_pairs_gene_finish_kernel(int n_q, int n, long long N, int S, const unsigned long long *__restrict__ key,
+                                                 const int32_t *__restrict__ part, const int32_t *__restrict__ qrank,
+                                                 const int32_t *__restrict__ oq, const int32_t *__restrict__ cand,
+                                                 unsigned long long *__restrict__ n_out, int32_t *__restrict__ out_ids,
+                                                 double *__restrict__ out_scores)
+{
+    const long long m = N < n - 1 ? N : n - 1;
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (long long)n_q * m) return;
+    const long long qi = i / m, t = i % m;
+    const unsigned long long k = key[qi * (n - 1) + t];
+    if (k == 0) return;
+    const int x = part[qi * (n - 1) + t], r = qrank[qi];
+    const long long o = (long long)oq[qi] * N + t;
+    out_ids[2 * o + 0] = cand[x < r ? x : r];
+    out_ids[2 * o + 1] = cand[x < r ? r : x];
+    out_scores[o] = __longlong_as_double((long long)(k - 1)) / (double)S;
+    atomicAdd(n_out + oq[qi], 1ull);
+}
+
+// the test-set pair score of one parameter set (do_prediction's pair counterpart, rating 1, no eps)
+__global__ void tip_score_pairs_kernel(int K, const int32_t *__restrict__ a, const int32_t *__restrict__ b, long long T,
+                                       const double *__restrict__ theta, const double *__restrict__ q, double *__restrict__ out)
+{
+    for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < T; t += (long long)gridDim.x * blockDim.x) {
+        const double *ta = theta + (long long)a[t] * K, *tb = theta + (long long)b[t] * K;
+        double acc = 0.0;
+        for (int i = 0; i < K; ++i) {
+            double v = 0.0;
+            for (int j = 0; j < K; ++j) v = fma(q[(i * K + j) * 2 + 1], tb[j], v);
+            acc = fma(ta[i], v, acc);
+        }
+        out[t] = acc;
+    }
+}
+
+// rows of the global sweep: row tiles of 64 over ranks 0 .. n-2, each with ceil((n - a0) / 128) column items
+int tp_tiles(int n) { return n < 2 ? 0 : (n - 1 + kTpRows - 1) / kTpRows; }
+
+struct TopPairLayout {
+    size_t o_tcat, o_V, o_tile, o_thr, o_cnt, o_bits, o_pk, o_bits2, o_pk2, o_cub, cub_bytes, total;
+    int n_pad, SKP;
+    long long cap;
+};
+
+TopPairLayout top_pair_layout(int n, int K, int S, long long N)
+{
+    TopPairLayout L{};
+    L.n_pad = (n + 63) / 64 * 64 + 64;
+    L.SKP = (S * K + 3) / 4 * 4;
+    L.cap = N + kTpChunk;
+    size_t cb1 = 0, cb2 = 0;
+    cub::DeviceRadixSort::SortPairs(nullptr, cb1, (const unsigned long long *)nullptr, (unsigned long long *)nullptr,
+                                    (const unsigned long long *)nullptr, (unsigned long long *)nullptr, (int)L.cap, 0,
+                                    2 * kRankBits, (cudaStream_t)0);
+    cub::DeviceRadixSort::SortPairsDescending(nullptr, cb2, (const unsigned long long *)nullptr, (unsigned long long *)nullptr,
+                                              (const unsigned long long *)nullptr, (unsigned long long *)nullptr, (int)L.cap, 0,
+                                              63, (cudaStream_t)0);
+    L.cub_bytes = std::max(cb1, cb2);
+    size_t off = 0;
+    L.o_tcat = off;  off += a256((size_t)L.n_pad * L.SKP * 8);
+    L.o_V = off;     off += a256((size_t)L.n_pad * L.SKP * 8);
+    L.o_tile = off;  off += a256(((size_t)tp_tiles(n) + 1) * 8);
+    L.o_thr = off;   off += 256;
+    L.o_cnt = off;   off += 256;
+    L.o_bits = off;  off += a256((size_t)L.cap * 8);
+    L.o_pk = off;    off += a256((size_t)L.cap * 8);
+    L.o_bits2 = off; off += a256((size_t)L.cap * 8);
+    L.o_pk2 = off;   off += a256((size_t)L.cap * 8);
+    L.o_cub = off;   off += a256(L.cub_bytes);
+    L.total = off + 256;
+    return L;
+}
+
+// queries per chunk: as many whole segments of n - 1 partners as TIP_PAIR_CHUNK holds, at least one
+int gp_chunk_queries(int n, int n_query)
+{
+    return (int)std::max(1ll, std::min<long long>(n_query, kTpChunk / std::max(1, n - 1)));
+}
+
+struct GenePairLayout {
+    size_t o_tcat, o_V, o_Tq, o_Vq, o_qs, o_oq, o_off, o_nout, o_key, o_part, o_key2, o_part2, o_cub, cub_bytes, total;
+    int n_pad, nq_pad, SKP, qc;
+};
+
+GenePairLayout gene_pair_layout(int n, int n_query, int K, int S)
+{
+    GenePairLayout L{};
+    L.n_pad = (n + 63) / 64 * 64 + 64;
+    L.nq_pad = (n_query + 63) / 64 * 64 + 64;
+    L.SKP = (S * K + 3) / 4 * 4;
+    L.qc = gp_chunk_queries(n, n_query);
+    const long long items = (long long)L.qc * std::max(1, n - 1);
+    size_t cb = 0;
+    cub::DeviceSegmentedSort::StableSortPairsDescending(nullptr, cb, (const unsigned long long *)nullptr,
+                                                        (unsigned long long *)nullptr, (const int32_t *)nullptr, (int32_t *)nullptr,
+                                                        (int)items, L.qc, (const int *)nullptr, (const int *)nullptr, (cudaStream_t)0);
+    L.cub_bytes = cb;
+    size_t off = 0;
+    L.o_tcat = off;  off += a256((size_t)L.n_pad * L.SKP * 8);
+    L.o_V = off;     off += a256((size_t)L.n_pad * L.SKP * 8);
+    L.o_Tq = off;    off += a256((size_t)L.nq_pad * L.SKP * 8);
+    L.o_Vq = off;    off += a256((size_t)L.nq_pad * L.SKP * 8);
+    L.o_qs = off;    off += a256((size_t)std::max(n_query, 1) * 4);
+    L.o_oq = off;    off += a256((size_t)std::max(n_query, 1) * 4);
+    L.o_off = off;   off += a256(((size_t)L.qc + 1) * 4);
+    L.o_nout = off;  off += a256((size_t)std::max(n_query, 1) * 8);
+    L.o_key = off;   off += a256((size_t)items * 8);
+    L.o_part = off;  off += a256((size_t)items * 4);
+    L.o_key2 = off;  off += a256((size_t)items * 8);
+    L.o_part2 = off; off += a256((size_t)items * 4);
+    L.o_cub = off;   off += a256(L.cub_bytes);
+    L.total = off + 256;
+    return L;
+}
+
+__global__ void tip_pair_offsets_kernel(int m, int len, int *__restrict__ off)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i <= m) off[i] = i * len;
+}
+
+int launch_pair_prep(int S, int P, int K, int n, int n_pad, int SKP, const double *theta, const double *q, const int32_t *cand,
+                     int n_q, int nq_pad, const int32_t *qsorted, double *tcat, double *V, double *Tq, double *Vq, cudaStream_t st)
+{
+    const long long work = 2 * ((long long)n_pad + (n_q > 0 ? nq_pad : 0)) * SKP;
+    const long long want = (work + 255) / 256;
+    tip_pair_prep_kernel<<<(int)std::max(1ll, std::min<long long>(want, (long long)sm_count() * 16)), 256, 0, st>>>(
+        S, P, K, n, n_pad, SKP, theta, q, cand, n_q, n_q > 0 ? nq_pad : 0, qsorted, tcat, V, Tq, Vq);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    return 0;
+}
+
+}  // namespace
+}  // namespace tip
+
+static thread_local int g_last_pair_chunks = 0;
+static thread_local int g_last_gene_pair_chunks = 0;
+
+static bool top_pairs_args_ok(int n_cand, int K, int S, int64_t N)
+{
+    return n_cand >= 0 && n_cand <= (1 << kRankBits) && K >= 1 && K <= TIP_MAX_K && S >= 1 && (long long)S * K <= kPredMaxSK &&
+           N >= 0 && N < (1ll << 28);
+}
+
+#define TIP_TOP_PAIRS_LIMITS "n_cand <= 2^21, 1 <= K <= %d, S >= 1, S*K <= %d, 0 <= N < 2^28"
+#define TIP_GENE_PAIRS_LIMITS "n_cand <= 2^21, 0 <= n_query <= n_cand, 1 <= K <= %d, S >= 1, S*K <= %d, N >= 0, n_query*N <= 2^24"
+
+extern "C" int tip_score_pairs(int P, int K, const double *d_theta, const double *d_q, const int32_t *d_a, const int32_t *d_b,
+                               int64_t T, double *d_out, void *stream)
+{
+    TIP_REQUIRE(P > 0 && K >= 1 && K <= TIP_MAX_K && T >= 0, "tip_score_pairs: bad arguments (P > 0, 1 <= K <= %d, T >= 0)",
+                TIP_MAX_K);
+    TIP_REQUIRE(d_theta && d_q && (T == 0 || (d_a && d_b && d_out)), "tip_score_pairs: null pointer");
+    if (T == 0) return 0;
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    const long long want = (T + 255) / 256;
+    tip_score_pairs_kernel<<<(int)std::min<long long>(want, (long long)sm_count() * 32), 256, 0, st>>>(K, d_a, d_b, T, d_theta,
+                                                                                                     d_q, d_out);
+    TIP_CHECK_CUDA(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int tip_top_pairs_workspace_bytes(int n_cand, int K, int S, int64_t N, size_t *bytes)
+{
+    TIP_REQUIRE(bytes != nullptr && top_pairs_args_ok(n_cand, K, S, N),
+                "tip_top_pairs_workspace_bytes: bad arguments (" TIP_TOP_PAIRS_LIMITS ")", TIP_MAX_K, kPredMaxSK);
+    *bytes = top_pair_layout(n_cand, K, S, N).total;
+    return 0;
+}
+
+extern "C" int tip_top_pairs(int P, int K, int S, const double *d_theta, const double *d_q, const int32_t *d_cand, int n_cand,
+                             const uint64_t *d_known, int64_t n_known, int64_t N, void *d_ws, size_t ws_bytes, int32_t *d_out_ids,
+                             double *d_out_scores, int64_t *h_n_out, void *stream)
+{
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    TIP_REQUIRE(P > 0 && n_cand <= P && top_pairs_args_ok(n_cand, K, S, N) && n_known >= 0 && h_n_out != nullptr,
+                "tip_top_pairs: bad arguments (P > 0, n_known >= 0, " TIP_TOP_PAIRS_LIMITS ")", TIP_MAX_K, kPredMaxSK);
+    TIP_REQUIRE(d_theta && d_q && (d_cand || n_cand == 0) && (d_known || n_known == 0) && (N == 0 || (d_out_ids && d_out_scores)),
+                "tip_top_pairs: null pointer");
+    *h_n_out = 0;
+    g_last_pair_chunks = 0;
+    const int n = n_cand;
+    if (N == 0 || n < 2) return 0;
+    const TopPairLayout L = top_pair_layout(n, K, S, N);
+    TIP_REQUIRE(d_ws != nullptr && ws_bytes >= L.total, "tip_top_pairs: workspace too small (%zu < %zu)", ws_bytes, L.total);
+    char *base = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(d_ws) + 255) / 256 * 256);
+    double *tcat = reinterpret_cast<double *>(base + L.o_tcat), *V = reinterpret_cast<double *>(base + L.o_V);
+    auto *tile = reinterpret_cast<long long *>(base + L.o_tile);
+    auto *thr = reinterpret_cast<unsigned long long *>(base + L.o_thr), *cnt = reinterpret_cast<unsigned long long *>(base + L.o_cnt);
+    auto *bits = reinterpret_cast<unsigned long long *>(base + L.o_bits), *pk = reinterpret_cast<unsigned long long *>(base + L.o_pk);
+    auto *bits2 = reinterpret_cast<unsigned long long *>(base + L.o_bits2), *pk2 = reinterpret_cast<unsigned long long *>(base + L.o_pk2);
+    void *cub_tmp = base + L.o_cub;
+
+    if (int rc = launch_pair_prep(S, P, K, n, L.n_pad, L.SKP, d_theta, d_q, d_cand, 0, 0, nullptr, tcat, V, nullptr, nullptr, st))
+        return rc;
+    // items: row tile t holds ceil((n - 64 t) / 128) of them
+    const int n_tiles = tp_tiles(n);
+    std::vector<long long> h_tile((size_t)n_tiles + 1, 0);
+    for (int t = 0; t < n_tiles; ++t) h_tile[t + 1] = h_tile[t] + (n - t * kTpRows + kTpCols - 1) / kTpCols;
+    const long long n_items = h_tile[n_tiles];
+    TIP_CHECK_CUDA(cudaMemcpyAsync(tile, h_tile.data(), ((size_t)n_tiles + 1) * 8, cudaMemcpyHostToDevice, st));
+    TIP_CHECK_CUDA(cudaMemsetAsync(thr, 0, 8, st));
+
+    TopPairArgs A{};
+    A.n = n; A.SKP = L.SKP; A.V = V; A.tcat = tcat;
+    A.known = reinterpret_cast<const unsigned long long *>(d_known); A.n_known = n_known;
+    A.tile_item = tile; A.n_tiles = n_tiles; A.thr = thr; A.counter = cnt;
+    const long long per_chunk = kTpChunk / kTpItemPairs;
+    long long have = 0;          // running best, sorted, at bits[0, have) / pk[0, have)
+    for (long long i0 = 0; i0 < n_items; i0 += per_chunk) {
+        const long long items = std::min(per_chunk, n_items - i0);
+        TIP_CHECK_CUDA(cudaMemsetAsync(cnt, 0, 8, st));
+        A.item0 = i0; A.out_bits = bits + have; A.out_packed = pk + have;
+        tip_top_pairs_pass_kernel<<<(int)items, kPredThreads, 0, st>>>(A);
+        TIP_CHECK_CUDA(cudaGetLastError());
+        unsigned long long h_cnt = 0;
+        TIP_CHECK_CUDA(cudaMemcpyAsync(&h_cnt, cnt, 8, cudaMemcpyDeviceToHost, st));
+        TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+        ++g_last_pair_chunks;
+        if (h_cnt == 0) continue;
+        const int total = (int)(have + (long long)h_cnt);
+        // packed ranks ascending, then (stable) bits descending: the running best N come first
+        size_t cb = L.cub_bytes;
+        TIP_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(cub_tmp, cb, pk, pk2, bits, bits2, total, 0, 2 * kRankBits, st));
+        cb = L.cub_bytes;
+        TIP_CHECK_CUDA(cub::DeviceRadixSort::SortPairsDescending(cub_tmp, cb, bits2, bits, pk2, pk, total, 0, 63, st));
+        have = std::min<long long>(N, total);
+        if (have == N) TIP_CHECK_CUDA(cudaMemcpyAsync(thr, bits + N - 1, 8, cudaMemcpyDeviceToDevice, st));
+    }
+    if (have > 0) {
+        tip_top_pairs_finish_kernel<<<(int)((have + 255) / 256), 256, 0, st>>>(have, S, bits, pk, d_cand, d_out_ids, d_out_scores);
+        TIP_CHECK_CUDA(cudaGetLastError());
+    }
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    *h_n_out = have;
+    return 0;
+}
+
+extern "C" int tip_top_pairs_last_chunks(void) { return g_last_pair_chunks; }
+
+static bool gene_pairs_args_ok(int n_cand, int n_query, int K, int S, int64_t N)
+{
+    return n_cand >= 0 && n_cand <= (1 << kRankBits) && K >= 1 && K <= TIP_MAX_K && S >= 1 && (long long)S * K <= kPredMaxSK &&
+           n_query >= 0 && n_query <= n_cand && N >= 0 && (long long)n_query * N <= kTpMaxRows;
+}
+
+extern "C" int tip_top_pairs_per_gene_workspace_bytes(int n_cand, int n_query, int K, int S, int64_t N, size_t *bytes)
+{
+    TIP_REQUIRE(bytes != nullptr && gene_pairs_args_ok(n_cand, n_query, K, S, N),
+                "tip_top_pairs_per_gene_workspace_bytes: bad arguments (" TIP_GENE_PAIRS_LIMITS ")", TIP_MAX_K, kPredMaxSK);
+    *bytes = gene_pair_layout(n_cand, n_query, K, S).total;
+    return 0;
+}
+
+extern "C" int tip_top_pairs_per_gene(int P, int K, int S, const double *d_theta, const double *d_q, const int32_t *d_cand,
+                                      int n_cand, const int32_t *d_query_ranks, int n_query, const uint64_t *d_known,
+                                      int64_t n_known, int64_t N, void *d_ws, size_t ws_bytes, int32_t *d_out_ids,
+                                      double *d_out_scores, int64_t *h_n_out, void *stream)
+{
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    TIP_REQUIRE(P > 0 && n_cand <= P && gene_pairs_args_ok(n_cand, n_query, K, S, N) && n_known >= 0 && (h_n_out || n_query == 0),
+                "tip_top_pairs_per_gene: bad arguments (P > 0, n_known >= 0, " TIP_GENE_PAIRS_LIMITS ")", TIP_MAX_K, kPredMaxSK);
+    TIP_REQUIRE(d_theta && d_q && (d_cand || n_cand == 0) && (d_query_ranks || n_query == 0) && (d_known || n_known == 0) &&
+                    (N == 0 || n_query == 0 || (d_out_ids && d_out_scores)),
+                "tip_top_pairs_per_gene: null pointer");
+    g_last_gene_pair_chunks = 0;
+    if (n_query == 0) return 0;
+    const int n = n_cand, nq = n_query;
+    // the query ranks are checked on the host before any device work
+    std::vector<int32_t> qr(nq);
+    TIP_CHECK_CUDA(cudaMemcpyAsync(qr.data(), d_query_ranks, (size_t)nq * 4, cudaMemcpyDeviceToHost, st));
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    {
+        std::vector<char> seen(n, 0);
+        for (int i = 0; i < nq; ++i) {
+            TIP_REQUIRE(qr[i] >= 0 && qr[i] < n, "tip_top_pairs_per_gene: query rank %d of query %d is not in [0, %d)", qr[i], i, n);
+            TIP_REQUIRE(!seen[qr[i]], "tip_top_pairs_per_gene: query rank %d appears twice", qr[i]);
+            seen[qr[i]] = 1;
+        }
+    }
+    for (int i = 0; i < nq; ++i) h_n_out[i] = 0;
+    if (N == 0 || n < 2) return 0;
+    const GenePairLayout L = gene_pair_layout(n, nq, K, S);
+    TIP_REQUIRE(d_ws != nullptr && ws_bytes >= L.total, "tip_top_pairs_per_gene: workspace too small (%zu < %zu)", ws_bytes,
+                L.total);
+    char *base = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(d_ws) + 255) / 256 * 256);
+    double *tcat = reinterpret_cast<double *>(base + L.o_tcat), *V = reinterpret_cast<double *>(base + L.o_V);
+    double *Tq = reinterpret_cast<double *>(base + L.o_Tq), *Vq = reinterpret_cast<double *>(base + L.o_Vq);
+    auto *qs = reinterpret_cast<int32_t *>(base + L.o_qs), *oq = reinterpret_cast<int32_t *>(base + L.o_oq);
+    auto *off = reinterpret_cast<int *>(base + L.o_off);
+    auto *n_out = reinterpret_cast<unsigned long long *>(base + L.o_nout);
+    auto *key = reinterpret_cast<unsigned long long *>(base + L.o_key), *key2 = reinterpret_cast<unsigned long long *>(base + L.o_key2);
+    auto *part = reinterpret_cast<int32_t *>(base + L.o_part), *part2 = reinterpret_cast<int32_t *>(base + L.o_part2);
+    void *cub_tmp = base + L.o_cub;
+
+    // queries in ascending rank order, so that a warp's rows span a short range of ranks; oq maps them back
+    std::vector<int32_t> order(nq);
+    for (int i = 0; i < nq; ++i) order[i] = i;
+    std::sort(order.begin(), order.end(), [&](int a, int b) { return qr[a] < qr[b]; });
+    std::vector<int32_t> h_qs(nq);
+    for (int i = 0; i < nq; ++i) h_qs[i] = qr[order[i]];
+    TIP_CHECK_CUDA(cudaMemcpyAsync(qs, h_qs.data(), (size_t)nq * 4, cudaMemcpyHostToDevice, st));
+    TIP_CHECK_CUDA(cudaMemcpyAsync(oq, order.data(), (size_t)nq * 4, cudaMemcpyHostToDevice, st));
+    TIP_CHECK_CUDA(cudaMemsetAsync(n_out, 0, (size_t)nq * 8, st));
+    if (int rc = launch_pair_prep(S, P, K, n, L.n_pad, L.SKP, d_theta, d_q, d_cand, nq, L.nq_pad, qs, tcat, V, Tq, Vq, st))
+        return rc;
+    tip_pair_offsets_kernel<<<(L.qc + 256) / 256, 256, 0, st>>>(L.qc, n - 1, off);
+    TIP_CHECK_CUDA(cudaGetLastError());
+
+    GenePairArgs A{};
+    A.n = n; A.SKP = L.SKP; A.V = V; A.tcat = tcat;
+    A.known = reinterpret_cast<const unsigned long long *>(d_known); A.n_known = n_known;
+    A.key = key; A.part = part;
+    const int col_tiles = (n + kTpCols - 1) / kTpCols;
+    const long long m = std::min<long long>(N, n - 1);
+    for (int c = 0; c < nq; c += L.qc) {
+        const int cq = std::min(L.qc, nq - c);
+        A.n_q = cq; A.qrank = qs + c; A.Vq = Vq + (long long)c * L.SKP; A.Tq = Tq + (long long)c * L.SKP;
+        tip_top_pairs_gene_kernel<<<dim3(col_tiles, (cq + kTpRows - 1) / kTpRows), kPredThreads, 0, st>>>(A);
+        TIP_CHECK_CUDA(cudaGetLastError());
+        const int items = cq * (n - 1);
+        size_t cb = L.cub_bytes;
+        TIP_CHECK_CUDA(cub::DeviceSegmentedSort::StableSortPairsDescending(cub_tmp, cb, key, key2, part, part2, items, cq, off,
+                                                                          off + 1, st));
+        const long long rows = (long long)cq * m;
+        tip_top_pairs_gene_finish_kernel<<<(int)((rows + 255) / 256), 256, 0, st>>>(cq, n, N, S, key2, part2, qs + c, oq + c, d_cand,
+                                                                                   n_out, d_out_ids, d_out_scores);
+        TIP_CHECK_CUDA(cudaGetLastError());
+        ++g_last_gene_pair_chunks;
+    }
+    std::vector<unsigned long long> h_out(nq);
+    TIP_CHECK_CUDA(cudaMemcpyAsync(h_out.data(), n_out, (size_t)nq * 8, cudaMemcpyDeviceToHost, st));
+    TIP_CHECK_CUDA(cudaStreamSynchronize(st));
+    for (int i = 0; i < nq; ++i) h_n_out[i] = (int64_t)h_out[i];
+    return 0;
+}
+
+extern "C" int tip_top_pairs_per_gene_last_chunks(void) { return g_last_gene_pair_chunks; }

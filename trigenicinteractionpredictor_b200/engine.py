@@ -13,6 +13,8 @@ CUDA kernels behind the C ABI (include/tip.h).  There is no CPU path.
     eng.score_histogram(thetas, ps, cand)              # histogram of all C(n, 3) scores (tip_score_histogram)
     eng.rank_per_pair(thetas, ps, cand, pr, known, tp, trc)   # held-out ranks per query pair (tip_rank_per_pair)
     eng.rank_per_gene(thetas, ps, cand, q, known, tq, tu, tv)   # held-out ranks per query gene (tip_rank_per_gene)
+    eng.top_pairs(thetas, qs, cand, known, n)           # digenic: exhaustive top-n of unseen gene pairs (tip_top_pairs)
+    eng.top_pairs_per_gene(thetas, qs, cand, q, known, n)   # the same per query gene (tip_top_pairs_per_gene)
 """
 from __future__ import annotations
 
@@ -137,6 +139,7 @@ class EMEngine:
         self.test_ids = None      # (g1, g2, g3, labels) int32 tensors in test order
         self.em_ws = None
         self.pairs = None         # digenic extension: int32 [n][4] rows {a, b, n0, n1}
+        self.test_pairs = None    # its held-out pair links, same rows
         self.q = None             # its rating tensor q[K][K][2] and the statistic Sq[2][K*K]
         self.sq = None
         self._graphs = None
@@ -248,9 +251,17 @@ class EMEngine:
         self._graphs = None
 
     @_on_device
+    def set_test_pair_links(self, a, b, n0, n1):
+        """Digenic extension: held-out pair links; loglik("test") adds their term (tip_pairs_loglik)."""
+        a, b, n0, n1 = (self._as_dev_i32(x) for x in (a, b, n0, n1))
+        self.test_pairs = torch.stack([a, b, n0, n1], dim=1).contiguous()
+
+    @_on_device
     def set_q(self, q):
         qq = torch.from_numpy(np.ascontiguousarray(q, dtype=np.float64).reshape(-1))
         assert qq.numel() == 2 * self.K * self.K
+        if self.q is None:            # pair scores without pair links (score_pairs)
+            self.q = torch.empty(2 * self.K * self.K, dtype=torch.float64, device=self.device)
         self.q.copy_(qq, non_blocking=False)
 
     @_on_device
@@ -459,15 +470,19 @@ class EMEngine:
     @_on_device
     def loglik(self, which: str = "train") -> float:
         links = self.train if which == "train" else self.test
-        if links is None:
+        pairs = self.pairs if which == "train" else self.test_pairs
+        if links is None and pairs is None:
             raise ValueError("no %s links set" % which)
-        _cabi.check(self.lib.tip_loglik(self.P, self.K, _ptr(links.rows), links.n_rows, links.n_rows_r0, _ptr(self.theta),
-                                        _ptr(self.p), _ptr(self.ll_out), _ptr(self.ll_ws),
-                                        self.flags & _cabi.TIP_EM_FORCE_GENERIC, self._stream()),
-                    "tip_loglik")
-        self.launches += 2 if (self.K <= 10 and not (self.flags & _cabi.TIP_EM_FORCE_GENERIC)) else 1
-        if self.pairs is not None and which == "train":
-            _cabi.check(self.lib.tip_pairs_loglik(self.P, self.K, _ptr(self.pairs), int(self.pairs.shape[0]), _ptr(self.theta),
+        if links is not None:
+            _cabi.check(self.lib.tip_loglik(self.P, self.K, _ptr(links.rows), links.n_rows, links.n_rows_r0, _ptr(self.theta),
+                                            _ptr(self.p), _ptr(self.ll_out), _ptr(self.ll_ws),
+                                            self.flags & _cabi.TIP_EM_FORCE_GENERIC, self._stream()),
+                        "tip_loglik")
+            self.launches += 2 if (self.K <= 10 and not (self.flags & _cabi.TIP_EM_FORCE_GENERIC)) else 1
+        else:
+            self.ll_out.zero_()           # held-out pair links without held-out triplets
+        if pairs is not None:
+            _cabi.check(self.lib.tip_pairs_loglik(self.P, self.K, _ptr(pairs), int(pairs.shape[0]), _ptr(self.theta),
                                                   _ptr(self.q), _ptr(self.ll_out), self._stream()), "tip_pairs_loglik")
             self.launches += 1
         if self.world > 1 and which == "train":
@@ -610,6 +625,82 @@ class EMEngine:
         return ids, sc, counts
 
     @_on_device
+    def score_pairs(self, ids_a, ids_b) -> torch.Tensor:
+        """tip_score_pairs: the pair score (rating 1, no eps) of (ids_a[t], ids_b[t]), ids_a in the key's first slot, under
+        the engine's theta and q.  Returns a float64 device tensor [T]."""
+        a, b = self._as_dev_i32(ids_a).reshape(-1), self._as_dev_i32(ids_b).reshape(-1)
+        assert a.numel() == b.numel()
+        T = int(a.numel())
+        out = torch.empty(T, dtype=torch.float64, device=self.device)
+        _cabi.check(self.lib.tip_score_pairs(self.P, self.K, _ptr(self.theta), _ptr(self.q), _ptr(a), _ptr(b), T, _ptr(out),
+                                             self._stream()), "tip_score_pairs")
+        self.launches += 1 if T else 0
+        return out
+
+    def _pair_sets(self, theta_stack, q_stack):
+        th = np.ascontiguousarray(theta_stack, dtype=np.float64)
+        qq = np.ascontiguousarray(q_stack, dtype=np.float64)
+        S = int(th.shape[0])
+        assert th.shape == (S, self.P, self.K) and qq.shape == (S, self.K, self.K, 2)
+        return S, torch.from_numpy(th.reshape(-1)).to(self.device), torch.from_numpy(qq.reshape(-1)).to(self.device)
+
+    @_on_device
+    def top_pairs(self, theta_stack, q_stack, cand, known, n: int):
+        """tip_top_pairs: the `n` best pairs of the candidate genes under the mean of S digenic models.
+        theta_stack [S][P][K], q_stack [S][K][K][2] (numpy fp64); cand: gene ids in decimal-string order; known: sorted
+        packed rank pairs (ra << 21 | rb) to leave out.  Returns (ids [m][2] int32 in slot order, scores [m] float64), best
+        first."""
+        S, d_th, d_q = self._pair_sets(theta_stack, q_stack)
+        cand = np.ascontiguousarray(cand, dtype=np.int32)
+        known = np.ascontiguousarray(known, dtype=np.uint64)
+        n_cand, n_known, n = int(cand.shape[0]), int(known.shape[0]), int(n)
+        nb = ctypes.c_size_t(0)
+        _cabi.check(self.lib.tip_top_pairs_workspace_bytes(n_cand, self.K, S, n, ctypes.byref(nb)),
+                    "tip_top_pairs_workspace_bytes")
+        d_cand = torch.from_numpy(cand).to(self.device)
+        d_known = torch.from_numpy(known.view(np.int64)).to(self.device) if n_known else None
+        ws = torch.empty(max(nb.value, 1), dtype=torch.uint8, device=self.device)
+        out_ids = torch.empty((max(n, 1), 2), dtype=torch.int32, device=self.device)
+        out_sc = torch.empty(max(n, 1), dtype=torch.float64, device=self.device)
+        m = ctypes.c_int64(0)
+        _cabi.check(self.lib.tip_top_pairs(self.P, self.K, S, _ptr(d_th), _ptr(d_q), _ptr(d_cand), n_cand, _ptr(d_known),
+                                           n_known, n, _ptr(ws), nb.value, _ptr(out_ids), _ptr(out_sc), ctypes.byref(m),
+                                           self._stream()), "tip_top_pairs")
+        m = int(m.value)
+        return out_ids[:m].cpu().numpy(), out_sc[:m].cpu().numpy()
+
+    @_on_device
+    def top_pairs_per_gene(self, theta_stack, q_stack, cand, query_ranks, known, n: int):
+        """tip_top_pairs_per_gene: for every query rank (into `cand`), the `n` best pairs of it with another candidate,
+        under the mean of S digenic models; arguments otherwise as top_pairs.  Returns (ids [Q][m][2] int32 in slot order,
+        scores [Q][m] float64, counts [Q]), best first per query, m = the largest count; a query's rows past its count are
+        -1 / NaN."""
+        S, d_th, d_q = self._pair_sets(theta_stack, q_stack)
+        cand = np.ascontiguousarray(cand, dtype=np.int32)
+        qr = np.ascontiguousarray(query_ranks, dtype=np.int32).reshape(-1)
+        known = np.ascontiguousarray(known, dtype=np.uint64)
+        n_cand, n_query, n_known, n = int(cand.shape[0]), int(qr.shape[0]), int(known.shape[0]), int(n)
+        nb = ctypes.c_size_t(0)
+        _cabi.check(self.lib.tip_top_pairs_per_gene_workspace_bytes(n_cand, n_query, self.K, S, n, ctypes.byref(nb)),
+                    "tip_top_pairs_per_gene_workspace_bytes")
+        d_cand = torch.from_numpy(cand).to(self.device)
+        d_qr = torch.from_numpy(qr).to(self.device)
+        d_known = torch.from_numpy(known.view(np.int64)).to(self.device) if n_known else None
+        ws = torch.empty(max(nb.value, 1), dtype=torch.uint8, device=self.device)
+        out_ids = torch.full((max(n_query * n, 1), 2), -1, dtype=torch.int32, device=self.device)
+        out_sc = torch.full((max(n_query * n, 1),), float("nan"), dtype=torch.float64, device=self.device)
+        counts = np.zeros(max(n_query, 1), dtype=np.int64)
+        _cabi.check(self.lib.tip_top_pairs_per_gene(
+            self.P, self.K, S, _ptr(d_th), _ptr(d_q), _ptr(d_cand), n_cand, _ptr(d_qr), n_query, _ptr(d_known), n_known, n,
+            _ptr(ws), nb.value, _ptr(out_ids), _ptr(out_sc), counts.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)),
+            self._stream()), "tip_top_pairs_per_gene")
+        counts = counts[:n_query]
+        m = int(counts.max()) if n_query else 0
+        ids = out_ids[:n_query * n].reshape(n_query, n, 2)[:, :m].cpu().numpy()
+        sc = out_sc[:n_query * n].reshape(n_query, n)[:, :m].cpu().numpy()
+        return ids, sc, counts
+
+    @_on_device
     def rank_per_pair(self, theta_stack, p_stack, cand, pair_ranks, known, test_pair, test_rc):
         """tip_rank_per_pair: the exact rank of every test entry (test_pair[j], an index into `pair_ranks`; test_rc[j], the
         partner's rank) among its pair's partners whose triplet is not a key of `known`, in the order of
@@ -743,9 +834,10 @@ class EMEngine:
         return torch.where(sk[i] == q, perm[i], torch.full_like(i, -1)).cpu().numpy()
 
     @_on_device
-    def metric_counts(self, scores: torch.Tensor, positives_number: int) -> dict:
-        """Integer ingredients of calculate_metrics (TIP.py:583-637); ratios are formed by the caller."""
-        labels = self.test_ids[3]
+    def metric_counts(self, scores: torch.Tensor, positives_number: int, labels: torch.Tensor | None = None) -> dict:
+        """Integer ingredients of calculate_metrics (TIP.py:583-637); ratios are formed by the caller.  `labels` (int32,
+        1 = positive) default to those of the test triplets."""
+        labels = self.test_ids[3] if labels is None else labels
         T = int(scores.numel())
         nb = ctypes.c_size_t(0)
         _cabi.check(self.lib.tip_metrics_workspace_bytes(T, ctypes.byref(nb)), "tip_metrics_workspace_bytes")
