@@ -95,7 +95,8 @@ LEFT_OUT = {
 # source files not scanned, and where their kernels are tested
 FILES_ELSEWHERE = {
     "tip_em.cu": "E-step and log-likelihood kernels: test_estep_coverage.py",
-    "tip_predict.cu": "predict kernels: test_predict.py, test_predict_per_gene.py, test_predict_per_pair.py",
+    "tip_predict.cu": "prediction, ranking and gene-pair kernels: test_predict*.py, test_rank_*.py, "
+                      "test_digenic_predict.py; at the sizes their limits accept: SCALE_COVERAGE in test_predict_scale.py",
     "tip_peer.cu": "peer_* and normalise_peers_kernel need two GPUs: test_gpu_dist.py",
 }
 
